@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
-"""bench.py -- throughput of the conv-stack hot path on B200 (driver contract in the task statement).
+"""bench.py -- throughput of the conv-stack hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the conv stack (128x128 u8 -> 64x16x16 u8, shipped weights.bin, shifts 2/4/6)
 over one batch of B synthetic images per GPU -- B = 4096 by default, BASELINE.json's configs[1].  The steps walk
@@ -13,7 +13,10 @@ four host batches in flight), with the plain synchronous cnnacc_run_batch loop n
 N > 1: launched by torchrun, one rank per GPU, batch sharded by rank with no data-path collective (weak
 scaling: B images per GPU); times are CUDA-event times, max over ranks.
 `--impl reference` times the reference's own arm_cnn.c (oracle/_ref, one process per host core because
-its static scratch buffers make it non-re-entrant) on the same workload.
+its static scratch buffers make it non-re-entrant) on the same workload; where oracle/_ref/arm_cnn.so is not built it
+times the C restatement oracle/cnn_oracle.c instead, and `cpu_baseline.kind` / `sample` say which.
+`--dump-outputs DIR` writes the features the last timed step computed (rank 0's shard) to DIR/features.npy as float32,
+so that two builds can be compared output for output: the inputs depend only on the arguments.
 
 Beside the contract line's `value` / `e2e` / `roofline` / `cpu_baseline` the line carries, at every N:
   `sustained`  >= 2 s of back-to-back conv-stack launches with the clocks / power / throttle reasons seen inside them;
@@ -79,6 +82,21 @@ def gather_counts(count, dist):
     out = [torch.zeros_like(t) for _ in range(dist.get_world_size())]
     dist.all_gather(out, t)
     return [int(o.item()) for o in out]
+
+
+DUMP_IMAGES = 512                       # 512 x 64x16x16 float32 = 32 MiB
+
+
+def dump_outputs(out_dir, feats):
+    """--dump-outputs: `feats` (torch u8 [n,64,16,16]) -> out_dir/features.npy, float32.  A batch of more than DUMP_IMAGES
+    images is sampled at fixed, seeded, sorted image indices, so runs with the same --batch dump the same images."""
+    import torch
+    n = feats.shape[0]
+    idx = np.arange(n) if n <= DUMP_IMAGES else np.sort(np.random.default_rng(0).choice(n, DUMP_IMAGES, replace=False))
+    sample = feats[torch.from_numpy(idx).to(feats.device)].cpu().numpy().astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "features.npy"), sample)
+    return idx
 
 
 def ncu_dram_bytes_per_image(kernel_tag="conv"):
@@ -212,6 +230,11 @@ class ClockSampler:
 # ------------------------------------------------------------------------------------------------
 # reference arm: arm_cnn.c on the host cores
 # ------------------------------------------------------------------------------------------------
+# what the CPU arm timed, by the `kind` _ref_worker reports
+CPU_PROGRAMS = {"reference": "the reference's own arm_cnn.c (oracle/_ref/arm_cnn.so)",
+                "port": "oracle/cnn_oracle.c, the C restatement of arm_cnn.c (oracle/_ref/arm_cnn.so is not built)"}
+
+
 def _ref_worker(args):
     """One process = one private mapping of the reference .so (static buffers => never threads)."""
     seed, n_images, weights, shifts, seconds = args
@@ -294,8 +317,8 @@ def run_reference_arm(args, weights):
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u8*s8->s32", "data": "synthetic",
         "config": ours_config(args.batch, args.gpus, False),       # the same keys and values as our arm's line
         "cpu_baseline": {"value": value, "unit": "images/s", "cores": cores, "kind": kind,
-                         "sample": f"arm_cnn.c on the host CPU, {cores} processes x {per_core} images per step (a bounded sample "
-                                   f"of the batch), {total_imgs} images in all, gcc -O3 (the reference's own flags)",
+                         "sample": f"{CPU_PROGRAMS[kind]} on the host CPU, {cores} processes x {per_core} images per step (a bounded "
+                                   f"sample of the batch), {total_imgs} images in all, gcc -O3 (the reference's own flags)",
                          "cpu_model": _cpu_model()},
         "e2e": {"value": value, "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
@@ -530,6 +553,14 @@ def bind_to_gpu_numa_node(gpu_index):
         return f"unavailable ({type(e).__name__})"
 
 
+def synthetic_batches(torch, nb, nbuf, rank):
+    """The timed loop's `nbuf` device-resident batches of `nb` images from a generator seeded by the rank: the same images on
+    every run, and the first k batches do not depend on nbuf.  Returns (generator, batches); later legs draw on."""
+    g = torch.Generator(device="cuda")
+    g.manual_seed(1234 + rank)
+    return g, [torch.randint(0, 256, (nb, 128, 128), dtype=torch.uint8, device="cuda", generator=g) for _ in range(nbuf)]
+
+
 def run_ours(args, weights):
     import torch
     import torch.distributed as dist
@@ -559,9 +590,7 @@ def run_ours(args, weights):
     lo, hi = shard_range(B * world, rank, world)
     nb = hi - lo
     nbuf = max(2, -(-(2 << 30) // (nb * BYTES_PER_IMAGE)))
-    g = torch.Generator(device="cuda")
-    g.manual_seed(1234 + rank)
-    imgs = [torch.randint(0, 256, (nb, 128, 128), dtype=torch.uint8, device="cuda", generator=g) for _ in range(nbuf)]
+    g, imgs = synthetic_batches(torch, nb, nbuf, rank)
     feats = [torch.empty((nb, 64, 16, 16), dtype=torch.uint8, device="cuda") for _ in range(nbuf)]
     torch.cuda.synchronize()
 
@@ -589,6 +618,8 @@ def run_ours(args, weights):
     t_end = time.time()
     launches = acc.launch_count - launches0
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, feats[(args.steps - 1) % nbuf])
     ms = reduce_max(ms, ddist)
     total_images = sum(gather_counts(nb, ddist)) * args.steps
     value = total_images / (ms / 1000.0)
@@ -815,7 +846,7 @@ def run_ours(args, weights):
             rate, kind, n_img, wall = cpu_reference_rate(weights, cores, seconds=2.0)
             rate1, _, n1, _ = cpu_reference_rate(weights, 1, seconds=1.0)
             cpu = {"value": rate, "unit": "images/s", "cores": cores, "kind": kind,
-                   "sample": f"{n_img} images of the same workload in a 2 s window, one process per core, gcc -O3",
+                   "sample": f"{CPU_PROGRAMS[kind]}: {n_img} images of the same workload in a 2 s window, one process per core, gcc -O3",
                    "single_core_images_per_s": rate1, "single_core_ms_per_image": 1000.0 / rate1 if rate1 else None,
                    "numpy_port_ms_per_image": numpy_port_ms(weights), "cpu_model": _cpu_model()}
         line = {
@@ -858,7 +889,13 @@ def main():
     ap.add_argument("--no-stream", action="store_true", help="skip the 1M-image stream block")
     ap.add_argument("--sustained-s", type=float, default=2.2, help="length of the sustained leg in seconds")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's features (rank 0's shard, at most %d images) to DIR/features.npy" % DUMP_IMAGES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     weights = np.fromfile(os.path.join(ROOT, "tests", "golden", "weights.bin"), dtype=np.uint8)
     if args.impl == "reference":

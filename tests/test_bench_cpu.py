@@ -56,6 +56,7 @@ def test_reference_arm_prints_contract_line():
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "images/s" and line["value"] > 0
     assert line["cpu_baseline"]["kind"] in ("reference", "port") and line["cpu_baseline"]["cores"] >= 1
+    assert line["cpu_baseline"]["sample"].startswith(bench.CPU_PROGRAMS[line["cpu_baseline"]["kind"]])   # names what was timed
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["gpu_launches"] == 0
 
 
@@ -73,6 +74,25 @@ def test_both_arms_describe_the_same_config():
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["config"] == bench.ours_config(4096, 1, False, 16)
     assert "sample" not in line["config"] and "sample" in line["cpu_baseline"]
+
+
+def test_dump_outputs_writes_a_fixed_float32_sample(tmp_path):
+    import numpy as np
+    import torch
+    feats = torch.randint(0, 256, (3000, 64, 16, 16), dtype=torch.uint8, generator=torch.Generator().manual_seed(5))
+    idx = bench.dump_outputs(str(tmp_path / "a"), feats)
+    got = np.load(tmp_path / "a" / "features.npy")
+    assert got.dtype == np.float32 and got.shape == (bench.DUMP_IMAGES, 64, 16, 16) and got.nbytes <= 64 << 20
+    assert np.all(np.diff(idx) > 0) and np.array_equal(got, feats.numpy()[idx])
+    assert np.array_equal(bench.dump_outputs(str(tmp_path / "b"), feats), idx)           # the same images on every run
+    bench.dump_outputs(str(tmp_path / "c"), feats[:100])                                  # a small batch is written whole
+    assert np.array_equal(np.load(tmp_path / "c" / "features.npy"), feats[:100].numpy())
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bad_arguments_are_refused(argv):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and r.stdout == "" and argv[-2] in r.stderr
 
 
 def test_roofline_traffic_comes_from_the_newest_committed_capture():

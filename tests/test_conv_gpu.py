@@ -1,6 +1,9 @@
 """Parity of the CUDA conv stack with the oracle, through the C ABI.  Bit-exact (integer path)."""
 import ctypes
+import json
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -519,3 +522,20 @@ def test_misaligned_device_pointers_are_refused(fc, shipped_weights):
     assert a.run_batch(good).shape == (2, 64, 16, 16)                    # the context is intact
     a.synchronize()
     a.close()
+
+
+def test_bench_dump_is_the_last_timed_step(port, shipped_weights, tmp_path):
+    """bench.py --dump-outputs: features.npy holds what the last of --steps timed steps computed from its seeded batch."""
+    import torch
+    import bench
+    nb, steps = bench.DUMP_IMAGES, 3
+    r = subprocess.run([sys.executable, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py"),
+                        "--steps", str(steps), "--warmup", "0", "--batch", str(nb), "--quick", "--no-stream", "--no-cpu-baseline",
+                        "--sustained-s", "0", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+    got = np.load(tmp_path / "features.npy")
+    assert got.dtype == np.float32 and got.shape == (nb, 64, 16, 16)
+    _, batches = bench.synthetic_batches(torch, nb, steps, 0)
+    want = oracle.port_infer_batch(port, batches[steps - 1].cpu().numpy(), shipped_weights, bench.SHIFTS)
+    assert np.array_equal(got.reshape(nb, 64, 256), want)
