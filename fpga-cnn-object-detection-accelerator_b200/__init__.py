@@ -6,9 +6,9 @@ the host-side mirror of the reference's engine objects; the work happens in libc
 """
 from . import _lib
 from ._lib import build, load
-from .accelerator import (ARMEngine, B200Engine, CNNAccelerator, Classifier, NAMES, alloc_host, bbox_vec, classify_vec,
-                          dump_features, load_arm_cnn_lib, load_features, load_image_any, register_host,
+from .accelerator import (ARMEngine, B200Engine, CNNAccelerator, Classifier, MultiAccelerator, NAMES, alloc_host, bbox_vec,
+                          classify_vec, dump_features, load_arm_cnn_lib, load_features, load_image_any, register_host,
                           train_linear_classifier)
 
-__all__ = ["ARMEngine", "B200Engine", "CNNAccelerator", "Classifier", "dump_features", "load_features", "NAMES", "alloc_host", "register_host", "load_image_any", "train_linear_classifier", "bbox_vec", "classify_vec",
+__all__ = ["ARMEngine", "B200Engine", "CNNAccelerator", "Classifier", "MultiAccelerator", "dump_features", "load_features", "NAMES", "alloc_host", "register_host", "load_image_any", "train_linear_classifier", "bbox_vec", "classify_vec",
            "load_arm_cnn_lib", "build", "load", "_lib"]

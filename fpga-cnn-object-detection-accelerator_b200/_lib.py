@@ -51,6 +51,13 @@ SYMBOLS = {
     "cnnacc_detect_frames": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p,
                                         _c.c_void_p, _c.c_uint32]),
     "cnnacc_image_to_gray128": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p, _c.c_uint32]),
+    "cnnacc_run_batch_sharded": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p,
+                                            _c.c_uint32, _c.POINTER(_c.c_int)]),
+    "cnnacc_infer_batch_sharded": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_void_p, _c.c_void_p,
+                                              _c.c_void_p, _c.c_uint32, _c.POINTER(_c.c_int)]),
+    "cnnacc_detect_frames_sharded": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p,
+                                                _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_uint32, _c.POINTER(_c.c_int)]),
+    "cnnacc_shard_plan_host": (_c.c_int, [_c.c_int64, _c.c_int, _c.c_int64, _c.c_void_p, _c.c_int]),
     "cnnacc_alloc_host": (_c.c_int, [_c.c_size_t, _c.POINTER(_c.c_void_p)]),
     "cnnacc_free_host": (_c.c_int, [_c.c_void_p]),
     "cnnacc_register_host": (_c.c_int, [_c.c_void_p, _c.c_size_t]),
@@ -91,12 +98,12 @@ def load():
     return lib
 
 
-def check(rc, handle=None):
-    """Map C status codes to the reference's Python exceptions (SURVEY.md 8b)."""
+def check(rc, handle=None, prefix=""):
+    """Map C status codes to the reference's Python exceptions (SURVEY.md 8b); `prefix` goes in front of the error text."""
     if rc == OK:
         return
     msg = load().cnnacc_last_error(handle)
-    msg = msg.decode() if msg else ""
+    msg = prefix + (msg.decode() if msg else "")
     if rc == ERR_TIMEOUT:
         raise TimeoutError(msg or "timed out")
     if rc == ERR_ARG:

@@ -443,6 +443,130 @@ class CNNAccelerator:
         return feat, c._obj.value, r._obj.value
 
 
+class MultiAccelerator:
+    """One host batch over several GPUs in one call: a CNNAccelerator per entry of `devices` (None = every visible GPU; a
+    device may repeat), run through the cnnacc_*_sharded calls.  Each call cuts the batch into contiguous shards, runs shard
+    i on member i's own thread and returns once every prediction / feature is in the host arrays -- the same values, byte for
+    byte, as one CNNAccelerator.  Host arrays from alloc_host() are pinned for every GPU; ordinary numpy arrays work, slowly.
+
+    Configuration (load_weights, set_shifts, set_accumulator_bits, load_classifier) goes to every member.  Everything that
+    stays per device -- torch tensors, run_batch_async tickets, the register protocol -- is on `.members[i]`."""
+
+    def __init__(self, devices=None):
+        if devices is None:
+            import torch
+            devices = list(range(torch.cuda.device_count())) or [0]     # [0]: no GPU -> CNNAccelerator raises "no CUDA device"
+        devices = [int(d) for d in devices]
+        if not devices:
+            raise ValueError("devices must name at least one GPU")
+        self._libc = _lib.load()
+        self.members = []
+        try:
+            for d in devices:
+                self.members.append(CNNAccelerator(device=d))
+        except BaseException:
+            self.close()
+            raise
+        self._hs = (ctypes.c_void_p * len(self.members))(*[m._h.value for m in self.members])
+
+    def close(self):
+        for m in self.members:
+            m.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def _call(self, fn, *args):
+        failed = ctypes.c_int(-1)
+        rc = fn(self._hs, len(self.members), *args, ctypes.byref(failed))
+        i = failed.value
+        if rc != _lib.OK and 0 <= i < len(self.members):
+            _lib.check(rc, self.members[i]._h, prefix=f"member {i} (cuda:{self.members[i].device}): ")
+        _lib.check(rc)
+
+    @staticmethod
+    def _host_only(x):
+        if _is_torch_cuda(x):
+            raise ValueError("MultiAccelerator takes host arrays; run a CUDA tensor on the accelerator of its GPU, .members[i]")
+
+    # -- configuration, broadcast to every member ----------------------------------------------------------------------
+    def load_weights(self, weights_path):
+        for m in self.members:
+            m.load_weights(weights_path)
+
+    def set_shifts(self, s0=SHIFT_L0, s1=SHIFT_L1, s2=SHIFT_L2):
+        for m in self.members:
+            m.set_shifts(s0, s1, s2)
+
+    def set_accumulator_bits(self, bits=32):
+        for m in self.members:
+            m.set_accumulator_bits(bits)
+
+    def load_classifier(self, fc_w, fc_b):
+        for m in self.members:
+            m.load_classifier(fc_w, fc_b)
+
+    # -- sharded host-batch calls: same arguments and results as CNNAccelerator's for host arrays -----------------------
+    def run_batch(self, images, out=None, direct=False):
+        """images [N,H,W] u8 (host) -> features [N,64,H/8,W/8] u8."""
+        self._host_only(images)
+        images = np.ascontiguousarray(images, dtype=np.uint8)
+        if images.ndim != 3:
+            raise ValueError("images must be [N,H,W]")
+        n, H, W = images.shape
+        if out is None:
+            out = np.empty((n, 64, H // 8, W // 8), dtype=np.uint8)
+        elif not (isinstance(out, np.ndarray) and out.dtype == np.uint8 and out.flags.c_contiguous and out.size == n * 64 * (H // 8) * (W // 8)):
+            raise ValueError("out must be a C-contiguous uint8 numpy array of n*64*(H/8)*(W/8) elements")
+        self._call(self._libc.cnnacc_run_batch_sharded, _vp(images), n, H, W, _vp(out), _lib.FLAG_DIRECT if direct else 0)
+        return out
+
+    def _n_cls(self):
+        n_cls = self.members[0]._n_cls
+        if n_cls == 0:
+            raise RuntimeError("classifier not loaded")
+        return n_cls
+
+    def infer_batch(self, images, direct=False, bbox="vec", logits=False, two_kernels=False):
+        """images [N,128,128] u8 (host) -> (cls [N] i32, probs [N,n_cls] f32, bbox [N,4] i32)."""
+        self._host_only(images)
+        if bbox not in ("vec", "upsampled"):
+            raise ValueError("bbox must be 'vec' (realtime_detect.bbox_vec) or 'upsampled' (Classifier.get_cam_bbox)")
+        flags = (_lib.FLAG_DIRECT if direct else 0) | (_lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0) | \
+                (_lib.FLAG_LOGITS if logits else 0) | (_lib.FLAG_TWO_KERNELS if two_kernels else 0)
+        n_cls = self._n_cls()
+        x = np.ascontiguousarray(images, dtype=np.uint8)
+        if _item_bytes(x) != 16384:
+            raise ValueError("expected [N,128,128] images")
+        n = x.shape[0]
+        probs = np.empty((n, n_cls), dtype=np.float32)
+        cls = np.empty((n,), dtype=np.int32)
+        box = np.empty((n, 4), dtype=np.int32)
+        self._call(self._libc.cnnacc_infer_batch_sharded, _vp(x), n, _vp(probs), _vp(cls), _vp(box), flags)
+        return cls, probs, box
+
+    def detect_frames(self, frames, bbox="vec", return_gray=False):
+        """Camera frames [N,h,w,3] u8 BGR (host) -> (cls, probs, bbox[, gray128]), as CNNAccelerator.detect_frames."""
+        self._host_only(frames)
+        if bbox not in ("vec", "upsampled"):
+            raise ValueError("bbox must be 'vec' or 'upsampled'")
+        n_cls = self._n_cls()
+        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        if frames.ndim != 4 or frames.shape[3] != 3:
+            raise ValueError("expected [N,h,w,3] BGR frames")
+        n, fh, fw = frames.shape[:3]
+        probs = np.empty((n, n_cls), dtype=np.float32)
+        cls = np.empty((n,), dtype=np.int32)
+        box = np.empty((n, 4), dtype=np.int32)
+        gray = np.empty((n, 128, 128), dtype=np.uint8) if return_gray else None
+        self._call(self._libc.cnnacc_detect_frames_sharded, _vp(frames), n, fh, fw, _vp(gray) if return_gray else None,
+                   _vp(probs), _vp(cls), _vp(box), _lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0)
+        return (cls, probs, box, gray) if return_gray else (cls, probs, box)
+
+
 class B200Engine:
     """FPGAEngine's surface (realtime_detect.py:246-363): run(gray128) -> (feat, conv_ms, read_ms)."""
 

@@ -9,6 +9,8 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <system_error>
+#include <thread>
 #include <vector>
 
 #include "conv_direct.cuh"
@@ -20,6 +22,7 @@
 #include "pil_resize.cuh"
 #include "host_chunks.h"
 #include "pdl_chain.h"
+#include "shard_plan.h"
 #include "tiling.cuh"
 #include "weights_pack.h"
 
@@ -59,6 +62,7 @@ struct cnnacc_handle {
     uint32_t* d_wdirect = nullptr; size_t wdirect_off[3] = {0, 0, 0};
     FusedWeights fused;                         // packed operands of the fused kernel (conv_fused.cuh)
     float *d_fcw = nullptr, *d_fcb = nullptr; int n_cls = 0;
+    float fcw_host[kMaxClasses * 1024], fcb_host[kMaxClasses];   // what d_fcw / d_fcb hold: sharded calls compare members
     // workspaces (grown on demand) for the per-layer path and for infer_batch
     uint8_t *d_l0 = nullptr, *d_l1 = nullptr, *d_feat = nullptr;
     size_t cap_l0 = 0, cap_l1 = 0, cap_feat = 0;
@@ -397,6 +401,76 @@ int enqueue_host_batch(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int H, 
     }
     if (pipelined) h->ring_ci = (ring0 + ci) % kSlots;
     return 0;
+}
+
+// ---- sharded host-batch calls (cnnacc_*_sharded, shard_plan.h) ----------------------------------------------------------
+
+// Checked on the calling thread before any member starts work: the member array, the flags, and that every member computes the
+// same function as member 0 (members that silently disagreed would make a prediction depend on which shard its image fell
+// in).  Returns 0 or a code; *bad = the index of the member concerned (its cnnacc_last_error holds the text), -1 for none.
+int check_members(cnnacc_handle* const* hs, int n_handles, uint32_t flags, bool predictions, int* bad) {
+    *bad = -1;
+    if (!hs || n_handles < 1) return CNNACC_ERR_ARG;
+    for (int i = 0; i < n_handles; i++) {
+        *bad = i;
+        if (!hs[i]) return CNNACC_ERR_ARG;
+        for (int j = 0; j < i; j++)
+            if (hs[j] == hs[i])
+                return fail(hs[i], CNNACC_ERR_ARG, "sharded call: members " + std::to_string(j) + " and " + std::to_string(i) +
+                                                       " are the same handle (one handle is used by one thread only)");
+    }
+    *bad = 0;
+    if (flags & (CNNACC_FLAG_DEVICE_PTRS | CNNACC_FLAG_KEEP_MAPS))
+        return fail(hs[0], CNNACC_ERR_ARG, "sharded call: CNNACC_FLAG_DEVICE_PTRS / CNNACC_FLAG_KEEP_MAPS have no sharded form");
+    const cnnacc_handle* h0 = hs[0];
+    for (int i = 0; i < n_handles; i++) {
+        cnnacc_handle* h = hs[i];
+        const std::string who = "sharded call: member " + std::to_string(i);
+        *bad = i;
+        if (!h->weights_loaded) return fail(h, CNNACC_ERR_STATE, who + ": weights not loaded (call cnnacc_load_weights)");
+        if (predictions && !h->fc_loaded) return fail(h, CNNACC_ERR_STATE, who + ": classifier not loaded (call cnnacc_load_classifier)");
+        if (std::memcmp(h->wbin, h0->wbin, CNNACC_WEIGHT_BYTES) != 0) return fail(h, CNNACC_ERR_ARG, who + ": weights differ from member 0's");
+        if (std::memcmp(h->shifts, h0->shifts, sizeof(h->shifts)) != 0) return fail(h, CNNACC_ERR_ARG, who + ": shifts differ from member 0's");
+        if (h->acc24 != h0->acc24) return fail(h, CNNACC_ERR_ARG, who + ": accumulator bits differ from member 0's");
+        if (predictions && (h->n_cls != h0->n_cls || std::memcmp(h->fcw_host, h0->fcw_host, (size_t)h->n_cls * 1024 * sizeof(float)) != 0 ||
+                            std::memcmp(h->fcb_host, h0->fcb_host, (size_t)h->n_cls * sizeof(float)) != 0))
+            return fail(h, CNNACC_ERR_ARG, who + ": classifier differs from member 0's");
+    }
+    *bad = -1;
+    return 0;
+}
+
+// One sharded call: checks, then run(h, lo, hi) -- the member's own single-handle call on units [lo, hi) -- for every shard of
+// the plan: shard 0 on the calling thread, shards 1 .. m-1 on a thread each, joined before it returns, so every started
+// shard runs to completion and each member handle is used by exactly one thread.  `args_ok`: the pointers are usable and
+// `unit_bytes` means something (otherwise member 0 alone runs the call, which reports the bad argument).  Returns the code
+// of the lowest-index failing member and stores its index in *failed (-1: success, or no member to blame).
+template <class Run>
+int run_sharded(cnnacc_handle* const* hs, int n_handles, int64_t n, int64_t unit_bytes, bool args_ok, uint32_t flags,
+                bool predictions, int* failed, Run run) {
+    int bad = -1;
+    int rc = check_members(hs, n_handles, flags, predictions, &bad);
+    if (!rc && n < 0) { bad = 0; rc = fail(hs[0], CNNACC_ERR_ARG, "sharded call: negative n"); }
+    if (!rc && n > 0 && !args_ok) { bad = 0; rc = fail(hs[0], CNNACC_ERR_ARG, "sharded call: bad size or NULL input / output pointer"); }
+    if (!rc) {
+        const ShardPlan plan = make_shard_plan(n, n_handles, unit_bytes);
+        std::vector<int> rcs(plan.m, CNNACC_OK);
+        std::vector<std::thread> workers;
+        workers.reserve(plan.m);
+        for (int i = 1; i < plan.m; i++) {
+            try {
+                workers.emplace_back([&, i] { rcs[i] = run(hs[i], plan.begin(i), plan.begin(i + 1)); });
+            } catch (const std::system_error& e) {
+                rcs[i] = fail(hs[i], CNNACC_ERR_CUDA, std::string("sharded call: could not start the member's thread: ") + e.what());
+            }
+        }
+        rcs[0] = run(hs[0], plan.begin(0), plan.begin(1));
+        for (auto& t : workers) t.join();
+        for (int i = plan.m - 1; i >= 0; i--)
+            if (rcs[i]) { rc = rcs[i]; bad = i; }
+    }
+    if (failed) *failed = rc ? bad : -1;
+    return rc;
 }
 
 }  // namespace
@@ -782,6 +856,8 @@ int cnnacc_load_classifier(cnnacc_handle* h, const float* fc_w, const float* fc_
     if (!h->d_fcb) CU(h, cudaMalloc(&h->d_fcb, kMaxClasses * sizeof(float)));
     CU(h, cudaMemcpy(h->d_fcw, fc_w, (size_t)n_cls * 1024 * sizeof(float), cudaMemcpyHostToDevice));
     CU(h, cudaMemcpy(h->d_fcb, fc_b, n_cls * sizeof(float), cudaMemcpyHostToDevice));
+    std::memcpy(h->fcw_host, fc_w, (size_t)n_cls * 1024 * sizeof(float));
+    std::memcpy(h->fcb_host, fc_b, n_cls * sizeof(float));
     h->n_cls = n_cls;
     h->fc_loaded = true;
     return CNNACC_OK;
@@ -1118,6 +1194,44 @@ int cnnacc_preprocess_bgr(cnnacc_handle* h, const uint8_t* frames, int64_t n, in
 int cnnacc_detect_frames(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, uint8_t* gray128,
                          float* probs, int32_t* cls, int32_t* bbox, uint32_t flags) {
     return frames_impl(h, frames, n, fh, fw, gray128, probs, cls, bbox, true, flags);
+}
+
+int cnnacc_shard_plan_host(int64_t n, int n_handles, int64_t unit_bytes, int64_t* begin, int cap) {
+    if (n < 0 || n_handles < 1 || unit_bytes < 1 || !begin) return CNNACC_ERR_ARG;
+    const ShardPlan plan = make_shard_plan(n, n_handles, unit_bytes);
+    if (cap < plan.m + 1) return CNNACC_ERR_ARG;
+    for (int i = 0; i <= plan.m; i++) begin[i] = plan.begin(i);
+    return plan.m;
+}
+
+int cnnacc_run_batch_sharded(cnnacc_handle* const* hs, int n_handles, const uint8_t* imgs, int64_t n, int H, int W,
+                             uint8_t* feats, uint32_t flags, int* failed) {
+    const bool ok = valid_hw(H, W) && imgs && feats;
+    const size_t in_sz = ok ? (size_t)H * W : 0, out_sz = ok ? (size_t)64 * (H / 8) * (W / 8) : 0;
+    return run_sharded(hs, n_handles, n, (int64_t)in_sz, ok, flags, false, failed, [=](cnnacc_handle* h, int64_t lo, int64_t hi) {
+        return cnnacc_run_batch(h, imgs + lo * in_sz, hi - lo, H, W, feats + lo * out_sz, flags);
+    });
+}
+
+int cnnacc_infer_batch_sharded(cnnacc_handle* const* hs, int n_handles, const uint8_t* imgs, int64_t n,
+                               float* probs, int32_t* cls, int32_t* bbox, uint32_t flags, int* failed) {
+    const size_t img_sz = CNNACC_FEAT_BYTES;
+    return run_sharded(hs, n_handles, n, (int64_t)img_sz, imgs != nullptr, flags, true, failed, [=](cnnacc_handle* h, int64_t lo, int64_t hi) {
+        const int nc = h->n_cls;                                    // the same on every member (check_members)
+        return cnnacc_infer_batch(h, imgs + lo * img_sz, hi - lo, probs ? probs + lo * nc : nullptr, cls ? cls + lo : nullptr,
+                                  bbox ? bbox + lo * 4 : nullptr, flags);
+    });
+}
+
+int cnnacc_detect_frames_sharded(cnnacc_handle* const* hs, int n_handles, const uint8_t* frames, int64_t n, int fh, int fw,
+                                 uint8_t* gray128, float* probs, int32_t* cls, int32_t* bbox, uint32_t flags, int* failed) {
+    const bool ok = fh > 0 && fw > 0 && (int64_t)fh * fw <= ((int64_t)1 << 40) && frames;
+    const size_t frame_sz = ok ? (size_t)fh * fw * 3 : 0, img_sz = CNNACC_FEAT_BYTES;
+    return run_sharded(hs, n_handles, n, (int64_t)frame_sz, ok, flags, true, failed, [=](cnnacc_handle* h, int64_t lo, int64_t hi) {
+        const int nc = h->n_cls;
+        return cnnacc_detect_frames(h, frames + lo * frame_sz, hi - lo, fh, fw, gray128 ? gray128 + lo * img_sz : nullptr,
+                                    probs ? probs + lo * nc : nullptr, cls ? cls + lo : nullptr, bbox ? bbox + lo * 4 : nullptr, flags);
+    });
 }
 
 int cnnacc_probe_int8_peak(cnnacc_handle* h, double target_ms, double* tops, double* ms_out) {

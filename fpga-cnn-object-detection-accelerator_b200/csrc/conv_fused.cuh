@@ -932,15 +932,15 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+// Looked up once per process; the initialisation of a function-local static is thread-safe (handles of a sharded call encode
+// tensor maps from several threads at once).
 inline PFN_encodeTiled get_encode_tiled() {
-    static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
+    static const PFN_encodeTiled fn = [] {
         void* p = nullptr;
         cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = (PFN_encodeTiled)p;
-    }
+        return (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
+                qres == cudaDriverEntryPointSuccess) ? (PFN_encodeTiled)p : nullptr;
+    }();
     return fn;
 }
 

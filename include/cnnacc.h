@@ -19,7 +19,8 @@
  * cam pointers 4-byte aligned (they feed TMA descriptors, bulk stores and 128-bit accesses); anything else returns -2.
  *
  * Threading: one handle = one device + one stream.  A handle is not thread-safe (neither is the
- * reference: arm_cnn.c:30-32 static scratch); distinct handles are independent.
+ * reference: arm_cnn.c:30-32 static scratch); distinct handles are independent.  The cnnacc_*_sharded calls spread one host
+ * batch over several handles, one thread per handle.
  */
 #ifndef CNNACC_H
 #define CNNACC_H
@@ -201,6 +202,34 @@ int cnnacc_detect_frames(cnnacc_handle *h, const uint8_t *frames, int64_t n, int
  *                 12.2.0).  File decoding itself stays on the host. */
 int cnnacc_image_to_gray128(cnnacc_handle *h, const uint8_t *img, int64_t n, int H, int W, int C,
                             uint8_t *gray128, uint32_t flags);
+
+/* ---- one host batch over several GPUs ------------------------------------------------------------------------------------
+ * The sharded forms of cnnacc_run_batch / cnnacc_infer_batch / cnnacc_detect_frames for HOST pointers take an array of
+ * n_handles member handles the caller created and configured (usually one per GPU; two handles on one GPU are allowed) and
+ * cut the n images / frames into contiguous shards: shard i = [begin[i], begin[i+1]) runs through member i's own
+ * single-handle host path with every pointer offset to that slice, so the outputs are those of one handle, byte for byte.
+ * The calling thread runs shard 0; shards 1 .. m-1 run on a thread each that the call starts and joins before it returns (a
+ * call small enough for one member starts none), so every member handle is used by one thread only.
+ *   Plan (csrc/shard_plan.h): m = min(n_handles, max(1, n * unit_bytes / kMinShardBytes)) members, begin[i] = n*i/m, where
+ *   unit_bytes is the input size of one image (H*W) or frame (fh*fw*3).
+ *   Checked before any member starts (nothing is launched; -2 or -4): hs / an entry NULL, n_handles < 1, a handle listed
+ *   twice, CNNACC_FLAG_DEVICE_PTRS or CNNACC_FLAG_KEEP_MAPS set, a member without weights (-4) or -- for the prediction
+ *   calls -- without a classifier (-4), and members configured unlike member 0: weights, shifts, accumulator bits and, for
+ *   the prediction calls, the classifier (-2).  The other flags pass through to every member unchanged.
+ *   Errors: every started shard runs to completion; the call returns the code of the lowest-index failing member and, when
+ *   failed != NULL, stores that index there (-1 on success, or when no member is at fault: hs NULL / n_handles < 1).  The text
+ *   stays in that member's cnnacc_last_error.  After a failure the outputs of the whole call are undefined.
+ *   Host buffers should be page-locked (cnnacc_alloc_host / cnnacc_register_host pin memory for every GPU at once); pageable
+ *   memory works but makes each member's copies synchronous and slow. */
+int cnnacc_run_batch_sharded(cnnacc_handle *const *hs, int n_handles, const uint8_t *imgs, int64_t n, int H, int W,
+                             uint8_t *feats, uint32_t flags, int *failed);
+int cnnacc_infer_batch_sharded(cnnacc_handle *const *hs, int n_handles, const uint8_t *imgs, int64_t n,
+                               float *probs, int32_t *cls, int32_t *bbox, uint32_t flags, int *failed);
+int cnnacc_detect_frames_sharded(cnnacc_handle *const *hs, int n_handles, const uint8_t *frames, int64_t n, int fh, int fw,
+                                 uint8_t *gray128, float *probs, int32_t *cls, int32_t *bbox, uint32_t flags, int *failed);
+/* Host-only view of the shard plan: begin[0 .. m] (m + 1 entries, begin[m] = n).  Returns m, or a negative code when n < 0,
+ * n_handles < 1, unit_bytes < 1 or cap < m + 1.  No GPU needed; tests/ check that every plan covers the call exactly once. */
+int cnnacc_shard_plan_host(int64_t n, int n_handles, int64_t unit_bytes, int64_t *begin, int cap);
 
 /* ---- host memory the DMA engines can stream from (pynq.allocate, realtime_detect.py:293,301) */
 int cnnacc_alloc_host(size_t bytes, void **out);
