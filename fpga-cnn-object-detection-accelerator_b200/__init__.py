@@ -7,8 +7,9 @@ the host-side mirror of the reference's engine objects; the work happens in libc
 from . import _lib
 from ._lib import build, load
 from .accelerator import (ARMEngine, B200Engine, CNNAccelerator, Classifier, MultiAccelerator, NAMES, alloc_host, bbox_vec,
-                          classify_vec, dump_features, load_arm_cnn_lib, load_features, load_image_any, register_host,
-                          train_linear_classifier)
+                          classify_vec, dump_features, grid_regions, load_arm_cnn_lib, load_features, load_image_any,
+                          region_boxes_to_frame, register_host, train_linear_classifier)
 
 __all__ = ["ARMEngine", "B200Engine", "CNNAccelerator", "Classifier", "MultiAccelerator", "dump_features", "load_features", "NAMES", "alloc_host", "register_host", "load_image_any", "train_linear_classifier", "bbox_vec", "classify_vec",
+           "grid_regions", "region_boxes_to_frame",
            "load_arm_cnn_lib", "build", "load", "_lib"]

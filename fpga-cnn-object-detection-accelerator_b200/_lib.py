@@ -50,6 +50,12 @@ SYMBOLS = {
     "cnnacc_preprocess_bgr": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_uint32]),
     "cnnacc_detect_frames": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p,
                                         _c.c_void_p, _c.c_uint32]),
+    "cnnacc_preprocess_regions": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int64,
+                                             _c.c_void_p, _c.c_uint32]),
+    "cnnacc_detect_regions": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_void_p,
+                                         _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_uint32]),
+    "cnnacc_region_plan_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int]),
+    "cnnacc_area_tab_host": (_c.c_int, [_c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_int]),
     "cnnacc_image_to_gray128": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p, _c.c_uint32]),
     "cnnacc_run_batch_sharded": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p,
                                             _c.c_uint32, _c.POINTER(_c.c_int)]),

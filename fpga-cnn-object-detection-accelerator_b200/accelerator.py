@@ -430,6 +430,73 @@ class CNNAccelerator:
                                                     _lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0))
         return (cls, probs, box, gray) if return_gray else (cls, probs, box)
 
+    def detect_regions(self, frames, regions, bbox="vec", logits=False, return_gray=False):
+        """detect_frames on caller-chosen square regions: frames [F,h,w,3] u8 BGR (numpy, or a contiguous CUDA uint8 tensor run
+        on torch's current stream), regions (R,4) integers (frame, x, y, side) in any order, side 128..8192, inside its
+        frame.  Region r's results are those detect_frames gives for frames[f][y:y+side, x:x+side] as a frame of its own; its
+        box is in that square's 128x128 coordinates (region_boxes_to_frame maps it to frame pixels).
+        -> (cls [R], probs [R,n_cls], bbox [R,4][, gray128 [R,128,128]]) in the order of `regions`, numpy or torch like frames."""
+        if bbox not in ("vec", "upsampled"):
+            raise ValueError("bbox must be 'vec' or 'upsampled'")
+        if self._n_cls == 0:
+            raise RuntimeError("classifier not loaded")
+        flags = (_lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0) | (_lib.FLAG_LOGITS if logits else 0)
+        return self._regions(frames, regions, True, return_gray, flags)
+
+    def preprocess_regions(self, frames, regions):
+        """preprocess on caller-chosen square regions (see detect_regions) -> gray128 [R,128,128] u8 in the order of `regions`."""
+        return self._regions(frames, regions, False, True, 0)[0]
+
+    def _regions(self, frames, regions, detect, want_gray, flags):
+        reg = np.asarray(regions)
+        if reg.ndim != 2 or reg.shape[1] != 4 or not (reg.size == 0 or np.issubdtype(reg.dtype, np.integer)):
+            raise ValueError("regions must be an (R, 4) integer array of (frame, x, y, side)")
+        reg = reg.astype(np.int64)
+        if reg.size and (reg.min() < -2 ** 31 or reg.max() >= 2 ** 31):
+            raise ValueError("region values must fit int32")
+        order = np.argsort(reg[:, 0], kind="stable")         # the library takes regions grouped by frame
+        shuffled = bool((order != np.arange(len(order))).any())
+        reg = np.ascontiguousarray(reg[order], dtype=np.int32)
+        n = reg.shape[0]
+        nc = self._n_cls
+        if _is_torch_cuda(frames):
+            import torch
+            if frames.dim() != 4 or frames.shape[3] != 3 or frames.dtype != torch.uint8 or not frames.is_contiguous():
+                raise ValueError("expected a contiguous [F,h,w,3] uint8 tensor")
+            nf, fh, fw = frames.shape[:3]
+            new = lambda shape, dt: torch.empty(shape, dtype=dt, device=frames.device)
+            gray = new((n, 128, 128), torch.uint8) if want_gray else None
+            outs = (new((n,), torch.int32), new((n, nc), torch.float32), new((n, 4), torch.int32)) if detect else ()
+            ptr = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+            with self._on_stream_of(frames):
+                self._call_regions(ptr(frames), nf, fh, fw, reg, ptr(gray), [ptr(t) for t in outs], detect,
+                                   flags | _lib.FLAG_DEVICE_PTRS)
+            res = outs + ((gray,) if want_gray else ())
+            if shuffled:
+                inv = torch.from_numpy(np.argsort(order)).to(frames.device)
+                res = tuple(t[inv] for t in res)
+            return res
+        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        if frames.ndim != 4 or frames.shape[3] != 3:
+            raise ValueError("expected [F,h,w,3] BGR frames")
+        nf, fh, fw = frames.shape[:3]
+        gray = np.empty((n, 128, 128), dtype=np.uint8) if want_gray else None
+        outs = (np.empty((n,), np.int32), np.empty((n, nc), np.float32), np.empty((n, 4), np.int32)) if detect else ()
+        self._call_regions(_vp(frames), nf, fh, fw, reg, _vp(gray) if want_gray else None, [_vp(a) for a in outs], detect, flags)
+        res = outs + ((gray,) if want_gray else ())
+        if shuffled:
+            inv = np.argsort(order)
+            res = tuple(a[inv] for a in res)
+        return res
+
+    def _call_regions(self, frames_p, nf, fh, fw, reg, gray_p, outs_p, detect, flags):
+        if detect:
+            cls_p, probs_p, box_p = outs_p
+            self._check(self._libc.cnnacc_detect_regions(self._h, frames_p, nf, fh, fw, _vp(reg), reg.shape[0], gray_p,
+                                                         probs_p, cls_p, box_p, flags))
+        else:
+            self._check(self._libc.cnnacc_preprocess_regions(self._h, frames_p, nf, fh, fw, _vp(reg), reg.shape[0], gray_p, flags))
+
     def infer_one(self, gray128):
         """One image, lowest latency.  -> (feat (64,256) u8, conv_ms, read_ms)."""
         img = gray128 if (type(gray128) is np.ndarray and gray128.dtype == np.uint8 and gray128.flags.c_contiguous) \
@@ -441,6 +508,49 @@ class CNNAccelerator:
         if rc:
             self._check(rc)
         return feat, c._obj.value, r._obj.value
+
+
+def _tile_origins(size, side, stride):
+    pos = list(range(0, size - side + 1, stride))
+    if pos[-1] != size - side:
+        pos.append(size - side)                              # one tile flush with the far edge
+    return pos
+
+
+def grid_regions(n_frames, fh, fw, sides, strides):
+    """Regions (frame, x, y, side) tiling every frame of a [n_frames, fh, fw, 3] batch at each side: tiles at x = 0, stride,
+    2 stride, ... plus one flush with the right edge (x = fw - side) when that position is missing, the same for y.  `sides`
+    and `strides` are ints or equal-length sequences.  Frame-major (frame, then side in the given order, then y, then x): the
+    order CNNAccelerator.detect_regions hands to the library unchanged.  -> (R, 4) int32."""
+    sides = [int(s) for s in np.atleast_1d(sides)]
+    strides = [int(s) for s in np.atleast_1d(strides)]
+    if len(strides) == 1:
+        strides = strides * len(sides)
+    if len(strides) != len(sides):
+        raise ValueError("sides and strides must have the same length")
+    per_frame = []
+    for side, stride in zip(sides, strides):
+        if side < 1 or side > min(fh, fw) or stride < 1:
+            raise ValueError(f"side {side} / stride {stride} does not fit a {fh}x{fw} frame")
+        for y in _tile_origins(fh, side, stride):
+            for x in _tile_origins(fw, side, stride):
+                per_frame.append((x, y, side))
+    tiles = np.array(per_frame, dtype=np.int32).reshape(-1, 3)
+    out = np.empty((int(n_frames), len(tiles), 4), dtype=np.int32)
+    out[:, :, 0] = np.arange(int(n_frames), dtype=np.int32)[:, None]
+    out[:, :, 1:] = tiles[None]
+    return out.reshape(-1, 4)
+
+
+def region_boxes_to_frame(regions, bbox):
+    """Boxes of detect_regions (x1, y1, x2, y2 on the region's 128x128 grid) in frame pixels: x + b * side / 128 for x1 and
+    x2, y + b * side / 128 for y1 and y2, as float64.  This is the one mapping the library documents; it merges nothing
+    (no NMS).  -> (R, 4) float64."""
+    reg = np.asarray(regions, dtype=np.float64).reshape(-1, 4)
+    b = np.asarray(bbox, dtype=np.float64).reshape(-1, 4)
+    scale = reg[:, 3:4] / 128.0
+    origin = np.concatenate([reg[:, 1:3], reg[:, 1:3]], axis=1)
+    return origin + b * scale
 
 
 class MultiAccelerator:

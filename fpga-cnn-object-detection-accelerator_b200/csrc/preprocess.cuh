@@ -35,37 +35,66 @@ struct AreaTabHost {
     std::vector<float> alpha;                  // [128][taps]
 };
 
-// computeResizeAreaTab(ssize = S, dsize = 128, scale = S/128.) in OpenCV's order
+// The INTER_AREA taps of output index d for a square side S (128..8192): OpenCV's computeResizeAreaTab(ssize = S, dsize = 128,
+// scale = S/128.) for one d, in its order (double arithmetic, then float).  The taps are the consecutive source indices
+// first .. first+n-1; tap i weighs area_tap_weight(t, i).  Integer scales (S = 128 k) give k taps of weight 1 (their kernels
+// sum integers instead).  Host (make_area_tab, cnnacc_area_tab_host) and device (regions.cuh) get the same bits: scale = S/128
+// is exact, so are d * scale, fsx1 + scale and S - fsx1 for S <= 8192 (at most 20 significant bits) -- an FMA the compiler
+// forms from them rounds nothing -- ceil / floor / min are exact, and the three divisions are correctly rounded in IEEE double
+// on both sides.  Up to 65 taps per output at S = 8191: the weights stay three scalars (first partial, 1/cell, last partial)
+// instead of a table in registers.
+struct AreaTaps {
+    int first, n;
+    bool head, tail;                 // tap 0 / tap n-1 is a partial cell
+    float a_head, a_mid, a_tail;
+};
+
+__host__ __device__ __forceinline__ AreaTaps area_taps(int S, int d) {
+    AreaTaps t;
+    if (S % kPrepOut == 0) {
+        const int k = S / kPrepOut;
+        t.first = d * k; t.n = k; t.head = t.tail = false; t.a_head = t.a_mid = t.a_tail = 1.f;
+        return t;
+    }
+    const double scale = (double)S / kPrepOut;
+    const double fsx1 = d * scale, fsx2 = fsx1 + scale;
+    const double cell = scale < S - fsx1 ? scale : S - fsx1;
+    int sx1 = (int)ceil(fsx1), sx2 = (int)floor(fsx2);
+    sx2 = sx2 < S - 1 ? sx2 : S - 1;
+    sx1 = sx1 < sx2 ? sx1 : sx2;
+    t.head = sx1 - fsx1 > 1e-3;
+    t.tail = fsx2 - sx2 > 1e-3;
+    t.first = t.head ? sx1 - 1 : sx1;
+    t.n = (int)t.head + (sx2 - sx1) + (int)t.tail;
+    double last = fsx2 - sx2;
+    last = last < 1. ? last : 1.;
+    last = last < cell ? last : cell;
+    t.a_head = (float)((sx1 - fsx1) / cell);
+    t.a_mid = (float)(1.0 / cell);
+    t.a_tail = (float)(last / cell);
+    return t;
+}
+
+__host__ __device__ __forceinline__ float area_tap_weight(const AreaTaps& t, int i) {
+    return (t.head && i == 0) ? t.a_head : (t.tail && i == t.n - 1) ? t.a_tail : t.a_mid;
+}
+
+// The whole table of one side (the same for x and y: the crop is square)
 inline AreaTabHost make_area_tab(int S) {
     AreaTabHost t;
     t.start.assign(kPrepOut, 0); t.cnt.assign(kPrepOut, 1);
-    if (S == kPrepOut) {
-        t.mode = kPrepCopy; t.alpha.assign(kPrepOut, 1.f);
-        for (int d = 0; d < kPrepOut; d++) t.start[d] = d;
-        return t;
-    }
     if (S % kPrepOut == 0) {
-        t.k = S / kPrepOut; t.mode = t.k == 2 ? kPrepBox2 : kPrepBoxK; t.inv = 1.f / (float)(t.k * t.k);
-        for (int d = 0; d < kPrepOut; d++) { t.start[d] = d * t.k; t.cnt[d] = t.k; }
-        t.alpha.assign(kPrepOut, 1.f);
-        return t;
+        t.k = S / kPrepOut; t.mode = t.k == 1 ? kPrepCopy : t.k == 2 ? kPrepBox2 : kPrepBoxK; t.inv = 1.f / (float)(t.k * t.k);
+    } else {
+        t.mode = kPrepFrac;
+        t.taps = (int)std::ceil((double)S / kPrepOut) + 2;
     }
-    t.mode = kPrepFrac;
-    const double scale = (double)S / kPrepOut;
-    t.taps = (int)std::ceil(scale) + 2;
-    t.alpha.assign((size_t)kPrepOut * t.taps, 0.f);
-    for (int dx = 0; dx < kPrepOut; dx++) {
-        const double fsx1 = dx * scale, fsx2 = fsx1 + scale;
-        const double cell = std::min(scale, S - fsx1);
-        int sx1 = (int)std::ceil(fsx1), sx2 = (int)std::floor(fsx2);
-        sx2 = std::min(sx2, S - 1);
-        sx1 = std::min(sx1, sx2);
-        int n = 0, first = sx1;
-        float* a = &t.alpha[(size_t)dx * t.taps];
-        if (sx1 - fsx1 > 1e-3) { first = sx1 - 1; a[n++] = (float)((sx1 - fsx1) / cell); }
-        for (int sx = sx1; sx < sx2; sx++) a[n++] = float(1.0 / cell);
-        if (fsx2 - sx2 > 1e-3) a[n++] = (float)(std::min(std::min(fsx2 - sx2, 1.), cell) / cell);
-        t.start[dx] = first; t.cnt[dx] = n;         // the taps are consecutive source indices first .. first+n-1
+    t.alpha.assign((size_t)kPrepOut * t.taps, 1.f);
+    for (int d = 0; d < kPrepOut; d++) {
+        const AreaTaps a = area_taps(S, d);
+        t.start[d] = a.first; t.cnt[d] = a.n;
+        if (t.mode == kPrepFrac)
+            for (int i = 0; i < t.taps; i++) t.alpha[(size_t)d * t.taps + i] = i < a.n ? area_tap_weight(a, i) : 0.f;
     }
     return t;
 }

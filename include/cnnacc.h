@@ -195,6 +195,36 @@ int cnnacc_preprocess_bgr(cnnacc_handle *h, const uint8_t *frames, int64_t n, in
 int cnnacc_detect_frames(cnnacc_handle *h, const uint8_t *frames, int64_t n, int fh, int fw, uint8_t *gray128,
                          float *probs, int32_t *cls, int32_t *bbox, uint32_t flags);
 
+/* ---- the same loop body on caller-chosen square regions of each frame -------------------------------------------------
+ * A region is four int32 (frame, x, y, side): the square frames[frame][y:y+side, x:x+side, :] of the BGR frames
+ * [n_frames][fh][fw][3] u8.  For every region the calls produce exactly what preprocess_bgr / detect_frames produce for that
+ * square cut out as a frame of its own (a square is its own centre crop): gray128 / cls / bbox byte for byte, probs bit for
+ * bit.  Boxes stay in the region's own 128x128 coordinates.  One call mixes any sides: the INTER_AREA taps are computed in the
+ * kernel from each region's side.  Outputs are indexed by region, in the order of `regions`.
+ *   regions : [n_regions][4] int32 in HOST memory in both modes, read only during the call (reusable once it returns).  The
+ *             frame indices must not decrease (group the regions by frame).  frames / gray128 / probs / cls / bbox are host or
+ *             device memory as for detect_frames, with the same flags, alignment rules and NULL conventions (gray128 may be
+ *             NULL in detect_regions; any prediction array may be NULL).
+ *   -2, nothing launched: n_regions > 0 with regions or frames NULL, a frame index outside [0, n_frames), a side outside
+ *             128..8192, x < 0, y < 0, x + side > fw, y + side > fh, or frame indices that decrease.  n_regions == 0 returns 0.
+ *   detect_regions returns -4 without weights or without a classifier.
+ * Host pointers: the call copies each run of consecutive referenced frames once (about 16 MiB per staged chunk; unreferenced
+ * frames never cross the link) and runs all regions of a frame on that copy.  Device pointers: asynchronous on the handle's
+ * stream; the library keeps its own device copy of the descriptors alive until the call's kernels are done. */
+int cnnacc_preprocess_regions(cnnacc_handle *h, const uint8_t *frames, int64_t n_frames, int fh, int fw,
+                              const int32_t *regions, int64_t n_regions, uint8_t *gray128, uint32_t flags);
+int cnnacc_detect_regions(cnnacc_handle *h, const uint8_t *frames, int64_t n_frames, int fh, int fw,
+                          const int32_t *regions, int64_t n_regions, uint8_t *gray128,
+                          float *probs, int32_t *cls, int32_t *bbox, uint32_t flags);
+/* Host-only view of the staging plan of a host-pointer region call (csrc/region_plan.h): chunk i stages frames
+ * [chunks[4i], chunks[4i+1]) with one copy and runs regions [chunks[4i+2], chunks[4i+3]) on them.  Returns the number of chunks
+ * (<= cap), or -2 for a region array the real call refuses, or when cap is too small.  No GPU needed. */
+int cnnacc_region_plan_host(const int32_t *regions, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t *chunks, int cap);
+/* Host-only view of the INTER_AREA taps the kernels use for one crop side (128..8192): output index d reads source indices
+ * start[d] .. start[d]+cnt[d]-1 with weights alpha[d*taps_cap + i] (zero beyond cnt[d]; weight 1 at integer scales, whose
+ * kernels sum integers).  Returns the largest cnt, or -2 when it exceeds taps_cap.  No GPU needed. */
+int cnnacc_area_tab_host(int side, int *start, int *cnt, float *alpha, int taps_cap);
+
 /* image_to_gray128: the image-loading step of pynq_inference.py, load_image_any (:414-425), for n decoded images of one size:
  *                 img [n][H][W][C] u8 with C = 1 (mode L), 3 (RGB) or 4 (RGBA) -> gray128 [n][128][128] u8 =
  *                 Image.convert('L').resize((128, 128)): Pillow's ITU-R 601 integer luma and its default BICUBIC resampler
