@@ -1487,18 +1487,35 @@ int cnnacc_image_to_gray128(cnnacc_handle* h, const uint8_t* img, int64_t n, int
         CU(h, cudaMemcpyAsync(h->d_pil_in, img, in_bytes, cudaMemcpyHostToDevice, st));
         d_in = h->d_pil_in; d_out = h->d_pil_out;
     }
-    const bool need_v = H != kPilOut;
-    // the horizontal pass (or, at W == 128, the plain gray conversion) writes [n][H][128]: the result itself when H == 128
-    uint8_t* d_tmp = d_out;
-    if (need_v) {
-        if ((rc = grow(h, &h->d_pil_tmp, &h->cap_pil_tmp, (size_t)n * H * kPilOut))) return rc;
-        d_tmp = h->d_pil_tmp;
-    }
-    pil_horizontal_kernel<<<dim3((unsigned)H, (unsigned)n), kPilOut, 0, st>>>(d_in, d_tmp, h->d_pil_kx, h->d_pil_bx, h->pil_kw, H, W, C, W == kPilOut);
-    h->launches++;
-    if (need_v) {
-        pil_vertical_kernel<<<dim3(kPilOut, (unsigned)n), kPilOut, 0, st>>>(d_tmp, d_out, h->d_pil_ky, h->d_pil_by, h->pil_kh, H);
+    const unsigned nu = (unsigned)n;
+    if (H > 100 * W && H > kPilOut) {
+        // Pillow's order for a very tall image (H > 100 W, so W <= 327): the vertical pass over the source, gray conversion
+        // folded in, writes [n][128][W] -- the result itself when W == 128 -- and the horizontal pass reads that
+        uint8_t* d_tmp = d_out;
+        if (W != kPilOut) {
+            if ((rc = grow(h, &h->d_pil_tmp, &h->cap_pil_tmp, (size_t)n * kPilOut * W))) return rc;
+            d_tmp = h->d_pil_tmp;
+        }
+        pil_vertical_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_in, d_tmp, h->d_pil_ky, h->d_pil_by, h->pil_kh, H, W, C);
         h->launches++;
+        if (W != kPilOut) {
+            pil_horizontal_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_tmp, d_out, h->d_pil_kx, h->d_pil_bx, h->pil_kw, kPilOut, W, 1, 0);
+            h->launches++;
+        }
+    } else {
+        const bool need_v = H != kPilOut;
+        // the horizontal pass (or, at W == 128, the plain gray conversion) writes [n][H][128]: the result itself when H == 128
+        uint8_t* d_tmp = d_out;
+        if (need_v) {
+            if ((rc = grow(h, &h->d_pil_tmp, &h->cap_pil_tmp, (size_t)n * H * kPilOut))) return rc;
+            d_tmp = h->d_pil_tmp;
+        }
+        pil_horizontal_kernel<<<dim3((unsigned)H, nu), kPilOut, 0, st>>>(d_in, d_tmp, h->d_pil_kx, h->d_pil_bx, h->pil_kw, H, W, C, W == kPilOut);
+        h->launches++;
+        if (need_v) {
+            pil_vertical_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_tmp, d_out, h->d_pil_ky, h->d_pil_by, h->pil_kh, H, kPilOut, 1);
+            h->launches++;
+        }
     }
     CU(h, cudaGetLastError());
     if (!dev) {

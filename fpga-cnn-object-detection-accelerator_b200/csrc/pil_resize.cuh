@@ -8,8 +8,10 @@
 //   * resize() of a mode "L" image defaults to BICUBIC (a = -0.5, support 2); when shrinking, the support and the filter
 //     argument scale with the ratio (antialiasing).  8-bit images are resampled in integers (src/libImaging/Resample.c):
 //     per output index a window [xmin, xmin + xmax) and coefficients normalised in double precision, rounded to 22
-//     fractional bits; out = clip8((2^21 + sum in * k) >> 22); horizontal pass first (skipped when the width is already
-//     128), rounded to u8, then the vertical pass (skipped when the height is already 128).
+//     fractional bits; out = clip8((2^21 + sum in * k) >> 22); one pass rounded to u8, then the other; a pass is skipped
+//     when that side is already 128;
+//   * pass order (PIL/Image.py Image.resize): horizontal first, except that an image more than 100 times taller than wide
+//     (H > 100 W, H > 128) is first resized to (W, 128) and then to (128, 128), i.e. the vertical pass runs first.
 // The coefficient tables depend on the input size, so they are built on the host exactly as precompute_coeffs /
 // normalize_coeffs_8bpc do and cached per (H, W) in the handle.
 #pragma once
@@ -88,19 +90,24 @@ pil_horizontal_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ tmp,
     dst[xx] = pil_clip8_acc(acc);
 }
 
-// Vertical pass: one CTA per (output row, image), thread = column.  tmp [n][H][128] -> out [n][128][128].
+// Vertical pass (and the gray conversion): one CTA per (output row, image), thread = column, looping over the W columns.
+// in [n][H][W][C] -> out [n][128][W].  Horizontal-first runs it on the [n][H][128] u8 result of the horizontal pass (W = 128,
+// C = 1); vertical-first on the source image, and the horizontal pass then reads its [n][128][W] output (H = 128, C = 1).
 __global__ void __launch_bounds__(kPilOut)
-pil_vertical_kernel(const uint8_t* __restrict__ tmp, uint8_t* __restrict__ out, const int32_t* __restrict__ k,
-                    const int32_t* __restrict__ bounds, int ksize, int H)
+pil_vertical_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, const int32_t* __restrict__ k,
+                    const int32_t* __restrict__ bounds, int ksize, int H, int W, int C)
 {
-    const int xx = threadIdx.x, yy = blockIdx.x;
+    const int yy = blockIdx.x;
     const size_t img = blockIdx.y;
     const int ymin = bounds[2 * yy], cnt = bounds[2 * yy + 1];
     const int32_t* kk = k + (size_t)yy * ksize;
-    const uint8_t* src = tmp + (img * H + ymin) * kPilOut + xx;
-    int acc = 1 << (kPilCoefBits - 1);
-    for (int y = 0; y < cnt; y++) acc += (int)src[(size_t)y * kPilOut] * kk[y];
-    out[(img * kPilOut + yy) * kPilOut + xx] = pil_clip8_acc(acc);
+    const size_t row = (size_t)W * C;
+    for (int x = threadIdx.x; x < W; x += blockDim.x) {
+        const uint8_t* src = in + (img * H + ymin) * row + (size_t)x * C;
+        int acc = 1 << (kPilCoefBits - 1);
+        for (int y = 0; y < cnt; y++) acc += (int)pil_gray(src + (size_t)y * row, C) * kk[y];
+        out[(img * kPilOut + yy) * W + x] = pil_clip8_acc(acc);
+    }
 }
 
 }  // namespace cnnacc

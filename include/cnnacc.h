@@ -228,8 +228,8 @@ int cnnacc_area_tab_host(int side, int *start, int *cnt, float *alpha, int taps_
 /* image_to_gray128: the image-loading step of pynq_inference.py, load_image_any (:414-425), for n decoded images of one size:
  *                 img [n][H][W][C] u8 with C = 1 (mode L), 3 (RGB) or 4 (RGBA) -> gray128 [n][128][128] u8 =
  *                 Image.convert('L').resize((128, 128)): Pillow's ITU-R 601 integer luma and its default BICUBIC resampler
- *                 (22-bit fixed point, horizontal pass then vertical pass), reproduced bit for bit (pinned against Pillow
- *                 12.2.0).  File decoding itself stays on the host. */
+ *                 (22-bit fixed point, horizontal pass then vertical pass, or vertical first when H > 100 W as Image.resize
+ *                 does), reproduced bit for bit (pinned against Pillow 12.2.0).  File decoding itself stays on the host. */
 int cnnacc_image_to_gray128(cnnacc_handle *h, const uint8_t *img, int64_t n, int H, int W, int C,
                             uint8_t *gray128, uint32_t flags);
 

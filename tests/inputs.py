@@ -244,9 +244,88 @@ def make_pil_image(case):
     elif tag == "smooth":
         hh, ww = -(-h // 16) * 16, -(-w // 16) * 16
         planes = [smooth_images(seed * 5 + c, 1, hh, ww)[0, :h, :w] for c in range(ch)]
+    elif tag == "stripes":                          # saturated 0 / 255 diagonal stripes: the largest swings of the filter sums
+        rng = np.random.default_rng(seed)
+        yy, xx = np.ogrid[:h, :w]
+        planes = [((((xx + yy * int(rng.integers(1, 4))) // int(rng.integers(1, 4))) % 2) * 255).astype(np.uint8)
+                  for _ in range(ch)]
+    elif tag == "const":                            # ('const', value): every pixel of every channel; 255 gives the largest sums
+        planes = [np.full((h, w), seed, dtype=np.uint8) for _ in range(ch)]
     else:
         planes = [np.random.default_rng(seed * 5 + c).integers(0, 256, (h, w), dtype=np.uint8) for c in range(ch)]
     return planes[0] if ch == 1 else np.ascontiguousarray(np.stack(planes, axis=-1))
+
+
+def _resample_pil_cases():
+    """load_image_any at the edges of its domain, pinned by tests/golden/resample_edges.npz (make_resample_edges_golden.py runs
+    Pillow itself).  Image.resize runs the vertical pass first when H > 100 W, so both sides of that switch are here for several
+    widths (H is capped at the 32768 the loader accepts, so W = 328 has only 32768x328, which runs horizontal first), in every
+    mode, plus the extreme shapes and both orientations of a strip."""
+    cases, seed = [], 1000
+    def add(h, w, mode, tag):
+        nonlocal seed
+        content = ("const", 255) if tag == "full" else (tag, seed)
+        cases.append(dict(name=f"pil_{h}x{w}_{mode}_{tag}", mode=mode, images=content, h=h, w=w))
+        seed += 1
+    for w in (2, 3, 7, 64, 129, 327, 328):
+        for h in sorted({min(100 * w, 32768), min(100 * w + 1, 32768)}):
+            for mode, tag in (("L", "rng"), ("L", "stripes"), ("L", "full"), ("RGB", "rng"), ("RGBA", "stripes")):
+                add(h, w, mode, tag)
+    for h, w in ((1, 1), (1, 2), (2, 1), (1, 32768), (32768, 1), (3, 32768), (32768, 5), (32768, 128), (128, 32768)):
+        add(h, w, "L", "rng")
+    for h, w, mode, tag in ((3, 32768, "RGB", "rng"), (32768, 5, "RGB", "rng"), (32768, 5, "L", "full"),
+                            (17, 2000, "L", "rng"), (2000, 17, "L", "rng"), (17, 2000, "RGB", "stripes"), (2000, 17, "RGB", "stripes")):
+        add(h, w, mode, tag)
+    return cases
+
+
+RESAMPLE_PIL_CASES = _resample_pil_cases()
+
+# centre-crop pre-processing at the large crop sides, pinned by tests/golden/resample_edges.npz (cv2 4.13.0): integer scales
+# k = 9, 16, 32, 63, 64 (k != 2^j: the rounded 1/(k*k)), fractional sides up to 65 taps, 4K frames (one per 16 MiB staging
+# chunk) and 8192x8192 frames (201 MB, above the 64 MiB latency path)
+RESAMPLE_AREA_CASES = [
+    dict(name="area_k9_1152", frames=("rng", 1200), n=2, h=1152, w=1300),
+    dict(name="area_k16_2048", frames=("edges", 1201), n=1, h=2100, w=2048),
+    dict(name="area_k32_4096", frames=("rng", 1202), n=1, h=4096, w=4096),
+    dict(name="area_k63_8064", frames=("edges", 1203), n=1, h=8064, w=8100),
+    dict(name="area_k64_8192", frames=("rng", 1204), n=1, h=8192, w=8192),
+    dict(name="area_k64_8192_edges", frames=("edges", 1205), n=1, h=8192, w=8192),
+    dict(name="area_1081", frames=("rng", 1206), n=2, h=1081, w=1500),
+    dict(name="area_2047", frames=("edges", 1207), n=2, h=2047, w=2047),
+    dict(name="area_2049", frames=("rng", 1208), n=1, h=2200, w=2049),
+    dict(name="area_4095", frames=("edges", 1209), n=1, h=4095, w=4200),
+    dict(name="area_4097", frames=("rng", 1210), n=1, h=4097, w=4097),
+    dict(name="area_8191", frames=("edges", 1211), n=1, h=8191, w=8191),
+    dict(name="area_4k", frames=("rng", 1212), n=3, h=2160, w=3840),
+    dict(name="area_4k_edges", frames=("edges", 1213), n=2, h=2160, w=3840),
+]
+
+
+def make_area_frames(name):
+    """The seeded frames of the RESAMPLE_AREA_CASES case `name`."""
+    c = next(c for c in RESAMPLE_AREA_CASES if c["name"] == name)
+    return make_frames(c["frames"], c["n"], c["h"], c["w"])
+
+
+AREA_LARGE_SIDES = (1081, 1152, 2047, 2048, 2049, 4095, 4096, 4097, 8064, 8191, 8192)
+
+
+def corner_regions(frame, fh, fw, sides=AREA_LARGE_SIDES):
+    """(frame, x, y, side) for every side at the four corners of the frame."""
+    return np.array([(frame, x, y, s) for s in sides for x, y in ((0, 0), (fw - s, 0), (0, fh - s), (fw - s, fh - s))], np.int32)
+
+
+# regions of the 8192x8192 frames of area_k64_8192 and area_k64_8192_edges (201 MB each: one frame per staging chunk): every
+# large side at the four corners of the first, three odd sides on the second
+REGIONS_8192 = np.concatenate([corner_regions(0, 8192, 8192),
+                               np.array([(1, 1, 8192 - 8191, 8191), (1, 8192 - 4097, 3, 4097), (1, 2049, 4000, 2049)], np.int32)])
+
+
+# several regions of the frames of area_4k (frame 1 unreferenced), through host staging of one 4K frame per chunk
+REGIONS_4K = np.array([(0, 0, 0, 2160), (0, 3840 - 2049, 111, 2049), (0, 1000, 2160 - 1081, 1081), (0, 3840 - 128, 2160 - 128, 128),
+                       (0, 1680, 1, 2047), (2, 17, 3, 2047), (2, 3840 - 1152, 0, 1152), (2, 1500, 50, 2048), (2, 0, 2160 - 129, 129),
+                       (2, 1792, 1008, 1152)], np.int32)
 
 
 def make_training_set(seed=90, n=300, n_cls=6, noise=0.35):
