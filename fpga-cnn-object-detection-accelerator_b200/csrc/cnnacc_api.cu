@@ -50,7 +50,7 @@ struct DescBuf {
 struct Slot {
     cudaEvent_t ev_in = nullptr, ev_k = nullptr, ev_out = nullptr;   // H2D landed / kernels done / D2H drained
     uint8_t *d_in = nullptr, *d_out = nullptr;
-    float* d_probs = nullptr; int32_t* d_cls = nullptr; int32_t* d_bbox = nullptr;
+    int32_t *d_cls = nullptr, *d_bbox = nullptr;            // cnnacc_cam_bbox_batch's classes in and boxes out
     size_t cap_in = 0, cap_out = 0, cap_pred = 0;
 };
 
@@ -87,11 +87,8 @@ struct cnnacc_handle {
     int pil_h = 0, pil_w = 0, pil_kh = 0, pil_kw = 0;
     int32_t *d_pil_kx = nullptr, *d_pil_bx = nullptr, *d_pil_ky = nullptr, *d_pil_by = nullptr;
     uint8_t *d_pil_tmp = nullptr, *d_pil_in = nullptr, *d_pil_out = nullptr; size_t cap_pil_tmp = 0, cap_pil_in = 0, cap_pil_out = 0;
-    // small calls (<= kSmallN units): everything on one stream, predictions come back in one copy through pinned memory
-    // predictions of a host-pointer call: one device block the kernels write, one pinned block it is copied to in a single
-    // D2H, then plain memcpy into the caller's (usually pageable) arrays.  Copying straight into pageable memory would make
-    // every cudaMemcpyAsync synchronous and stall the H2D ring behind each chunk's kernels (tools/host_fed_probe.py).
-    uint8_t *d_pred_small = nullptr, *h_pred_small = nullptr;
+    // the prediction block of host-pointer calls (PredBlock): device block the kernels write, pinned block it is copied to
+    uint8_t *d_pred = nullptr, *h_pred = nullptr;
     size_t cap_pred = 0;                            // images the two blocks hold
     // single-image protocol state
     uint8_t *h_img = nullptr, *h_bram = nullptr;    // pinned + mapped: the batch-1 path runs zero-copy on them
@@ -144,10 +141,24 @@ bool aligned(const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p
 
 bool valid_hw(int H, int W) { return H >= 16 && W >= 16 && H % 16 == 0 && W % 16 == 0 && H <= 8192 && W <= 8192; }
 
-// Sizes from 128 up (other than 128x128 itself) run as overlapping windows through the fused kernel.
-bool tiled_ok(const cnnacc_handle* h, int H, int W, uint32_t flags) {
-    return H >= CNNACC_IMG && W >= CNNACC_IMG && !(H == CNNACC_IMG && W == CNNACC_IMG) && h->fused.ready &&
-           !(flags & (CNNACC_FLAG_DIRECT | CNNACC_FLAG_KEEP_MAPS));
+// The tuning overrides the sweeps in tools/ set (CNNACC_PDL, CNNACC_HOST_CHUNK_MB, CNNACC_HOST_RAMP, CNNACC_WS_CHUNK): the
+// variable's integer value, or dflt when it is unset.  Each is read once, into a function-local static where it is used.
+int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
+
+// Which kernels run the conv stack of an H x W call.  128x128 is one fused launch (its maps can also be kept); larger sizes
+// run as overlapping 128x128 windows through the fused kernel; everything else, and DIRECT, takes the per-layer kernels.
+enum class ConvPath { kFused128, kFusedWindows, kPerLayer };
+ConvPath conv_path(const cnnacc_handle* h, int H, int W, uint32_t flags) {
+    if (!h->fused.ready || (flags & CNNACC_FLAG_DIRECT)) return ConvPath::kPerLayer;
+    if (H == CNNACC_IMG && W == CNNACC_IMG) return ConvPath::kFused128;
+    if (H >= CNNACC_IMG && W >= CNNACC_IMG && !(flags & CNNACC_FLAG_KEEP_MAPS)) return ConvPath::kFusedWindows;
+    return ConvPath::kPerLayer;
+}
+
+// Does the classifier tail of a 128x128 call run inside the fused conv kernel, on the feature map still in shared memory?
+bool tail_in_conv(const cnnacc_handle* h, uint32_t flags) {
+    return conv_path(h, CNNACC_IMG, CNNACC_IMG, flags) == ConvPath::kFused128 &&
+           !(flags & (CNNACC_FLAG_KEEP_MAPS | CNNACC_FLAG_TWO_KERNELS));
 }
 
 // One layer of the generic per-layer path on `stream`.
@@ -168,11 +179,11 @@ int launch_direct_layer(cnnacc_handle* h, cudaStream_t stream, int layer, const 
 // Conv stack for n device-resident images on `stream`.  l0/l1 are workspaces for the per-layer path.
 int conv_stack_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_imgs, int64_t n, int H, int W,
                       uint8_t* d_feats, uint32_t flags, uint8_t* d_l0, uint8_t* d_l1) {
-    const bool fused_ok = (H == CNNACC_IMG && W == CNNACC_IMG) && !(flags & CNNACC_FLAG_DIRECT) && h->fused.ready;
-    if (fused_ok) {
+    const ConvPath path = conv_path(h, H, W, flags);
+    if (path == ConvPath::kFused128) {
         // May this launch overlap the previous conv-stack launch (no griddepcontrol.wait)?  Only if that one is the last thing
         // this handle launched, on the same stream, and none of the launches since the last full wait shares memory with it.
-        static const bool pdl_on = [] { const char* e = getenv("CNNACC_PDL"); return !(e && e[0] == '0'); }();
+        static const bool pdl_on = env_int("CNNACC_PDL", 1) != 0;
         // Why a waiting launch is enough of a fence: every launch in such a chain fills all SMs with one CTA each, so a CTA of
         // launch B only starts on an SM after the CTAs of A, A-1, ... there have exited -- "A complete" implies the whole chain
         // is.  Launches smaller than the SM count therefore always wait and break the chain, and so does any other kernel of
@@ -193,7 +204,7 @@ int conv_stack_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_im
         if (rc != 0) return fail(h, CNNACC_ERR_CUDA, std::string("fused launch: ") + cudaGetErrorString((cudaError_t)rc));
         return 0;
     }
-    if (tiled_ok(h, H, W, flags)) {
+    if (path == ConvPath::kFusedWindows) {
         // larger images: overlapping 128x128 windows through the fused kernel (tiling.cuh)
         const TilePlan py = make_tile_plan(H / 8), px = make_tile_plan(W / 8);
         const int64_t n_t = n * py.n * px.n;
@@ -219,8 +230,7 @@ int conv_stack_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_im
 }
 
 bool needs_maps(const cnnacc_handle* h, int H, int W, uint32_t flags) {   // only the per-layer path has intermediate maps in HBM
-    const bool fused_ok = (H == CNNACC_IMG && W == CNNACC_IMG) && !(flags & CNNACC_FLAG_DIRECT) && h->fused.ready;
-    return !(fused_ok || tiled_ok(h, H, W, flags)) || (flags & CNNACC_FLAG_KEEP_MAPS);
+    return conv_path(h, H, W, flags) == ConvPath::kPerLayer || (flags & CNNACC_FLAG_KEEP_MAPS);
 }
 
 // images per chunk so that the per-layer workspaces stay around 512 MiB
@@ -266,8 +276,7 @@ int launch_tail(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_feats, i
 // the features afterwards (want_feats) or the per-layer kernels are in use.
 int infer_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_imgs, int64_t m, uint8_t* d_feat_ws, bool want_feats,
                  const TailArgs& A, uint32_t flags) {
-    const bool fused_ok = !(flags & (CNNACC_FLAG_DIRECT | CNNACC_FLAG_KEEP_MAPS | CNNACC_FLAG_TWO_KERNELS)) && h->fused.ready;
-    if (fused_ok) {
+    if (tail_in_conv(h, flags)) {
         int rc = launch_fused(h->fused, stream, d_imgs, m, want_feats ? d_feat_ws : nullptr, h->shifts, h->sm_count, nullptr, nullptr, &A);
         h->launches++;
         if (rc != 0) return fail(h, CNNACC_ERR_CUDA, std::string("fused launch: ") + cudaGetErrorString((cudaError_t)rc));
@@ -278,7 +287,7 @@ int infer_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_imgs, i
     return launch_tail(h, stream, d_feat_ws, m, A);
 }
 bool infer_needs_feat_ws(const cnnacc_handle* h, bool want_feats, uint32_t flags) {
-    return want_feats || (flags & (CNNACC_FLAG_DIRECT | CNNACC_FLAG_KEEP_MAPS | CNNACC_FLAG_TWO_KERNELS)) || !h->fused.ready;
+    return want_feats || !tail_in_conv(h, flags);
 }
 
 // Classifier.get_cam_bbox per image (cam_upsampled.cuh); d_cam may be null
@@ -329,23 +338,6 @@ int launch_preprocess(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_fr
     return 0;
 }
 
-int slot_reserve(cnnacc_handle* h, Slot& s, size_t in_bytes, size_t out_bytes, size_t n_pred) {
-    int rc;
-    if ((rc = grow(h, &s.d_in, &s.cap_in, in_bytes))) return rc;
-    if ((rc = grow(h, &s.d_out, &s.cap_out, out_bytes))) return rc;
-    if (n_pred > s.cap_pred) {
-        if (s.d_probs) cudaFree(s.d_probs);
-        if (s.d_cls) cudaFree(s.d_cls);
-        if (s.d_bbox) cudaFree(s.d_bbox);
-        s.d_probs = nullptr; s.d_cls = nullptr; s.d_bbox = nullptr; s.cap_pred = 0;
-        CU(h, cudaMalloc(&s.d_probs, n_pred * kMaxClasses * sizeof(float)));
-        CU(h, cudaMalloc(&s.d_cls, n_pred * sizeof(int32_t)));
-        CU(h, cudaMalloc(&s.d_bbox, n_pred * 4 * sizeof(int32_t)));
-        s.cap_pred = n_pred;
-    }
-    return 0;
-}
-
 // A fused launch whose internal waits timed out reports it through a device status word.
 int check_fused_status(cnnacc_handle* h) {
     int bits = 0;
@@ -355,63 +347,145 @@ int check_fused_status(cnnacc_handle* h) {
     return 0;
 }
 
-// Host-pointer calls queue copies that read and write the CALLER's buffers.  If such a call returns early with an error the
-// queued work must not outlive it: the guard drains the ring's streams on every exit it was not dismissed on.
-struct RingDrain {
-    cnnacc_handle* h;
-    bool armed = true;
-    explicit RingDrain(cnnacc_handle* h_) : h(h_) {}
-    ~RingDrain() {
-        if (!armed) return;
-        for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) cudaStreamSynchronize(st);
-    }
-    int done(int rc) { armed = false; return rc; }       // normal exit: the call has synchronised already
-};
-
 int check_ready(cnnacc_handle* h) {
     if (!h) return CNNACC_ERR_ARG;
     if (!h->weights_loaded) return fail(h, CNNACC_ERR_STATE, "weights not loaded (call cnnacc_load_weights)");
     return 0;
 }
 
-// The host-pointer conv stack: queue the staged copies and kernels of one call on the ring; does not wait for anything.
-// `pipelined`: the call belongs to a stream of asynchronous calls -- no ramped chunk sizes (the neighbouring calls keep both
-// copy directions busy at its edges) and the slots continue from where the previous call left the ring.
-int enqueue_host_batch(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int H, int W, uint8_t* feats, uint32_t flags, bool pipelined) {
+// Waits for the handle's stream and the three ring streams.
+int sync_all(cnnacc_handle* h) {
+    CU(h, cudaStreamSynchronize(h->stream));
+    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));
+    return 0;
+}
+
+// One host-pointer call on the staging ring, the one place the ring's protocol is written.  kSlots slots are driven through
+// one stream per engine (st_h2d copies in, st_k runs the kernels, st_d2h copies out) so that copies in both directions and
+// kernels of different chunks overlap.  Each chunk takes its slot through
+//   acquire   reserve the buffers; st_h2d waits for ev_out, i.e. until the slot's previous chunk is done with it
+//   staged    after the copies in: ev_in on st_h2d, st_k waits for it
+//   computed  after the kernels: ev_k on st_k, st_d2h waits for it (calls that copy nothing out per slot skip it)
+//   released  ev_out on the stream of the last operation that reads or writes the slot
+// The call queues copies that read and write the CALLER's buffers: until finish() or done() ends it, the destructor drains
+// the ring's streams, so a call that returns early with an error leaves none of those copies in flight.
+struct HostCall {
+    cnnacc_handle* const h;
+    const bool pipelined;       // cnnacc_run_batch_async: the call continues the ring where the previous one left it, and
+    const int64_t ring0;        // a slot's last user may be an earlier call still in flight
+    int64_t ci = 0;             // chunks acquired so far
+    bool armed = true;
+
+    explicit HostCall(cnnacc_handle* h_, bool pipelined_ = false)
+        : h(h_), pipelined(pipelined_), ring0(pipelined_ ? h_->ring_ci : 0) {}
+    ~HostCall() { if (armed) for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) cudaStreamSynchronize(st); }
+    // a synchronous call starts on an idle handle (the ring is idle already unless asynchronous calls are pending)
+    int begin() { return sync_all(h); }
+    // the call's last operation is queued on `st`: wait for it and end the call; `fused`: the call ran the conv stack
+    int finish(cudaStream_t st, bool fused) { CU(h, cudaStreamSynchronize(st)); return done(fused); }
+    // end a call that has waited for its last operation already, or leaves it in flight on purpose (asynchronous calls)
+    int done(bool fused) { armed = false; return fused ? check_fused_status(h) : 0; }
+
+    // the call's next slot, with room for in_bytes / out_bytes and for the classes and boxes of n_pred units
+    int acquire(Slot*& out, size_t in_bytes, size_t out_bytes, size_t n_pred = 0) {
+        Slot& s = h->slots[(ring0 + ci) % kSlots];
+        int rc;
+        if ((rc = grow(h, &s.d_in, &s.cap_in, in_bytes)) || (rc = grow(h, &s.d_out, &s.cap_out, out_bytes))) return rc;
+        if (n_pred > s.cap_pred) {
+            cudaFree(s.d_cls); cudaFree(s.d_bbox);
+            s.d_cls = s.d_bbox = nullptr; s.cap_pred = 0;
+            CU(h, cudaMalloc(&s.d_cls, n_pred * sizeof(int32_t)));
+            CU(h, cudaMalloc(&s.d_bbox, n_pred * 4 * sizeof(int32_t)));
+            s.cap_pred = n_pred;
+        }
+        if ((ci >= kSlots || pipelined) && (rc = wait_released(s, h->st_h2d))) return rc;   // an unrecorded event is complete
+        ci++;
+        if (pipelined) h->ring_ci = (ring0 + ci) % kSlots;
+        out = &s;
+        return 0;
+    }
+    int wait_released(const Slot& s, cudaStream_t st) { CU(h, cudaStreamWaitEvent(st, s.ev_out, 0)); return 0; }
+    int staged(const Slot& s) { CU(h, cudaEventRecord(s.ev_in, h->st_h2d)); CU(h, cudaStreamWaitEvent(h->st_k, s.ev_in, 0)); return 0; }
+    int computed(const Slot& s) { CU(h, cudaEventRecord(s.ev_k, h->st_k)); CU(h, cudaStreamWaitEvent(h->st_d2h, s.ev_k, 0)); return 0; }
+    int released(const Slot& s, cudaStream_t st) { CU(h, cudaEventRecord(s.ev_out, st)); return 0; }
+};
+
+// The predictions of a host-pointer call come back in blocks of up to kPredSuper units.  The kernels write the block of units
+// [s0, s0 + m) into h->d_pred as [bbox m x 4 i32 | probs m x nc f32 | cls m i32]; flush() brings it with one D2H into the
+// pinned h->h_pred, then with plain memcpy into the caller's (usually pageable) arrays.  Copying straight into pageable
+// memory would make every cudaMemcpyAsync synchronous and stall the H2D ring behind each chunk's kernels
+// (tools/host_fed_probe.py).
+struct PredBlock {
+    cnnacc_handle* const h;
+    int64_t s0 = 0, m = 0;
+
+    explicit PredBlock(cnnacc_handle* h_) : h(h_) {}
+    // lay the block out for units [first, first + count), growing the handle's two buffers when they are too small
+    int start(int64_t first, int64_t count) {
+        if ((size_t)count > h->cap_pred) {
+            CU(h, cudaStreamSynchronize(h->st_d2h));
+            cudaFree(h->d_pred); cudaFreeHost(h->h_pred);
+            h->d_pred = h->h_pred = nullptr; h->cap_pred = 0;
+            CU(h, cudaMalloc(&h->d_pred, (size_t)count * kPredBytesPerImage));
+            CU(h, cudaHostAlloc(&h->h_pred, (size_t)count * kPredBytesPerImage, cudaHostAllocDefault));
+            h->cap_pred = (size_t)count;
+        }
+        s0 = first; m = count;
+        return 0;
+    }
+    int64_t end() const { return s0 + m; }
+    size_t off_probs() const { return (size_t)m * 16; }
+    size_t off_cls() const { return off_probs() + (size_t)m * h->n_cls * 4; }
+    // where the kernels write the predictions of unit u, s0 <= u < end()
+    int32_t* bbox(int64_t u) const { return reinterpret_cast<int32_t*>(h->d_pred) + (u - s0) * 4; }
+    float* probs(int64_t u) const { return reinterpret_cast<float*>(h->d_pred + off_probs()) + (u - s0) * h->n_cls; }
+    int32_t* cls(int64_t u) const { return reinterpret_cast<int32_t*>(h->d_pred + off_cls()) + (u - s0); }
+    // the block, after the kernels queued on `st`, into the caller's arrays (indexed from unit 0); waits for st
+    int flush(cudaStream_t st, float* probs_out, int32_t* cls_out, int32_t* bbox_out, bool cls_given) {
+        CU(h, cudaMemcpyAsync(h->h_pred, h->d_pred, off_cls() + (size_t)m * 4, cudaMemcpyDeviceToHost, st));
+        CU(h, cudaStreamSynchronize(st));
+        if (bbox_out) std::memcpy(bbox_out + s0 * 4, h->h_pred, (size_t)m * 16);
+        if (probs_out) std::memcpy(probs_out + s0 * h->n_cls, h->h_pred + off_probs(), (size_t)m * h->n_cls * 4);
+        if (cls_out && !cls_given) std::memcpy(cls_out + s0, h->h_pred + off_cls(), (size_t)m * 4);
+        return 0;
+    }
+};
+
+// The cut of a host-pointer call into staging chunks (host_chunks.h) under the CNNACC_HOST_CHUNK_MB / CNNACC_HOST_RAMP
+// overrides.  `ramp`: the call may ramp its chunk sizes up and down at its edges.
+HostChunkPlan host_chunk_plan(int64_t n, size_t in_sz, int64_t cap_images, bool pipelined, bool ramp) {
+    static const size_t chunk_mb = (size_t)std::max(0, env_int("CNNACC_HOST_CHUNK_MB", 0));
+    static const int depth = std::clamp(env_int("CNNACC_HOST_RAMP", 2), 0, 4);
+    return make_host_chunk_plan(n, in_sz, cap_images, pipelined, chunk_mb, ramp ? depth : 0);
+}
+
+// The host-pointer conv stack: queue the staged copies and kernels of one call on the ring; does not wait for anything.  A
+// pipelined call has no ramped chunk sizes: the neighbouring calls keep both copy directions busy at its edges.
+int enqueue_host_batch(HostCall& call, const uint8_t* imgs, int64_t n, int H, int W, uint8_t* feats, uint32_t flags) {
+    cnnacc_handle* h = call.h;
     int rc;
     const size_t in_sz = (size_t)H * W, out_sz = (size_t)64 * (H / 8) * (W / 8);
-    const bool maps = needs_maps(h, H, W, flags);
-    // the cut into staging chunks: host_chunks.h (CNNACC_HOST_CHUNK_MB / CNNACC_HOST_RAMP override it)
-    static const size_t chunk_mb = [] { const char* e = getenv("CNNACC_HOST_CHUNK_MB"); int v = e ? atoi(e) : 0; return (size_t)(v > 0 ? v : 0); }();
-    static const int ramp = [] { const char* e = getenv("CNNACC_HOST_RAMP"); int v = e ? atoi(e) : 2; return v < 0 ? 0 : (v > 4 ? 4 : v); }();
-    const HostChunkPlan plan = make_host_chunk_plan(n, in_sz, chunk_images(H, W), pipelined, chunk_mb, ramp);
+    const HostChunkPlan plan = host_chunk_plan(n, in_sz, chunk_images(H, W), call.pipelined, true);
     const int64_t hchunk = plan.full;
-    if (maps && (rc = ensure_maps(h, hchunk, H, W))) return rc;
-    if (pipelined) {
+    if (needs_maps(h, H, W, flags) && (rc = ensure_maps(h, hchunk, H, W))) return rc;
+    if (call.pipelined) {
         // earlier calls may still be using the slots: growing one (free + malloc) waits for the device first
         bool grows = false;
         for (const Slot& s : h->slots) grows |= s.cap_in < hchunk * in_sz || s.cap_out < hchunk * out_sz;
         if (grows) CU(h, cudaDeviceSynchronize());
     }
-    const int64_t ring0 = pipelined ? h->ring_ci : 0;                                // where this call enters the slot ring
-    int64_t ci = 0, m = 0;
-    for (int64_t i0 = 0; i0 < n; i0 += m, ci++) {
+    int64_t m = 0;
+    for (int64_t i0 = 0, ci = 0; i0 < n; i0 += m, ci++) {
         m = plan.next(i0, ci);
-        Slot& s = h->slots[(ring0 + ci) % kSlots];
-        if ((rc = slot_reserve(h, s, hchunk * in_sz, hchunk * out_sz, 0))) return rc;
-        // slot drained (its kernels ended earlier); in a pipelined stream its last user may be an earlier call (an event that
-        // was never recorded counts as complete)
-        if (ci >= kSlots || pipelined) CU(h, cudaStreamWaitEvent(h->st_h2d, s.ev_out, 0));
-        CU(h, cudaMemcpyAsync(s.d_in, imgs + i0 * in_sz, m * in_sz, cudaMemcpyHostToDevice, h->st_h2d));
-        CU(h, cudaEventRecord(s.ev_in, h->st_h2d));
-        CU(h, cudaStreamWaitEvent(h->st_k, s.ev_in, 0));
-        if ((rc = conv_stack_device(h, h->st_k, s.d_in, m, H, W, s.d_out, flags, h->d_l0, h->d_l1))) return rc;
-        CU(h, cudaEventRecord(s.ev_k, h->st_k));
-        CU(h, cudaStreamWaitEvent(h->st_d2h, s.ev_k, 0));
-        CU(h, cudaMemcpyAsync(feats + i0 * out_sz, s.d_out, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
-        CU(h, cudaEventRecord(s.ev_out, h->st_d2h));
+        Slot* s;
+        if ((rc = call.acquire(s, hchunk * in_sz, hchunk * out_sz))) return rc;
+        CU(h, cudaMemcpyAsync(s->d_in, imgs + i0 * in_sz, m * in_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        if ((rc = call.staged(*s)) || (rc = conv_stack_device(h, h->st_k, s->d_in, m, H, W, s->d_out, flags, h->d_l0, h->d_l1)) ||
+            (rc = call.computed(*s)))
+            return rc;
+        CU(h, cudaMemcpyAsync(feats + i0 * out_sz, s->d_out, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+        if ((rc = call.released(*s, h->st_d2h))) return rc;
     }
-    if (pipelined) h->ring_ci = (ring0 + ci) % kSlots;
     return 0;
 }
 
@@ -537,8 +611,8 @@ int cnnacc_create(int device_id, cnnacc_handle** out) {
     if ((e = cudaHostAlloc(&h->h_done, 64, cudaHostAllocMapped)) != cudaSuccess) return bail("cudaHostAlloc", e);
     *h->h_done = 0;
     if ((e = cudaHostGetDevicePointer(&h->h_done_dev, h->h_done, 0)) != cudaSuccess) return bail("cudaHostGetDevicePointer", e);
-    if ((e = cudaHostAlloc(&h->h_pred_small, kSmallN * kPredBytesPerImage, cudaHostAllocDefault)) != cudaSuccess) return bail("cudaHostAlloc", e);
-    if ((e = cudaMalloc(&h->d_pred_small, kSmallN * kPredBytesPerImage)) != cudaSuccess) return bail("cudaMalloc", e);
+    if ((e = cudaHostAlloc(&h->h_pred, kSmallN * kPredBytesPerImage, cudaHostAllocDefault)) != cudaSuccess) return bail("cudaHostAlloc", e);
+    if ((e = cudaMalloc(&h->d_pred, kSmallN * kPredBytesPerImage)) != cudaSuccess) return bail("cudaMalloc", e);
     h->cap_pred = kSmallN;
     if ((e = cudaMalloc(&h->d_img1, CNNACC_IMG * CNNACC_IMG)) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMalloc(&h->d_bram, kBramBytes)) != cudaSuccess) return bail("cudaMalloc", e);
@@ -551,7 +625,7 @@ int cnnacc_destroy(cnnacc_handle* h) {
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
     for (auto& s : h->slots) {
-        cudaFree(s.d_in); cudaFree(s.d_out); cudaFree(s.d_probs); cudaFree(s.d_cls); cudaFree(s.d_bbox);
+        cudaFree(s.d_in); cudaFree(s.d_out); cudaFree(s.d_cls); cudaFree(s.d_bbox);
         for (auto ev : {s.ev_in, s.ev_k, s.ev_out}) if (ev) cudaEventDestroy(ev);
     }
     for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) if (st) cudaStreamDestroy(st);
@@ -566,7 +640,7 @@ int cnnacc_destroy(cnnacc_handle* h) {
     cudaFree(h->d_wdirect); cudaFree(h->d_fcw); cudaFree(h->d_fcb);
     cudaFree(h->d_l0); cudaFree(h->d_l1); cudaFree(h->d_feat); cudaFree(h->d_img1); cudaFree(h->d_bram);
     fused_free(h->fused);
-    cudaFreeHost(h->h_img); cudaFreeHost(h->h_bram); cudaFreeHost(h->h_done); cudaFreeHost(h->h_pred_small); cudaFree(h->d_pred_small);
+    cudaFreeHost(h->h_img); cudaFreeHost(h->h_bram); cudaFreeHost(h->h_done); cudaFreeHost(h->h_pred); cudaFree(h->d_pred);
     cudaEvent_t evs[] = {h->ev_t0, h->ev_t1, h->ev_a, h->ev_b, h->ev_c, h->ev_done};
     for (auto ev : evs) if (ev) cudaEventDestroy(ev);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
@@ -692,12 +766,9 @@ int cnnacc_run_batch(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int H, in
     }
 
     // host pointers: returns when feats is complete
-    CU(h, cudaStreamSynchronize(h->stream));
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));   // idle already unless asynchronous calls are pending
-    RingDrain drain(h);
-    if ((rc = enqueue_host_batch(h, imgs, n, H, W, feats, flags, /*pipelined=*/false))) return rc;
-    CU(h, cudaStreamSynchronize(h->st_d2h));            // the last D2H is the last operation of the whole chain
-    return drain.done(check_fused_status(h));
+    HostCall call(h);
+    if ((rc = call.begin()) || (rc = enqueue_host_batch(call, imgs, n, H, W, feats, flags))) return rc;
+    return call.finish(h->st_d2h, true);                // the last D2H is the last operation of the whole chain
 }
 
 int cnnacc_run_batch_async(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int H, int W, uint8_t* feats, uint32_t flags,
@@ -714,11 +785,11 @@ int cnnacc_run_batch_async(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int
     // the event of the call submitted CNNACC_MAX_PENDING calls ago is about to be reused: that call must have completed
     cudaEvent_t ev = h->ev_ticket[h->next_ticket % CNNACC_MAX_PENDING];
     if (h->next_ticket >= CNNACC_MAX_PENDING) CU(h, cudaEventSynchronize(ev));
-    RingDrain drain(h);
-    if (n > 0 && (rc = enqueue_host_batch(h, imgs, n, H, W, feats, flags, /*pipelined=*/true))) return rc;
+    HostCall call(h, /*pipelined=*/true);
+    if (n > 0 && (rc = enqueue_host_batch(call, imgs, n, H, W, feats, flags))) return rc;
     CU(h, cudaEventRecord(ev, h->st_d2h));
     *ticket = h->next_ticket++;
-    return drain.done(CNNACC_OK);
+    return call.done(false);
 }
 
 int cnnacc_wait_batch(cnnacc_handle* h, int64_t ticket) {
@@ -881,35 +952,6 @@ int cnnacc_load_classifier(cnnacc_handle* h, const float* fc_w, const float* fc_
     return CNNACC_OK;
 }
 
-// Predictions of a small call: one contiguous device block [bbox m x 4 i32 | probs m x nc f32 | cls m i32], one D2H into
-// pinned memory, then plain copies into the caller's arrays.
-struct SmallPred {
-    float* d_probs; int32_t* d_cls; int32_t* d_bbox; size_t bytes; size_t off_probs, off_cls;
-};
-static int ensure_pred(cnnacc_handle* h, int64_t m) {       // grow the prediction blocks to hold m images
-    if ((size_t)m <= h->cap_pred) return 0;
-    CU(h, cudaStreamSynchronize(h->st_d2h));
-    cudaFree(h->d_pred_small); cudaFreeHost(h->h_pred_small);
-    h->d_pred_small = h->h_pred_small = nullptr; h->cap_pred = 0;
-    CU(h, cudaMalloc(&h->d_pred_small, (size_t)m * kPredBytesPerImage));
-    CU(h, cudaHostAlloc(&h->h_pred_small, (size_t)m * kPredBytesPerImage, cudaHostAllocDefault));
-    h->cap_pred = (size_t)m;
-    return 0;
-}
-static SmallPred small_pred(cnnacc_handle* h, int64_t m) {
-    SmallPred p;
-    p.off_probs = (size_t)m * 16; p.off_cls = p.off_probs + (size_t)m * h->n_cls * 4; p.bytes = p.off_cls + (size_t)m * 4;
-    p.d_bbox = reinterpret_cast<int32_t*>(h->d_pred_small);
-    p.d_probs = reinterpret_cast<float*>(h->d_pred_small + p.off_probs);
-    p.d_cls = reinterpret_cast<int32_t*>(h->d_pred_small + p.off_cls);
-    return p;
-}
-static void small_pred_unpack(cnnacc_handle* h, const SmallPred& p, int64_t m, float* probs, int32_t* cls, int32_t* bbox, bool cls_given) {
-    if (bbox) std::memcpy(bbox, h->h_pred_small, (size_t)m * 16);
-    if (probs) std::memcpy(probs, h->h_pred_small + p.off_probs, (size_t)m * h->n_cls * 4);
-    if (cls && !cls_given) std::memcpy(cls, h->h_pred_small + p.off_cls, (size_t)m * 4);
-}
-
 // shared body of classify_batch / infer_batch
 static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool src_is_images,
                         float* probs, int32_t* cls, int32_t* bbox, uint32_t flags) {
@@ -938,8 +980,8 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
         REQUIRE_ALIGNED(h, probs, 4, "probs");
         REQUIRE_ALIGNED(h, cls, 4, "cls");
         // one fused launch covers the whole call unless a workspace bounds the chunk
-        static const int64_t ws_chunk = [] { const char* e = getenv("CNNACC_WS_CHUNK"); int v = e ? atoi(e) : 0; return (int64_t)(v > 0 ? v : 16384); }();
-        const int64_t chunk = feat_ws ? std::min<int64_t>(n, ws_chunk) : n;
+        static const int ws_chunk = env_int("CNNACC_WS_CHUNK", 0);
+        const int64_t chunk = feat_ws ? std::min<int64_t>(n, ws_chunk > 0 ? ws_chunk : 16384) : n;
         if (feat_ws) {
             if ((rc = grow(h, &h->d_feat, &h->cap_feat, (size_t)chunk * img_sz))) return rc;
             if (maps && (rc = ensure_maps(h, chunk, CNNACC_IMG, CNNACC_IMG))) return rc;
@@ -958,65 +1000,46 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
         return CNNACC_OK;
     }
 
-    CU(h, cudaStreamSynchronize(h->stream));
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));
-    RingDrain drain(h);
-    if (n <= kSmallN) {                                      // latency path: one stream, one result copy
-        Slot& s = h->slots[0];
-        cudaStream_t st = h->st_k;
-        if ((rc = slot_reserve(h, s, n * img_sz, feat_ws ? n * img_sz : 0, 0))) return rc;
-        if (maps && (rc = ensure_maps(h, n, CNNACC_IMG, CNNACC_IMG))) return rc;
-        const SmallPred p = small_pred(h, n);
-        CU(h, cudaMemcpyAsync(s.d_in, src, n * img_sz, cudaMemcpyHostToDevice, st));
-        if (cls_given) CU(h, cudaMemcpyAsync(p.d_cls, cls, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        const TailArgs A = make_tail(h, p.d_probs, p.d_cls, upsampled ? nullptr : p.d_bbox, cls_given, flags);
+    HostCall call(h);
+    if ((rc = call.begin())) return rc;
+    PredBlock pred(h);
+    auto kernels = [&](cudaStream_t st, const Slot& s, int64_t i0, int64_t m) -> int {   // units [i0, i0 + m), staged in s
+        const TailArgs A = make_tail(h, pred.probs(i0), pred.cls(i0), upsampled ? nullptr : pred.bbox(i0), cls_given, flags);
         const uint8_t* f = s.d_in;
+        int r;
         if (src_is_images) {
-            if ((rc = infer_device(h, st, s.d_in, n, s.d_out, upsampled, A, flags))) return rc;
+            if ((r = infer_device(h, st, s.d_in, m, s.d_out, upsampled, A, flags))) return r;
             f = s.d_out;
-        } else if ((rc = launch_tail(h, st, f, n, A))) return rc;
-        if (upsampled && (rc = launch_cam_upsampled(h, st, f, n, p.d_cls, p.d_bbox, nullptr))) return rc;
-        CU(h, cudaMemcpyAsync(h->h_pred_small, h->d_pred_small, p.bytes, cudaMemcpyDeviceToHost, st));
-        CU(h, cudaStreamSynchronize(st));
-        small_pred_unpack(h, p, n, probs, cls, bbox, cls_given);
-        return drain.done(src_is_images ? check_fused_status(h) : CNNACC_OK);
+        } else if ((r = launch_tail(h, st, f, m, A))) return r;
+        return upsampled ? launch_cam_upsampled(h, st, f, m, pred.cls(i0), pred.bbox(i0), nullptr) : 0;
+    };
+    Slot* s;
+    if (n <= kSmallN) {                                      // latency path: one stream, one result copy
+        cudaStream_t st = h->st_k;
+        if ((rc = call.acquire(s, n * img_sz, feat_ws ? n * img_sz : 0))) return rc;
+        if (maps && (rc = ensure_maps(h, n, CNNACC_IMG, CNNACC_IMG))) return rc;
+        if ((rc = pred.start(0, n))) return rc;
+        CU(h, cudaMemcpyAsync(s->d_in, src, n * img_sz, cudaMemcpyHostToDevice, st));
+        if (cls_given) CU(h, cudaMemcpyAsync(pred.cls(0), cls, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        if ((rc = kernels(st, *s, 0, n)) || (rc = pred.flush(st, probs, cls, bbox, cls_given))) return rc;
+        return call.done(src_is_images);
     }
-    // Same ring as cnnacc_run_batch's host path; only the predictions (44 B per image) come back, so the link carries
-    // H2D traffic alone and the chunks can be a quarter of the call, clamped to 4..32 MiB.  The kernels write the
-    // predictions of up to kPredSuper images into one device block; one D2H into pinned memory ends the block.
-    static const size_t env_chunk_mb = [] { const char* e = getenv("CNNACC_HOST_CHUNK_MB"); int v = e ? atoi(e) : 0; return (size_t)(v > 0 ? v : 0); }();
-    const size_t chunk_bytes = env_chunk_mb ? (env_chunk_mb << 20)
-                                            : std::min<size_t>((size_t)32 << 20, std::max<size_t>((size_t)4 << 20, (size_t)n * img_sz / 4));
-    const int64_t hchunk = std::min<int64_t>(n, std::max<int64_t>(1, (int64_t)(chunk_bytes / img_sz)));
+    // Only the predictions (44 B per image) come back, so the link carries H2D traffic alone: no ramp, and no cap beyond the
+    // call's own size.  Nothing is copied out per slot, so a slot is released once its kernels have ended.
+    const int64_t hchunk = host_chunk_plan(n, img_sz, INT64_MAX, false, false).full;
     if (maps && (rc = ensure_maps(h, hchunk, CNNACC_IMG, CNNACC_IMG))) return rc;
-    if ((rc = ensure_pred(h, std::min<int64_t>(n, kPredSuper)))) return rc;
-    int64_t ci = 0;
     for (int64_t s0 = 0; s0 < n; s0 += kPredSuper) {
-        const int64_t sn = std::min<int64_t>(kPredSuper, n - s0);
-        const SmallPred p = small_pred(h, sn);
-        for (int64_t i0 = 0; i0 < sn; i0 += hchunk, ci++) {
-            const int64_t m = std::min(hchunk, sn - i0);
-            Slot& s = h->slots[ci % kSlots];
-            if ((rc = slot_reserve(h, s, hchunk * img_sz, feat_ws ? hchunk * img_sz : 0, 0))) return rc;
-            if (ci >= kSlots) CU(h, cudaStreamWaitEvent(h->st_h2d, s.ev_k, 0));      // the kernels that read this slot have ended
-            CU(h, cudaMemcpyAsync(s.d_in, src + (s0 + i0) * img_sz, m * img_sz, cudaMemcpyHostToDevice, h->st_h2d));
-            if (cls_given) CU(h, cudaMemcpyAsync(p.d_cls + i0, cls + s0 + i0, m * sizeof(int32_t), cudaMemcpyHostToDevice, h->st_h2d));
-            CU(h, cudaEventRecord(s.ev_in, h->st_h2d));
-            CU(h, cudaStreamWaitEvent(h->st_k, s.ev_in, 0));
-            const TailArgs A = make_tail(h, p.d_probs + i0 * nc, p.d_cls + i0, upsampled ? nullptr : p.d_bbox + i0 * 4, cls_given, flags);
-            const uint8_t* f = s.d_in;
-            if (src_is_images) {
-                if ((rc = infer_device(h, h->st_k, s.d_in, m, s.d_out, upsampled, A, flags))) return rc;
-                f = s.d_out;
-            } else if ((rc = launch_tail(h, h->st_k, f, m, A))) return rc;
-            if (upsampled && (rc = launch_cam_upsampled(h, h->st_k, f, m, p.d_cls + i0, p.d_bbox + i0 * 4, nullptr))) return rc;
-            CU(h, cudaEventRecord(s.ev_k, h->st_k));
+        if ((rc = pred.start(s0, std::min<int64_t>(kPredSuper, n - s0)))) return rc;
+        for (int64_t i0 = s0; i0 < pred.end(); i0 += hchunk) {
+            const int64_t m = std::min(hchunk, pred.end() - i0);
+            if ((rc = call.acquire(s, hchunk * img_sz, feat_ws ? hchunk * img_sz : 0))) return rc;
+            CU(h, cudaMemcpyAsync(s->d_in, src + i0 * img_sz, m * img_sz, cudaMemcpyHostToDevice, h->st_h2d));
+            if (cls_given) CU(h, cudaMemcpyAsync(pred.cls(i0), cls + i0, m * sizeof(int32_t), cudaMemcpyHostToDevice, h->st_h2d));
+            if ((rc = call.staged(*s)) || (rc = kernels(h->st_k, *s, i0, m)) || (rc = call.released(*s, h->st_k))) return rc;
         }
-        CU(h, cudaMemcpyAsync(h->h_pred_small, h->d_pred_small, p.bytes, cudaMemcpyDeviceToHost, h->st_k));
-        CU(h, cudaStreamSynchronize(h->st_k));
-        small_pred_unpack(h, p, sn, probs ? probs + s0 * nc : nullptr, cls ? cls + s0 : nullptr, bbox ? bbox + s0 * 4 : nullptr, cls_given);
+        if ((rc = pred.flush(h->st_k, probs, cls, bbox, cls_given))) return rc;
     }
-    return drain.done(src_is_images ? check_fused_status(h) : CNNACC_OK);
+    return call.done(src_is_images);
 }
 
 int cnnacc_classify_batch(cnnacc_handle* h, const uint8_t* feats, int64_t n, float* probs, int32_t* cls, int32_t* bbox, uint32_t flags) {
@@ -1043,29 +1066,23 @@ int cnnacc_pool_features(cnnacc_handle* h, const uint8_t* feats, int64_t n, floa
         CU(h, cudaGetLastError());
         return CNNACC_OK;
     }
-    CU(h, cudaStreamSynchronize(h->stream));
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));
-    RingDrain drain(h);
+    HostCall call(h);
+    if ((rc = call.begin())) return rc;
     const int64_t hchunk = std::min<int64_t>(n, 2048);
-    int64_t ci = 0;
-    for (int64_t i0 = 0; i0 < n; i0 += hchunk, ci++) {      // same ring as cnnacc_run_batch's host path
+    for (int64_t i0 = 0; i0 < n; i0 += hchunk) {
         const int64_t m = std::min(hchunk, n - i0);
-        Slot& s = h->slots[ci % kSlots];
-        if ((rc = slot_reserve(h, s, hchunk * feat_sz, hchunk * out_sz, 0))) return rc;
-        if (ci >= kSlots) CU(h, cudaStreamWaitEvent(h->st_h2d, s.ev_out, 0));
-        CU(h, cudaMemcpyAsync(s.d_in, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
-        CU(h, cudaEventRecord(s.ev_in, h->st_h2d));
-        CU(h, cudaStreamWaitEvent(h->st_k, s.ev_in, 0));
-        pool_features_kernel<<<(unsigned)m, 256, 0, h->st_k>>>(s.d_in, reinterpret_cast<float*>(s.d_out));
+        Slot* s;
+        if ((rc = call.acquire(s, hchunk * feat_sz, hchunk * out_sz))) return rc;
+        CU(h, cudaMemcpyAsync(s->d_in, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        if ((rc = call.staged(*s))) return rc;
+        pool_features_kernel<<<(unsigned)m, 256, 0, h->st_k>>>(s->d_in, reinterpret_cast<float*>(s->d_out));
         h->launches++;
         CU(h, cudaGetLastError());
-        CU(h, cudaEventRecord(s.ev_k, h->st_k));
-        CU(h, cudaStreamWaitEvent(h->st_d2h, s.ev_k, 0));
-        CU(h, cudaMemcpyAsync(pooled + i0 * 1024, s.d_out, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
-        CU(h, cudaEventRecord(s.ev_out, h->st_d2h));
+        if ((rc = call.computed(*s))) return rc;
+        CU(h, cudaMemcpyAsync(pooled + i0 * 1024, s->d_out, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+        if ((rc = call.released(*s, h->st_d2h))) return rc;
     }
-    CU(h, cudaStreamSynchronize(h->st_d2h));
-    return drain.done(CNNACC_OK);
+    return call.finish(h->st_d2h, false);
 }
 
 int cnnacc_cam_bbox_batch(cnnacc_handle* h, const uint8_t* feats, int64_t n, const int32_t* cls, int32_t* bbox, uint8_t* cam,
@@ -1086,29 +1103,24 @@ int cnnacc_cam_bbox_batch(cnnacc_handle* h, const uint8_t* feats, int64_t n, con
         return launch_cam_upsampled(h, h->stream, feats, n, cls, bbox, cam);
     }
 
-    CU(h, cudaStreamSynchronize(h->stream));
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));
-    RingDrain drain(h);
+    HostCall call(h);
+    if ((rc = call.begin())) return rc;
     const int64_t hchunk = std::min<int64_t>(n, 4096);
-    int64_t ci = 0;
-    for (int64_t i0 = 0; i0 < n; i0 += hchunk, ci++) {      // same ring as cnnacc_run_batch's host path
+    for (int64_t i0 = 0; i0 < n; i0 += hchunk) {
         const int64_t m = std::min(hchunk, n - i0);
-        Slot& s = h->slots[ci % kSlots];
-        if ((rc = slot_reserve(h, s, hchunk * feat_sz, cam ? hchunk * cam_sz : 0, hchunk))) return rc;
-        if (ci >= kSlots) CU(h, cudaStreamWaitEvent(h->st_h2d, s.ev_out, 0));
-        CU(h, cudaMemcpyAsync(s.d_in, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
-        CU(h, cudaMemcpyAsync(s.d_cls, cls + i0, m * sizeof(int32_t), cudaMemcpyHostToDevice, h->st_h2d));
-        CU(h, cudaEventRecord(s.ev_in, h->st_h2d));
-        CU(h, cudaStreamWaitEvent(h->st_k, s.ev_in, 0));
-        if ((rc = launch_cam_upsampled(h, h->st_k, s.d_in, m, s.d_cls, bbox ? s.d_bbox : nullptr, cam ? s.d_out : nullptr))) return rc;
-        CU(h, cudaEventRecord(s.ev_k, h->st_k));
-        CU(h, cudaStreamWaitEvent(h->st_d2h, s.ev_k, 0));
-        if (bbox) CU(h, cudaMemcpyAsync(bbox + i0 * 4, s.d_bbox, m * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st_d2h));
-        if (cam)  CU(h, cudaMemcpyAsync(cam + i0 * cam_sz, s.d_out, m * cam_sz, cudaMemcpyDeviceToHost, h->st_d2h));
-        CU(h, cudaEventRecord(s.ev_out, h->st_d2h));
+        Slot* s;
+        if ((rc = call.acquire(s, hchunk * feat_sz, cam ? hchunk * cam_sz : 0, hchunk))) return rc;
+        CU(h, cudaMemcpyAsync(s->d_in, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        CU(h, cudaMemcpyAsync(s->d_cls, cls + i0, m * sizeof(int32_t), cudaMemcpyHostToDevice, h->st_h2d));
+        if ((rc = call.staged(*s)) ||
+            (rc = launch_cam_upsampled(h, h->st_k, s->d_in, m, s->d_cls, bbox ? s->d_bbox : nullptr, cam ? s->d_out : nullptr)) ||
+            (rc = call.computed(*s)))
+            return rc;
+        if (bbox) CU(h, cudaMemcpyAsync(bbox + i0 * 4, s->d_bbox, m * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st_d2h));
+        if (cam)  CU(h, cudaMemcpyAsync(cam + i0 * cam_sz, s->d_out, m * cam_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+        if ((rc = call.released(*s, h->st_d2h))) return rc;
     }
-    CU(h, cudaStreamSynchronize(h->st_d2h));
-    return drain.done(CNNACC_OK);
+    return call.finish(h->st_d2h, false);
 }
 
 // Pre-processing of m square regions of frames already on the device into d_gray: base.desc = their descriptors (frame
@@ -1223,9 +1235,8 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         return rc;
     }
 
-    CU(h, cudaStreamSynchronize(h->stream));
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));
-    RingDrain drain(h);
+    HostCall call(h);
+    if ((rc = call.begin())) return rc;
     const std::vector<RegionChunk> plan =
         make_region_plan([&](int64_t r) -> int64_t { return centre ? r : regions[4 * r]; }, n, frame_sz, kPredSuper);
     size_t staged = 0, max_stage = 0;
@@ -1258,72 +1269,56 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         return P;
     };
 
+    PredBlock pred(h);
+    Slot* s;
     if (small) {
-        Slot& s = h->slots[0];
         cudaStream_t st = h->st_k;
-        if ((rc = slot_reserve(h, s, staged, n * img_sz, 0))) return rc;
-        const SmallPred p = small_pred(h, n);
+        if ((rc = call.acquire(s, staged, n * img_sz)) || (rc = pred.start(0, n))) return rc;
         // one copy per run of consecutive staged frames (the chunks of one run are adjacent in the buffer)
         size_t off = 0;
         for (size_t k = 0; k < plan.size();) {
             size_t j = k + 1;
             while (j < plan.size() && plan[j].f0 == plan[j - 1].f1) j++;
             const size_t bytes = (size_t)(plan[j - 1].f1 - plan[k].f0) * frame_sz;
-            CU(h, cudaMemcpyAsync(s.d_in + off, frames + plan[k].f0 * frame_sz, bytes, cudaMemcpyHostToDevice, st));
+            CU(h, cudaMemcpyAsync(s->d_in + off, frames + plan[k].f0 * frame_sz, bytes, cudaMemcpyHostToDevice, st));
             off += bytes;
             k = j;
         }
-        if ((rc = prep_then_tail(h, st, region_base(s.d_in, 0, 0, s.d_out), n, detect, p.d_probs, p.d_cls, p.d_bbox, flags))) return rc;
+        if ((rc = prep_then_tail(h, st, region_base(s->d_in, 0, 0, s->d_out), n, detect, pred.probs(0), pred.cls(0), pred.bbox(0), flags)))
+            return rc;
         if (db) CU(h, cudaEventRecord(db->ev, st));
-        if (gray128) CU(h, cudaMemcpyAsync(gray128, s.d_out, n * img_sz, cudaMemcpyDeviceToHost, st));
-        if (detect) CU(h, cudaMemcpyAsync(h->h_pred_small, h->d_pred_small, p.bytes, cudaMemcpyDeviceToHost, st));
-        CU(h, cudaStreamSynchronize(st));
-        if (detect) small_pred_unpack(h, p, n, probs, cls, bbox, false);
-        return drain.done(detect ? check_fused_status(h) : CNNACC_OK);
+        if (gray128) CU(h, cudaMemcpyAsync(gray128, s->d_out, n * img_sz, cudaMemcpyDeviceToHost, st));
+        if (detect && (rc = pred.flush(st, probs, cls, bbox, false))) return rc;
+        return detect ? call.done(true) : call.finish(st, false);
     }
-    // staged chunks of about 16 MiB of frames through the ring of cnnacc_run_batch's host path; a chunk's regions run in
-    // launches of up to kRegionLaunch (their gray images fill the slot's output buffer); predictions as in predict_impl
+    // Staged chunks of about 16 MiB of frames through the ring (HostCall).  A chunk's regions run in launches of up to
+    // kRegionLaunch: their gray images fill the slot's output buffer, so a launch after the first waits for the gray copy of
+    // the launch before.
     const int64_t per_launch = std::min<int64_t>(max_regions, kRegionLaunch);
-    if (detect && (rc = ensure_pred(h, std::min<int64_t>(n, kPredSuper)))) return rc;
-    int64_t s0 = 0;
-    SmallPred p = detect ? small_pred(h, std::min<int64_t>(kPredSuper, n)) : SmallPred();
-    auto flush = [&](int64_t sn) -> int {                // predictions of regions [s0, s0 + sn) to the caller
-        if (!detect) return 0;
-        CU(h, cudaMemcpyAsync(h->h_pred_small, h->d_pred_small, p.bytes, cudaMemcpyDeviceToHost, h->st_k));
-        CU(h, cudaStreamSynchronize(h->st_k));
-        small_pred_unpack(h, p, sn, probs ? probs + s0 * nc : nullptr, cls ? cls + s0 : nullptr, bbox ? bbox + s0 * 4 : nullptr, false);
-        return 0;
-    };
-    int64_t ci = 0;
+    if (detect && (rc = pred.start(0, std::min<int64_t>(kPredSuper, n)))) return rc;
     for (const RegionChunk& c : plan) {
-        if (c.r0 >= s0 + kPredSuper) {                   // the plan never lets a chunk straddle a block edge
-            if ((rc = flush(kPredSuper))) return rc;
-            s0 += kPredSuper;
-            if (detect) p = small_pred(h, std::min<int64_t>(kPredSuper, n - s0));
+        if (detect && c.r0 >= pred.end()) {              // the plan never lets a chunk straddle a block edge
+            if ((rc = pred.flush(h->st_k, probs, cls, bbox, false)) ||
+                (rc = pred.start(pred.end(), std::min<int64_t>(kPredSuper, n - pred.end()))))
+                return rc;
         }
-        Slot& s = h->slots[ci % kSlots];
-        if ((rc = slot_reserve(h, s, max_stage, per_launch * img_sz, 0))) return rc;
-        if (ci >= kSlots) CU(h, cudaStreamWaitEvent(h->st_h2d, s.ev_out, 0));
-        CU(h, cudaMemcpyAsync(s.d_in, frames + c.f0 * frame_sz, (size_t)(c.f1 - c.f0) * frame_sz, cudaMemcpyHostToDevice, h->st_h2d));
-        CU(h, cudaEventRecord(s.ev_in, h->st_h2d));
-        CU(h, cudaStreamWaitEvent(h->st_k, s.ev_in, 0));
+        if ((rc = call.acquire(s, max_stage, per_launch * img_sz))) return rc;
+        CU(h, cudaMemcpyAsync(s->d_in, frames + c.f0 * frame_sz, (size_t)(c.f1 - c.f0) * frame_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        if ((rc = call.staged(*s))) return rc;
         for (int64_t r = c.r0; r < c.r1; r += per_launch) {
             const int64_t m = std::min(per_launch, c.r1 - r);
-            if (r > c.r0 && gray128) CU(h, cudaStreamWaitEvent(h->st_k, s.ev_out, 0));   // the last gray copy has left s.d_out
-            if ((rc = prep_then_tail(h, h->st_k, region_base(s.d_in, r, c.r0, s.d_out), m, detect,
-                                     detect ? p.d_probs + (r - s0) * nc : nullptr, detect ? p.d_cls + (r - s0) : nullptr,
-                                     detect ? p.d_bbox + (r - s0) * 4 : nullptr, flags))) return rc;
-            CU(h, cudaEventRecord(s.ev_k, h->st_k));
-            CU(h, cudaStreamWaitEvent(h->st_d2h, s.ev_k, 0));
-            if (gray128) CU(h, cudaMemcpyAsync(gray128 + r * img_sz, s.d_out, m * img_sz, cudaMemcpyDeviceToHost, h->st_d2h));
-            CU(h, cudaEventRecord(s.ev_out, h->st_d2h));
+            if (r > c.r0 && gray128 && (rc = call.wait_released(*s, h->st_k))) return rc;
+            if ((rc = prep_then_tail(h, h->st_k, region_base(s->d_in, r, c.r0, s->d_out), m, detect, detect ? pred.probs(r) : nullptr,
+                                     detect ? pred.cls(r) : nullptr, detect ? pred.bbox(r) : nullptr, flags)) ||
+                (rc = call.computed(*s)))
+                return rc;
+            if (gray128) CU(h, cudaMemcpyAsync(gray128 + r * img_sz, s->d_out, m * img_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+            if ((rc = call.released(*s, h->st_d2h))) return rc;
         }
-        ci++;
     }
     if (db) CU(h, cudaEventRecord(db->ev, h->st_k));
-    if ((rc = flush(n - s0))) return rc;
-    CU(h, cudaStreamSynchronize(h->st_d2h));
-    return drain.done(detect ? check_fused_status(h) : CNNACC_OK);
+    if (detect && (rc = pred.flush(h->st_k, probs, cls, bbox, false))) return rc;
+    return call.finish(h->st_d2h, detect);
 }
 
 int cnnacc_preprocess_bgr(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, uint8_t* gray128, uint32_t flags) {
@@ -1556,9 +1551,8 @@ int cnnacc_timer_stop(cnnacc_handle* h, float* ms) {
 int cnnacc_synchronize(cnnacc_handle* h) {
     if (!h) return CNNACC_ERR_ARG;
     CU(h, cudaSetDevice(h->device));
-    CU(h, cudaStreamSynchronize(h->stream));
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));
-    return check_fused_status(h);
+    int rc = sync_all(h);
+    return rc ? rc : check_fused_status(h);
 }
 
 // ---- drop-in for arm_cnn.c:159-162 -------------------------------------------------------------
