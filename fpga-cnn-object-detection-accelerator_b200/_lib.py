@@ -4,7 +4,7 @@ import os
 import subprocess
 
 _DIR = os.path.dirname(os.path.abspath(__file__))
-# CNNACC_LIB_PATH: tuning experiments load an alternative build of the same library (tools/build_variants.sh)
+# CNNACC_LIB_PATH: load another build of the same library instead (the -DCNNACC_TRACE build of tools/trace_run.py)
 LIB_PATH = os.environ.get("CNNACC_LIB_PATH") or os.path.join(_DIR, "libcnnacc.so")
 CSRC = os.path.join(_DIR, "csrc")
 

@@ -63,7 +63,7 @@ struct cnnacc_handle {
     int device = 0;
     cudaStream_t own_stream = nullptr, stream = nullptr;
     cudaStream_t st_h2d = nullptr, st_k = nullptr, st_d2h = nullptr;   // one stream per engine for host-pointer batches
-    cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_a = nullptr, ev_b = nullptr, ev_c = nullptr, ev_done = nullptr;
+    cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_a = nullptr, ev_b = nullptr, ev_done = nullptr;
     int sm_count = 0;
     bool weights_loaded = false, fc_loaded = false, tail_attr_set = false;
     int shifts[3] = {2, 4, 6};                  // SHIFT_L0..2 defaults, pynq_inference.py:83-85
@@ -141,23 +141,23 @@ bool aligned(const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p
 
 bool valid_hw(int H, int W) { return H >= 16 && W >= 16 && H % 16 == 0 && W % 16 == 0 && H <= 8192 && W <= 8192; }
 
-// The tuning overrides the sweeps in tools/ set (CNNACC_PDL, CNNACC_HOST_CHUNK_MB, CNNACC_HOST_RAMP, CNNACC_WS_CHUNK): the
-// variable's integer value, or dflt when it is unset.  Each is read once, into a function-local static where it is used.
+// An integer environment setting (CNNACC_PDL, INTEGRATION.md): the variable's value, or dflt when it is unset.  Read once,
+// into a function-local static where it is used.
 int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
 
 // Which kernels run the conv stack of an H x W call.  128x128 is one fused launch (its maps can also be kept); larger sizes
 // run as overlapping 128x128 windows through the fused kernel; everything else, and DIRECT, takes the per-layer kernels.
 enum class ConvPath { kFused128, kFusedWindows, kPerLayer };
-ConvPath conv_path(const cnnacc_handle* h, int H, int W, uint32_t flags) {
-    if (!h->fused.ready || (flags & CNNACC_FLAG_DIRECT)) return ConvPath::kPerLayer;
+ConvPath conv_path(int H, int W, uint32_t flags) {
+    if (flags & CNNACC_FLAG_DIRECT) return ConvPath::kPerLayer;
     if (H == CNNACC_IMG && W == CNNACC_IMG) return ConvPath::kFused128;
     if (H >= CNNACC_IMG && W >= CNNACC_IMG && !(flags & CNNACC_FLAG_KEEP_MAPS)) return ConvPath::kFusedWindows;
     return ConvPath::kPerLayer;
 }
 
 // Does the classifier tail of a 128x128 call run inside the fused conv kernel, on the feature map still in shared memory?
-bool tail_in_conv(const cnnacc_handle* h, uint32_t flags) {
-    return conv_path(h, CNNACC_IMG, CNNACC_IMG, flags) == ConvPath::kFused128 &&
+bool tail_in_conv(uint32_t flags) {
+    return conv_path(CNNACC_IMG, CNNACC_IMG, flags) == ConvPath::kFused128 &&
            !(flags & (CNNACC_FLAG_KEEP_MAPS | CNNACC_FLAG_TWO_KERNELS));
 }
 
@@ -179,7 +179,7 @@ int launch_direct_layer(cnnacc_handle* h, cudaStream_t stream, int layer, const 
 // Conv stack for n device-resident images on `stream`.  l0/l1 are workspaces for the per-layer path.
 int conv_stack_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_imgs, int64_t n, int H, int W,
                       uint8_t* d_feats, uint32_t flags, uint8_t* d_l0, uint8_t* d_l1) {
-    const ConvPath path = conv_path(h, H, W, flags);
+    const ConvPath path = conv_path(H, W, flags);
     if (path == ConvPath::kFused128) {
         // May this launch overlap the previous conv-stack launch (no griddepcontrol.wait)?  Only if that one is the last thing
         // this handle launched, on the same stream, and none of the launches since the last full wait shares memory with it.
@@ -229,8 +229,8 @@ int conv_stack_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_im
     return 0;
 }
 
-bool needs_maps(const cnnacc_handle* h, int H, int W, uint32_t flags) {   // only the per-layer path has intermediate maps in HBM
-    return conv_path(h, H, W, flags) == ConvPath::kPerLayer || (flags & CNNACC_FLAG_KEEP_MAPS);
+bool needs_maps(int H, int W, uint32_t flags) {   // only the per-layer path has intermediate maps in HBM
+    return conv_path(H, W, flags) == ConvPath::kPerLayer || (flags & CNNACC_FLAG_KEEP_MAPS);
 }
 
 // images per chunk so that the per-layer workspaces stay around 512 MiB
@@ -276,7 +276,7 @@ int launch_tail(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_feats, i
 // the features afterwards (want_feats) or the per-layer kernels are in use.
 int infer_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_imgs, int64_t m, uint8_t* d_feat_ws, bool want_feats,
                  const TailArgs& A, uint32_t flags) {
-    if (tail_in_conv(h, flags)) {
+    if (tail_in_conv(flags)) {
         int rc = launch_fused(h->fused, stream, d_imgs, m, want_feats ? d_feat_ws : nullptr, h->shifts, h->sm_count, nullptr, nullptr, &A);
         h->launches++;
         if (rc != 0) return fail(h, CNNACC_ERR_CUDA, std::string("fused launch: ") + cudaGetErrorString((cudaError_t)rc));
@@ -286,8 +286,8 @@ int infer_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_imgs, i
     if ((rc = conv_stack_device(h, stream, d_imgs, m, CNNACC_IMG, CNNACC_IMG, d_feat_ws, flags, h->d_l0, h->d_l1))) return rc;
     return launch_tail(h, stream, d_feat_ws, m, A);
 }
-bool infer_needs_feat_ws(const cnnacc_handle* h, bool want_feats, uint32_t flags) {
-    return want_feats || !tail_in_conv(h, flags);
+bool infer_needs_feat_ws(bool want_feats, uint32_t flags) {
+    return want_feats || !tail_in_conv(flags);
 }
 
 // Classifier.get_cam_bbox per image (cam_upsampled.cuh); d_cam may be null
@@ -451,23 +451,15 @@ struct PredBlock {
     }
 };
 
-// The cut of a host-pointer call into staging chunks (host_chunks.h) under the CNNACC_HOST_CHUNK_MB / CNNACC_HOST_RAMP
-// overrides.  `ramp`: the call may ramp its chunk sizes up and down at its edges.
-HostChunkPlan host_chunk_plan(int64_t n, size_t in_sz, int64_t cap_images, bool pipelined, bool ramp) {
-    static const size_t chunk_mb = (size_t)std::max(0, env_int("CNNACC_HOST_CHUNK_MB", 0));
-    static const int depth = std::clamp(env_int("CNNACC_HOST_RAMP", 2), 0, 4);
-    return make_host_chunk_plan(n, in_sz, cap_images, pipelined, chunk_mb, ramp ? depth : 0);
-}
-
 // The host-pointer conv stack: queue the staged copies and kernels of one call on the ring; does not wait for anything.  A
 // pipelined call has no ramped chunk sizes: the neighbouring calls keep both copy directions busy at its edges.
 int enqueue_host_batch(HostCall& call, const uint8_t* imgs, int64_t n, int H, int W, uint8_t* feats, uint32_t flags) {
     cnnacc_handle* h = call.h;
     int rc;
     const size_t in_sz = (size_t)H * W, out_sz = (size_t)64 * (H / 8) * (W / 8);
-    const HostChunkPlan plan = host_chunk_plan(n, in_sz, chunk_images(H, W), call.pipelined, true);
+    const HostChunkPlan plan = make_host_chunk_plan(n, in_sz, chunk_images(H, W), call.pipelined);
     const int64_t hchunk = plan.full;
-    if (needs_maps(h, H, W, flags) && (rc = ensure_maps(h, hchunk, H, W))) return rc;
+    if (needs_maps(H, W, flags) && (rc = ensure_maps(h, hchunk, H, W))) return rc;
     if (call.pipelined) {
         // earlier calls may still be using the slots: growing one (free + malloc) waits for the device first
         bool grows = false;
@@ -591,7 +583,7 @@ int cnnacc_create(int device_id, cnnacc_handle** out) {
     h->sm_count = prop.multiProcessorCount;
     if ((e = cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
     h->stream = h->own_stream;
-    cudaEvent_t* evs[] = {&h->ev_t0, &h->ev_t1, &h->ev_a, &h->ev_b, &h->ev_c, &h->ev_done};
+    cudaEvent_t* evs[] = {&h->ev_t0, &h->ev_t1, &h->ev_a, &h->ev_b, &h->ev_done};
     for (auto ev : evs)
         if ((e = cudaEventCreate(ev)) != cudaSuccess) return bail("cudaEventCreate", e);
     for (auto& s : h->slots) {
@@ -641,7 +633,7 @@ int cnnacc_destroy(cnnacc_handle* h) {
     cudaFree(h->d_l0); cudaFree(h->d_l1); cudaFree(h->d_feat); cudaFree(h->d_img1); cudaFree(h->d_bram);
     fused_free(h->fused);
     cudaFreeHost(h->h_img); cudaFreeHost(h->h_bram); cudaFreeHost(h->h_done); cudaFreeHost(h->h_pred); cudaFree(h->d_pred);
-    cudaEvent_t evs[] = {h->ev_t0, h->ev_t1, h->ev_a, h->ev_b, h->ev_c, h->ev_done};
+    cudaEvent_t evs[] = {h->ev_t0, h->ev_t1, h->ev_a, h->ev_b, h->ev_done};
     for (auto ev : evs) if (ev) cudaEventDestroy(ev);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
@@ -661,6 +653,7 @@ int cnnacc_load_weights(cnnacc_handle* h, const uint8_t* weights_bin, size_t n) 
     if (!h || !weights_bin) return fail(h, CNNACC_ERR_ARG, "NULL argument");
     if (n != CNNACC_WEIGHT_BYTES)
         return fail(h, CNNACC_ERR_ARG, "Expected 23184 weights, got " + std::to_string(n));   // pynq_inference.py:189
+    h->weights_loaded = false;           // a reload that fails partway leaves a handle that refuses calls
     CU(h, cudaSetDevice(h->device));
     CU(h, cudaDeviceSynchronize());      // weights may be in use by queued launches
     std::memcpy(h->wbin, weights_bin, n);
@@ -717,7 +710,7 @@ int cnnacc_pdl_chain_host(int n_launches, const uint64_t* ranges, const int64_t*
 
 int cnnacc_chunk_plan_host(int64_t n, int H, int W, int pipelined, int64_t* sizes, int cap) {
     if (n < 1 || !valid_hw(H, W) || !sizes || cap < 1) return CNNACC_ERR_ARG;
-    const HostChunkPlan plan = make_host_chunk_plan(n, (size_t)H * W, chunk_images(H, W), pipelined != 0, 0, 2);
+    const HostChunkPlan plan = make_host_chunk_plan(n, (size_t)H * W, chunk_images(H, W), pipelined != 0);
     int count = 0;
     for (int64_t i0 = 0; i0 < n; count++) {
         const int64_t m = plan.next(i0, count);
@@ -750,7 +743,7 @@ int cnnacc_run_batch(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int H, in
     if (!imgs || !feats) return fail(h, CNNACC_ERR_ARG, "NULL image / feature pointer");
     CU(h, cudaSetDevice(h->device));
     const size_t in_sz = (size_t)H * W, out_sz = (size_t)64 * (H / 8) * (W / 8);
-    const bool maps = needs_maps(h, H, W, flags);
+    const bool maps = needs_maps(H, W, flags);
     const int64_t chunk = maps ? std::min<int64_t>(n, chunk_images(H, W)) : n;
 
     if (flags & CNNACC_FLAG_DEVICE_PTRS) {
@@ -780,7 +773,7 @@ int cnnacc_run_batch_async(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int
     if (flags & CNNACC_FLAG_DEVICE_PTRS) return fail(h, CNNACC_ERR_ARG, "device-pointer calls are asynchronous already (cnnacc_run_batch)");
     if (n > 0 && (!imgs || !feats)) return fail(h, CNNACC_ERR_ARG, "NULL image / feature pointer");
     // the per-layer kernels share two workspaces between chunks; only the paths without them can overlap calls
-    if (needs_maps(h, H, W, flags)) return fail(h, CNNACC_ERR_ARG, "this size / flag combination has no asynchronous form: use cnnacc_run_batch");
+    if (needs_maps(H, W, flags)) return fail(h, CNNACC_ERR_ARG, "this size / flag combination has no asynchronous form: use cnnacc_run_batch");
     CU(h, cudaSetDevice(h->device));
     // the event of the call submitted CNNACC_MAX_PENDING calls ago is about to be reused: that call must have completed
     cudaEvent_t ev = h->ev_ticket[h->next_ticket % CNNACC_MAX_PENDING];
@@ -883,52 +876,37 @@ int cnnacc_infer_one(cnnacc_handle* h, const uint8_t* img, uint8_t* feat, float*
     uint8_t* h_l2 = h->h_bram + 16 * 4096 + 32 * 1024;
     const auto t0 = std::chrono::steady_clock::now();
     std::memcpy(h->h_img, img, CNNACC_FEAT_BYTES);
-    if (h->fused.ready) {
-        // Zero-copy: the kernel TMA-loads the image straight from mapped pinned host memory and its 16 KiB bulk
-        // store lands in mapped pinned host memory -- one launch, one stream sync, no copy-engine round trips.
-        if (!h->one_map_ok) {
-            if (fused_encode_map(h->h_img_dev, 1, &h->one_map)) return fail(h, CNNACC_ERR_CUDA, "tensor map over the pinned image buffer");
-            h->one_map_ok = true;
-        }
-        uint8_t* l2_dev = h->h_bram_dev + 16 * 4096 + 32 * 1024;
-        const int seq = ++h->done_seq;
-        rc = launch_fused_map(h->fused, h->stream, h->one_map, 1, l2_dev, h->shifts, h->sm_count, nullptr, nullptr, nullptr, nullptr,
-                              h->h_done_dev, seq);
-        h->launches++;
-        if (rc != 0) return fail(h, CNNACC_ERR_CUDA, std::string("fused launch: ") + cudaGetErrorString((cudaError_t)rc));
-        // The kernel stores `seq` into a mapped host word after its feature store has landed: spinning on that word skips the
-        // driver's wake-up path of a stream synchronise (~8 us of the ~36).  Bounded: after 2 s fall back to the synchronise.
-        {
-            const volatile int* flag = h->h_done;
-            const auto spin0 = std::chrono::steady_clock::now();
-            for (unsigned it = 0; *flag != seq; it++) {
+    // Zero-copy: the kernel TMA-loads the image straight from mapped pinned host memory and its 16 KiB bulk
+    // store lands in mapped pinned host memory -- one launch, one stream sync, no copy-engine round trips.
+    if (!h->one_map_ok) {
+        if (fused_encode_map(h->h_img_dev, 1, &h->one_map)) return fail(h, CNNACC_ERR_CUDA, "tensor map over the pinned image buffer");
+        h->one_map_ok = true;
+    }
+    uint8_t* l2_dev = h->h_bram_dev + 16 * 4096 + 32 * 1024;
+    const int seq = ++h->done_seq;
+    rc = launch_fused_map(h->fused, h->stream, h->one_map, 1, l2_dev, h->shifts, h->sm_count, nullptr, nullptr, nullptr, nullptr,
+                          h->h_done_dev, seq);
+    h->launches++;
+    if (rc != 0) return fail(h, CNNACC_ERR_CUDA, std::string("fused launch: ") + cudaGetErrorString((cudaError_t)rc));
+    // The kernel stores `seq` into a mapped host word after its feature store has landed: spinning on that word skips the
+    // driver's wake-up path of a stream synchronise (~8 us of the ~36).  Bounded: after 2 s fall back to the synchronise.
+    {
+        const volatile int* flag = h->h_done;
+        const auto spin0 = std::chrono::steady_clock::now();
+        for (unsigned it = 0; *flag != seq; it++) {
 #if defined(__x86_64__)
-                __builtin_ia32_pause();
+            __builtin_ia32_pause();
 #endif
-                if ((it & 0xFFFF) == 0xFFFF && std::chrono::steady_clock::now() - spin0 > std::chrono::seconds(2)) {
-                    CU(h, cudaStreamSynchronize(h->stream));
-                    break;
-                }
+            if ((it & 0xFFFF) == 0xFFFF && std::chrono::steady_clock::now() - spin0 > std::chrono::seconds(2)) {
+                CU(h, cudaStreamSynchronize(h->stream));
+                break;
             }
         }
-        const auto t1 = std::chrono::steady_clock::now();
-        std::memcpy(feat, h_l2, CNNACC_FEAT_BYTES);
-        if (conv_ms) *conv_ms = std::chrono::duration<float, std::milli>(t1 - t0).count();
-        if (read_ms) *read_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t1).count();
-        return check_fused_status(h);
     }
-    // generic path (no fused kernel): staged copies around the per-layer kernels
-    uint8_t *l0 = h->d_bram, *l1 = h->d_bram + 16 * 4096, *l2 = l1 + 32 * 1024;
-    CU(h, cudaMemcpyAsync(h->d_img1, h->h_img, CNNACC_IMG * CNNACC_IMG, cudaMemcpyHostToDevice, h->stream));
-    CU(h, cudaEventRecord(h->ev_a, h->stream));
-    if ((rc = conv_stack_device(h, h->stream, h->d_img1, 1, CNNACC_IMG, CNNACC_IMG, l2, 0, l0, l1))) return rc;
-    CU(h, cudaEventRecord(h->ev_b, h->stream));
-    CU(h, cudaMemcpyAsync(h_l2, l2, CNNACC_FEAT_BYTES, cudaMemcpyDeviceToHost, h->stream));
-    CU(h, cudaEventRecord(h->ev_c, h->stream));
-    CU(h, cudaStreamSynchronize(h->stream));
+    const auto t1 = std::chrono::steady_clock::now();
     std::memcpy(feat, h_l2, CNNACC_FEAT_BYTES);
-    if (conv_ms) CU(h, cudaEventElapsedTime(conv_ms, h->ev_a, h->ev_b));
-    if (read_ms) CU(h, cudaEventElapsedTime(read_ms, h->ev_b, h->ev_c));
+    if (conv_ms) *conv_ms = std::chrono::duration<float, std::milli>(t1 - t0).count();
+    if (read_ms) *read_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t1).count();
     return check_fused_status(h);
 }
 
@@ -965,14 +943,14 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
     CU(h, cudaSetDevice(h->device));
     const size_t img_sz = CNNACC_FEAT_BYTES;        // 128*128 image and 64*256 feature map are both 16 KiB
     const int nc = h->n_cls;
-    const bool maps = src_is_images && needs_maps(h, CNNACC_IMG, CNNACC_IMG, flags);
+    const bool maps = src_is_images && needs_maps(CNNACC_IMG, CNNACC_IMG, flags);
     const bool cls_given = (flags & CNNACC_FLAG_CLS_GIVEN) != 0;
     if (cls_given && !cls) return fail(h, CNNACC_ERR_ARG, "CNNACC_FLAG_CLS_GIVEN without a cls array");
     const bool upsampled = (flags & CNNACC_FLAG_BBOX_UPSAMPLED) != 0 && bbox;
     if (upsampled && !cls && (flags & CNNACC_FLAG_DEVICE_PTRS))
         return fail(h, CNNACC_ERR_ARG, "CNNACC_FLAG_BBOX_UPSAMPLED with device pointers needs a cls array");
     // images in: does anything after the conv stack need the feature maps in HBM?
-    const bool feat_ws = src_is_images && infer_needs_feat_ws(h, upsampled, flags);
+    const bool feat_ws = src_is_images && infer_needs_feat_ws(upsampled, flags);
 
     if (flags & CNNACC_FLAG_DEVICE_PTRS) {
         REQUIRE_ALIGNED(h, src, 16, "image / feature");
@@ -980,8 +958,7 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
         REQUIRE_ALIGNED(h, probs, 4, "probs");
         REQUIRE_ALIGNED(h, cls, 4, "cls");
         // one fused launch covers the whole call unless a workspace bounds the chunk
-        static const int ws_chunk = env_int("CNNACC_WS_CHUNK", 0);
-        const int64_t chunk = feat_ws ? std::min<int64_t>(n, ws_chunk > 0 ? ws_chunk : 16384) : n;
+        const int64_t chunk = feat_ws ? std::min<int64_t>(n, 16384) : n;
         if (feat_ws) {
             if ((rc = grow(h, &h->d_feat, &h->cap_feat, (size_t)chunk * img_sz))) return rc;
             if (maps && (rc = ensure_maps(h, chunk, CNNACC_IMG, CNNACC_IMG))) return rc;
@@ -1026,7 +1003,7 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
     }
     // Only the predictions (44 B per image) come back, so the link carries H2D traffic alone: no ramp, and no cap beyond the
     // call's own size.  Nothing is copied out per slot, so a slot is released once its kernels have ended.
-    const int64_t hchunk = host_chunk_plan(n, img_sz, INT64_MAX, false, false).full;
+    const int64_t hchunk = make_host_chunk_plan(n, img_sz, INT64_MAX, false).full;
     if (maps && (rc = ensure_maps(h, hchunk, CNNACC_IMG, CNNACC_IMG))) return rc;
     for (int64_t s0 = 0; s0 < n; s0 += kPredSuper) {
         if ((rc = pred.start(s0, std::min<int64_t>(kPredSuper, n - s0)))) return rc;
@@ -1150,7 +1127,7 @@ static int prep_then_tail(cnnacc_handle* h, cudaStream_t st, const RegionPrep& b
     if (!detect) return 0;
     const size_t img_sz = CNNACC_FEAT_BYTES;
     const bool ups = (flags & CNNACC_FLAG_BBOX_UPSAMPLED) && d_bbox;
-    if (infer_needs_feat_ws(h, ups, 0) && (rc = grow(h, &h->d_feat, &h->cap_feat, (size_t)m * img_sz))) return rc;
+    if (infer_needs_feat_ws(ups, 0) && (rc = grow(h, &h->d_feat, &h->cap_feat, (size_t)m * img_sz))) return rc;
     const TailArgs A = make_tail(h, d_probs, d_cls, ups ? nullptr : d_bbox, false, flags);
     if ((rc = infer_device(h, st, base.out, m, h->d_feat, ups, A, 0))) return rc;
     if (ups && (rc = launch_cam_upsampled(h, st, h->d_feat, m, d_cls, d_bbox, nullptr))) return rc;

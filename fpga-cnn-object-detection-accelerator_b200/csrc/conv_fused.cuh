@@ -115,29 +115,14 @@ constexpr int kTraceMax = 90, kTraceRoles = 6;
 #define TRACE_END(role) do { } while (0)
 #endif
 
-#ifndef CNNACC_TAIL_WARPS_FIRST
-#define CNNACC_TAIL_WARPS_FIRST 0
-#endif
-#ifndef CNNACC_L0_DP4A_WARPS
-#define CNNACC_L0_DP4A_WARPS 8     // layer-0 warps that use dp4a; the rest use mma.sync (0 and 16 = the single-pipe ablations)
-#endif
-#ifndef CNNACC_L0_WARPS
-#define CNNACC_L0_WARPS 16
-#endif
-#ifndef CNNACC_EPI_WARPS
-#define CNNACC_EPI_WARPS 4
-#endif
-constexpr int kL0Dp4aWarps = CNNACC_L0_DP4A_WARPS;
-constexpr int kL0Warps = CNNACC_L0_WARPS, kEpiWarps = CNNACC_EPI_WARPS;   // multiples of 4 (TMEM lane quarter == warp % 4)
-static_assert(kL0Warps % 4 == 0 && kL0Warps <= 24 && (kEpiWarps == 4 || kEpiWarps == 8), "warp split");
+constexpr int kL0Warps = 16;                          // layer 0 (a multiple of 4: TMEM lane quarter == warp % 4)
+constexpr int kL0Dp4aWarps = 8;                       // ... of which these use dp4a, the rest mma.sync
+constexpr int kEpiWarps = 4;                          // one per TMEM lane quarter
 constexpr int kWarpMma = kL0Warps + kEpiWarps;       // the last warp: MMA issue and TMA loads
-// 4 epilogue warps: 21 warps at 80 registers.  8 epilogue warps (experiment, CNNACC_EPI_WARPS=8): 25 working warps only fit
-// with the setmaxnreg hand-over, so the grid is padded to 28 warps (warpgroup 6 = MMA warp + three idle ones).
-constexpr int kFusedThreads = (kEpiWarps == 8 ? 28 : kWarpMma + 1) * 32;    // 21 warps = 672
+constexpr int kFusedThreads = (kWarpMma + 1) * 32;    // 21 warps = 672
 constexpr int kTailWarps = kTailThreads / 32;         // 4 tail warps = warpgroup 6 of the kTail instantiation
 constexpr int kWarpTail0 = 24;                        // first tail warp (warpgroup aligned: setmaxnreg acts on warpgroups)
 constexpr int kTailKernelThreads = (kWarpTail0 + kTailWarps) * 32;   // 896
-static_assert(kWarpMma == 20 || kWarpMma == 24, "register hand-over below assumes warpgroups 0-4 heavy, 5-6 light");
 constexpr uint32_t kTmemCols = 512;
 #ifndef CNNACC_WAIT_BUDGET_CLK
 #define CNNACC_WAIT_BUDGET_CLK 8000000000LL            // bounded pipeline waits: ~4 s of SM clocks
@@ -161,7 +146,7 @@ constexpr int kErrInputTimeout = 1, kErrMmaTimeout = 2, kErrEmptyTimeout = 4, kE
               kErrAct1Timeout = 16, kErrAct2Timeout = 32, kErrSlotTimeout = 64, kErrStageTimeout = 128;
 
 struct FusedParams {
-    uint32_t w0[16][6];          // layer-0 dp4a words per out-channel: lo[dy], hi[dy]  (constant bank; CNNACC_L0_DP4A build)
+    uint32_t w0[16][6];          // layer-0 dp4a words per out-channel: lo[dy], hi[dy]  (constant bank)
     uint32_t w0f[8][32];         // layer-0 mma.sync B fragments: [block = py*4 + ol][lane]
     int shift0, shift1, shift2;
     int acc24;                   // layer-2 accumulators wrap at 24 bits before the pool (RTL / trainer width, accumulator.v:15,
@@ -200,38 +185,24 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(bytes) : "memory");
 }
-// 0 = plain try_wait (shipped).  With a suspend-time hint every failed try_wait costs a NANOSLEEP.SYNCS that wakes on ANY
-// barrier event of the CTA (ncu: ~100 wake-ups per image per waiting warp, 16.8 k polling instructions per image in the
-// round-1 kernel); without it the hardware holds the warp on this barrier alone: +2.5-4 % images/s
-// (profiles/r2_trywait_hint_sweep.txt).
-#ifndef CNNACC_TRYWAIT_HINT
-#define CNNACC_TRYWAIT_HINT 0
-#endif
+// Plain SYNCS.TRYWAIT: the hardware holds the warp until this barrier's phase completes or its own time limit passes.
+// With a suspend-time hint every failed try_wait cost a NANOSLEEP.SYNCS that woke on ANY barrier event of the CTA (ncu:
+// ~100 wake-ups per image per waiting warp, 16.8 k polling instructions per image in the round-1 kernel); without it the
+// kernel ran 2.5-4 % more images/s (profiles/r2_trywait_hint_sweep.txt).
 __device__ __forceinline__ uint32_t mbar_try(uint32_t bar, uint32_t parity) {
     uint32_t ok;
-#if CNNACC_TRYWAIT_HINT > 0
-    // with a suspend-time hint: SYNCS.TRYWAIT; NANOSLEEP.SYNCS hint; SYNCS.PHASECHK (the sleep ends on any barrier event)
-    asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n selp.u32 %0, 1, 0, p;\n}\n"
-                 : "=r"(ok) : "r"(bar), "r"(parity), "r"((uint32_t)CNNACC_TRYWAIT_HINT) : "memory");
-#else
-    // plain SYNCS.TRYWAIT: the hardware holds the warp until this barrier's phase completes or its own time limit passes
     asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
                  : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-#endif
     return ok;
 }
 // Bounded wait: a broken pipeline must never hang the GPU.  Returns false on timeout.  Every try_wait parks the warp in
-// hardware for a while, and the clock is only consulted every 32 unsuccessful polls.  kSleepNs > 0: a plain nanosleep
-// between polls (for the sixteen layer-0 warps, which otherwise out-poll the one epilogue warp of their sub-partition).
-template <int kSleepNs = 0>
+// hardware for a while, and the clock is only consulted every 32 unsuccessful polls.
 __device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity, long long budget) {
     const long long t0 = clock64();
     for (;;) {
 #pragma unroll 1
-        for (int i = 0; i < 32; i++) {
+        for (int i = 0; i < 32; i++)
             if (mbar_try(bar, parity)) return true;
-            if constexpr (kSleepNs > 0) __nanosleep(kSleepNs);
-        }
         if (clock64() - t0 > budget) return false;
     }
 }
@@ -292,18 +263,8 @@ __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, %0;" 
 // side costs no issue slots at all (an mbarrier wait polls, and NANOSLEEP.SYNCS wakes on every barrier event of the CTA:
 // ncu counted ~100 wake-ups per image per waiting warp).  The two barriers strictly alternate -- full(k), free(k),
 // full(k+1) ... -- and both sides run the same n_local iterations, so arrivals can never run a phase ahead.
-#ifndef CNNACC_L0_WAIT_SLEEP_NS
-#define CNNACC_L0_WAIT_SLEEP_NS 0
-#endif
-#ifndef CNNACC_L0_RENDEZVOUS
-#define CNNACC_L0_RENDEZVOUS 4     // kTail instantiation: sixteen layer-0 warps behind one poller at the A1BotFree point only
-#endif
-constexpr int kNamedL0Top = 8, kNamedL0Bot = 9;       // the sixteen layer-0 warps behind one poller (see the layer-0 loop)
+constexpr int kNamedL0Bot = 9;                        // kTail: the sixteen layer-0 warps behind one poller (see the layer-0 loop)
 __device__ __forceinline__ void l0_bar_sync(int id) { asm volatile("bar.sync %0, %1;" :: "r"(id), "n"(kL0Warps * 32) : "memory"); }
-__device__ __forceinline__ void l0_group_bar_sync(int id) { asm volatile("bar.sync %0, %1;" :: "r"(id), "n"(kL0Warps * 8) : "memory"); }
-#ifndef CNNACC_L0_RENDEZVOUS_CONV
-#define CNNACC_L0_RENDEZVOUS_CONV 0
-#endif
 constexpr int kNamedStageFull = 3, kNamedStageFree = 4;
 // ... and the same between the tail's front warps (24-27) and back warps (22-23) for the 1 KiB CAM buffer; 2 and 5 are the
 // front's and the back's own barriers.
@@ -360,15 +321,7 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
     int* s_err = reinterpret_cast<int*>(smem + kOffBar + 8 * kNumBars + 8);
 
     const int tid = threadIdx.x, lane = tid & 31;
-    // Role index.  In the kTail instantiation the light roles sit on the LOWEST hardware warp ids (CNNACC_TAIL_WARPS_FIRST):
-    // hardware warps 0-3 = tail front (role 24-27), 4-7 = MMA / idle / tail back (20-23), 8-11 = epilogues (16-19, TMEM
-    // lane quarter = hardware warp % 4 still holds), 12-27 = layer 0 (0-15).  Warpgroups stay aligned for setmaxnreg.
-    const int hw_warp = __shfl_sync(0xffffffffu, tid >> 5, 0);       // warp-uniform in the compiler's eyes
-#if CNNACC_TAIL_WARPS_FIRST
-    const int warp = !kTail ? hw_warp : (hw_warp < 4 ? hw_warp + 24 : hw_warp < 8 ? hw_warp + 16 : hw_warp < 12 ? hw_warp + 8 : hw_warp - 12);
-#else
-    const int warp = hw_warp;
-#endif
+    const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);          // warp-uniform in the compiler's eyes
     const int n_local = (P.n_images - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // images of this CTA
 #ifdef CNNACC_TRACE
     __shared__ unsigned trace_buf[kTraceRoles * kTraceMax];
@@ -410,23 +363,12 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
         asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
         if (P.pdl_wait) asm volatile("griddepcontrol.wait;" ::: "memory");
     }
-#ifndef CNNACC_REGS_EPI8
-#define CNNACC_REGS_EPI8 80
-#define CNNACC_REGS_MMA8 24
-#endif
-    if constexpr (!kTail && kEpiWarps == 8) {
-        if (warp >= kWarpMma)      asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" :: "n"(CNNACC_REGS_MMA8));
-        else if (warp >= kL0Warps) { if (CNNACC_REGS_EPI8 > 72) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" :: "n"(CNNACC_REGS_EPI8)); }
-        else                       asm volatile("setmaxnreg.inc.sync.aligned.u32 80;");
-    }
     if constexpr (kTail) {
-        // register hand-over (see the warp-role table): the light warpgroups release first, the heavy ones then grow
-#ifndef CNNACC_REGS_WG5
-#define CNNACC_REGS_WG5 48
-#define CNNACC_REGS_WG6 48
-#endif
-        if (warp >= kWarpTail0)    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" :: "n"(CNNACC_REGS_WG6));
-        else if (warp >= kWarpMma) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" :: "n"(CNNACC_REGS_WG5));
+        // register hand-over (see the warp-role table): the light warpgroups release first, the heavy ones then grow.
+        // The two dec branches stay separate: merged into one `warp >= kWarpMma` branch they compile to one
+        // USETMAXREG.DEALLOC instead of two, i.e. to a kernel other than the measured one.
+        if (warp >= kWarpTail0)    asm volatile("setmaxnreg.dec.sync.aligned.u32 48;");
+        else if (warp >= kWarpMma) asm volatile("setmaxnreg.dec.sync.aligned.u32 48;");
         else                       asm volatile("setmaxnreg.inc.sync.aligned.u32 80;");
     }
 
@@ -435,10 +377,6 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
         // ~4 s budget (a wait this long means a broken pipeline, not time-slicing or a debugger); once any wait has timed
         // out every later wait gives up quickly so the CTA drains.  A reported timeout invalidates the whole launch.
         if (!mbar_wait(b, parity, *reinterpret_cast<volatile int*>(s_err) ? 2000LL : kWaitBudgetClk)) atomicOr(s_err, code);
-    };
-    auto wait_or_flag_l0 = [&](uint32_t b, uint32_t parity, int code) {      // the same with a short sleep between polls
-        if (mbar_try(b, parity)) return;
-        if (!mbar_wait<CNNACC_L0_WAIT_SLEEP_NS>(b, parity, *reinterpret_cast<volatile int*>(s_err) ? 2000LL : kWaitBudgetClk)) atomicOr(s_err, code);
     };
 
     // TMA load of unit u (an image, or a window of a larger image) into an input slot; the box starts one pixel row above
@@ -477,29 +415,19 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
             for (int yp = warp; yp < 64; yp += kL0Warps) {
                 // act1 rows still being read by image k-1's layer-1 MMAs: rows 0-33 by the top tiles, 32-65 by the bottom
                 // ones.  This unit writes row yp+1.
-                // One warp polls the mbarrier for all sixteen; the others park on a hardware named barrier and cost no issue
-                // slots while they wait.  (ncu, profiles/r2a_conv_*: sixteen warps polling A1TopFree executed 2 166 try_waits
-                // per image -- four pollers per sub-partition next to the one epilogue warp whose progress they wait for.)
-                // Every layer-0 warp reaches each of the two points exactly once per image, so the barriers stay in step.
-                // Measured (tools/pipe_timing_short.py, M img/s conv-only / infer_batch when BOTH instantiations use the mode):
-                // none 19.73 / 15.67, both points 17.88 / 16.09, per sub-partition groups 18.82 / 15.62, top point only
-                // 19.29 / 16.02, bottom point only 19.08 / 16.23.  Without the tail warps any rendezvous costs throughput (the
-                // warps then move in lockstep behind the slowest); with them the bottom-only one is worth +3.5 %.  So the
-                // conv-only instantiation uses none and the kTail instantiation mode 4.
-                // CNNACC_L0_RENDEZVOUS: 0 none, 1 all sixteen warps behind warp 0 (both points), 2 per sub-partition group of four
-                // (warps s, s+4, s+8, s+12 behind warp s), 3 = 1 for the top point only, 4 = 1 for the bottom point only
-                constexpr int kRv = kTail ? CNNACC_L0_RENDEZVOUS : CNNACC_L0_RENDEZVOUS_CONV;
-                if (k > 0 && yp == warp) {
-                    const bool rv = kRv == 1 || kRv == 2 || kRv == 3;
-                    const bool poller = !rv || (kRv == 2 ? warp < 4 : warp == 0);
-                    if (poller) wait_or_flag_l0(bar(kBarA1TopFree), (uint32_t)(k - 1) & 1, kErrAct1Timeout);
-                    if (rv) { if (kRv == 2) l0_group_bar_sync(8 + (warp & 3)); else l0_bar_sync(kNamedL0Top); }
-                }
+                // Sixteen warps polling one mbarrier are costly (ncu, profiles/r2a_conv_*: 2 166 try_waits per image at
+                // A1TopFree -- four pollers per sub-partition next to the one epilogue warp whose progress they wait for).  The
+                // alternative is a rendezvous: warp 0 polls and the others park on a hardware named barrier, which costs no
+                // issue slots but moves the warps in lockstep behind the slowest.  Measured (tools/pipe_timing_short.py, M img/s
+                // conv-only / infer_batch with the same choice in both instantiations): no rendezvous 19.73 / 15.67, at both
+                // points 17.88 / 16.09, per sub-partition groups of four 18.82 / 15.62, top point only 19.29 / 16.02, bottom
+                // point only 19.08 / 16.23.  So the conv-only and window kernels have every warp poll, and the kTail kernel
+                // (+3.5 %) meets at the bottom point only.  Every layer-0 warp reaches each point exactly once per image, so the
+                // named barrier stays in step.
+                if (k > 0 && yp == warp) wait_or_flag(bar(kBarA1TopFree), (uint32_t)(k - 1) & 1, kErrAct1Timeout);
                 if (k > 0 && yp >= 31 && yp - kL0Warps < 31) {
-                    const bool rv = kRv == 1 || kRv == 2 || kRv == 4;
-                    const bool poller = !rv || (kRv == 2 ? warp < 4 : warp == 0);
-                    if (poller) wait_or_flag_l0(bar(kBarA1BotFree), (uint32_t)(k - 1) & 1, kErrAct1Timeout);
-                    if (rv) { if (kRv == 2) l0_group_bar_sync(12 + (warp & 3)); else l0_bar_sync(kNamedL0Bot); }
+                    if (!kTail || warp == 0) wait_or_flag(bar(kBarA1BotFree), (uint32_t)(k - 1) & 1, kErrAct1Timeout);
+                    if constexpr (kTail) l0_bar_sync(kNamedL0Bot);
                 }
                 if (warp == 0) TRACE(2, 1); else if (warp == kL0Warps - 1) TRACE(3, 1);
                 if (use_dp4a) {
@@ -606,8 +534,6 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
         // =============== epilogue warps ==========================================================================
         const int e = warp - kL0Warps;
         const int q = e & 3;                             // TMEM lane quarter (== warp % 4)
-        constexpr int kGStep = kEpiWarps / 4;            // 8 warps: each takes one channel half; 4 warps: both
-        const int g0 = e >> 2;
         const int L = q * 32 + lane;
         const uint32_t t_lane = tm + ((uint32_t)(q * 32) << 16);
         uint32_t use0 = 0, use1 = 0;                     // completed uses of each TMEM half (scalars: an array indexed by the
@@ -624,8 +550,10 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
                 if (e == 0) TRACE2(1, 20 + t);
                 tc_fence_after();
                 const int i = i0 + (L >> 3), j = j0 + (L & 7);
+                // channel half: 16 of the 32 output channels.  e >> 2 is always 0, but a literal 0 here schedules the window
+                // instantiation differently; this start keeps the measured code.
 #pragma unroll
-                for (int g = g0; g < 2; g += kGStep) {   // channel half: 16 of the 32 output channels
+                for (int g = e >> 2; g < 2; g++) {
                     const uint32_t taddr = t_lane + h * 256 + g * 16;
                     int mx[16];
                     {
@@ -641,7 +569,7 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
 #pragma unroll
                         for (int c = 0; c < 16; c++) mx[c] = max(mx[c], max(v0[c], v1[c]));
                     }
-                    if (g + kGStep >= 2) {               // last read of this TMEM half by this warp
+                    if (g == 1) {                        // last read of this TMEM half by this warp
                         tc_fence_before();
                         __syncwarp();
                         if (lane == 0) mbar_arrive(bar(kBarTmEmpty0 + h));
@@ -698,9 +626,7 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
                 tc_fence_after();
                 const int i = L >> 3, j = j0 + (L & 7);
 #pragma unroll
-                for (int c4 = 0; c4 < 4 / kGStep; c4++) {
-                    const int cg = (kGStep == 2) ? 2 * g0 + c4 : c4;     // group of 16 output channels
-                    const bool last_cg = (c4 == 4 / kGStep - 1);
+                for (int cg = 0; cg < 4; cg++) {         // group of 16 output channels
                     const uint32_t taddr = t_lane + h * 256 + cg * 16;
                     int m[16];
                     {
@@ -724,7 +650,7 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
 #pragma unroll
                         for (int c = 0; c < 16; c++) m[c] = max(m[c], max(v0[c], v1[c]));
                     }
-                    if (last_cg) {
+                    if (cg == 3) {                       // last read of this TMEM half by this warp
                         tc_fence_before();
                         __syncwarp();
                         if (lane == 0) mbar_arrive(bar(kBarTmEmpty0 + h));
@@ -916,7 +842,6 @@ conv_stack_fused_kernel(const __grid_constant__ CUtensorMap in_map, const __grid
 
 // ---- host side ------------------------------------------------------------------------------------------------
 struct FusedWeights {
-    bool ready = false;
     uint32_t w0[16][6];
     uint32_t w0f[8][32];
     uint8_t* d_b1 = nullptr;
@@ -996,7 +921,6 @@ inline void fused_pack_weights(const uint8_t* wbin, uint32_t w0[16][6], uint32_t
 
 // Pack and upload.  Returns a cudaError_t as int.
 inline int fused_load_weights(FusedWeights& fw, const uint8_t* wbin) {
-    fw.ready = false;
     std::vector<uint8_t> b1(kB1Bytes), b2(kB2Bytes);
     fused_pack_weights(wbin, fw.w0, fw.w0f, b1.data(), b2.data());
     cudaError_t e;
@@ -1018,14 +942,13 @@ inline int fused_load_weights(FusedWeights& fw, const uint8_t* wbin) {
         fw.attr_set = true;
     }
     if (!get_encode_tiled()) return (int)cudaErrorNotSupported;
-    fw.ready = true;
     return 0;
 }
 
 inline void fused_free(FusedWeights& fw) {
     cudaFree(fw.d_b1); cudaFree(fw.d_b2); cudaFree(fw.d_status);
     if (fw.h_status) cudaFreeHost(fw.h_status);
-    fw.d_b1 = fw.d_b2 = nullptr; fw.d_status = nullptr; fw.h_status = fw.h_status_dev = nullptr; fw.ready = false;
+    fw.d_b1 = fw.d_b2 = nullptr; fw.d_status = nullptr; fw.h_status = fw.h_status_dev = nullptr;
 }
 
 // Tensor map over n images [n][H][W] u8 (W a multiple of 16) at a device-accessible address (device memory or mapped
@@ -1055,7 +978,6 @@ inline int launch_fused_map(const FusedWeights& fw, cudaStream_t stream, const C
     P.done_flag = (n == 1 && !win && !tail) ? done_flag : nullptr;
     P.done_seq = done_seq;
     if (win && tail) return (int)cudaErrorInvalidValue;
-    if (tail && kEpiWarps != 4) return (int)cudaErrorNotSupported;       // the tail's warp layout assumes 4 epilogue warps
     if (!tail && !d_feats) return (int)cudaErrorInvalidValue;
     std::memset(&P.tail, 0, sizeof(P.tail));
     if (tail) P.tail = *tail;

@@ -41,17 +41,17 @@ struct HostChunkPlan {
     }
 };
 
-// in_sz: bytes per image; cap_images: most images a chunk may hold (workspace bound of the per-layer path); forced_mb / ramp:
-// the CNNACC_HOST_CHUNK_MB / CNNACC_HOST_RAMP overrides (0 / 2 by default)
-inline HostChunkPlan make_host_chunk_plan(int64_t n, size_t in_sz, int64_t cap_images, bool pipelined, size_t forced_mb, int ramp) {
+constexpr int kHostRampDepth = 2;   // ramp steps at each end of a synchronous call (see above)
+
+// in_sz: bytes per image; cap_images: most images a chunk may hold (workspace bound of the per-layer path)
+inline HostChunkPlan make_host_chunk_plan(int64_t n, size_t in_sz, int64_t cap_images, bool pipelined) {
     HostChunkPlan p;
     p.n = n;
     const size_t call_bytes = (size_t)n * in_sz;
     size_t chunk_bytes = std::min<size_t>((size_t)32 << 20, std::max<size_t>((size_t)4 << 20, call_bytes / 4));
     if (pipelined) chunk_bytes = std::min<size_t>((size_t)64 << 20, std::max<size_t>((size_t)4 << 20, call_bytes));
-    if (forced_mb) chunk_bytes = forced_mb << 20;
     p.full = std::min<int64_t>(n, std::max<int64_t>(1, std::min<int64_t>(cap_images, (int64_t)(chunk_bytes / in_sz))));
-    p.depth = (!pipelined && n >= 4 * p.full && (p.full >> ramp) >= 1) ? ramp : 0;
+    p.depth = (!pipelined && n >= 4 * p.full && (p.full >> kHostRampDepth) >= 1) ? kHostRampDepth : 0;
     p.tail_total = p.full - (p.full >> p.depth);
     return p;
 }

@@ -75,7 +75,8 @@ int64_t cnnacc_launch_count(const cnnacc_handle *h);
 /* ---- configuration -------------------------------------------------------------------------
  * load_weights: the one-off DMA of weights.bin into weight BRAM (pynq_inference.py:186-207,
  * realtime_detect.py:288-296); n must be 23184.  parse_kernels (arm_cnn.c:43-59) runs here once,
- * not per image (arm_cnn.c:186). */
+ * not per image (arm_cnn.c:186).  A load that fails after its argument checks leaves the handle
+ * without weights: calls that need them return -4 until a load succeeds. */
 int cnnacc_load_weights(cnnacc_handle *h, const uint8_t *weights_bin, size_t n);
 /* set_shifts: AXI reg 10 write, s0 | s1<<5 | s2<<10 (pynq_inference.py:226-229).  The hardware
  * masks with 0x1F; here values outside 0..31 are rejected with -2 (C >> by >=32 is undefined). */

@@ -1,4 +1,4 @@
-import os, sys, time
+import sys
 sys.path[:0] = ['.', 'tests']
 import numpy as np, torch
 import fpga_cnn_b200 as fc
@@ -16,7 +16,3 @@ for B in (4096, 16384, 65536):
     ms = acc.timer_stop()
     print(f"batch {B}: {nbuf} rotating buffers, {steps} steps: {ms/steps*1e3:.1f} us/step, {B*steps/ms/1e3:.3f} M img/s")
     del ins, outs
-for B in (4096,):
-    h_i = fc.alloc_host((B,128,128)); h_o = fc.alloc_host((B,64,16,16)); h_i[:] = 7
-    for mb in (4, 8, 16, 32):
-        os.environ['CNNACC_HOST_CHUNK_MB'] = str(mb)

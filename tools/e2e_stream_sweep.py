@@ -1,5 +1,4 @@
-"""Streaming host-buffer calls (run_batch_async / wait_batch): throughput against the number of batches in flight.
-The staging chunk size is CNNACC_HOST_CHUNK_MB (read once per process): run once per value, see tools/e2e_stream_sweep.sh."""
+"""Streaming host-buffer calls (run_batch_async / wait_batch): throughput against the number of batches in flight."""
 import os, sys, time, numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
@@ -23,7 +22,7 @@ def streamed(n, depth):
     while pend: a.wait_batch(pend.pop(0))
 sync_loop(3)
 t0 = time.perf_counter(); sync_loop(steps); dt = time.perf_counter() - t0
-res = [f"chunk_mb={os.environ.get('CNNACC_HOST_CHUNK_MB', 'auto')} batch={B}: synchronous {steps * B / dt / 1e6:.3f}"]
+res = [f"batch={B}: synchronous {steps * B / dt / 1e6:.3f}"]
 for depth in (2, 3, 4, 5):
     streamed(depth + 2, depth)
     t0 = time.perf_counter(); streamed(steps, depth); dt = time.perf_counter() - t0

@@ -1,8 +1,3 @@
 #!/bin/bash
 # usage: tools/e2e_stream_sweep.sh > gpurun_out/e2e_stream_sweep.txt
-for mb in auto 8 16 32 64; do
-  if [ $mb = auto ]; then timeout 120 python tools/e2e_stream_sweep.py 4096
-  else CNNACC_HOST_CHUNK_MB=$mb timeout 120 python tools/e2e_stream_sweep.py 4096; fi
-done
-timeout 120 python tools/e2e_stream_sweep.py 1024
-timeout 120 python tools/e2e_stream_sweep.py 16384
+for B in 1024 4096 16384; do timeout 120 python tools/e2e_stream_sweep.py $B; done

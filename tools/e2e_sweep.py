@@ -11,4 +11,4 @@ for _ in range(2): acc.run_batch(h_imgs, out=h_feats)
 t0 = time.perf_counter()
 for _ in range(20): acc.run_batch(h_imgs, out=h_feats)
 dt = (time.perf_counter() - t0) / 20
-print(os.environ.get('CNNACC_HOST_CHUNK_MB', 'default'), 'MB chunks:', f'{B/dt/1e6:.3f} M img/s', f'{2*B*16384/dt/1e9:.1f} GB/s both ways')
+print(f'batch {B}:', f'{B/dt/1e6:.3f} M img/s', f'{2*B*16384/dt/1e9:.1f} GB/s both ways')

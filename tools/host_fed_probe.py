@@ -19,7 +19,7 @@ for rep in range(2):
     t0 = time.perf_counter()
     for _ in range(3): acc.infer_batch(h)
     dt = time.perf_counter() - t0
-    print(f"infer_batch host-fed (CNNACC_HOST_CHUNK_MB={os.environ.get('CNNACC_HOST_CHUNK_MB', 'default')}): {3 * n / dt / 1e6:.2f} M img/s = {3 * n * 16384 / dt / 1e9:.1f} GB/s")
+    print(f"infer_batch host-fed: {3 * n / dt / 1e6:.2f} M img/s = {3 * n * 16384 / dt / 1e9:.1f} GB/s")
 t0 = time.perf_counter()
 for _ in range(3): acc.infer_batch(h, two_kernels=True)
 dt = time.perf_counter() - t0

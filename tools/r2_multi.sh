@@ -1,5 +1,5 @@
 #!/bin/bash
-# 8-GPU evidence of round 2 (run under `gpurun --gpus 8`): concurrent-copy ceiling, bench lines at N = 8 / 4 / 2, e2e chunk knobs.
+# 8-GPU evidence of round 2 (run on an 8-GPU machine): concurrent-copy ceiling, bench lines at N = 8 / 4 / 2.
 set -u
 OUT=gpurun_out; mkdir -p $OUT
 TR="python -m torch.distributed.run --nnodes=1 --master-addr 127.0.0.1"
@@ -14,12 +14,6 @@ import json,sys
 d=json.loads(open('$OUT/r2f_bench_n$n.json').read().strip().splitlines()[-1])
 print('N=$n value %.2fM e2e %.2fM (%.2f of raw ceiling %.2fM) stream_1m %.2fM host_fed %.2fM sustained %.2fM' % (d['value']/1e6, d['e2e']['value']/1e6, d['e2e']['frac_of_raw_copy_ceiling'], d['e2e']['raw_copy_ceiling_images_per_s']/1e6, d['stream_1m']['images_per_s']/1e6, d['stream_1m']['host_fed']['images_per_s']/1e6, d['sustained']['images_per_s']/1e6), d['stream_1m']['oracle_spot_check'])
 " 2>&1 | tail -2
-done
-for mb in 8 32; do
-  CNNACC_HOST_CHUNK_MB=$mb timeout 200 $TR --nproc-per-node 8 --master-port $((29640 + mb)) bench.py --gpus 8 --steps 30 --warmup 3 --quick --no-stream > $OUT/r2f_bench_n8_chunk$mb.json 2> $OUT/r2f_bench_n8_chunk$mb.err; echo "chunk $mb rc=$?"
-  python -c "
-import json
-d=json.loads(open('$OUT/r2f_bench_n8_chunk$mb.json').read().strip().splitlines()[-1]); print('chunk $mb MB: e2e %.2fM' % (d['e2e']['value']/1e6))" 2>&1 | tail -1
 done
 timeout 120 python bench.py --steps 50 --warmup 3 > $OUT/r2f_bench_n1_on8box.json 2> $OUT/r2f_bench_n1_on8box.err; echo "bench n1 rc=$?"
 ls -la $OUT | tail -12
