@@ -37,8 +37,50 @@ def _is_torch_cuda(x):
     return hasattr(x, "data_ptr") and getattr(x, "is_cuda", False)
 
 
+class _ArrayPtr(ctypes.c_void_p):
+    """c_void_p to a numpy array's data that holds the array: an argument tuple may keep the only reference to a copy that
+    np.ascontiguousarray made.  a.ctypes.data_as(c_void_p) holds it as well, but its ctypes.cast about doubles the cost of
+    a pointer, and every batch call builds several."""
+    __slots__ = ("_array",)
+
+
 def _vp(a):
-    return a.ctypes.data_as(ctypes.c_void_p)
+    p = _ArrayPtr(a.ctypes.data)
+    p._array = a
+    return p
+
+
+def _tp(t):
+    return ctypes.c_void_p(t.data_ptr())
+
+
+_NO_STREAM = contextlib.nullcontext()                # host-pointer calls run on the handle's own stream
+
+
+def _pred_flags(bbox, logits=False, direct=False, two_kernels=False):
+    if bbox not in ("vec", "upsampled"):
+        raise ValueError("bbox must be 'vec' (realtime_detect.bbox_vec) or 'upsampled' (Classifier.get_cam_bbox)")
+    return (_lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0) | (_lib.FLAG_LOGITS if logits else 0) | \
+        (_lib.FLAG_DIRECT if direct else 0) | (_lib.FLAG_TWO_KERNELS if two_kernels else 0)
+
+
+def _pred_outputs(new, n, n_cls):
+    """The (cls [n] i32, probs [n,n_cls] f32, bbox [n,4] i32) of a prediction call, allocated by new(shape, dtype)."""
+    return new((n,), np.int32), new((n, n_cls), np.float32), new((n, 4), np.int32)
+
+
+def _check_features_out(images, out):
+    """run_batch's `out`: C-contiguous uint8 of n*64*(H/8)*(W/8) elements, a numpy array for host images and a CUDA tensor
+    for CUDA images.  The library writes exactly that many bytes from out's first one."""
+    n, H, W = images.shape
+    size = n * 64 * (H // 8) * (W // 8)
+    if isinstance(images, np.ndarray):
+        ok = isinstance(out, np.ndarray) and out.dtype == np.uint8 and out.flags.c_contiguous and out.size == size
+    else:
+        ok = _is_torch_cuda(out) and out.dtype == images.dtype and out.is_contiguous() and out.numel() == size
+    if not ok:
+        raise ValueError("out must be a C-contiguous uint8 array of n*64*(H/8)*(W/8) elements, of the images' kind "
+                         "(numpy array or CUDA tensor)")
 
 
 def _item_bytes(x):
@@ -123,6 +165,25 @@ class CNNAccelerator:
             yield
         finally:
             self._check(self._libc.cnnacc_set_stream(self._h, ctypes.c_void_p(0)))
+
+    def _host_or_device(self, x, *more):
+        """How a call that takes host arrays or CUDA tensors passes `x` to the library -> (x, new, ptr, kind, ctx):
+        x C-contiguous uint8, new(shape, dtype) allocating outputs of x's kind on x's device, ptr(a) -> c_void_p, kind the
+        flag that says which (FLAG_DEVICE_PTRS or 0), and the context to call in (for tensors _on_stream_of(x, *more))."""
+        if not _is_torch_cuda(x):
+            return np.ascontiguousarray(x, dtype=np.uint8), np.empty, _vp, 0, _NO_STREAM
+        import torch
+        # the kernels read the tensor in place through 128-bit loads / TMA boxes: dtype and layout must be exact
+        if x.dtype != torch.uint8 or not x.is_contiguous():
+            raise ValueError("expected a contiguous CUDA uint8 tensor")
+        dev = x.device
+        new = lambda shape, dt: torch.empty(shape, dtype=getattr(torch, np.dtype(dt).name), device=dev)
+        return x, new, _tp, _lib.FLAG_DEVICE_PTRS, self._on_stream_of(x, *more)
+
+    def _classes(self):
+        if self._n_cls == 0:
+            raise RuntimeError("classifier not loaded")
+        return self._n_cls
 
     def synchronize(self):
         self._check(self._libc.cnnacc_synchronize(self._h))
@@ -231,27 +292,22 @@ class CNNAccelerator:
     # -- batch entry points -----------------------------------------------------------------------
     def run_batch(self, images, out=None, direct=False):
         """images [N,H,W] u8 (numpy, host) or a torch CUDA tensor -> features [N,64,H/8,W/8] u8 of the same kind."""
-        flags = _lib.FLAG_DIRECT if direct else 0
-        if _is_torch_cuda(images):
-            import torch
-            assert images.dtype == torch.uint8 and images.is_contiguous() and images.dim() == 3
-            n, H, W = images.shape
-            if out is None:
-                out = torch.empty((n, 64, H // 8, W // 8), dtype=torch.uint8, device=images.device)
-            elif not (_is_torch_cuda(out) and out.dtype == torch.uint8 and out.is_contiguous() and out.numel() == n * 64 * (H // 8) * (W // 8)):
-                raise ValueError("out must be a contiguous CUDA uint8 tensor of n*64*(H/8)*(W/8) elements")
-            with self._on_stream_of(images, out):
-                self._check(self._libc.cnnacc_run_batch(self._h, ctypes.c_void_p(images.data_ptr()), n, H, W,
-                                                        ctypes.c_void_p(out.data_ptr()), flags | _lib.FLAG_DEVICE_PTRS))
-            return out
-        images = np.ascontiguousarray(images, dtype=np.uint8)
+        c_args, out, ctx = self._run_batch_args(images, out, direct)
+        with ctx:
+            self._check(self._libc.cnnacc_run_batch(self._h, *c_args))
+        return out
+
+    def _run_batch_args(self, images, out, direct):
+        """run_batch's arguments checked -> (C arguments after the handle(s), features, context to call in)."""
+        images, new, ptr, kind, ctx = self._host_or_device(images, out)
         if images.ndim != 3:
             raise ValueError("images must be [N,H,W]")
         n, H, W = images.shape
         if out is None:
-            out = np.empty((n, 64, H // 8, W // 8), dtype=np.uint8)
-        self._check(self._libc.cnnacc_run_batch(self._h, _vp(images), n, H, W, _vp(out), flags))
-        return out
+            out = new((n, 64, H // 8, W // 8), np.uint8)
+        else:
+            _check_features_out(images, out)
+        return (ptr(images), n, H, W, ptr(out), kind | (_lib.FLAG_DIRECT if direct else 0)), out, ctx
 
     def run_batch_async(self, images, out=None):
         """Queue one HOST batch (images [N,H,W] u8, C-contiguous, ideally from alloc_host) and return a ticket at once;
@@ -262,8 +318,8 @@ class CNNAccelerator:
         n, H, W = images.shape
         if out is None:
             out = alloc_host((n, 64, H // 8, W // 8), np.uint8)
-        elif not (isinstance(out, np.ndarray) and out.dtype == np.uint8 and out.flags.c_contiguous and out.size == n * 64 * (H // 8) * (W // 8)):
-            raise ValueError("out must be a C-contiguous uint8 numpy array of n*64*(H/8)*(W/8) elements")
+        else:
+            _check_features_out(images, out)
         ticket = ctypes.c_int64(-1)
         self._check(self._libc.cnnacc_run_batch_async(self._h, _vp(images), n, H, W, _vp(out), 0, ctypes.byref(ticket)))
         self._pending[ticket.value] = (images, out)          # keep both alive while the copy engines use them
@@ -285,35 +341,21 @@ class CNNAccelerator:
         self._n_cls = fc_w.shape[0]
 
     def _predict(self, fn, x, direct=False, bbox="vec", logits=False, two_kernels=False):
-        if bbox not in ("vec", "upsampled"):
-            raise ValueError("bbox must be 'vec' (realtime_detect.bbox_vec) or 'upsampled' (Classifier.get_cam_bbox)")
-        flags = (_lib.FLAG_DIRECT if direct else 0) | (_lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0) | \
-                (_lib.FLAG_LOGITS if logits else 0) | (_lib.FLAG_TWO_KERNELS if two_kernels else 0)
-        if self._n_cls == 0:
-            raise RuntimeError("classifier not loaded")
-        if _is_torch_cuda(x):
-            import torch
-            # the kernels read each item through 128-bit loads / a TMA box: shape, dtype and layout must be exact
-            if x.dtype != torch.uint8 or not x.is_contiguous() or _item_bytes(x) != 16384:
-                raise ValueError("expected a contiguous CUDA uint8 tensor of [N,128,128] images or [N,64,256] features")
-            n = x.shape[0]
-            probs = torch.empty((n, self._n_cls), dtype=torch.float32, device=x.device)
-            cls = torch.empty((n,), dtype=torch.int32, device=x.device)
-            bbox = torch.empty((n, 4), dtype=torch.int32, device=x.device)
-            with self._on_stream_of(x):
-                self._check(fn(self._h, ctypes.c_void_p(x.data_ptr()), n, ctypes.c_void_p(probs.data_ptr()),
-                               ctypes.c_void_p(cls.data_ptr()), ctypes.c_void_p(bbox.data_ptr()),
-                               flags | _lib.FLAG_DEVICE_PTRS))
-            return cls, probs, bbox
-        x = np.ascontiguousarray(x, dtype=np.uint8)
+        c_args, res, ctx = self._predict_args(x, direct, bbox, logits, two_kernels)
+        with ctx:
+            self._check(fn(self._h, *c_args))
+        return res
+
+    def _predict_args(self, x, direct=False, bbox="vec", logits=False, two_kernels=False):
+        """A prediction call's arguments checked -> (C arguments after the handle(s), (cls, probs, bbox), context to call in)."""
+        flags = _pred_flags(bbox, logits, direct, two_kernels)
+        n_cls = self._classes()
+        x, new, ptr, kind, ctx = self._host_or_device(x)
         if _item_bytes(x) != 16384:
             raise ValueError("expected [N,128,128] images or [N,64,256] features")
         n = x.shape[0]
-        probs = np.empty((n, self._n_cls), dtype=np.float32)
-        cls = np.empty((n,), dtype=np.int32)
-        bbox = np.empty((n, 4), dtype=np.int32)
-        self._check(fn(self._h, _vp(x), n, _vp(probs), _vp(cls), _vp(bbox), flags))
-        return cls, probs, bbox
+        cls, probs, box = _pred_outputs(new, n, n_cls)
+        return (ptr(x), n, ptr(probs), ptr(cls), ptr(box), flags | kind), (cls, probs, box), ctx
 
     def classify_batch(self, features, bbox="vec", logits=False):
         """features [N,64,256] (or [N,64,16,16]) u8 -> (cls [N] i32, probs [N,n_cls] f32, bbox [N,4] i32).
@@ -334,13 +376,7 @@ class CNNAccelerator:
     def cam_bbox_batch(self, features, cls, return_cam=False):
         """Classifier.get_cam_bbox (pynq_inference.py:349-408) for given classes: features [N,64,256] u8 + cls [N] i32
         -> bbox [N,4] i32 (x1,y1,x2,y2), and with return_cam the upsampled maps [N,128,128] u8 (cam_full = maps/255)."""
-        if self._n_cls == 0:
-            raise RuntimeError("classifier not loaded")
-        x = np.ascontiguousarray(features, dtype=np.uint8)
-        cls = np.ascontiguousarray(cls, dtype=np.int32)
-        n = x.shape[0] if x.ndim else -1
-        if _item_bytes(x) != 16384 or cls.shape != (n,):
-            raise ValueError("expected [N,64,256] features and [N] classes")
+        x, cls, n = self._features_and_classes(features, cls)
         bbox = np.empty((n, 4), dtype=np.int32)
         cam = np.empty((n, 128, 128), dtype=np.uint8) if return_cam else None
         self._check(self._libc.cnnacc_cam_bbox_batch(self._h, _vp(x), n, _vp(cls), _vp(bbox), _vp(cam) if return_cam else None, 0))
@@ -348,16 +384,20 @@ class CNNAccelerator:
 
     def bbox_batch(self, features, cls):
         """bbox_vec for given classes: features [N,64,256] u8 + cls [N] i32 -> bbox [N,4] i32 (host arrays)."""
-        if self._n_cls == 0:
-            raise RuntimeError("classifier not loaded")
+        x, cls, n = self._features_and_classes(features, cls)
+        bbox = np.empty((n, 4), dtype=np.int32)
+        self._check(self._libc.cnnacc_classify_batch(self._h, _vp(x), n, None, _vp(cls), _vp(bbox), _lib.FLAG_CLS_GIVEN))
+        return bbox
+
+    def _features_and_classes(self, features, cls):
+        """The host inputs of cam_bbox_batch / bbox_batch checked -> (features, classes, N)."""
+        self._classes()
         x = np.ascontiguousarray(features, dtype=np.uint8)
         cls = np.ascontiguousarray(cls, dtype=np.int32)
         n = x.shape[0] if x.ndim else -1
         if _item_bytes(x) != 16384 or cls.shape != (n,):
             raise ValueError("expected [N,64,256] features and [N] classes")
-        bbox = np.empty((n, 4), dtype=np.int32)
-        self._check(self._libc.cnnacc_classify_batch(self._h, _vp(x), n, None, _vp(cls), _vp(bbox), _lib.FLAG_CLS_GIVEN))
-        return bbox
+        return x, cls, n
 
     def infer_batch(self, images, direct=False, bbox="vec", logits=False, two_kernels=False):
         """images [N,128,128] u8 -> (cls, probs, bbox).  The classifier / CAM-box tail runs inside the conv-stack kernel on
@@ -368,67 +408,48 @@ class CNNAccelerator:
     def preprocess(self, frames):
         """realtime_detect.py:582-591 for a batch: frames [N,h,w,3] u8 BGR -> [N,128,128] u8 (centre-crop, BGR2GRAY,
         INTER_AREA), bit-identical to cv2 4.13.  numpy in -> numpy out; torch CUDA tensor in -> torch CUDA tensor out."""
-        if _is_torch_cuda(frames):
-            import torch
-            if frames.dim() != 4 or frames.shape[3] != 3 or frames.dtype != torch.uint8 or not frames.is_contiguous():
-                raise ValueError("expected a contiguous [N,h,w,3] uint8 tensor")
-            n, fh, fw = frames.shape[:3]
-            out = torch.empty((n, 128, 128), dtype=torch.uint8, device=frames.device)
-            with self._on_stream_of(frames):
-                self._check(self._libc.cnnacc_preprocess_bgr(self._h, ctypes.c_void_p(frames.data_ptr()), n, fh, fw,
-                                                             ctypes.c_void_p(out.data_ptr()), _lib.FLAG_DEVICE_PTRS))
-            return out
-        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
         if frames.ndim != 4 or frames.shape[3] != 3:
             raise ValueError("expected [N,h,w,3] BGR frames")
         n, fh, fw = frames.shape[:3]
-        out = np.empty((n, 128, 128), dtype=np.uint8)
-        self._check(self._libc.cnnacc_preprocess_bgr(self._h, _vp(frames), n, fh, fw, _vp(out), 0))
+        out = new((n, 128, 128), np.uint8)
+        with ctx:
+            self._check(self._libc.cnnacc_preprocess_bgr(self._h, ptr(frames), n, fh, fw, ptr(out), kind))
         return out
 
     def image_to_gray128(self, images):
         """The arithmetic of pynq_inference.load_image_any (:414-425) for decoded images of one size: [N,H,W] (mode L),
         [N,H,W,3] (RGB) or [N,H,W,4] (RGBA) u8 -> [N,128,128] u8 = PIL convert('L').resize((128,128)), bit-identical to
         Pillow 12.2 (integer luma, default BICUBIC resampler).  numpy in -> numpy out; torch CUDA tensor in -> tensor out."""
-        if _is_torch_cuda(images):
-            import torch
-            if images.dtype != torch.uint8 or not images.is_contiguous() or images.dim() not in (3, 4):
-                raise ValueError("expected a contiguous uint8 tensor [N,H,W] or [N,H,W,C]")
-            n, H, W = images.shape[:3]
-            C = images.shape[3] if images.dim() == 4 else 1
-            out = torch.empty((n, 128, 128), dtype=torch.uint8, device=images.device)
-            with self._on_stream_of(images):
-                self._check(self._libc.cnnacc_image_to_gray128(self._h, ctypes.c_void_p(images.data_ptr()), n, H, W, C,
-                                                               ctypes.c_void_p(out.data_ptr()), _lib.FLAG_DEVICE_PTRS))
-            return out
-        images = np.ascontiguousarray(images, dtype=np.uint8)
+        images, new, ptr, kind, ctx = self._host_or_device(images)
         if images.ndim not in (3, 4):
             raise ValueError("expected [N,H,W] or [N,H,W,C] images")
         n, H, W = images.shape[:3]
         C = images.shape[3] if images.ndim == 4 else 1
-        out = np.empty((n, 128, 128), dtype=np.uint8)
-        self._check(self._libc.cnnacc_image_to_gray128(self._h, _vp(images), n, H, W, C, _vp(out), 0))
+        out = new((n, 128, 128), np.uint8)
+        with ctx:
+            self._check(self._libc.cnnacc_image_to_gray128(self._h, ptr(images), n, H, W, C, ptr(out), kind))
         return out
 
     def detect_frames(self, frames, bbox="vec", return_gray=False):
         """The loop body of realtime_detect.py:582-598 for a batch of camera frames [N,h,w,3] u8 BGR (host array):
         preprocess -> conv stack -> classify -> CAM box on the GPU.  -> (cls, probs, bbox[, gray128])."""
-        if bbox not in ("vec", "upsampled"):
-            raise ValueError("bbox must be 'vec' or 'upsampled'")
-        if self._n_cls == 0:
-            raise RuntimeError("classifier not loaded")
+        c_args, res = self._detect_frames_args(frames, bbox, return_gray)
+        self._check(self._libc.cnnacc_detect_frames(self._h, *c_args))
+        return res
+
+    def _detect_frames_args(self, frames, bbox, return_gray):
+        """detect_frames' arguments checked -> (C arguments after the handle(s), (cls, probs, bbox[, gray128]))."""
+        flags = _pred_flags(bbox)
+        n_cls = self._classes()
         frames = np.ascontiguousarray(frames, dtype=np.uint8)
         if frames.ndim != 4 or frames.shape[3] != 3:
             raise ValueError("expected [N,h,w,3] BGR frames")
         n, fh, fw = frames.shape[:3]
-        probs = np.empty((n, self._n_cls), dtype=np.float32)
-        cls = np.empty((n,), dtype=np.int32)
-        box = np.empty((n, 4), dtype=np.int32)
+        cls, probs, box = _pred_outputs(np.empty, n, n_cls)
         gray = np.empty((n, 128, 128), dtype=np.uint8) if return_gray else None
-        self._check(self._libc.cnnacc_detect_frames(self._h, _vp(frames), n, fh, fw, _vp(gray) if return_gray else None,
-                                                    _vp(probs), _vp(cls), _vp(box),
-                                                    _lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0))
-        return (cls, probs, box, gray) if return_gray else (cls, probs, box)
+        c_args = (_vp(frames), n, fh, fw, _vp(gray) if return_gray else None, _vp(probs), _vp(cls), _vp(box), flags)
+        return c_args, ((cls, probs, box, gray) if return_gray else (cls, probs, box))
 
     def detect_regions(self, frames, regions, bbox="vec", logits=False, return_gray=False):
         """detect_frames on caller-chosen square regions: frames [F,h,w,3] u8 BGR (numpy, or a contiguous CUDA uint8 tensor run
@@ -436,11 +457,8 @@ class CNNAccelerator:
         frame.  Region r's results are those detect_frames gives for frames[f][y:y+side, x:x+side] as a frame of its own; its
         box is in that square's 128x128 coordinates (region_boxes_to_frame maps it to frame pixels).
         -> (cls [R], probs [R,n_cls], bbox [R,4][, gray128 [R,128,128]]) in the order of `regions`, numpy or torch like frames."""
-        if bbox not in ("vec", "upsampled"):
-            raise ValueError("bbox must be 'vec' or 'upsampled'")
-        if self._n_cls == 0:
-            raise RuntimeError("classifier not loaded")
-        flags = (_lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0) | (_lib.FLAG_LOGITS if logits else 0)
+        flags = _pred_flags(bbox, logits)
+        self._classes()
         return self._regions(frames, regions, True, return_gray, flags)
 
     def preprocess_regions(self, frames, regions):
@@ -458,34 +476,18 @@ class CNNAccelerator:
         shuffled = bool((order != np.arange(len(order))).any())
         reg = np.ascontiguousarray(reg[order], dtype=np.int32)
         n = reg.shape[0]
-        nc = self._n_cls
-        if _is_torch_cuda(frames):
-            import torch
-            if frames.dim() != 4 or frames.shape[3] != 3 or frames.dtype != torch.uint8 or not frames.is_contiguous():
-                raise ValueError("expected a contiguous [F,h,w,3] uint8 tensor")
-            nf, fh, fw = frames.shape[:3]
-            new = lambda shape, dt: torch.empty(shape, dtype=dt, device=frames.device)
-            gray = new((n, 128, 128), torch.uint8) if want_gray else None
-            outs = (new((n,), torch.int32), new((n, nc), torch.float32), new((n, 4), torch.int32)) if detect else ()
-            ptr = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
-            with self._on_stream_of(frames):
-                self._call_regions(ptr(frames), nf, fh, fw, reg, ptr(gray), [ptr(t) for t in outs], detect,
-                                   flags | _lib.FLAG_DEVICE_PTRS)
-            res = outs + ((gray,) if want_gray else ())
-            if shuffled:
-                inv = torch.from_numpy(np.argsort(order)).to(frames.device)
-                res = tuple(t[inv] for t in res)
-            return res
-        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
         if frames.ndim != 4 or frames.shape[3] != 3:
             raise ValueError("expected [F,h,w,3] BGR frames")
         nf, fh, fw = frames.shape[:3]
-        gray = np.empty((n, 128, 128), dtype=np.uint8) if want_gray else None
-        outs = (np.empty((n,), np.int32), np.empty((n, nc), np.float32), np.empty((n, 4), np.int32)) if detect else ()
-        self._call_regions(_vp(frames), nf, fh, fw, reg, _vp(gray) if want_gray else None, [_vp(a) for a in outs], detect, flags)
+        gray = new((n, 128, 128), np.uint8) if want_gray else None
+        outs = _pred_outputs(new, n, self._n_cls) if detect else ()
+        with ctx:
+            self._call_regions(ptr(frames), nf, fh, fw, reg, ptr(gray) if want_gray else None, [ptr(a) for a in outs], detect,
+                               flags | kind)
         res = outs + ((gray,) if want_gray else ())
         if shuffled:
-            inv = np.argsort(order)
+            inv = np.argsort(order)                          # also indexes CUDA tensors: torch moves the index to their device
             res = tuple(a[inv] for a in res)
         return res
 
@@ -623,58 +625,23 @@ class MultiAccelerator:
     def run_batch(self, images, out=None, direct=False):
         """images [N,H,W] u8 (host) -> features [N,64,H/8,W/8] u8."""
         self._host_only(images)
-        images = np.ascontiguousarray(images, dtype=np.uint8)
-        if images.ndim != 3:
-            raise ValueError("images must be [N,H,W]")
-        n, H, W = images.shape
-        if out is None:
-            out = np.empty((n, 64, H // 8, W // 8), dtype=np.uint8)
-        elif not (isinstance(out, np.ndarray) and out.dtype == np.uint8 and out.flags.c_contiguous and out.size == n * 64 * (H // 8) * (W // 8)):
-            raise ValueError("out must be a C-contiguous uint8 numpy array of n*64*(H/8)*(W/8) elements")
-        self._call(self._libc.cnnacc_run_batch_sharded, _vp(images), n, H, W, _vp(out), _lib.FLAG_DIRECT if direct else 0)
+        c_args, out, _ = self.members[0]._run_batch_args(images, out, direct)
+        self._call(self._libc.cnnacc_run_batch_sharded, *c_args)
         return out
-
-    def _n_cls(self):
-        n_cls = self.members[0]._n_cls
-        if n_cls == 0:
-            raise RuntimeError("classifier not loaded")
-        return n_cls
 
     def infer_batch(self, images, direct=False, bbox="vec", logits=False, two_kernels=False):
         """images [N,128,128] u8 (host) -> (cls [N] i32, probs [N,n_cls] f32, bbox [N,4] i32)."""
         self._host_only(images)
-        if bbox not in ("vec", "upsampled"):
-            raise ValueError("bbox must be 'vec' (realtime_detect.bbox_vec) or 'upsampled' (Classifier.get_cam_bbox)")
-        flags = (_lib.FLAG_DIRECT if direct else 0) | (_lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0) | \
-                (_lib.FLAG_LOGITS if logits else 0) | (_lib.FLAG_TWO_KERNELS if two_kernels else 0)
-        n_cls = self._n_cls()
-        x = np.ascontiguousarray(images, dtype=np.uint8)
-        if _item_bytes(x) != 16384:
-            raise ValueError("expected [N,128,128] images")
-        n = x.shape[0]
-        probs = np.empty((n, n_cls), dtype=np.float32)
-        cls = np.empty((n,), dtype=np.int32)
-        box = np.empty((n, 4), dtype=np.int32)
-        self._call(self._libc.cnnacc_infer_batch_sharded, _vp(x), n, _vp(probs), _vp(cls), _vp(box), flags)
-        return cls, probs, box
+        c_args, res, _ = self.members[0]._predict_args(images, direct, bbox, logits, two_kernels)
+        self._call(self._libc.cnnacc_infer_batch_sharded, *c_args)
+        return res
 
     def detect_frames(self, frames, bbox="vec", return_gray=False):
         """Camera frames [N,h,w,3] u8 BGR (host) -> (cls, probs, bbox[, gray128]), as CNNAccelerator.detect_frames."""
         self._host_only(frames)
-        if bbox not in ("vec", "upsampled"):
-            raise ValueError("bbox must be 'vec' or 'upsampled'")
-        n_cls = self._n_cls()
-        frames = np.ascontiguousarray(frames, dtype=np.uint8)
-        if frames.ndim != 4 or frames.shape[3] != 3:
-            raise ValueError("expected [N,h,w,3] BGR frames")
-        n, fh, fw = frames.shape[:3]
-        probs = np.empty((n, n_cls), dtype=np.float32)
-        cls = np.empty((n,), dtype=np.int32)
-        box = np.empty((n, 4), dtype=np.int32)
-        gray = np.empty((n, 128, 128), dtype=np.uint8) if return_gray else None
-        self._call(self._libc.cnnacc_detect_frames_sharded, _vp(frames), n, fh, fw, _vp(gray) if return_gray else None,
-                   _vp(probs), _vp(cls), _vp(box), _lib.FLAG_BBOX_UPSAMPLED if bbox == "upsampled" else 0)
-        return (cls, probs, box, gray) if return_gray else (cls, probs, box)
+        c_args, res = self.members[0]._detect_frames_args(frames, bbox, return_gray)
+        self._call(self._libc.cnnacc_detect_frames_sharded, *c_args)
+        return res
 
 
 class B200Engine:
@@ -776,17 +743,20 @@ def dump_features(acc, images, labels, names, output, shifts=None):
     return feats
 
 
-_tail_acc = {}
+_module_acc = {}
 
 
-def _tail_accelerator(fc_w, fc_b, device=0):
-    key = (device, fc_w.shape, fc_w.tobytes(), fc_b.tobytes())
-    acc = _tail_acc.get("acc")
+def _module_accelerator(fc_w=None, fc_b=None):
+    """The CNNAccelerator on cuda:0 behind classify_vec, bbox_vec and load_image_any, created on first use.  Given fc_w and
+    fc_b it holds that classifier, loaded again only when they change."""
+    acc = _module_acc.get("acc")
     if acc is None:
-        acc = _tail_acc["acc"] = CNNAccelerator(device=device)
-    if _tail_acc.get("key") != key:
-        acc.load_classifier(fc_w, fc_b)
-        _tail_acc["key"] = key
+        acc = _module_acc["acc"] = CNNAccelerator()
+    if fc_w is not None:
+        key = (fc_w.shape, fc_w.tobytes(), fc_b.tobytes())
+        if _module_acc.get("key") != key:
+            acc.load_classifier(fc_w, fc_b)
+            _module_acc["key"] = key
     return acc
 
 
@@ -794,7 +764,7 @@ def classify_vec(feat_flat, fc_w, fc_b, names=NAMES):
     """realtime_detect.py:68-82 on the GPU: (64,256) u8 -> (idx, name, conf, probs)."""
     fc_w = np.ascontiguousarray(fc_w, dtype=np.float32)
     fc_b = np.ascontiguousarray(fc_b, dtype=np.float32)
-    acc = _tail_accelerator(fc_w, fc_b)
+    acc = _module_accelerator(fc_w, fc_b)
     cls, probs, _ = acc.classify_batch(np.asarray(feat_flat, dtype=np.uint8).reshape(1, 64, 256))
     i = int(cls[0])
     return i, names[i], float(probs[0, i]), probs[0]
@@ -804,13 +774,10 @@ def bbox_vec(feat_flat, cls_idx, fc_w, fc_b=None):
     """realtime_detect.py:85-116 on the GPU: bbox of the CAM of class cls_idx."""
     fc_w = np.ascontiguousarray(fc_w, dtype=np.float32)
     fc_b = np.zeros(fc_w.shape[0], np.float32) if fc_b is None else np.ascontiguousarray(fc_b, dtype=np.float32)
-    acc = _tail_accelerator(fc_w, fc_b)
+    acc = _module_accelerator(fc_w, fc_b)
     feats = np.ascontiguousarray(feat_flat, dtype=np.uint8).reshape(1, 64, 256)
     bbox = acc.bbox_batch(feats, np.array([cls_idx], dtype=np.int32))
     return tuple(int(v) for v in bbox[0])
-
-
-_loader_acc = {}
 
 
 def load_image_any(image_path, acc=None):
@@ -829,9 +796,7 @@ def load_image_any(image_path, acc=None):
         img = img.convert("L")
     arr = np.asarray(img, dtype=np.uint8)
     if acc is None:
-        acc = _loader_acc.get("acc")
-        if acc is None:
-            acc = _loader_acc["acc"] = CNNAccelerator()
+        acc = _module_accelerator()
     return acc.image_to_gray128(arr[None]).reshape(-1)
 
 

@@ -198,6 +198,12 @@ def test_error_conventions(fc, shipped_weights):
         a.set_shifts(2, 4, 32)
     with pytest.raises(ValueError):
         a.run_batch(np.zeros((1, 100, 128), np.uint8))
+    n0 = a.launch_count
+    for out in (np.zeros(2 * 16384, np.float32),                 # the right element count, of the wrong dtype
+                np.zeros(4 * 16384, np.uint8)[::2]):             # a strided view over a buffer large enough for 2*16384
+        with pytest.raises(ValueError):
+            a.run_batch(np.zeros((2, 128, 128), np.uint8), out=out)
+    assert a.launch_count == n0
     with pytest.raises(RuntimeError):
         a.start_inference()                                      # no image loaded
     assert a.run_batch(np.zeros((0, 128, 128), np.uint8)).shape == (0, 64, 16, 16)   # empty batch
@@ -214,6 +220,10 @@ def test_device_pointer_path_with_torch(fc, shipped_weights, conv_golden):
     out = a.run_batch(imgs)
     torch.cuda.synchronize()
     assert np.array_equal(out.cpu().numpy().reshape(8, 64, 256), conv_golden["rng_shipped_mid"])
+    n0 = a.launch_count
+    with pytest.raises(ValueError):
+        a.run_batch(imgs.float())
+    assert a.launch_count == n0
     a.close()
 
 
