@@ -66,7 +66,8 @@ def pack_weights(kernels):
 
 
 def make_weights(kind, shipped=None):
-    """kind: 'shipped' | 'identity' | ('rng', seed) | ('const', byte) | ('sparse', seed) | ('acc24', seed) | 'acc24_extreme'."""
+    """kind: 'shipped' | 'identity' | ('rng', seed) | ('const', byte) | ('sparse', seed) | ('acc24', seed) | 'acc24_extreme' |
+    ('ternary', seed)."""
     if kind == "shipped":
         assert shipped is not None and shipped.size == NUM_WEIGHT_BYTES
         return np.array(shipped, dtype=np.uint8)
@@ -78,6 +79,9 @@ def make_weights(kind, shipped=None):
         k2 = np.where((np.arange(64) % 2 == 0)[:, None, None, None], 127, -127) * np.ones((64, 32, 3, 3), dtype=np.int64)
         return pack_weights([np.full((16, 1, 3, 3), 127), np.full((32, 16, 3, 3), 127), k2])
     tag, arg = kind
+    if tag == "ternary":                        # weights in {-1, 0, 1}: with shifts near (1,3,3) every layer's sums straddle 2^shift
+        rng = np.random.default_rng(arg)
+        return pack_weights([rng.integers(-1, 2, s) for s in ((16, 1, 3, 3), (32, 16, 3, 3), (64, 32, 3, 3))])
     if tag == "acc24":                          # large same-sign layer-2 kernels on near-saturated inputs: sums straddle 2^23
         rng = np.random.default_rng(arg)
         k0 = rng.integers(64, 128, (16, 1, 3, 3))
@@ -140,6 +144,58 @@ HW_CASES = [
     dict(name="hw_64x32", weights=("rng", 21), images=("rng", 22), H=64, W=32, shifts=(9, 12, 13)),
     dict(name="hw_512x512", weights="shipped", images=("smooth", 23), H=512, W=512, shifts=(6, 9, 10)),
 ]
+
+
+# Workloads on which a one-LSB error shows.  Every layer ends in >> shift and a clip to 0..255, so an accumulator that is off
+# by one changes an output byte only when its sum sits next to a multiple of 2^shift and its byte is not clipped: with the
+# shipped weights at shifts (7,10,11) a +1 on every layer-2 accumulator changes about one final byte in 10 000.  Weights in
+# {-1, 0, 1} at shifts near (1,3,3) keep 30-70 % of every layer's bytes strictly inside (0, 255) and let such a +1 change
+# 3-25 % of the final bytes; tests/test_exposure_cpu.py measures both with the numpy oracle and holds every entry to them.
+# images: (kind, count) pieces in order; more: the kind that workload_images() draws further images (or other sizes) from.
+# acc24_wrap runs with 24-bit accumulators and is built to wrap, not to expose one LSB: a wrapped layer-2 sum is at least
+# 2^24 - 9.4 M = 7.4 M away from zero, so only shifts of 15 and up give bytes inside (0, 255), and a +1 crosses a multiple of
+# 2^15 once in 32 768 sums.  Its test is that the wraps happen and move many final bytes.
+EXPOSED_WORKLOADS = [
+    dict(name="tern_rng", weights=("ternary", 1), shifts=(1, 3, 3), images=[(("rng", 5), 32)], more=("rng", 105)),
+    dict(name="tern_smooth", weights=("ternary", 2), shifts=(1, 3, 4), images=[(("smooth", 6), 32)], more=("smooth", 106)),
+    dict(name="tern_tb", weights=("ternary", 3), shifts=(1, 3, 3), images=[("tb", 1), (("smooth", 7), 31)], more=("rng", 107)),
+    dict(name="acc24_wrap", weights=("acc24", 31), shifts=(0, 14, 15), images=[(("bright", 32), 16)], more=("bright", 132),
+         acc_bits=24),
+]
+
+
+def shift_triple_draws(trials=8):
+    """Seeded random shift triples, each with its own ternary weights and image kind (smooth for every third trial, else
+    uniform): shifts drawn from the ranges where those weights' sums reach 2^shift at every layer, so that each draw keeps
+    its bytes informative (tests/test_exposure_cpu.py holds every draw to the EXPOSED_WORKLOADS criteria).
+    -> [(name, weights kind, shifts, images kind)]."""
+    rng = np.random.default_rng(77)
+    out = []
+    for t in range(trials):
+        sh = (int(rng.integers(1, 3)), int(rng.integers(3, 5)), int(rng.integers(3, 5)))
+        out.append((f"triple{t}", ("ternary", 500 + t), sh, ("smooth", 600 + t) if t % 3 == 0 else ("rng", 600 + t)))
+    return out
+
+
+def all_zero_triples(trials=4):
+    """Seeded shift triples of 24..31 at every layer with full-range weights: no sum reaches 2^24 (32*9*255*128 = 9.4 M), so
+    every byte of every layer is 0.  -> [(weights kind, shifts, images kind)]."""
+    rng = np.random.default_rng(78)
+    return [(("rng", 520 + t) if t % 2 else ("const", 0x7F), tuple(int(v) for v in rng.integers(24, 32, 3)),
+             ("rng", 620 + t) if t % 2 else ("const", 255)) for t in range(trials)]
+
+
+def workload_images(w, n=None, H=128, W=128):
+    """The images of an EXPOSED_WORKLOADS entry: its own pieces for n = None; the first n of them, followed by further images
+    of kind w["more"] (drawn 512 at a time) when n is larger; at any other size n images of kind w["more"]."""
+    if (H, W) != (128, 128):
+        return make_images(w["more"], n, H, W)
+    own = np.concatenate([make_images(kind, k) for kind, k in w["images"]])
+    if n is None or n <= len(own):
+        return own[:n]
+    tag, seed = w["more"]
+    extra = [make_images((tag, seed * 1000 + b), min(512, n - len(own) - 512 * b)) for b in range(-(-(n - len(own)) // 512))]
+    return np.concatenate([own] + extra)
 
 
 def make_features(kind, n):
