@@ -69,6 +69,46 @@ def _pred_outputs(new, n, n_cls):
     return new((n,), np.int32), new((n, n_cls), np.float32), new((n, 4), np.int32)
 
 
+def _grouped_regions(regions):
+    """An (R, 4) integer array of (frame, x, y, side) in any order -> (the regions as int32 grouped by frame, stably, as the
+    library takes them; the caller's index of each, or None when they were grouped already)."""
+    reg = np.asarray(regions)
+    if reg.ndim != 2 or reg.shape[1] != 4 or not (reg.size == 0 or np.issubdtype(reg.dtype, np.integer)):
+        raise ValueError("regions must be an (R, 4) integer array of (frame, x, y, side)")
+    reg = reg.astype(np.int64)
+    if reg.size and (reg.min() < -2 ** 31 or reg.max() >= 2 ** 31):
+        raise ValueError("region values must fit int32")
+    order = np.argsort(reg[:, 0], kind="stable")
+    shuffled = bool((order != np.arange(len(order))).any())
+    return np.ascontiguousarray(reg[order], dtype=np.int32), (order.astype(np.int32) if shuffled else None)
+
+
+def _merge_flags(max_det, class_agnostic):
+    if not 1 <= int(max_det) <= _lib.MERGE_MAX_DET:
+        raise ValueError(f"max_det must be 1..{_lib.MERGE_MAX_DET}")
+    return _lib.FLAG_CLASS_AGNOSTIC if class_agnostic else 0
+
+
+def _det_outputs(new, n_frames, max_det):
+    """The (n_det [F] i32, region [F,D] i32, cls [F,D] i32, score [F,D] f32, box [F,D,4] f32) of a merging call."""
+    return (new((n_frames,), np.int32), new((n_frames, max_det), np.int32), new((n_frames, max_det), np.int32),
+            new((n_frames, max_det), np.float32), new((n_frames, max_det, 4), np.float32))
+
+
+def _callers_regions(dets, order):
+    """The detections with det_region mapped from the library's (grouped) region index back to the caller's."""
+    if order is None:
+        return dets
+    region = dets[1]
+    if isinstance(region, np.ndarray):
+        region = np.where(region >= 0, order[np.maximum(region, 0)], region).astype(np.int32)
+    else:
+        import torch
+        idx = torch.from_numpy(order).to(region.device)
+        region = torch.where(region >= 0, idx[region.clamp(min=0).long()], region)
+    return (dets[0], region) + tuple(dets[2:])
+
+
 def _check_features_out(images, out):
     """run_batch's `out`: C-contiguous uint8 of n*64*(H/8)*(W/8) elements, a numpy array for host images and a CUDA tensor
     for CUDA images.  The library writes exactly that many bytes from out's first one."""
@@ -466,15 +506,7 @@ class CNNAccelerator:
         return self._regions(frames, regions, False, True, 0)[0]
 
     def _regions(self, frames, regions, detect, want_gray, flags):
-        reg = np.asarray(regions)
-        if reg.ndim != 2 or reg.shape[1] != 4 or not (reg.size == 0 or np.issubdtype(reg.dtype, np.integer)):
-            raise ValueError("regions must be an (R, 4) integer array of (frame, x, y, side)")
-        reg = reg.astype(np.int64)
-        if reg.size and (reg.min() < -2 ** 31 or reg.max() >= 2 ** 31):
-            raise ValueError("region values must fit int32")
-        order = np.argsort(reg[:, 0], kind="stable")         # the library takes regions grouped by frame
-        shuffled = bool((order != np.arange(len(order))).any())
-        reg = np.ascontiguousarray(reg[order], dtype=np.int32)
+        reg, order = _grouped_regions(regions)              # the library takes regions grouped by frame
         n = reg.shape[0]
         frames, new, ptr, kind, ctx = self._host_or_device(frames)
         if frames.ndim != 4 or frames.shape[3] != 3:
@@ -486,7 +518,7 @@ class CNNAccelerator:
             self._call_regions(ptr(frames), nf, fh, fw, reg, ptr(gray) if want_gray else None, [ptr(a) for a in outs], detect,
                                flags | kind)
         res = outs + ((gray,) if want_gray else ())
-        if shuffled:
+        if order is not None:
             inv = np.argsort(order)                          # also indexes CUDA tensors: torch moves the index to their device
             res = tuple(a[inv] for a in res)
         return res
@@ -498,6 +530,65 @@ class CNNAccelerator:
                                                          probs_p, cls_p, box_p, flags))
         else:
             self._check(self._libc.cnnacc_preprocess_regions(self._h, frames_p, nf, fh, fw, _vp(reg), reg.shape[0], gray_p, flags))
+
+    def detect_objects(self, frames, regions, score_min=0.0, iou_max=0.5, max_det=100, class_agnostic=False, bbox="vec",
+                       logits=False):
+        """detect_regions followed by per-frame greedy NMS on the GPU (include/cnnacc.h, csrc/region_merge.h): a region is a
+        candidate when its score -- the probability of its class, or the logit with logits=True -- is >= score_min; candidates
+        are kept by score descending (ties: lower region index first) unless a kept box of the same class (any class with
+        class_agnostic) has IoU > iou_max with it, at most max_det per frame.  The per-region predictions never leave the GPU.
+        frames / regions as for detect_regions (numpy or a CUDA tensor on torch's current stream; regions in any order).
+        -> (n_det [F] i32, region [F,max_det] i32 index into `regions`, cls [F,max_det] i32, score [F,max_det] f32,
+        box [F,max_det,4] f32 frame pixels), rows past n_det[f] hold -1 / -1 / 0 / 0; numpy or torch like frames."""
+        flags = _pred_flags(bbox, logits) | _merge_flags(max_det, class_agnostic)
+        self._classes()
+        reg, order = _grouped_regions(regions)
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
+        if frames.ndim != 4 or frames.shape[3] != 3:
+            raise ValueError("expected [F,h,w,3] BGR frames")
+        nf, fh, fw = frames.shape[:3]
+        dets = _det_outputs(new, nf, int(max_det))
+        with ctx:
+            self._check(self._libc.cnnacc_detect_objects(self._h, ptr(frames), nf, fh, fw, _vp(reg), reg.shape[0], float(score_min),
+                                                         float(iou_max), int(max_det), *[ptr(a) for a in dets], flags | kind))
+        return _callers_regions(dets, order)
+
+    def merge_regions(self, regions, cls, scores, bbox, n_frames, score_min=0.0, iou_max=0.5, max_det=100, class_agnostic=False):
+        """The merge of detect_objects alone, on predictions the caller already has: regions (R,4) (frame, x, y, side) in any
+        order, cls [R] i32, scores [R] f32, bbox [R,4] i32 on each region's 128 grid, as numpy arrays or CUDA tensors (scores
+        decides which; tensors run on torch's current stream).  Needs no weights or classifier.  -> as detect_objects."""
+        if int(n_frames) < 0:
+            raise ValueError("n_frames must be >= 0")
+        flags = _merge_flags(max_det, class_agnostic)
+        reg, order = _grouped_regions(regions)
+        n = reg.shape[0]
+        if _is_torch_cuda(scores):
+            import torch
+            idx = None if order is None else torch.from_numpy(order.astype(np.int64)).to(scores.device)
+
+            def arg(t, dtype, shape):
+                if not _is_torch_cuda(t) or tuple(t.shape) != shape:
+                    raise ValueError(f"expected a CUDA tensor of shape {shape}")
+                t = t.to(dtype=dtype)
+                return (t if idx is None else t[idx]).contiguous()
+            scores, cls, bbox = arg(scores, torch.float32, (n,)), arg(cls, torch.int32, (n,)), arg(bbox, torch.int32, (n, 4))
+            dev = scores.device
+            new = lambda shape, dt: torch.empty(shape, dtype=getattr(torch, np.dtype(dt).name), device=dev)
+            ptr, kind, ctx = _tp, _lib.FLAG_DEVICE_PTRS, self._on_stream_of(scores, cls, bbox)
+        else:
+            def arg(a, dtype, shape):
+                a = np.asarray(a, dtype=dtype)
+                if a.shape != shape:
+                    raise ValueError(f"expected an array of shape {shape}")
+                return np.ascontiguousarray(a if order is None else a[order])
+            scores, cls, bbox = arg(scores, np.float32, (n,)), arg(cls, np.int32, (n,)), arg(bbox, np.int32, (n, 4))
+            new, ptr, kind, ctx = np.empty, _vp, 0, _NO_STREAM
+        dets = _det_outputs(new, int(n_frames), int(max_det))
+        with ctx:
+            self._check(self._libc.cnnacc_merge_regions(self._h, _vp(reg), n, int(n_frames), ptr(scores), ptr(cls), ptr(bbox),
+                                                        float(score_min), float(iou_max), int(max_det), *[ptr(a) for a in dets],
+                                                        flags | kind))
+        return _callers_regions(dets, order)
 
     def infer_one(self, gray128):
         """One image, lowest latency.  -> (feat (64,256) u8, conv_ms, read_ms)."""
@@ -546,8 +637,9 @@ def grid_regions(n_frames, fh, fw, sides, strides):
 
 def region_boxes_to_frame(regions, bbox):
     """Boxes of detect_regions (x1, y1, x2, y2 on the region's 128x128 grid) in frame pixels: x + b * side / 128 for x1 and
-    x2, y + b * side / 128 for y1 and y2, as float64.  This is the one mapping the library documents; it merges nothing
-    (no NMS).  -> (R, 4) float64."""
+    x2, y + b * side / 128 for y1 and y2, as float64, exact.  Its float32 cast equals, bit for bit, the boxes
+    CNNAccelerator.detect_objects / merge_regions return for boxes inside the 128 grid (those calls clamp to [0, 127] and
+    merge the regions of each frame by greedy NMS; this function only maps).  -> (R, 4) float64."""
     reg = np.asarray(regions, dtype=np.float64).reshape(-1, 4)
     b = np.asarray(bbox, dtype=np.float64).reshape(-1, 4)
     scale = reg[:, 3:4] / 128.0

@@ -21,6 +21,7 @@
 #include "preprocess.cuh"
 #include "regions.cuh"
 #include "region_plan.h"
+#include "region_merge.cuh"
 #include "pil_resize.cuh"
 #include "host_chunks.h"
 #include "pdl_chain.h"
@@ -40,10 +41,13 @@ constexpr size_t kBramBytes = 16 * 4096 + 32 * 1024 + 64 * 256;   // 112-channel
 constexpr int64_t kRegionLaunch = 1024;         // host-pointer region calls: regions per launch (16 MiB of gray per slot)
 constexpr int kDescRing = 4;                    // region-descriptor buffers in flight
 
-// Pinned host and device copies of one call's region descriptors; ev is recorded after the call's last launch that reads them.
+// Pinned host and device copies of one call's region descriptors (and, for the merging calls, of its per-frame region
+// ranges); ev is recorded after the call's last launch that reads them.
 struct DescBuf {
     int4 *host = nullptr, *dev = nullptr;
     size_t cap = 0;
+    long long *first_host = nullptr, *first_dev = nullptr;
+    size_t cap_first = 0;
     cudaEvent_t ev = nullptr;
 };
 
@@ -83,6 +87,11 @@ struct cnnacc_handle {
     int *d_prep_start = nullptr, *d_prep_cnt = nullptr; float* d_prep_alpha = nullptr; size_t cap_prep_alpha = 0;
     uint8_t* d_gray = nullptr; size_t cap_gray = 0;
     DescBuf rdesc[kDescRing]; int rdesc_next = 0;   // region calls (regions_impl)
+    // merging calls (region_merge.cuh): device predictions of detect_objects' device-pointer path, and the detections of
+    // host-pointer merges on the device and in pinned memory
+    uint8_t* d_mpred = nullptr; size_t cap_mpred = 0;
+    uint8_t *d_det = nullptr, *h_det = nullptr; size_t cap_det = 0;
+    bool merge_attr_set = false;
     // load_image_any (pil_resize.cuh): Pillow coefficient tables of the last (H, W) seen, on the device
     int pil_h = 0, pil_w = 0, pil_kh = 0, pil_kw = 0;
     int32_t *d_pil_kx = nullptr, *d_pil_bx = nullptr, *d_pil_ky = nullptr, *d_pil_by = nullptr;
@@ -623,9 +632,10 @@ int cnnacc_destroy(cnnacc_handle* h) {
     for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) if (st) cudaStreamDestroy(st);
     for (auto ev : h->ev_ticket) if (ev) cudaEventDestroy(ev);
     for (auto& b : h->rdesc) {
-        cudaFreeHost(b.host); cudaFree(b.dev);
+        cudaFreeHost(b.host); cudaFree(b.dev); cudaFreeHost(b.first_host); cudaFree(b.first_dev);
         if (b.ev) cudaEventDestroy(b.ev);
     }
+    cudaFree(h->d_mpred); cudaFree(h->d_det); cudaFreeHost(h->h_det);
     cudaFree(h->d_prep_start); cudaFree(h->d_prep_cnt); cudaFree(h->d_prep_alpha); cudaFree(h->d_gray);
     cudaFree(h->d_pil_kx); cudaFree(h->d_pil_bx); cudaFree(h->d_pil_ky); cudaFree(h->d_pil_by);
     cudaFree(h->d_pil_tmp); cudaFree(h->d_pil_in); cudaFree(h->d_pil_out);
@@ -1134,9 +1144,10 @@ static int prep_then_tail(cnnacc_handle* h, cudaStream_t st, const RegionPrep& b
     return 0;
 }
 
-// The next entry of the descriptor ring, with room for n descriptors.  Its previous user -- kDescRing calls ago, possibly an
-// asynchronous device-pointer call on any stream -- recorded the entry's event after its last launch that reads it.
-static int desc_acquire(cnnacc_handle* h, int64_t n, DescBuf** out) {
+// The next entry of the descriptor ring, with room for n descriptors and n_first frame-range entries.  Its previous user --
+// kDescRing calls ago, possibly an asynchronous device-pointer call on any stream -- recorded the entry's event after its last
+// launch that reads it.
+static int desc_acquire(cnnacc_handle* h, int64_t n, DescBuf** out, int64_t n_first = 0) {
     DescBuf& b = h->rdesc[h->rdesc_next];
     h->rdesc_next = (h->rdesc_next + 1) % kDescRing;
     CU(h, cudaEventSynchronize(b.ev));                   // an event never recorded counts as complete
@@ -1147,15 +1158,160 @@ static int desc_acquire(cnnacc_handle* h, int64_t n, DescBuf** out) {
         CU(h, cudaMalloc(&b.dev, (size_t)n * sizeof(int4)));
         b.cap = (size_t)n;
     }
+    if ((int64_t)b.cap_first < n_first) {
+        cudaFreeHost(b.first_host); cudaFree(b.first_dev);
+        b.first_host = nullptr; b.first_dev = nullptr; b.cap_first = 0;
+        CU(h, cudaHostAlloc(&b.first_host, (size_t)n_first * sizeof(long long), cudaHostAllocDefault));
+        CU(h, cudaMalloc(&b.first_dev, (size_t)n_first * sizeof(long long)));
+        b.cap_first = (size_t)n_first;
+    }
     *out = &b;
     return 0;
 }
 
+// ---- merging region detections into per-frame detections (region_merge.h / region_merge.cuh) -----------------------------
+
+// The merge of one call: its arguments, the caller's five outputs (rows of frame 0) and the per-frame region ranges.
+struct MergeSpec {
+    float score_min = 0.f, iou_max = 0.f;
+    int max_det = 1;
+    bool agnostic = false;
+    int32_t *n_det = nullptr, *det_region = nullptr, *det_cls = nullptr;
+    float *det_score = nullptr, *det_box = nullptr;
+    std::vector<int64_t> first;                 // [n_frames + 1]: frame f holds regions first[f] .. first[f+1]-1
+};
+
+// Checks shared by cnnacc_detect_objects and the cnnacc_merge_regions calls once the regions themselves passed their checks:
+// the merge limits, n_det, and at most kMergeMaxPerFrame regions per frame.  Fills M.first.  "" or why not.
+static std::string merge_error(const int32_t* regions, int64_t n, int64_t n_frames, MergeSpec& M) {
+    if (!M.n_det) return "NULL n_det";
+    if (const char* why = merge_limits_error(M.iou_max, M.max_det)) return why;
+    if (n > 0x7fffffffLL) return "more than 2^31-1 regions in one merging call";
+    int64_t most, bad;
+    if (const char* why = merge_frame_ranges([&](int64_t r) -> int64_t { return regions[4 * r]; }, n, n_frames, M.first, &most, &bad))
+        return "frame " + std::to_string(bad) + ": " + why;
+    return "";
+}
+static int merge_check(cnnacc_handle* h, const int32_t* regions, int64_t n, int64_t n_frames, MergeSpec& M) {
+    const std::string why = merge_error(regions, n, n_frames, M);
+    return why.empty() ? 0 : fail(h, CNNACC_ERR_ARG, why);
+}
+
+// The arguments of cnnacc_merge_regions / cnnacc_merge_regions_host: "" or why not.  There is no frame size, so a region's
+// frame, position and side are checked, not that it lies inside its frame.
+static std::string merge_call_error(const int32_t* regions, int64_t n, int64_t n_frames, const float* scores, const int32_t* cls,
+                                    const int32_t* bbox, MergeSpec& M) {
+    if (n < 0 || n_frames < 0) return "negative n_frames / n_regions";
+    if (n > 0 && (!regions || !scores || !cls || !bbox)) return "NULL region / score / class / box pointer";
+    for (int64_t r = 0; r < n; r++) {
+        const int64_t f = regions[4 * r], x = regions[4 * r + 1], y = regions[4 * r + 2], side = regions[4 * r + 3];
+        const std::string at = "region " + std::to_string(r) + ": ";
+        if (f < 0 || f >= n_frames) return at + "frame index outside [0, n_frames)";
+        if (side < kRegionMinSide || side > kRegionMaxSide) return at + "side outside 128..8192";
+        if (x < 0 || y < 0) return at + "negative position";
+        if (r > 0 && f < regions[4 * (r - 1)]) return at + "frame indices decrease (group the regions by frame, in non-decreasing order)";
+    }
+    return merge_error(regions, n, n_frames, M);
+}
+
+static MergeSpec make_merge_spec(float score_min, float iou_max, int max_det, int32_t* n_det, int32_t* det_region, int32_t* det_cls,
+                          float* det_score, float* det_box, uint32_t flags) {
+    MergeSpec M;
+    M.score_min = score_min; M.iou_max = iou_max; M.max_det = max_det;
+    M.agnostic = (flags & CNNACC_FLAG_CLASS_AGNOSTIC) != 0;
+    M.n_det = n_det; M.det_region = det_region; M.det_cls = det_cls; M.det_score = det_score; M.det_box = det_box;
+    return M;
+}
+
+// Merge frames [fa, fb) on `st`: A carries the region data (desc, predictions) and the outputs of frame fa; d_first is the
+// device copy of M.first.  The shared memory follows the largest frame of the launch.
+static int launch_merge(cnnacc_handle* h, cudaStream_t st, MergeArgs A, const MergeSpec& M, const long long* d_first,
+                        int64_t fa, int64_t fb) {
+    if (!h->merge_attr_set) {
+        CU(h, cudaFuncSetAttribute(merge_regions_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)merge_smem_bytes(kMergeMaxPerFrame, kMergeMaxDet)));
+        h->merge_attr_set = true;
+    }
+    A.score_min = M.score_min; A.iou_max = M.iou_max; A.max_det = M.max_det; A.agnostic = M.agnostic ? 1 : 0;
+    constexpr int64_t kFramesPerLaunch = 1 << 20;
+    for (int64_t g0 = fa; g0 < fb; g0 += kFramesPerLaunch) {
+        const int64_t g1 = std::min(fb, g0 + kFramesPerLaunch);
+        int64_t most = 0;
+        for (int64_t f = g0; f < g1; f++) most = std::max(most, M.first[f + 1] - M.first[f]);
+        int cap = 1;
+        while (cap < most) cap <<= 1;
+        MergeArgs L = A;
+        const size_t o = (size_t)(g0 - fa) * M.max_det;
+        L.first = d_first + g0;
+        L.key_cap = cap; L.kept_cap = std::min(M.max_det, cap);
+        L.n_det = A.n_det + (g0 - fa);
+        L.det_region = A.det_region ? A.det_region + o : nullptr;
+        L.det_cls = A.det_cls ? A.det_cls + o : nullptr;
+        L.det_score = A.det_score ? A.det_score + o : nullptr;
+        L.det_box = A.det_box ? A.det_box + o : nullptr;
+        merge_regions_kernel<<<(unsigned)(g1 - g0), kMergeThreads, merge_smem_bytes(L.key_cap, L.kept_cap), st>>>(L);
+        h->launches++;
+        CU(h, cudaGetLastError());
+    }
+    return 0;
+}
+
+// Merge frames [fa, fb) of a host-pointer call into the caller's host arrays: the kernel writes a group of frames into h->d_det
+// as [box | region | cls | score | n_det], one D2H brings it to the pinned h->h_det, memcpy to the caller.  Waits for st.
+static int merge_to_host(cnnacc_handle* h, cudaStream_t st, MergeArgs A, const MergeSpec& M, const long long* d_first,
+                         int64_t fa, int64_t fb) {
+    const size_t D = (size_t)M.max_det, per_frame = 4 + D * 28;
+    const int64_t step = std::max<int64_t>(1, std::min<int64_t>(fb - fa, ((size_t)8 << 20) / per_frame));
+    const size_t need = (size_t)step * per_frame;
+    if (need > h->cap_det) {
+        cudaFree(h->d_det); cudaFreeHost(h->h_det);
+        h->d_det = h->h_det = nullptr; h->cap_det = 0;
+        CU(h, cudaMalloc(&h->d_det, need));
+        CU(h, cudaHostAlloc(&h->h_det, need, cudaHostAllocDefault));
+        h->cap_det = need;
+    }
+    for (int64_t g0 = fa; g0 < fb; g0 += step) {
+        const int64_t m = std::min(step, fb - g0);
+        const size_t md = (size_t)m * D, o_reg = md * 16, o_cls = o_reg + md * 4, o_score = o_cls + md * 4, o_n = o_score + md * 4;
+        A.det_box = reinterpret_cast<float4*>(h->d_det);
+        A.det_region = reinterpret_cast<int32_t*>(h->d_det + o_reg);
+        A.det_cls = reinterpret_cast<int32_t*>(h->d_det + o_cls);
+        A.det_score = reinterpret_cast<float*>(h->d_det + o_score);
+        A.n_det = reinterpret_cast<int32_t*>(h->d_det + o_n);
+        int rc;
+        if ((rc = launch_merge(h, st, A, M, d_first, g0, g0 + m))) return rc;
+        CU(h, cudaMemcpyAsync(h->h_det, h->d_det, o_n + (size_t)m * 4, cudaMemcpyDeviceToHost, st));
+        CU(h, cudaStreamSynchronize(st));
+        const size_t at = (size_t)g0 * D;
+        std::memcpy(M.n_det + g0, h->h_det + o_n, (size_t)m * 4);
+        if (M.det_box) std::memcpy(M.det_box + at * 4, h->h_det, md * 16);
+        if (M.det_region) std::memcpy(M.det_region + at, h->h_det + o_reg, md * 4);
+        if (M.det_cls) std::memcpy(M.det_cls + at, h->h_det + o_cls, md * 4);
+        if (M.det_score) std::memcpy(M.det_score + at, h->h_det + o_score, md * 4);
+    }
+    return 0;
+}
+
+// The region data of a merge over predictions laid out as PredBlock's [bbox | probs | cls] for regions r_pred0 ..: the score
+// of a region is its probability (or logit) of its own class.
+static MergeArgs merge_args_of_predictions(const int4* d_desc, int64_t r_pred0, const int32_t* bbox, const float* probs,
+                                           const int32_t* cls, int n_cls, const MergeSpec& M) {
+    MergeArgs A = {};
+    A.desc = d_desc; A.r_pred0 = r_pred0;
+    A.score = probs; A.score_stride = n_cls; A.score_by_cls = 1;
+    A.cls = cls; A.bbox = bbox;
+    A.n_det = M.n_det; A.det_region = M.det_region; A.det_cls = M.det_cls; A.det_score = M.det_score;
+    A.det_box = reinterpret_cast<float4*>(M.det_box);
+    return A;
+}
+
 // Shared body of preprocess_bgr / detect_frames (centre: n frames, one centre crop each) and of
-// preprocess_regions / detect_regions (n regions over n_frames frames).  gray128 out, predictions out, or both.
+// preprocess_regions / detect_regions (n regions over n_frames frames).  gray128 out, predictions out, or both.  With `mg`
+// (detect_objects, n > 0) the predictions stay on the device and are merged into mg's per-frame detections instead; pieces of
+// the call then end at frame edges, so no frame is merged before all of its regions are predicted.
 static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frames, int fh, int fw, bool centre,
                         const int32_t* regions, int64_t n, uint8_t* gray128, float* probs, int32_t* cls, int32_t* bbox,
-                        bool detect, uint32_t flags) {
+                        bool detect, uint32_t flags, MergeSpec* mg = nullptr) {
     int rc;
     if (!h) return CNNACC_ERR_ARG;
     if (detect) {
@@ -1171,6 +1327,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         int64_t bad;
         if (const char* why = region_error(regions, n, n_frames, fh, fw, &bad))
             return fail(h, CNNACC_ERR_ARG, "region " + std::to_string(bad) + ": " + why);
+        if (mg && (rc = merge_check(h, regions, n, n_frames, *mg))) return rc;
     }
     CU(h, cudaSetDevice(h->device));
     const size_t frame_sz = (size_t)fh * fw * 3, img_sz = CNNACC_FEAT_BYTES;
@@ -1185,25 +1342,61 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         REQUIRE_ALIGNED(h, bbox, 16, "bbox");
         REQUIRE_ALIGNED(h, probs, 4, "probs");
         REQUIRE_ALIGNED(h, cls, 4, "cls");
+        if (mg) {
+            REQUIRE_ALIGNED(h, mg->det_box, 16, "det_box");
+            REQUIRE_ALIGNED(h, mg->n_det, 4, "n_det");
+            REQUIRE_ALIGNED(h, mg->det_region, 4, "det_region");
+            REQUIRE_ALIGNED(h, mg->det_cls, 4, "det_cls");
+            REQUIRE_ALIGNED(h, mg->det_score, 4, "det_score");
+        }
         DescBuf* db = nullptr;
         if (!centre) {
-            if ((rc = desc_acquire(h, n, &db))) return rc;
+            if ((rc = desc_acquire(h, n, &db, mg ? n_frames + 1 : 0))) return rc;
             std::memcpy(db->host, regions, (size_t)n * sizeof(int4));
             CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
+            if (mg) {
+                std::memcpy(db->first_host, mg->first.data(), (size_t)(n_frames + 1) * sizeof(long long));
+                CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, (size_t)(n_frames + 1) * sizeof(long long),
+                                      cudaMemcpyHostToDevice, h->stream));
+            }
         }
         auto run = [&]() -> int {
             const int64_t chunk = std::min<int64_t>(n, 16384);
             uint8_t* g = gray128;
             int r;
             if (!g && (r = grow(h, &h->d_gray, &h->cap_gray, (size_t)chunk * img_sz))) return r;
-            for (int64_t i0 = 0; i0 < n; i0 += chunk) {
-                const int64_t m = std::min(chunk, n - i0);
+            // detect_objects: the predictions of a piece go to a workspace laid out as PredBlock's, then the piece's frames
+            // are merged; a piece is the whole frames that fit `chunk` regions (a frame has at most kMergeMaxPerFrame)
+            const size_t w_probs = (size_t)chunk * 16, w_cls = w_probs + (size_t)chunk * nc * 4;
+            if (mg && (r = grow(h, &h->d_mpred, &h->cap_mpred, (size_t)chunk * kPredBytesPerImage))) return r;
+            int64_t m = 0;
+            for (int64_t i0 = 0, fa = 0; i0 < n; i0 += m) {
+                m = std::min(chunk, n - i0);
+                if (mg && i0 + m < n) m = mg->first[regions[4 * (i0 + m)]] - i0;
                 RegionPrep P = base;
                 P.frames = centre ? frames + i0 * frame_sz : frames;
                 P.desc = centre ? nullptr : db->dev + i0;
                 P.out = g ? g + i0 * img_sz : h->d_gray;
-                if ((r = prep_then_tail(h, h->stream, P, m, detect, probs ? probs + i0 * nc : nullptr, cls ? cls + i0 : nullptr,
-                                        bbox ? bbox + i0 * 4 : nullptr, flags))) return r;
+                if (mg) {
+                    int32_t* wb = reinterpret_cast<int32_t*>(h->d_mpred);
+                    float* wp = reinterpret_cast<float*>(h->d_mpred + w_probs);
+                    int32_t* wc = reinterpret_cast<int32_t*>(h->d_mpred + w_cls);
+                    const int64_t fb = i0 + m == n ? n_frames : regions[4 * (i0 + m)];
+                    MergeArgs A = merge_args_of_predictions(db->dev, i0, wb, wp, wc, nc, *mg);
+                    A.n_det += fa;
+                    const size_t o = (size_t)fa * mg->max_det;
+                    if (A.det_region) A.det_region += o;
+                    if (A.det_cls) A.det_cls += o;
+                    if (A.det_score) A.det_score += o;
+                    if (A.det_box) A.det_box += o;
+                    if ((r = prep_then_tail(h, h->stream, P, m, detect, wp, wc, wb, flags)) ||
+                        (r = launch_merge(h, h->stream, A, *mg, db->first_dev, fa, fb)))
+                        return r;
+                    fa = fb;
+                } else if ((r = prep_then_tail(h, h->stream, P, m, detect, probs ? probs + i0 * nc : nullptr, cls ? cls + i0 : nullptr,
+                                               bbox ? bbox + i0 * 4 : nullptr, flags))) {
+                    return r;
+                }
             }
             return 0;
         };
@@ -1214,8 +1407,17 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
 
     HostCall call(h);
     if ((rc = call.begin())) return rc;
-    const std::vector<RegionChunk> plan =
-        make_region_plan([&](int64_t r) -> int64_t { return centre ? r : regions[4 * r]; }, n, frame_sz, kPredSuper);
+    // prediction blocks: kPredSuper regions each, or for detect_objects the whole frames that fit in kPredSuper
+    auto frame_of = [&](int64_t r) -> int64_t { return centre ? r : regions[4 * r]; };
+    std::vector<int64_t> blocks;
+    if (mg) {
+        blocks = frame_aligned_blocks(frame_of, n, kPredSuper);
+    } else {
+        for (int64_t b = 0; b < n; b += kPredSuper) blocks.push_back(b);
+        blocks.push_back(n);
+    }
+    auto block_end = [&](int64_t r) { return *std::upper_bound(blocks.begin(), blocks.end(), r); };
+    const std::vector<RegionChunk> plan = make_region_plan_blocks(frame_of, n, frame_sz, block_end);
     size_t staged = 0, max_stage = 0;
     int64_t max_regions = 0;
     for (const RegionChunk& c : plan) {
@@ -1227,7 +1429,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
     // descriptors with the frame index relative to the staging buffer of the region's chunk
     DescBuf* db = nullptr;
     if (!centre) {
-        if ((rc = desc_acquire(h, n, &db))) return rc;
+        if ((rc = desc_acquire(h, n, &db, mg ? n_frames + 1 : 0))) return rc;
         int64_t below = 0;                               // small: frames staged ahead of the chunk in the one buffer
         for (const RegionChunk& c : plan) {
             for (int64_t r = c.r0; r < c.r1; r++) {
@@ -1237,7 +1439,22 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
             below += c.f1 - c.f0;
         }
         CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, small ? h->st_k : h->st_h2d));
+        if (mg) {
+            std::memcpy(db->first_host, mg->first.data(), (size_t)(n_frames + 1) * sizeof(long long));
+            CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, (size_t)(n_frames + 1) * sizeof(long long), cudaMemcpyHostToDevice,
+                                  small ? h->st_k : h->st_h2d));
+        }
     }
+    // detect_objects: merge the block of predictions [pred.s0, pred.end()) -- whole frames -- into the caller's arrays, up to
+    // the frame of the next block (frames without regions in between belong to this block)
+    int64_t det_f = 0;
+    auto merge_block = [&](const PredBlock& pred, cudaStream_t st) -> int {
+        const int64_t fb = pred.end() == n ? n_frames : regions[4 * pred.end()];
+        const MergeArgs A = merge_args_of_predictions(db->dev, pred.s0, pred.bbox(pred.s0), pred.probs(pred.s0), pred.cls(pred.s0), nc, *mg);
+        const int r = merge_to_host(h, st, A, *mg, db->first_dev, det_f, fb);
+        det_f = fb;
+        return r;
+    };
     auto region_base = [&](const uint8_t* d_frames, int64_t r, int64_t r_frame0, uint8_t* d_gray) {
         RegionPrep P = base;
         P.frames = centre ? d_frames + (r - r_frame0) * frame_sz : d_frames;
@@ -1263,21 +1480,25 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         }
         if ((rc = prep_then_tail(h, st, region_base(s->d_in, 0, 0, s->d_out), n, detect, pred.probs(0), pred.cls(0), pred.bbox(0), flags)))
             return rc;
-        if (db) CU(h, cudaEventRecord(db->ev, st));
         if (gray128) CU(h, cudaMemcpyAsync(gray128, s->d_out, n * img_sz, cudaMemcpyDeviceToHost, st));
-        if (detect && (rc = pred.flush(st, probs, cls, bbox, false))) return rc;
+        if (mg) rc = merge_block(pred, st);
+        else if (detect) rc = pred.flush(st, probs, cls, bbox, false);
+        if (db) CU(h, cudaEventRecord(db->ev, st));
+        if (rc) return rc;
         return detect ? call.done(true) : call.finish(st, false);
     }
     // Staged chunks of about 16 MiB of frames through the ring (HostCall).  A chunk's regions run in launches of up to
     // kRegionLaunch: their gray images fill the slot's output buffer, so a launch after the first waits for the gray copy of
     // the launch before.
     const int64_t per_launch = std::min<int64_t>(max_regions, kRegionLaunch);
-    if (detect && (rc = pred.start(0, std::min<int64_t>(kPredSuper, n)))) return rc;
+    size_t bi = 1;                                       // pred holds block [blocks[bi - 1], blocks[bi])
+    if (detect && (rc = pred.start(0, blocks[1]))) return rc;
     for (const RegionChunk& c : plan) {
         if (detect && c.r0 >= pred.end()) {              // the plan never lets a chunk straddle a block edge
-            if ((rc = pred.flush(h->st_k, probs, cls, bbox, false)) ||
-                (rc = pred.start(pred.end(), std::min<int64_t>(kPredSuper, n - pred.end()))))
+            if ((rc = mg ? merge_block(pred, h->st_k) : pred.flush(h->st_k, probs, cls, bbox, false)) ||
+                (rc = pred.start(pred.end(), blocks[bi + 1] - blocks[bi])))
                 return rc;
+            bi++;
         }
         if ((rc = call.acquire(s, max_stage, per_launch * img_sz))) return rc;
         CU(h, cudaMemcpyAsync(s->d_in, frames + c.f0 * frame_sz, (size_t)(c.f1 - c.f0) * frame_sz, cudaMemcpyHostToDevice, h->st_h2d));
@@ -1293,8 +1514,10 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
             if ((rc = call.released(*s, h->st_d2h))) return rc;
         }
     }
+    if (mg) rc = merge_block(pred, h->st_k);
+    else if (detect) rc = pred.flush(h->st_k, probs, cls, bbox, false);
     if (db) CU(h, cudaEventRecord(db->ev, h->st_k));
-    if (detect && (rc = pred.flush(h->st_k, probs, cls, bbox, false))) return rc;
+    if (rc) return rc;
     return call.finish(h->st_d2h, detect);
 }
 
@@ -1316,6 +1539,112 @@ int cnnacc_detect_regions(cnnacc_handle* h, const uint8_t* frames, int64_t n_fra
                           const int32_t* regions, int64_t n_regions, uint8_t* gray128,
                           float* probs, int32_t* cls, int32_t* bbox, uint32_t flags) {
     return regions_impl(h, frames, n_frames, fh, fw, false, regions, n_regions, gray128, probs, cls, bbox, true, flags);
+}
+
+// cnnacc_merge_regions: the merge alone on predictions the caller has (n may be 0: every frame gets no detections)
+static int merge_impl(cnnacc_handle* h, const int32_t* regions, int64_t n, int64_t n_frames, const float* scores, const int32_t* cls,
+                      const int32_t* bbox, MergeSpec& M, uint32_t flags) {
+    int rc;
+    const std::string why = merge_call_error(regions, n, n_frames, scores, cls, bbox, M);
+    if (!why.empty()) return fail(h, CNNACC_ERR_ARG, why);
+    if (n_frames == 0) return CNNACC_OK;
+    CU(h, cudaSetDevice(h->device));
+    const size_t first_bytes = (size_t)(n_frames + 1) * sizeof(long long);
+    MergeArgs A = {};
+    A.score_stride = 1; A.score_by_cls = 0;
+    if (flags & CNNACC_FLAG_DEVICE_PTRS) {
+        REQUIRE_ALIGNED(h, scores, 4, "scores");
+        REQUIRE_ALIGNED(h, cls, 4, "cls");
+        REQUIRE_ALIGNED(h, bbox, 4, "bbox");
+        REQUIRE_ALIGNED(h, M.det_box, 16, "det_box");
+        REQUIRE_ALIGNED(h, M.n_det, 4, "n_det");
+        REQUIRE_ALIGNED(h, M.det_region, 4, "det_region");
+        REQUIRE_ALIGNED(h, M.det_cls, 4, "det_cls");
+        REQUIRE_ALIGNED(h, M.det_score, 4, "det_score");
+        DescBuf* db = nullptr;
+        if ((rc = desc_acquire(h, n, &db, n_frames + 1))) return rc;
+        if (n) std::memcpy(db->host, regions, (size_t)n * sizeof(int4));
+        std::memcpy(db->first_host, M.first.data(), first_bytes);
+        if (n) CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
+        CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, first_bytes, cudaMemcpyHostToDevice, h->stream));
+        A.desc = db->dev; A.r_pred0 = 0; A.score = scores; A.cls = cls; A.bbox = bbox;
+        A.n_det = M.n_det; A.det_region = M.det_region; A.det_cls = M.det_cls; A.det_score = M.det_score;
+        A.det_box = reinterpret_cast<float4*>(M.det_box);
+        rc = launch_merge(h, h->stream, A, M, db->first_dev, 0, n_frames);
+        CU(h, cudaEventRecord(db->ev, h->stream));     // also after a failed launch: earlier ones may still read it
+        return rc;
+    }
+    // Host pointers: blocks of whole frames (at most kPredSuper regions) go in, are merged, and their detections come out.
+    HostCall call(h);
+    if ((rc = call.begin())) return rc;
+    cudaStream_t st = h->st_k;
+    DescBuf* db = nullptr;
+    if ((rc = desc_acquire(h, n, &db, n_frames + 1))) return rc;
+    if (n) std::memcpy(db->host, regions, (size_t)n * sizeof(int4));
+    std::memcpy(db->first_host, M.first.data(), first_bytes);
+    if (n) CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, st));
+    CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, first_bytes, cudaMemcpyHostToDevice, st));
+    const std::vector<int64_t> blocks = frame_aligned_blocks([&](int64_t r) -> int64_t { return regions[4 * r]; }, n, kPredSuper);
+    int64_t most = 0;
+    for (size_t k = 1; k < blocks.size(); k++) most = std::max(most, blocks[k] - blocks[k - 1]);
+    if (most && (rc = grow(h, &h->d_mpred, &h->cap_mpred, (size_t)most * 24))) return rc;
+    A.desc = db->dev;
+    int64_t fa = 0;
+    for (size_t k = 0; k < std::max<size_t>(1, blocks.size() - 1); k++) {
+        const int64_t b0 = blocks[k], m = blocks.size() > 1 ? blocks[k + 1] - b0 : 0;
+        const int64_t fb = b0 + m == n ? n_frames : regions[4 * (b0 + m)];
+        if (m) {
+            CU(h, cudaMemcpyAsync(h->d_mpred, bbox + 4 * b0, (size_t)m * 16, cudaMemcpyHostToDevice, st));
+            CU(h, cudaMemcpyAsync(h->d_mpred + (size_t)m * 16, scores + b0, (size_t)m * 4, cudaMemcpyHostToDevice, st));
+            CU(h, cudaMemcpyAsync(h->d_mpred + (size_t)m * 20, cls + b0, (size_t)m * 4, cudaMemcpyHostToDevice, st));
+        }
+        A.r_pred0 = b0;
+        A.bbox = reinterpret_cast<const int32_t*>(h->d_mpred);
+        A.score = reinterpret_cast<const float*>(h->d_mpred + (size_t)m * 16);
+        A.cls = reinterpret_cast<const int32_t*>(h->d_mpred + (size_t)m * 20);
+        rc = merge_to_host(h, st, A, M, db->first_dev, fa, fb);
+        if (rc) break;
+        fa = fb;
+    }
+    CU(h, cudaEventRecord(db->ev, st));
+    if (rc) return rc;
+    return call.done(false);
+}
+
+int cnnacc_detect_objects(cnnacc_handle* h, const uint8_t* frames, int64_t n_frames, int fh, int fw, const int32_t* regions,
+                          int64_t n_regions, float score_min, float iou_max, int max_det, int32_t* n_det, int32_t* det_region,
+                          int32_t* det_cls, float* det_score, float* det_box, uint32_t flags) {
+    int rc;
+    if (!h) return CNNACC_ERR_ARG;
+    MergeSpec M = make_merge_spec(score_min, iou_max, max_det, n_det, det_region, det_cls, det_score, det_box, flags);
+    if (n_regions != 0)
+        return regions_impl(h, frames, n_frames, fh, fw, false, regions, n_regions, nullptr, nullptr, nullptr, nullptr, true, flags, &M);
+    // no regions: detect_regions' state checks, then every frame gets no detections
+    if ((rc = check_ready(h))) return rc;
+    if (!h->fc_loaded) return fail(h, CNNACC_ERR_STATE, "classifier not loaded (call cnnacc_load_classifier)");
+    return merge_impl(h, nullptr, 0, n_frames, nullptr, nullptr, nullptr, M, flags);
+}
+
+int cnnacc_merge_regions(cnnacc_handle* h, const int32_t* regions, int64_t n_regions, int64_t n_frames, const float* scores,
+                         const int32_t* cls, const int32_t* bbox, float score_min, float iou_max, int max_det, int32_t* n_det,
+                         int32_t* det_region, int32_t* det_cls, float* det_score, float* det_box, uint32_t flags) {
+    if (!h) return CNNACC_ERR_ARG;
+    MergeSpec M = make_merge_spec(score_min, iou_max, max_det, n_det, det_region, det_cls, det_score, det_box, flags);
+    return merge_impl(h, regions, n_regions, n_frames, scores, cls, bbox, M, flags);
+}
+
+int cnnacc_merge_regions_host(const int32_t* regions, int64_t n_regions, int64_t n_frames, const float* scores, const int32_t* cls,
+                              const int32_t* bbox, float score_min, float iou_max, int max_det, int32_t* n_det, int32_t* det_region,
+                              int32_t* det_cls, float* det_score, float* det_box, uint32_t flags) {
+    if (flags & CNNACC_FLAG_DEVICE_PTRS) return CNNACC_ERR_ARG;
+    MergeSpec M = make_merge_spec(score_min, iou_max, max_det, n_det, det_region, det_cls, det_score, det_box, flags);
+    if (!merge_call_error(regions, n_regions, n_frames, scores, cls, bbox, M).empty()) return CNNACC_ERR_ARG;
+    const size_t D = (size_t)max_det;
+    for (int64_t f = 0; f < n_frames; f++)
+        n_det[f] = merge_frame_host(regions, scores, cls, bbox, M.first[f], M.first[f + 1] - M.first[f], score_min, iou_max, max_det,
+                                    M.agnostic, det_region ? det_region + f * D : nullptr, det_cls ? det_cls + f * D : nullptr,
+                                    det_score ? det_score + f * D : nullptr, det_box ? det_box + f * D * 4 : nullptr);
+    return CNNACC_OK;
 }
 
 int cnnacc_region_plan_host(const int32_t* regions, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t* chunks, int cap) {

@@ -39,10 +39,10 @@ inline const char* region_error(const int32_t* rg, int64_t n, int64_t n_frames, 
 
 struct RegionChunk { int64_t f0, f1, r0, r1; };
 
-// frame_of(r): the frame of region r, non-decreasing in r.  `super`: chunks never straddle a multiple of it (the call brings
-// the predictions of up to `super` regions back in one block).
-template <class FrameOf>
-std::vector<RegionChunk> make_region_plan(FrameOf frame_of, int64_t n, size_t frame_bytes, int64_t super) {
+// frame_of(r): the frame of region r, non-decreasing in r.  block_end(r) > r: the end of the prediction block that holds
+// region r; chunks never straddle a block edge (the call brings the predictions of a block back, or merges them, at once).
+template <class FrameOf, class BlockEnd>
+std::vector<RegionChunk> make_region_plan_blocks(FrameOf frame_of, int64_t n, size_t frame_bytes, BlockEnd block_end) {
     const int64_t per_chunk = frame_bytes >= kRegionChunkBytes ? 1 : (int64_t)(kRegionChunkBytes / frame_bytes);
     std::vector<RegionChunk> plan;
     for (int64_t r = 0; r < n;) {
@@ -50,7 +50,7 @@ std::vector<RegionChunk> make_region_plan(FrameOf frame_of, int64_t n, size_t fr
         c.r0 = r;
         c.f0 = frame_of(r);
         int64_t last = c.f0;
-        const int64_t end = std::min<int64_t>(n, (r / super + 1) * super);
+        const int64_t end = std::min<int64_t>(n, block_end(r));
         for (; r < end; r++) {
             const int64_t f = frame_of(r);
             if (f != last && (f != last + 1 || f - c.f0 >= per_chunk)) break;
@@ -61,6 +61,31 @@ std::vector<RegionChunk> make_region_plan(FrameOf frame_of, int64_t n, size_t fr
         plan.push_back(c);
     }
     return plan;
+}
+
+// The plan of cnnacc_detect_regions / cnnacc_detect_frames: prediction blocks of `super` regions each.
+template <class FrameOf>
+std::vector<RegionChunk> make_region_plan(FrameOf frame_of, int64_t n, size_t frame_bytes, int64_t super) {
+    return make_region_plan_blocks(frame_of, n, frame_bytes, [super](int64_t r) { return (r / super + 1) * super; });
+}
+
+// Prediction blocks of at most `super` regions that end at frame edges (cnnacc_detect_objects merges a block once all of its
+// frames are predicted): bounds[0] = 0 < bounds[1] < ... = n.  Always possible while a frame has fewer than `super` regions.
+template <class FrameOf>
+std::vector<int64_t> frame_aligned_blocks(FrameOf frame_of, int64_t n, int64_t super) {
+    std::vector<int64_t> bounds{0};
+    while (bounds.back() < n) {
+        const int64_t b0 = bounds.back();
+        int64_t e = b0 + super;
+        if (e >= n) {
+            e = n;
+        } else {
+            while (e > b0 && frame_of(e) == frame_of(e - 1)) e--;   // back to the first region of the frame that holds e
+            if (e == b0) e = b0 + super;                          // a frame of super regions or more: cut inside it
+        }
+        bounds.push_back(e);
+    }
+    return bounds;
 }
 
 }  // namespace cnnacc

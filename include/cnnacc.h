@@ -217,6 +217,39 @@ int cnnacc_preprocess_regions(cnnacc_handle *h, const uint8_t *frames, int64_t n
 int cnnacc_detect_regions(cnnacc_handle *h, const uint8_t *frames, int64_t n_frames, int fh, int fw,
                           const int32_t *regions, int64_t n_regions, uint8_t *gray128,
                           float *probs, int32_t *cls, int32_t *bbox, uint32_t flags);
+/* ---- merging region detections into per-frame detections --------------------------------------------------------------
+ * The rule (csrc/region_merge.h), per frame, independently: clamp every box coordinate to [0, 127]; map the box to the frame
+ * exactly, in 1/128 pixel (X = 128 x + bx * side, the same for y); candidates are the regions with score >= score_min (a NaN
+ * score never is; -0.0 equals +0.0); walk them by score descending, ties by region index ascending, and keep a candidate
+ * unless an already-kept box of the same class (of any class with CNNACC_FLAG_CLASS_AGNOSTIC) has IoU > iou_max with it, where
+ * IoU = (double)inter / (double)union of the exact integer areas (0 when union == 0); stop after max_det kept boxes.
+ * Outputs per frame f, in kept order: n_det [F] i32, det_region [F][max_det] i32 (index into `regions`), det_cls [F][max_det]
+ * i32, det_score [F][max_det] f32, det_box [F][max_det][4] f32 frame pixels (x1, y1, x2, y2) = the float nearest X / 128.
+ * Rows k >= n_det[f] hold region -1, class -1, score 0 and box 0.  n_det is required; the other four may be NULL.
+ *   -2, nothing launched: max_det outside 1..CNNACC_MERGE_MAX_DET, iou_max NaN or outside [0, 1], a frame with more than
+ *       CNNACC_MERGE_MAX_PER_FRAME regions, n_det NULL, more than 2^31-1 regions; device pointers with det_box not 16-byte
+ *       aligned or another array not 4-byte aligned.
+ * detect_objects: detect_regions followed by the merge with score[r] = probs[r][cls[r]] (the logit with CNNACC_FLAG_LOGITS); the
+ *       per-region predictions never leave the GPU.  Same flags, regions and refusals as detect_regions (-2, -4), plus the
+ *       merge's.  n_regions == 0 gives every frame no detections.
+ * merge_regions: the merge alone on predictions the caller has, scores [R] f32, cls [R] i32, bbox [R][4] i32, host or device
+ *       memory (CNNACC_FLAG_DEVICE_PTRS); needs no weights or classifier.  Regions as above, in host memory; checked: a frame
+ *       in [0, n_frames), frame indices that do not decrease, x, y >= 0, side 128..8192 (there is no frame size to check them
+ *       against).  Device pointers: asynchronous on the handle's stream.
+ * merge_regions_host: the same rule on the CPU (host arrays only), for tests. */
+#define CNNACC_FLAG_CLASS_AGNOSTIC  0x80u  /* detect_objects / merge_regions: suppression across classes */
+#define CNNACC_MERGE_MAX_DET        1024
+#define CNNACC_MERGE_MAX_PER_FRAME  16384
+int cnnacc_detect_objects(cnnacc_handle *h, const uint8_t *frames, int64_t n_frames, int fh, int fw,
+                          const int32_t *regions, int64_t n_regions, float score_min, float iou_max, int max_det,
+                          int32_t *n_det, int32_t *det_region, int32_t *det_cls, float *det_score, float *det_box, uint32_t flags);
+int cnnacc_merge_regions(cnnacc_handle *h, const int32_t *regions, int64_t n_regions, int64_t n_frames,
+                         const float *scores, const int32_t *cls, const int32_t *bbox, float score_min, float iou_max, int max_det,
+                         int32_t *n_det, int32_t *det_region, int32_t *det_cls, float *det_score, float *det_box, uint32_t flags);
+int cnnacc_merge_regions_host(const int32_t *regions, int64_t n_regions, int64_t n_frames,
+                              const float *scores, const int32_t *cls, const int32_t *bbox, float score_min, float iou_max,
+                              int max_det, int32_t *n_det, int32_t *det_region, int32_t *det_cls, float *det_score,
+                              float *det_box, uint32_t flags);
 /* Host-only view of the staging plan of a host-pointer region call (csrc/region_plan.h): chunk i stages frames
  * [chunks[4i], chunks[4i+1]) with one copy and runs regions [chunks[4i+2], chunks[4i+3]) on them.  Returns the number of chunks
  * (<= cap), or -2 for a region array the real call refuses, or when cap is too small.  No GPU needed. */

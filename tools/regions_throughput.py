@@ -10,6 +10,9 @@ the predictions on the host), and device-resident frames/s and regions/s (CUDA e
 (preprocess_regions) and conv + tail (infer_batch on the same number of 128x128 images).  Beside them from the same run:
 detect_frames frames/s host-fed and device-resident, device-resident infer_batch images/s, and batch-1 p50 / p99 of one VGA
 frame with grid (a) against detect_frames of one frame.  The card's name and power limit are read in the same run.
+--objects adds the merging calls: detect_objects (detect_regions + per-frame greedy NMS on the GPU) host-fed and
+device-resident beside detect_regions for grid (a) and pyramid (b), merge_regions alone on device tensors at 63 and at
+2925 regions per frame (side 128, stride 8), and batch-1 p50 / p99 of detect_objects on one VGA frame with grid (a).
 
     python tools/regions_throughput.py [--frames 2048] [--dev-frames 1024] [--seconds 2] [--out FILE]
 """
@@ -79,6 +82,7 @@ def main():
     ap.add_argument("--dev-frames", type=int, default=1024, help="device-resident frames (0.9 GiB at 1024)")
     ap.add_argument("--seconds", type=float, default=2.0)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--objects", action="store_true", help="measure the merging calls (detect_objects / merge_regions)")
     a = ap.parse_args()
     import torch
     dev = torch.device("cuda", 0)
@@ -99,6 +103,10 @@ def main():
     block = inputs.make_frames(("smooth", 1), 16, H, W)
     for i in range(0, a.frames, 16):
         host[i:i + 16] = block[:a.frames - i]
+
+    if a.objects:
+        objects(a, acc, host, emit)
+        return write(a, lines)
 
     # host-fed
     per_s = wall_rate(lambda: acc.detect_frames(host), a.seconds)
@@ -156,11 +164,75 @@ def main():
         ts = np.array(ts) * 1e6
         emit({"what": "batch1", "path": path, "p50_us": float(np.percentile(ts, 50)), "p99_us": float(np.percentile(ts, 99))})
 
+    write(a, lines)
+
+
+def write(a, lines):
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
             for d in lines:
                 f.write(json.dumps(d) + "\n")
+
+
+def objects(a, acc, host, emit):
+    """detect_objects beside detect_regions (host-fed and device-resident, alternated in one run), merge_regions alone, batch 1."""
+    import torch
+    dev = torch.device("cuda", 0)
+    kw = dict(score_min=0.0, iou_max=0.5, max_det=100)
+    for name in ("grid", "pyramid"):
+        reg = workloads(a.frames)[name]
+        rates = {}
+        for rep in range(2):                                 # alternate the two calls to see the spread
+            for path, fn in (("detect_regions", lambda: acc.detect_regions(host, reg)),
+                             ("detect_objects", lambda: acc.detect_objects(host, reg, **kw))):
+                rates.setdefault(path, []).append(wall_rate(fn, a.seconds) * a.frames)
+        for path, r in rates.items():
+            emit({"what": "host_fed", "path": path, "workload": name, "regions_per_frame": len(reg) / a.frames,
+                  "frames_per_s": max(r), "frames_per_s_runs": r})
+        emit({"what": "host_fed", "ratio": "detect_objects/detect_regions", "workload": name,
+              "value": max(rates["detect_objects"]) / max(rates["detect_regions"])})
+    t = torch.from_numpy(host[:a.dev_frames]).to(dev)
+    nd = a.dev_frames
+    for name in ("grid", "pyramid"):
+        reg = workloads(nd)[name]
+        ms = {}
+        for rep in range(2):
+            for path, fn in (("detect_regions", lambda: acc.detect_regions(t, reg)),
+                             ("detect_objects", lambda: acc.detect_objects(t, reg, **kw))):
+                ms.setdefault(path, []).append(event_ms(fn, a.seconds))
+        for path, m in ms.items():
+            emit({"what": "device_resident", "path": path, "workload": name, "regions": len(reg), "ms": min(m), "ms_runs": m,
+                  "frames_per_s": nd / min(m) * 1e3})
+        emit({"what": "device_resident", "ratio": "detect_objects/detect_regions (frames/s)", "workload": name,
+              "value": min(ms["detect_regions"]) / min(ms["detect_objects"])})
+    del t
+    # the merge alone on device predictions: 63 regions per frame (stride 64) and 2925 (stride 8)
+    for stride, frames in ((64, 16384), (8, 1024)):
+        reg = fc.grid_regions(frames, H, W, 128, stride)
+        n = len(reg)
+        rng = np.random.default_rng(stride)
+        cls = torch.from_numpy(rng.integers(0, 6, n).astype(np.int32)).to(dev)
+        scores = torch.from_numpy(rng.random(n, np.float32)).to(dev)
+        b1 = rng.integers(0, 64, (n, 2))
+        bbox = torch.from_numpy(np.concatenate([b1, b1 + rng.integers(8, 64, (n, 2))], 1).astype(np.int32)).to(dev)
+        ms = event_ms(lambda: acc.merge_regions(reg, cls, scores, bbox, frames, **kw), a.seconds)
+        emit({"what": "device_resident", "path": "merge_regions", "regions_per_frame": n // frames, "frames": frames, "ms": ms,
+              "frames_per_s": frames / ms * 1e3, "regions_per_s": n / ms * 1e3, "us_per_frame": ms * 1e3 / frames})
+    # batch 1: one VGA frame (pageable, as a camera loop has it)
+    one = np.ascontiguousarray(host[:1])
+    grid1 = fc.grid_regions(1, H, W, 128, 64)
+    for path, fn in (("detect_objects_grid63", lambda: acc.detect_objects(one, grid1, **kw)),
+                     ("detect_regions_grid63", lambda: acc.detect_regions(one, grid1))):
+        for _ in range(50):
+            fn()
+        ts = []
+        for _ in range(2000):
+            t0 = time.perf_counter()
+            fn()
+            ts.append(time.perf_counter() - t0)
+        ts = np.array(ts) * 1e6
+        emit({"what": "batch1", "path": path, "p50_us": float(np.percentile(ts, 50)), "p99_us": float(np.percentile(ts, 99))})
 
 
 if __name__ == "__main__":
