@@ -12,6 +12,7 @@ OK, ERR_TIMEOUT, ERR_ARG, ERR_CUDA, ERR_STATE = 0, -1, -2, -3, -4
 FLAG_DEVICE_PTRS, FLAG_DIRECT, FLAG_KEEP_MAPS, FLAG_CLS_GIVEN, FLAG_BBOX_UPSAMPLED, FLAG_LOGITS = 0x1, 0x2, 0x4, 0x8, 0x10, 0x20
 FLAG_TWO_KERNELS = 0x40
 FLAG_CLASS_AGNOSTIC = 0x80
+FLAG_RECTS = 0x100
 MERGE_MAX_DET, MERGE_MAX_PER_FRAME = 1024, 16384
 MAX_PENDING = 8
 
@@ -63,6 +64,7 @@ SYMBOLS = {
     "cnnacc_merge_regions_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_float,
                                              _c.c_float, _c.c_int] + [_c.c_void_p] * 5 + [_c.c_uint32]),
     "cnnacc_region_plan_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int]),
+    "cnnacc_rect_plan_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int]),
     "cnnacc_area_tab_host": (_c.c_int, [_c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_int]),
     "cnnacc_image_to_gray128": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p, _c.c_uint32]),
     "cnnacc_run_batch_sharded": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p,

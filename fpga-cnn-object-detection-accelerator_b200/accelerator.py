@@ -70,17 +70,19 @@ def _pred_outputs(new, n, n_cls):
 
 
 def _grouped_regions(regions):
-    """An (R, 4) integer array of (frame, x, y, side) in any order -> (the regions as int32 grouped by frame, stably, as the
-    library takes them; the caller's index of each, or None when they were grouped already)."""
+    """An (R, 4) integer array of squares (frame, x, y, side) or an (R, 5) one of rectangles (frame, x, y, w, h), in any order
+    -> (the regions as int32 grouped by frame, stably, as the library takes them; the caller's index of each, or None when
+    they were grouped already; FLAG_RECTS for rectangles, else 0)."""
     reg = np.asarray(regions)
-    if reg.ndim != 2 or reg.shape[1] != 4 or not (reg.size == 0 or np.issubdtype(reg.dtype, np.integer)):
-        raise ValueError("regions must be an (R, 4) integer array of (frame, x, y, side)")
+    if reg.ndim != 2 or reg.shape[1] not in (4, 5) or not (reg.size == 0 or np.issubdtype(reg.dtype, np.integer)):
+        raise ValueError("regions must be an (R, 4) integer array of (frame, x, y, side) or an (R, 5) one of (frame, x, y, w, h)")
     reg = reg.astype(np.int64)
     if reg.size and (reg.min() < -2 ** 31 or reg.max() >= 2 ** 31):
         raise ValueError("region values must fit int32")
     order = np.argsort(reg[:, 0], kind="stable")
     shuffled = bool((order != np.arange(len(order))).any())
-    return np.ascontiguousarray(reg[order], dtype=np.int32), (order.astype(np.int32) if shuffled else None)
+    return (np.ascontiguousarray(reg[order], dtype=np.int32), (order.astype(np.int32) if shuffled else None),
+            _lib.FLAG_RECTS if reg.shape[1] == 5 else 0)
 
 
 def _merge_flags(max_det, class_agnostic):
@@ -496,17 +498,21 @@ class CNNAccelerator:
         on torch's current stream), regions (R,4) integers (frame, x, y, side) in any order, side 128..8192, inside its
         frame.  Region r's results are those detect_frames gives for frames[f][y:y+side, x:x+side] as a frame of its own; its
         box is in that square's 128x128 coordinates (region_boxes_to_frame maps it to frame pixels).
+        Rectangles: regions (R,5) integers (frame, x, y, w, h), w and h 128..8192; region r's gray128 is
+        cv2.resize(cv2.cvtColor(frames[f][y:y+h, x:x+w], COLOR_BGR2GRAY), (128, 128), interpolation=INTER_AREA) byte for
+        byte, its predictions are infer_batch's for that gray128, and its box is on the rectangle's 128 grid.
         -> (cls [R], probs [R,n_cls], bbox [R,4][, gray128 [R,128,128]]) in the order of `regions`, numpy or torch like frames."""
         flags = _pred_flags(bbox, logits)
         self._classes()
         return self._regions(frames, regions, True, return_gray, flags)
 
     def preprocess_regions(self, frames, regions):
-        """preprocess on caller-chosen square regions (see detect_regions) -> gray128 [R,128,128] u8 in the order of `regions`."""
+        """preprocess on caller-chosen square (R,4) or rectangular (R,5) regions (see detect_regions) -> gray128 [R,128,128] u8
+        in the order of `regions`."""
         return self._regions(frames, regions, False, True, 0)[0]
 
     def _regions(self, frames, regions, detect, want_gray, flags):
-        reg, order = _grouped_regions(regions)              # the library takes regions grouped by frame
+        reg, order, rects = _grouped_regions(regions)       # the library takes regions grouped by frame
         n = reg.shape[0]
         frames, new, ptr, kind, ctx = self._host_or_device(frames)
         if frames.ndim != 4 or frames.shape[3] != 3:
@@ -516,7 +522,7 @@ class CNNAccelerator:
         outs = _pred_outputs(new, n, self._n_cls) if detect else ()
         with ctx:
             self._call_regions(ptr(frames), nf, fh, fw, reg, ptr(gray) if want_gray else None, [ptr(a) for a in outs], detect,
-                               flags | kind)
+                               flags | kind | rects)
         res = outs + ((gray,) if want_gray else ())
         if order is not None:
             inv = np.argsort(order)                          # also indexes CUDA tensors: torch moves the index to their device
@@ -537,12 +543,13 @@ class CNNAccelerator:
         candidate when its score -- the probability of its class, or the logit with logits=True -- is >= score_min; candidates
         are kept by score descending (ties: lower region index first) unless a kept box of the same class (any class with
         class_agnostic) has IoU > iou_max with it, at most max_det per frame.  The per-region predictions never leave the GPU.
-        frames / regions as for detect_regions (numpy or a CUDA tensor on torch's current stream; regions in any order).
+        frames / regions as for detect_regions (numpy or a CUDA tensor on torch's current stream; regions in any order, (R,4)
+        squares or (R,5) rectangles, whose boxes map to the frame as region_boxes_to_frame's do).
         -> (n_det [F] i32, region [F,max_det] i32 index into `regions`, cls [F,max_det] i32, score [F,max_det] f32,
         box [F,max_det,4] f32 frame pixels), rows past n_det[f] hold -1 / -1 / 0 / 0; numpy or torch like frames."""
         flags = _pred_flags(bbox, logits) | _merge_flags(max_det, class_agnostic)
         self._classes()
-        reg, order = _grouped_regions(regions)
+        reg, order, rects = _grouped_regions(regions)
         frames, new, ptr, kind, ctx = self._host_or_device(frames)
         if frames.ndim != 4 or frames.shape[3] != 3:
             raise ValueError("expected [F,h,w,3] BGR frames")
@@ -550,17 +557,18 @@ class CNNAccelerator:
         dets = _det_outputs(new, nf, int(max_det))
         with ctx:
             self._check(self._libc.cnnacc_detect_objects(self._h, ptr(frames), nf, fh, fw, _vp(reg), reg.shape[0], float(score_min),
-                                                         float(iou_max), int(max_det), *[ptr(a) for a in dets], flags | kind))
+                                                         float(iou_max), int(max_det), *[ptr(a) for a in dets],
+                                                         flags | kind | rects))
         return _callers_regions(dets, order)
 
     def merge_regions(self, regions, cls, scores, bbox, n_frames, score_min=0.0, iou_max=0.5, max_det=100, class_agnostic=False):
-        """The merge of detect_objects alone, on predictions the caller already has: regions (R,4) (frame, x, y, side) in any
-        order, cls [R] i32, scores [R] f32, bbox [R,4] i32 on each region's 128 grid, as numpy arrays or CUDA tensors (scores
+        """The merge of detect_objects alone, on predictions the caller already has: regions (R,4) (frame, x, y, side) or (R,5)
+        (frame, x, y, w, h) in any order, cls [R] i32, scores [R] f32, bbox [R,4] i32 on each region's 128 grid, as numpy arrays or CUDA tensors (scores
         decides which; tensors run on torch's current stream).  Needs no weights or classifier.  -> as detect_objects."""
         if int(n_frames) < 0:
             raise ValueError("n_frames must be >= 0")
-        flags = _merge_flags(max_det, class_agnostic)
-        reg, order = _grouped_regions(regions)
+        reg, order, rects = _grouped_regions(regions)
+        flags = _merge_flags(max_det, class_agnostic) | rects
         n = reg.shape[0]
         if _is_torch_cuda(scores):
             import torch
@@ -635,14 +643,44 @@ def grid_regions(n_frames, fh, fw, sides, strides):
     return out.reshape(-1, 4)
 
 
+def grid_rects(n_frames, fh, fw, sizes, strides):
+    """Rectangles (frame, x, y, w, h) tiling every frame of a [n_frames, fh, fw, 3] batch at each size, as grid_regions does
+    for squares: tiles at x = 0, sx, 2 sx, ... plus one flush with the right edge (x = fw - w) when that position is missing,
+    the same for y with sy.  `sizes` is one (w, h) pair or a sequence of them; `strides` an int (sx = sy), one (sx, sy) pair
+    for every size, or one pair per size.  Frame-major (frame, then size in the given order, then y, then x).
+    -> (R, 5) int32."""
+    sizes = np.asarray(sizes, dtype=np.int64).reshape(-1, 2)
+    st = np.asarray(strides, dtype=np.int64)
+    if st.ndim == 0:
+        st = np.repeat(st, 2)
+    st = np.broadcast_to(st, sizes.shape) if st.shape == (2,) else st
+    if st.shape != sizes.shape:
+        raise ValueError("strides must be an int, an (sx, sy) pair or one (sx, sy) pair per size")
+    per_frame = []
+    for (w, h), (sx, sy) in zip(sizes.tolist(), st.tolist()):
+        if not (1 <= w <= fw and 1 <= h <= fh) or sx < 1 or sy < 1:
+            raise ValueError(f"size {w}x{h} / stride ({sx}, {sy}) does not fit a {fh}x{fw} frame")
+        for y in _tile_origins(fh, h, sy):
+            for x in _tile_origins(fw, w, sx):
+                per_frame.append((x, y, w, h))
+    tiles = np.array(per_frame, dtype=np.int32).reshape(-1, 4)
+    out = np.empty((int(n_frames), len(tiles), 5), dtype=np.int32)
+    out[:, :, 0] = np.arange(int(n_frames), dtype=np.int32)[:, None]
+    out[:, :, 1:] = tiles[None]
+    return out.reshape(-1, 5)
+
+
 def region_boxes_to_frame(regions, bbox):
     """Boxes of detect_regions (x1, y1, x2, y2 on the region's 128x128 grid) in frame pixels: x + b * side / 128 for x1 and
-    x2, y + b * side / 128 for y1 and y2, as float64, exact.  Its float32 cast equals, bit for bit, the boxes
-    CNNAccelerator.detect_objects / merge_regions return for boxes inside the 128 grid (those calls clamp to [0, 127] and
-    merge the regions of each frame by greedy NMS; this function only maps).  -> (R, 4) float64."""
-    reg = np.asarray(regions, dtype=np.float64).reshape(-1, 4)
+    x2, y + b * side / 128 for y1 and y2 -- for (R, 5) rectangles (frame, x, y, w, h), x + b * w / 128 and y + b * h / 128 --
+    as float64, exact.  Its float32 cast equals, bit for bit, the boxes CNNAccelerator.detect_objects / merge_regions return
+    for boxes inside the 128 grid (those calls clamp to [0, 127] and merge the regions of each frame by greedy NMS; this
+    function only maps).  -> (R, 4) float64."""
+    reg = np.asarray(regions, dtype=np.float64)
+    reg = reg.reshape(-1, 5) if reg.shape[-1:] == (5,) else reg.reshape(-1, 4)
     b = np.asarray(bbox, dtype=np.float64).reshape(-1, 4)
-    scale = reg[:, 3:4] / 128.0
+    w, h = reg[:, 3:4], reg[:, -1:]                         # a square's side is both
+    scale = np.concatenate([w, h, w, h], axis=1) / 128.0
     origin = np.concatenate([reg[:, 1:3], reg[:, 1:3]], axis=1)
     return origin + b * scale
 

@@ -1183,35 +1183,38 @@ struct MergeSpec {
 
 // Checks shared by cnnacc_detect_objects and the cnnacc_merge_regions calls once the regions themselves passed their checks:
 // the merge limits, n_det, and at most kMergeMaxPerFrame regions per frame.  Fills M.first.  "" or why not.
-static std::string merge_error(const int32_t* regions, int64_t n, int64_t n_frames, MergeSpec& M) {
+static std::string merge_error(const RegionRecords& rg, int64_t n, int64_t n_frames, MergeSpec& M) {
     if (!M.n_det) return "NULL n_det";
     if (const char* why = merge_limits_error(M.iou_max, M.max_det)) return why;
     if (n > 0x7fffffffLL) return "more than 2^31-1 regions in one merging call";
     int64_t most, bad;
-    if (const char* why = merge_frame_ranges([&](int64_t r) -> int64_t { return regions[4 * r]; }, n, n_frames, M.first, &most, &bad))
+    if (const char* why = merge_frame_ranges([&](int64_t r) { return rg.frame(r); }, n, n_frames, M.first, &most, &bad))
         return "frame " + std::to_string(bad) + ": " + why;
     return "";
 }
-static int merge_check(cnnacc_handle* h, const int32_t* regions, int64_t n, int64_t n_frames, MergeSpec& M) {
-    const std::string why = merge_error(regions, n, n_frames, M);
+static int merge_check(cnnacc_handle* h, const RegionRecords& rg, int64_t n, int64_t n_frames, MergeSpec& M) {
+    const std::string why = merge_error(rg, n, n_frames, M);
     return why.empty() ? 0 : fail(h, CNNACC_ERR_ARG, why);
 }
 
 // The arguments of cnnacc_merge_regions / cnnacc_merge_regions_host: "" or why not.  There is no frame size, so a region's
-// frame, position and side are checked, not that it lies inside its frame.
-static std::string merge_call_error(const int32_t* regions, int64_t n, int64_t n_frames, const float* scores, const int32_t* cls,
+// frame, position and sizes are checked, not that it lies inside its frame.
+static std::string merge_call_error(const RegionRecords& rg, int64_t n, int64_t n_frames, const float* scores, const int32_t* cls,
                                     const int32_t* bbox, MergeSpec& M) {
     if (n < 0 || n_frames < 0) return "negative n_frames / n_regions";
-    if (n > 0 && (!regions || !scores || !cls || !bbox)) return "NULL region / score / class / box pointer";
-    for (int64_t r = 0; r < n; r++) {
-        const int64_t f = regions[4 * r], x = regions[4 * r + 1], y = regions[4 * r + 2], side = regions[4 * r + 3];
-        const std::string at = "region " + std::to_string(r) + ": ";
-        if (f < 0 || f >= n_frames) return at + "frame index outside [0, n_frames)";
-        if (side < kRegionMinSide || side > kRegionMaxSide) return at + "side outside 128..8192";
-        if (x < 0 || y < 0) return at + "negative position";
-        if (r > 0 && f < regions[4 * (r - 1)]) return at + "frame indices decrease (group the regions by frame, in non-decreasing order)";
+    if (n > 0 && (!rg.p || !scores || !cls || !bbox)) return "NULL region / score / class / box pointer";
+    int64_t bad;
+    if (const char* why = region_error(rg, n, n_frames, false, 0, 0, &bad)) return "region " + std::to_string(bad) + ": " + why;
+    return merge_error(rg, n, n_frames, M);
+}
+
+// The device descriptors (regions.cuh, region_merge.cuh) of regions [0, n), frame indices as the caller gave them
+static void fill_desc(int4* d, const RegionRecords& rg, int64_t n) {
+    if (rg.stride == 4) {
+        if (n) std::memcpy(d, rg.p, (size_t)n * sizeof(int4));          // a square's record is its descriptor
+        return;
     }
-    return merge_error(regions, n, n_frames, M);
+    for (int64_t r = 0; r < n; r++) d[r] = make_int4((int)rg.frame(r), rg.x(r), rg.y(r), rg.wh(r));
 }
 
 static MergeSpec make_merge_spec(float score_min, float iou_max, int max_det, int32_t* n_det, int32_t* det_region, int32_t* det_cls,
@@ -1313,6 +1316,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
                         const int32_t* regions, int64_t n, uint8_t* gray128, float* probs, int32_t* cls, int32_t* bbox,
                         bool detect, uint32_t flags, MergeSpec* mg = nullptr) {
     int rc;
+    const RegionRecords rg(regions, (flags & CNNACC_FLAG_RECTS) != 0);
     if (!h) return CNNACC_ERR_ARG;
     if (detect) {
         if ((rc = check_ready(h))) return rc;
@@ -1325,9 +1329,9 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
     if (!frames || (!centre && !regions) || (!detect && !gray128)) return fail(h, CNNACC_ERR_ARG, "NULL frame / region / output pointer");
     if (!centre) {
         int64_t bad;
-        if (const char* why = region_error(regions, n, n_frames, fh, fw, &bad))
+        if (const char* why = region_error(rg, n, n_frames, true, fh, fw, &bad))
             return fail(h, CNNACC_ERR_ARG, "region " + std::to_string(bad) + ": " + why);
-        if (mg && (rc = merge_check(h, regions, n, n_frames, *mg))) return rc;
+        if (mg && (rc = merge_check(h, rg, n, n_frames, *mg))) return rc;
     }
     CU(h, cudaSetDevice(h->device));
     const size_t frame_sz = (size_t)fh * fw * 3, img_sz = CNNACC_FEAT_BYTES;
@@ -1352,7 +1356,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         DescBuf* db = nullptr;
         if (!centre) {
             if ((rc = desc_acquire(h, n, &db, mg ? n_frames + 1 : 0))) return rc;
-            std::memcpy(db->host, regions, (size_t)n * sizeof(int4));
+            fill_desc(db->host, rg, n);
             CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
             if (mg) {
                 std::memcpy(db->first_host, mg->first.data(), (size_t)(n_frames + 1) * sizeof(long long));
@@ -1372,7 +1376,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
             int64_t m = 0;
             for (int64_t i0 = 0, fa = 0; i0 < n; i0 += m) {
                 m = std::min(chunk, n - i0);
-                if (mg && i0 + m < n) m = mg->first[regions[4 * (i0 + m)]] - i0;
+                if (mg && i0 + m < n) m = mg->first[rg.frame(i0 + m)] - i0;
                 RegionPrep P = base;
                 P.frames = centre ? frames + i0 * frame_sz : frames;
                 P.desc = centre ? nullptr : db->dev + i0;
@@ -1381,7 +1385,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
                     int32_t* wb = reinterpret_cast<int32_t*>(h->d_mpred);
                     float* wp = reinterpret_cast<float*>(h->d_mpred + w_probs);
                     int32_t* wc = reinterpret_cast<int32_t*>(h->d_mpred + w_cls);
-                    const int64_t fb = i0 + m == n ? n_frames : regions[4 * (i0 + m)];
+                    const int64_t fb = i0 + m == n ? n_frames : rg.frame(i0 + m);
                     MergeArgs A = merge_args_of_predictions(db->dev, i0, wb, wp, wc, nc, *mg);
                     A.n_det += fa;
                     const size_t o = (size_t)fa * mg->max_det;
@@ -1408,7 +1412,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
     HostCall call(h);
     if ((rc = call.begin())) return rc;
     // prediction blocks: kPredSuper regions each, or for detect_objects the whole frames that fit in kPredSuper
-    auto frame_of = [&](int64_t r) -> int64_t { return centre ? r : regions[4 * r]; };
+    auto frame_of = [&](int64_t r) -> int64_t { return centre ? r : rg.frame(r); };
     std::vector<int64_t> blocks;
     if (mg) {
         blocks = frame_aligned_blocks(frame_of, n, kPredSuper);
@@ -1432,10 +1436,8 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         if ((rc = desc_acquire(h, n, &db, mg ? n_frames + 1 : 0))) return rc;
         int64_t below = 0;                               // small: frames staged ahead of the chunk in the one buffer
         for (const RegionChunk& c : plan) {
-            for (int64_t r = c.r0; r < c.r1; r++) {
-                const int32_t* g = regions + 4 * r;
-                db->host[r] = make_int4((int)(g[0] - c.f0 + (small ? below : 0)), g[1], g[2], g[3]);
-            }
+            for (int64_t r = c.r0; r < c.r1; r++)
+                db->host[r] = make_int4((int)(rg.frame(r) - c.f0 + (small ? below : 0)), rg.x(r), rg.y(r), rg.wh(r));
             below += c.f1 - c.f0;
         }
         CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, small ? h->st_k : h->st_h2d));
@@ -1449,7 +1451,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
     // the frame of the next block (frames without regions in between belong to this block)
     int64_t det_f = 0;
     auto merge_block = [&](const PredBlock& pred, cudaStream_t st) -> int {
-        const int64_t fb = pred.end() == n ? n_frames : regions[4 * pred.end()];
+        const int64_t fb = pred.end() == n ? n_frames : rg.frame(pred.end());
         const MergeArgs A = merge_args_of_predictions(db->dev, pred.s0, pred.bbox(pred.s0), pred.probs(pred.s0), pred.cls(pred.s0), nc, *mg);
         const int r = merge_to_host(h, st, A, *mg, db->first_dev, det_f, fb);
         det_f = fb;
@@ -1545,7 +1547,8 @@ int cnnacc_detect_regions(cnnacc_handle* h, const uint8_t* frames, int64_t n_fra
 static int merge_impl(cnnacc_handle* h, const int32_t* regions, int64_t n, int64_t n_frames, const float* scores, const int32_t* cls,
                       const int32_t* bbox, MergeSpec& M, uint32_t flags) {
     int rc;
-    const std::string why = merge_call_error(regions, n, n_frames, scores, cls, bbox, M);
+    const RegionRecords rg(regions, (flags & CNNACC_FLAG_RECTS) != 0);
+    const std::string why = merge_call_error(rg, n, n_frames, scores, cls, bbox, M);
     if (!why.empty()) return fail(h, CNNACC_ERR_ARG, why);
     if (n_frames == 0) return CNNACC_OK;
     CU(h, cudaSetDevice(h->device));
@@ -1563,7 +1566,7 @@ static int merge_impl(cnnacc_handle* h, const int32_t* regions, int64_t n, int64
         REQUIRE_ALIGNED(h, M.det_score, 4, "det_score");
         DescBuf* db = nullptr;
         if ((rc = desc_acquire(h, n, &db, n_frames + 1))) return rc;
-        if (n) std::memcpy(db->host, regions, (size_t)n * sizeof(int4));
+        fill_desc(db->host, rg, n);
         std::memcpy(db->first_host, M.first.data(), first_bytes);
         if (n) CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
         CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, first_bytes, cudaMemcpyHostToDevice, h->stream));
@@ -1580,11 +1583,11 @@ static int merge_impl(cnnacc_handle* h, const int32_t* regions, int64_t n, int64
     cudaStream_t st = h->st_k;
     DescBuf* db = nullptr;
     if ((rc = desc_acquire(h, n, &db, n_frames + 1))) return rc;
-    if (n) std::memcpy(db->host, regions, (size_t)n * sizeof(int4));
+    fill_desc(db->host, rg, n);
     std::memcpy(db->first_host, M.first.data(), first_bytes);
     if (n) CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, st));
     CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, first_bytes, cudaMemcpyHostToDevice, st));
-    const std::vector<int64_t> blocks = frame_aligned_blocks([&](int64_t r) -> int64_t { return regions[4 * r]; }, n, kPredSuper);
+    const std::vector<int64_t> blocks = frame_aligned_blocks([&](int64_t r) { return rg.frame(r); }, n, kPredSuper);
     int64_t most = 0;
     for (size_t k = 1; k < blocks.size(); k++) most = std::max(most, blocks[k] - blocks[k - 1]);
     if (most && (rc = grow(h, &h->d_mpred, &h->cap_mpred, (size_t)most * 24))) return rc;
@@ -1592,7 +1595,7 @@ static int merge_impl(cnnacc_handle* h, const int32_t* regions, int64_t n, int64
     int64_t fa = 0;
     for (size_t k = 0; k < std::max<size_t>(1, blocks.size() - 1); k++) {
         const int64_t b0 = blocks[k], m = blocks.size() > 1 ? blocks[k + 1] - b0 : 0;
-        const int64_t fb = b0 + m == n ? n_frames : regions[4 * (b0 + m)];
+        const int64_t fb = b0 + m == n ? n_frames : rg.frame(b0 + m);
         if (m) {
             CU(h, cudaMemcpyAsync(h->d_mpred, bbox + 4 * b0, (size_t)m * 16, cudaMemcpyHostToDevice, st));
             CU(h, cudaMemcpyAsync(h->d_mpred + (size_t)m * 16, scores + b0, (size_t)m * 4, cudaMemcpyHostToDevice, st));
@@ -1638,21 +1641,22 @@ int cnnacc_merge_regions_host(const int32_t* regions, int64_t n_regions, int64_t
                               int32_t* det_cls, float* det_score, float* det_box, uint32_t flags) {
     if (flags & CNNACC_FLAG_DEVICE_PTRS) return CNNACC_ERR_ARG;
     MergeSpec M = make_merge_spec(score_min, iou_max, max_det, n_det, det_region, det_cls, det_score, det_box, flags);
-    if (!merge_call_error(regions, n_regions, n_frames, scores, cls, bbox, M).empty()) return CNNACC_ERR_ARG;
+    const RegionRecords rg(regions, (flags & CNNACC_FLAG_RECTS) != 0);
+    if (!merge_call_error(rg, n_regions, n_frames, scores, cls, bbox, M).empty()) return CNNACC_ERR_ARG;
     const size_t D = (size_t)max_det;
     for (int64_t f = 0; f < n_frames; f++)
-        n_det[f] = merge_frame_host(regions, scores, cls, bbox, M.first[f], M.first[f + 1] - M.first[f], score_min, iou_max, max_det,
+        n_det[f] = merge_frame_host(rg, scores, cls, bbox, M.first[f], M.first[f + 1] - M.first[f], score_min, iou_max, max_det,
                                     M.agnostic, det_region ? det_region + f * D : nullptr, det_cls ? det_cls + f * D : nullptr,
                                     det_score ? det_score + f * D : nullptr, det_box ? det_box + f * D * 4 : nullptr);
     return CNNACC_OK;
 }
 
-int cnnacc_region_plan_host(const int32_t* regions, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t* chunks, int cap) {
-    if (n_regions < 0 || n_frames < 0 || (n_regions > 0 && !regions) || !chunks || cap < 0) return CNNACC_ERR_ARG;
+static int region_plan_host(const RegionRecords& rg, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t* chunks, int cap) {
+    if (n_regions < 0 || n_frames < 0 || (n_regions > 0 && !rg.p) || !chunks || cap < 0) return CNNACC_ERR_ARG;
     int64_t bad;
-    if (region_error(regions, n_regions, n_frames, fh, fw, &bad)) return CNNACC_ERR_ARG;
+    if (region_error(rg, n_regions, n_frames, true, fh, fw, &bad)) return CNNACC_ERR_ARG;
     const std::vector<RegionChunk> plan =
-        make_region_plan([&](int64_t r) -> int64_t { return regions[4 * r]; }, n_regions, (size_t)fh * fw * 3, kPredSuper);
+        make_region_plan([&](int64_t r) { return rg.frame(r); }, n_regions, (size_t)fh * fw * 3, kPredSuper);
     if ((int64_t)plan.size() > cap) return CNNACC_ERR_ARG;
     for (size_t i = 0; i < plan.size(); i++) {
         chunks[4 * i] = plan[i].f0; chunks[4 * i + 1] = plan[i].f1; chunks[4 * i + 2] = plan[i].r0; chunks[4 * i + 3] = plan[i].r1;
@@ -1660,11 +1664,19 @@ int cnnacc_region_plan_host(const int32_t* regions, int64_t n_regions, int64_t n
     return (int)plan.size();
 }
 
+int cnnacc_region_plan_host(const int32_t* regions, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t* chunks, int cap) {
+    return region_plan_host(RegionRecords(regions, false), n_regions, n_frames, fh, fw, chunks, cap);
+}
+
+int cnnacc_rect_plan_host(const int32_t* regions, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t* chunks, int cap) {
+    return region_plan_host(RegionRecords(regions, true), n_regions, n_frames, fh, fw, chunks, cap);
+}
+
 int cnnacc_area_tab_host(int side, int* start, int* cnt, float* alpha, int taps_cap) {
     if (side < kRegionMinSide || side > kRegionMaxSide || !start || !cnt || !alpha || taps_cap < 1) return CNNACC_ERR_ARG;
     int taps = 0;
     for (int d = 0; d < kPrepOut; d++) {
-        const AreaTaps a = area_taps(side, d);
+        const AreaTaps a = area_taps(side, d, side % kPrepOut == 0);
         if (a.n > taps_cap) return CNNACC_ERR_ARG;
         taps = std::max(taps, a.n);
         start[d] = a.first; cnt[d] = a.n;

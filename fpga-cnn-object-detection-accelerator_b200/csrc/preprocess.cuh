@@ -35,10 +35,11 @@ struct AreaTabHost {
     std::vector<float> alpha;                  // [128][taps]
 };
 
-// The INTER_AREA taps of output index d for a square side S (128..8192): OpenCV's computeResizeAreaTab(ssize = S, dsize = 128,
-// scale = S/128.) for one d, in its order (double arithmetic, then float).  The taps are the consecutive source indices
-// first .. first+n-1; tap i weighs area_tap_weight(t, i).  Integer scales (S = 128 k) give k taps of weight 1 (their kernels
-// sum integers instead).  Host (make_area_tab, cnnacc_area_tab_host) and device (regions.cuh) get the same bits: scale = S/128
+// The INTER_AREA taps of output index d for a side S (128..8192) of the source: OpenCV's computeResizeAreaTab(ssize = S,
+// dsize = 128, scale = S/128.) for one d, in its order (double arithmetic, then float).  The taps are the consecutive source
+// indices first .. first+n-1; tap i weighs area_tap_weight(t, i).  `box`: the source takes OpenCV's integer path
+// (ResizeAreaFast), which OpenCV decides from both sides (both multiples of 128); then S = 128 k gives k taps of weight 1
+// (the kernels sum integers instead).  Without it an integer S still takes the table: k taps of (float)(1.0 / k).  Host (make_area_tab, cnnacc_area_tab_host) and device (regions.cuh) get the same bits: scale = S/128
 // is exact, so are d * scale, fsx1 + scale and S - fsx1 for S <= 8192 (at most 20 significant bits) -- an FMA the compiler
 // forms from them rounds nothing -- ceil / floor / min are exact, and the three divisions are correctly rounded in IEEE double
 // on both sides.  Up to 65 taps per output at S = 8191: the weights stay three scalars (first partial, 1/cell, last partial)
@@ -49,9 +50,9 @@ struct AreaTaps {
     float a_head, a_mid, a_tail;
 };
 
-__host__ __device__ __forceinline__ AreaTaps area_taps(int S, int d) {
+__host__ __device__ __forceinline__ AreaTaps area_taps(int S, int d, bool box) {
     AreaTaps t;
-    if (S % kPrepOut == 0) {
+    if (box) {
         const int k = S / kPrepOut;
         t.first = d * k; t.n = k; t.head = t.tail = false; t.a_head = t.a_mid = t.a_tail = 1.f;
         return t;
@@ -91,7 +92,7 @@ inline AreaTabHost make_area_tab(int S) {
     }
     t.alpha.assign((size_t)kPrepOut * t.taps, 1.f);
     for (int d = 0; d < kPrepOut; d++) {
-        const AreaTaps a = area_taps(S, d);
+        const AreaTaps a = area_taps(S, d, S % kPrepOut == 0);
         t.start[d] = a.first; t.cnt[d] = a.n;
         if (t.mode == kPrepFrac)
             for (int i = 0; i < t.taps; i++) t.alpha[(size_t)d * t.taps + i] = i < a.n ? area_tap_weight(a, i) : 0.f;

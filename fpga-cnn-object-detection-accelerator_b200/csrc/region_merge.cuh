@@ -15,7 +15,7 @@ namespace cnnacc {
 constexpr int kMergeThreads = 256;
 
 struct MergeArgs {
-    const int4* desc;               // [r] (frame, x, y, side), indexed by region r of the call
+    const int4* desc;               // [r] (frame, x, y, wh) as in regions.cuh, indexed by region r of the call
     const long long* first;         // [F + 1] region ranges of this launch's F frames (absolute region indices)
     long long r_pred0;              // region index of element 0 of score / cls / bbox
     const float* score;             // score of region r: score[(r - r_pred0) * score_stride + (score_by_cls ? cls : 0)]
@@ -92,7 +92,7 @@ merge_regions_kernel(const MergeArgs A)
             const int4 d = __ldg(A.desc + r);
             const int32_t* b = A.bbox + 4 * (r - A.r_pred0);
             MergeCand m;
-            m.b = merge_box(d.y, d.z, d.w, __ldg(b), __ldg(b + 1), __ldg(b + 2), __ldg(b + 3));
+            m.b = merge_box(d.y, d.z, desc_w(d.w), desc_h(d.w), __ldg(b), __ldg(b + 1), __ldg(b + 2), __ldg(b + 3));
             m.area = merge_area(m.b);
             m.cls = __ldg(A.cls + (r - A.r_pred0));
             m.idx = idx;

@@ -2,10 +2,10 @@
 // (region_merge.cuh) and the CPU replay (merge_frame_host, cnnacc_merge_regions_host).
 //
 // Per frame, independently: clamp every box coordinate to [0, 127]; map it to the frame exactly, in 1/128 pixel as int64
-// (X = 128 x + b side); candidates are the regions with score >= score_min (never a NaN score); order them by score
+// (X = 128 x + bx w, Y = 128 y + by h for the region (x, y, w, h); w = h = side for a square); candidates are the regions with score >= score_min (never a NaN score); order them by score
 // descending, then region index ascending (-0.0 and +0.0 are equal); walk them in that order and keep a candidate unless an
 // already-kept box of the same class (any class with CNNACC_FLAG_CLASS_AGNOSTIC) has IoU > iou_max with it; stop at max_det.
-// IoU = (double)inter / (double)union from exact int64 areas (0 when union == 0).  With side <= 8192 a box spans at most
+// IoU = (double)inter / (double)union from exact int64 areas (0 when union == 0).  With w, h <= 8192 a box spans at most
 // 127 * 8192 < 2^20 units a side, so inter and union are below 2^40, both exact doubles: one IEEE division gives the same
 // bits on the device and on the host (the build has no fast-math).
 #pragma once
@@ -13,6 +13,7 @@
 #include <cstdint>
 #include <cstring>
 #include <vector>
+#include "region_plan.h"
 
 #if defined(__CUDACC__)
 #define CNNACC_MERGE_HD __host__ __device__ __forceinline__
@@ -30,13 +31,13 @@ struct MergeBox { long long x1, y1, x2, y2; };
 
 CNNACC_MERGE_HD int merge_clamp(int v) { return v < 0 ? 0 : (v > 127 ? 127 : v); }
 
-// box (x1, y1, x2, y2) on the 128 grid of the region (x, y, side), clamped, in 1/128 frame pixels
-CNNACC_MERGE_HD MergeBox merge_box(int x, int y, int side, int bx1, int by1, int bx2, int by2) {
+// box (x1, y1, x2, y2) on the 128 grid of the region (x, y, w, h), clamped, in 1/128 frame pixels
+CNNACC_MERGE_HD MergeBox merge_box(int x, int y, int w, int h, int bx1, int by1, int bx2, int by2) {
     MergeBox m;
-    m.x1 = 128LL * x + (long long)merge_clamp(bx1) * side;
-    m.y1 = 128LL * y + (long long)merge_clamp(by1) * side;
-    m.x2 = 128LL * x + (long long)merge_clamp(bx2) * side;
-    m.y2 = 128LL * y + (long long)merge_clamp(by2) * side;
+    m.x1 = 128LL * x + (long long)merge_clamp(bx1) * w;
+    m.y1 = 128LL * y + (long long)merge_clamp(by1) * h;
+    m.x2 = 128LL * x + (long long)merge_clamp(bx2) * w;
+    m.y2 = 128LL * y + (long long)merge_clamp(by2) * h;
     return m;
 }
 
@@ -108,9 +109,9 @@ const char* merge_frame_ranges(FrameOf frame_of, int64_t n, int64_t n_frames, st
     return nullptr;
 }
 
-// The merge rule on the CPU for one frame: regions r0 .. r0 + cnt - 1, region r at (x[r], y[r], side[r]) through `desc`
-// ((frame, x, y, side) int32 quadruples), score[r], cls[r], bbox[r][4].  Outputs hold max_det rows; returns n_det.
-inline int merge_frame_host(const int32_t* desc, const float* score, const int32_t* cls, const int32_t* bbox, int64_t r0,
+// The merge rule on the CPU for one frame: regions r0 .. r0 + cnt - 1 of `rg`, score[r], cls[r], bbox[r][4].  Outputs hold
+// max_det rows; returns n_det.
+inline int merge_frame_host(const RegionRecords& rg, const float* score, const int32_t* cls, const int32_t* bbox, int64_t r0,
                             int64_t cnt, float score_min, float iou_max, int max_det, bool agnostic, int32_t* det_region,
                             int32_t* det_cls, float* det_score, float* det_box) {
     std::vector<unsigned long long> keys;
@@ -124,9 +125,8 @@ inline int merge_frame_host(const int32_t* desc, const float* score, const int32
     for (unsigned long long k : keys) {
         if ((int)kept.size() >= max_det) break;
         const int64_t r = r0 + merge_key_index(k);
-        const int32_t* d = desc + 4 * r;
         const int32_t* b = bbox + 4 * r;
-        const MergeBox m = merge_box(d[1], d[2], d[3], b[0], b[1], b[2], b[3]);
+        const MergeBox m = merge_box(rg.x(r), rg.y(r), rg.w(r), rg.h(r), b[0], b[1], b[2], b[3]);
         const long long area = merge_area(m);
         bool sup = false;
         for (size_t j = 0; j < kept.size() && !sup; j++)

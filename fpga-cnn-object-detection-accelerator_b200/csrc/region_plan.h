@@ -1,6 +1,7 @@
 // region_plan.h -- checks of a region array and the staging plan of a host-pointer region call (cnnacc_detect_regions /
-// cnnacc_preprocess_regions; cnnacc_detect_frames / cnnacc_preprocess_bgr are the case of one centre region per frame).  Pure
-// host arithmetic, no CUDA; tests/test_regions_cpu.py replays it through cnnacc_region_plan_host.
+// cnnacc_preprocess_regions; cnnacc_detect_frames / cnnacc_preprocess_bgr are the case of one centre region per frame).  Host
+// arithmetic, plus the decoders of the descriptor's size field that the kernels share; tests/test_regions_cpu.py and tests/test_rect_regions_cpu.py replay it through
+// cnnacc_region_plan_host and cnnacc_rect_plan_host.
 //
 // A chunk stages the frames [f0, f1) with one copy and runs the regions [r0, r1) on them.  Its frames are a run of
 // consecutive frames that regions reference, at most about 16 MiB of them, so a frame that no region references never
@@ -21,17 +22,46 @@ namespace cnnacc {
 constexpr int kRegionMinSide = 128, kRegionMaxSide = 8192;
 constexpr size_t kRegionChunkBytes = (size_t)16 << 20;     // frames staged per chunk, as the centre-crop path always did
 
-// nullptr when regions [n][4] = (frame, x, y, side) are valid for n_frames frames of fh x fw, else why not; *bad = the index
-// of the first offending region.
-inline const char* region_error(const int32_t* rg, int64_t n, int64_t n_frames, int fh, int fw, int64_t* bad) {
+#if defined(__CUDACC__)
+#define CNNACC_REGION_HD __host__ __device__ __forceinline__
+#else
+#define CNNACC_REGION_HD inline
+#endif
+
+// The caller's region records, the one place that knows their two formats: [n][4] squares (frame, x, y, side), or with
+// CNNACC_FLAG_RECTS [n][5] rectangles (frame, x, y, w, h).  A square is the rectangle w = h = side, so everything past this
+// reads (frame, x, y, w, h).  The device descriptor of every region is the int4 (frame, x, y, wh) with wh = w | h << 16
+// (w, h <= 8192 fit 14 bits), where h = 0 stands for h = w: a square's record is its descriptor as it is, so square calls
+// copy their records as before instead of re-packing them.
+CNNACC_REGION_HD int desc_w(int wh) { return wh & 0xffff; }
+CNNACC_REGION_HD int desc_h(int wh) { return (wh >> 16) ? (wh >> 16) : (wh & 0xffff); }
+
+struct RegionRecords {
+    const int32_t* p;
+    int stride;                                            // 4 (squares) or 5 (rectangles)
+    RegionRecords(const int32_t* p_, bool rects) : p(p_), stride(rects ? 5 : 4) {}
+    int64_t frame(int64_t r) const { return p[stride * r]; }
+    int32_t x(int64_t r) const { return p[stride * r + 1]; }
+    int32_t y(int64_t r) const { return p[stride * r + 2]; }
+    int32_t w(int64_t r) const { return p[stride * r + 3]; }
+    int32_t h(int64_t r) const { return p[stride * r + stride - 1]; }
+    int32_t wh(int64_t r) const { return stride == 4 ? w(r) : w(r) | h(r) << 16; }   // the descriptor's, for checked records
+};
+
+// nullptr when the regions' frame, position and sizes are valid for n_frames frames and, when `sized` (the merging calls have
+// no frame size), they lie inside frames of fh x fw (in int64: x + w cannot wrap), else why not; *bad = the index of the
+// first offending region.
+inline const char* region_error(const RegionRecords& rg, int64_t n, int64_t n_frames, bool sized, int fh, int fw, int64_t* bad) {
     *bad = -1;
     for (int64_t r = 0; r < n; r++) {
-        const int64_t f = rg[4 * r], x = rg[4 * r + 1], y = rg[4 * r + 2], s = rg[4 * r + 3];
+        const int64_t f = rg.frame(r), x = rg.x(r), y = rg.y(r), w = rg.w(r), h = rg.h(r);
         *bad = r;
         if (f < 0 || f >= n_frames) return "frame index outside [0, n_frames)";
-        if (s < kRegionMinSide || s > kRegionMaxSide) return "side outside 128..8192";
-        if (x < 0 || y < 0 || x + s > fw || y + s > fh) return "region outside its frame";
-        if (r > 0 && f < rg[4 * (r - 1)]) return "frame indices decrease (group the regions by frame, in non-decreasing order)";
+        if (w < kRegionMinSide || w > kRegionMaxSide || h < kRegionMinSide || h > kRegionMaxSide)
+            return rg.stride == 4 ? "side outside 128..8192" : "width or height outside 128..8192";
+        if (x < 0 || y < 0) return sized ? "region outside its frame" : "negative position";
+        if (sized && (x + w > fw || y + h > fh)) return "region outside its frame";
+        if (r > 0 && f < rg.frame(r - 1)) return "frame indices decrease (group the regions by frame, in non-decreasing order)";
     }
     *bad = -1;
     return nullptr;

@@ -1,21 +1,27 @@
-// regions.cuh -- the pre-processing of preprocess.cuh on caller-chosen square regions of BGR frames, many sides in one launch.
+// regions.cuh -- the pre-processing of preprocess.cuh on caller-chosen regions of BGR frames, many sizes in one launch.
 //
-// Region r is the square frames[frame][y:y+side, x:x+side, :] with side 128..8192; its output is exactly what the centre-crop
-// path gives for that square cut out as a frame of its own (a square is its own centre crop): BGR2GRAY in OpenCV's 15-bit
-// fixed point, then INTER_AREA to 128x128 on whichever of the four paths the side selects (copy, 2x2, k x k, fractional).
-// The INTER_AREA taps are computed in the kernel from the side (area_taps, preprocess.cuh), so one launch mixes any sides and
-// nothing is uploaded per side.
+// Region r is the rectangle frames[frame][y:y+h, x:x+w, :] with w and h 128..8192 (a square region is w == h); its output is
+// exactly cv2.resize(cv2.cvtColor(rect, COLOR_BGR2GRAY), (128, 128), INTER_AREA): BGR2GRAY in OpenCV's 15-bit fixed point,
+// then INTER_AREA on the path OpenCV picks from both scales w/128 and h/128 (resize.cpp):
+//   * w and h both multiples of 128 (kx = w/128, ky = h/128): the integer box sum of kx x ky pixels, then
+//       kx = ky = 1 : copy;   kx = ky = 2 : (sum + 2) >> 2;   otherwise : saturate_cast<uchar>(float(sum) * (1.f / (kx*ky)))
+//   * otherwise: ResizeArea's float accumulation with x taps from computeResizeAreaTab(w) and y taps from
+//     computeResizeAreaTab(h); an axis that is an integer multiple takes the table too (kx taps of (float)(1.0/kx)).
+// For a square this is what the centre-crop path gives for the square cut out as a frame of its own.  The INTER_AREA taps are
+// computed in the kernel from the sizes (area_taps, preprocess.cuh), so one launch mixes any sizes and nothing is uploaded
+// per size.
 //
 // Work split as preprocess_bgr_kernel: one CTA of 128 threads per (output row, region), thread = output column.
 #pragma once
 #include "preprocess.cuh"
+#include "region_plan.h"
 
 namespace cnnacc {
 
 struct RegionPrep {
     const uint8_t* frames;        // [..][fh][fw][3] BGR
     uint8_t* out;                 // [n][128][128]
-    const int4* desc;             // [n] (frame, x, y, side), frame relative to `frames`
+    const int4* desc;             // [n] (frame, x, y, wh), frame relative to `frames` (wh: desc_w / desc_h, region_plan.h)
     int fh, fw;
 };
 
@@ -25,12 +31,13 @@ preprocess_regions_kernel(const RegionPrep P)
     const int dx = threadIdx.x, dy = blockIdx.x;
     const int r = blockIdx.y;
     const int4 d = __ldg(P.desc + r);
-    const int frame = d.x, x0 = d.y, y0 = d.z, S = d.w;
-    const AreaTaps tx = area_taps(S, dx), ty = area_taps(S, dy);
+    const int frame = d.x, x0 = d.y, y0 = d.z, W = desc_w(d.w), H = desc_h(d.w);
+    const bool box = W % kPrepOut == 0 && H % kPrepOut == 0;
+    const AreaTaps tx = area_taps(W, dx, box), ty = area_taps(H, dy, box);
     const uint8_t* src = P.frames + (size_t)frame * P.fh * P.fw * 3 + ((size_t)(y0 + ty.first) * P.fw + (x0 + tx.first)) * 3;
     const size_t pitch = (size_t)P.fw * 3;
     int v;
-    if (S % kPrepOut != 0) {
+    if (!box) {
         float sum = 0.f;
         for (int j = 0; j < ty.n; j++) {
             const uint8_t* row = src + j * pitch;
@@ -41,15 +48,15 @@ preprocess_regions_kernel(const RegionPrep P)
         }
         v = min(max(__float2int_rn(sum), 0), 255);
     } else {
-        const int k = S / kPrepOut;
+        const int kx = W / kPrepOut, ky = H / kPrepOut;
         int tot = 0;
-        for (int j = 0; j < k; j++) {
+        for (int j = 0; j < ky; j++) {
             const uint8_t* row = src + j * pitch;
-            for (int i = 0; i < k; i++) tot += bgr2gray(row + 3 * i);
+            for (int i = 0; i < kx; i++) tot += bgr2gray(row + 3 * i);
         }
-        if (k == 1)      v = tot;
-        else if (k == 2) v = (tot + 2) >> 2;
-        else             v = min(max(__float2int_rn(__fmul_rn((float)tot, 1.f / (float)(k * k))), 0), 255);
+        if (kx * ky == 1)           v = tot;
+        else if (kx == 2 && ky == 2) v = (tot + 2) >> 2;
+        else                         v = min(max(__float2int_rn(__fmul_rn((float)tot, 1.f / (float)(kx * ky))), 0), 255);
     }
     P.out[((size_t)r * kPrepOut + dy) * kPrepOut + dx] = (uint8_t)v;
 }

@@ -217,6 +217,26 @@ int cnnacc_preprocess_regions(cnnacc_handle *h, const uint8_t *frames, int64_t n
 int cnnacc_detect_regions(cnnacc_handle *h, const uint8_t *frames, int64_t n_frames, int fh, int fw,
                           const int32_t *regions, int64_t n_regions, uint8_t *gray128,
                           float *probs, int32_t *cls, int32_t *bbox, uint32_t flags);
+/* ---- rectangles: CNNACC_FLAG_RECTS -----------------------------------------------------------------------------------
+ * With CNNACC_FLAG_RECTS, `regions` of preprocess_regions, detect_regions, detect_objects, merge_regions and
+ * merge_regions_host is [n_regions][5] int32 (frame, x, y, w, h): the rectangle frames[frame][y:y+h, x:x+w, :], w and h each
+ * 128..8192 (a square is w == h).  Everything else is as for squares.  Its gray128 is, byte for byte,
+ *     cv2.resize(cv2.cvtColor(rect, COLOR_BGR2GRAY), (128, 128), interpolation=INTER_AREA)
+ * with OpenCV's INTER_AREA arithmetic picked from both scales, kx = w/128 and ky = h/128 (csrc/regions.cuh):
+ *   w == h == 128                          copy
+ *   w, h multiples of 128, kx = ky = 2     (sum of 4 + 2) >> 2
+ *   w, h multiples of 128, other kx, ky    rint(float(kx x ky box sum) * (1.f / float(kx*ky))), clamped to 0..255
+ *   otherwise (an axis is fractional)      ResizeArea's float accumulation, x taps from computeResizeAreaTab(w) and y taps
+ *                                          from computeResizeAreaTab(h); an integer axis takes that table too (kx taps of
+ *                                          (float)(1.0/kx) each)
+ * cls / probs / bbox are what infer_batch gives for that gray128; boxes stay on the rectangle's 128 grid.  The merge maps
+ * them with X = 128 x + clamp(bx) w and Y = 128 y + clamp(by) h.
+ *   -2, nothing launched: as for squares with w and h in place of side -- w or h outside 128..8192, x < 0, y < 0,
+ *       x + w > fw or y + h > fh (in 64-bit arithmetic), a frame index outside [0, n_frames), frame indices that decrease;
+ *       for the merging calls (no frame size): a frame outside [0, n_frames), x < 0, y < 0, w or h outside 128..8192.
+ * Regions below 128 on an axis (OpenCV upsamples them) are refused, as for squares.  One call takes squares or rectangles,
+ * not both: a square can be written as the rectangle w == h. */
+#define CNNACC_FLAG_RECTS           0x100u /* region calls: regions are [n][5] (frame, x, y, w, h) */
 /* ---- merging region detections into per-frame detections --------------------------------------------------------------
  * The rule (csrc/region_merge.h), per frame, independently: clamp every box coordinate to [0, 127]; map the box to the frame
  * exactly, in 1/128 pixel (X = 128 x + bx * side, the same for y); candidates are the regions with score >= score_min (a NaN
@@ -254,6 +274,8 @@ int cnnacc_merge_regions_host(const int32_t *regions, int64_t n_regions, int64_t
  * [chunks[4i], chunks[4i+1]) with one copy and runs regions [chunks[4i+2], chunks[4i+3]) on them.  Returns the number of chunks
  * (<= cap), or -2 for a region array the real call refuses, or when cap is too small.  No GPU needed. */
 int cnnacc_region_plan_host(const int32_t *regions, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t *chunks, int cap);
+/* The same for [n_regions][5] rectangles (frame, x, y, w, h), with the refusals of CNNACC_FLAG_RECTS. */
+int cnnacc_rect_plan_host(const int32_t *regions, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t *chunks, int cap);
 /* Host-only view of the INTER_AREA taps the kernels use for one crop side (128..8192): output index d reads source indices
  * start[d] .. start[d]+cnt[d]-1 with weights alpha[d*taps_cap + i] (zero beyond cnt[d]; weight 1 at integer scales, whose
  * kernels sum integers).  Returns the largest cnt, or -2 when it exceeds taps_cap.  No GPU needed. */

@@ -13,8 +13,13 @@ frame with grid (a) against detect_frames of one frame.  The card's name and pow
 --objects adds the merging calls: detect_objects (detect_regions + per-frame greedy NMS on the GPU) host-fed and
 device-resident beside detect_regions for grid (a) and pyramid (b), merge_regions alone on device tensors at 63 and at
 2925 regions per frame (side 128, stride 8), and batch-1 p50 / p99 of detect_objects on one VGA frame with grid (a).
+--rects measures rectangle regions (frame, x, y, w, h) instead: detect_regions and detect_objects host-fed and
+device-resident on
+  aspect  (d) 157 rectangles per frame: 128x128, 256x128 and 128x256 at stride 64 (grid_rects)
+  random  (e) 48 seeded random rectangles per frame, 128..640 wide and 128..480 tall
+beside grid (a) as squares in the same run, and batch-1 p50 / p99 of one VGA frame with aspect (d).
 
-    python tools/regions_throughput.py [--frames 2048] [--dev-frames 1024] [--seconds 2] [--out FILE]
+    python tools/regions_throughput.py [--frames 2048] [--dev-frames 1024] [--seconds 2] [--objects | --rects] [--out FILE]
 """
 import argparse
 import ctypes
@@ -83,6 +88,7 @@ def main():
     ap.add_argument("--seconds", type=float, default=2.0)
     ap.add_argument("--out", default=None)
     ap.add_argument("--objects", action="store_true", help="measure the merging calls (detect_objects / merge_regions)")
+    ap.add_argument("--rects", action="store_true", help="measure rectangle regions (detect_regions / detect_objects)")
     a = ap.parse_args()
     import torch
     dev = torch.device("cuda", 0)
@@ -106,6 +112,9 @@ def main():
 
     if a.objects:
         objects(a, acc, host, emit)
+        return write(a, lines)
+    if a.rects:
+        rects(a, acc, host, emit)
         return write(a, lines)
 
     # host-fed
@@ -224,6 +233,54 @@ def objects(a, acc, host, emit):
     grid1 = fc.grid_regions(1, H, W, 128, 64)
     for path, fn in (("detect_objects_grid63", lambda: acc.detect_objects(one, grid1, **kw)),
                      ("detect_regions_grid63", lambda: acc.detect_regions(one, grid1))):
+        for _ in range(50):
+            fn()
+        ts = []
+        for _ in range(2000):
+            t0 = time.perf_counter()
+            fn()
+            ts.append(time.perf_counter() - t0)
+        ts = np.array(ts) * 1e6
+        emit({"what": "batch1", "path": path, "p50_us": float(np.percentile(ts, 50)), "p99_us": float(np.percentile(ts, 99))})
+
+
+def rect_workloads(n):
+    rng = np.random.default_rng(6)
+    k = 48
+    w, h = rng.integers(128, W + 1, n * k), rng.integers(128, H + 1, n * k)
+    rnd = np.stack([np.repeat(np.arange(n), k), rng.integers(0, W + 1 - w), rng.integers(0, H + 1 - h), w, h], 1).astype(np.int32)
+    return {"aspect": fc.grid_rects(n, H, W, [(128, 128), (256, 128), (128, 256)], 64), "random": rnd,
+            "grid_squares": workloads(n)["grid"]}
+
+
+def rects(a, acc, host, emit):
+    """detect_regions and detect_objects on rectangles, host-fed and device-resident, with grid (a) as squares beside them."""
+    import torch
+    dev = torch.device("cuda", 0)
+    kw = dict(score_min=0.0, iou_max=0.5, max_det=100)
+    for name, reg in rect_workloads(a.frames).items():
+        for path, fn in (("detect_regions", lambda: acc.detect_regions(host, reg)),
+                         ("detect_objects", lambda: acc.detect_objects(host, reg, **kw))):
+            per_s = wall_rate(fn, a.seconds)
+            emit({"what": "host_fed", "path": path, "workload": name, "regions_per_frame": len(reg) / a.frames,
+                  "frames_per_s": per_s * a.frames, "regions_per_s": per_s * len(reg)})
+    t = torch.from_numpy(host[:a.dev_frames]).to(dev)
+    nd = a.dev_frames
+    for name, reg in rect_workloads(nd).items():
+        for path, fn in (("detect_regions", lambda: acc.detect_regions(t, reg)),
+                         ("detect_objects", lambda: acc.detect_objects(t, reg, **kw))):
+            ms = event_ms(fn, a.seconds)
+            emit({"what": "device_resident", "path": path, "workload": name, "regions": len(reg), "ms": ms,
+                  "frames_per_s": nd / ms * 1e3, "regions_per_s": len(reg) / ms * 1e3})
+        pre_ms = event_ms(lambda: acc.preprocess_regions(t, reg), a.seconds)
+        emit({"what": "device_resident", "path": "preprocess_regions", "workload": name, "regions": len(reg), "ms": pre_ms,
+              "regions_per_s": len(reg) / pre_ms * 1e3})
+    del t
+    torch.cuda.synchronize()
+    one = np.ascontiguousarray(host[:1])
+    aspect1 = rect_workloads(1)["aspect"]
+    for path, fn in (("detect_regions_aspect157", lambda: acc.detect_regions(one, aspect1)),
+                     ("detect_objects_aspect157", lambda: acc.detect_objects(one, aspect1, **kw))):
         for _ in range(50):
             fn()
         ts = []
