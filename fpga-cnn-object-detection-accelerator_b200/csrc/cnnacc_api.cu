@@ -7,10 +7,12 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <system_error>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "conv_direct.cuh"
@@ -41,21 +43,55 @@ constexpr size_t kBramBytes = 16 * 4096 + 32 * 1024 + 64 * 256;   // 112-channel
 constexpr int64_t kRegionLaunch = 1024;         // host-pointer region calls: regions per launch (16 MiB of gray per slot)
 constexpr int kDescRing = 4;                    // region-descriptor buffers in flight
 
+// ---- owners of the handle's CUDA resources: move-only, the destructor frees what they hold ------------------------------
+
+enum class Mem { kDevice, kPinned, kMapped };   // cudaMalloc / cudaHostAlloc default / cudaHostAlloc mapped
+
+// cap elements of T at p, or nothing; grow() (below) is the one place that allocates one.
+template <class T, Mem K = Mem::kDevice>
+struct Buf {
+    T* p = nullptr;
+    size_t cap = 0;
+    Buf() = default;
+    Buf(Buf&& o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    Buf& operator=(Buf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+    ~Buf() { release(); }
+    // frees the allocation; the buffer is empty afterwards whatever the free returned
+    cudaError_t release() {
+        const cudaError_t e = !p ? cudaSuccess : K == Mem::kDevice ? cudaFree(p) : cudaFreeHost(p);
+        p = nullptr; cap = 0;
+        return e;
+    }
+};
+
+// A CUDA event or stream, created by create(flags).
+template <class T, cudaError_t (*Create)(T*, unsigned), cudaError_t (*Destroy)(T)>
+struct Owned {
+    T raw = nullptr;
+    Owned() = default;
+    Owned(Owned&& o) noexcept : raw(std::exchange(o.raw, nullptr)) {}
+    Owned& operator=(Owned&& o) noexcept { std::swap(raw, o.raw); return *this; }
+    ~Owned() { if (raw) Destroy(raw); }
+    cudaError_t create(unsigned flags) { return Create(&raw, flags); }
+    operator T() const { return raw; }
+};
+using Event = Owned<cudaEvent_t, cudaEventCreateWithFlags, cudaEventDestroy>;
+using Stream = Owned<cudaStream_t, cudaStreamCreateWithFlags, cudaStreamDestroy>;
+
 // Pinned host and device copies of one call's region descriptors (and, for the merging calls, of its per-frame region
 // ranges); ev is recorded after the call's last launch that reads them.
 struct DescBuf {
-    int4 *host = nullptr, *dev = nullptr;
-    size_t cap = 0;
-    long long *first_host = nullptr, *first_dev = nullptr;
-    size_t cap_first = 0;
-    cudaEvent_t ev = nullptr;
+    Buf<int4, Mem::kPinned> host;
+    Buf<int4> dev;
+    Buf<long long, Mem::kPinned> first_host;
+    Buf<long long> first_dev;
+    Event ev;
 };
 
 struct Slot {
-    cudaEvent_t ev_in = nullptr, ev_k = nullptr, ev_out = nullptr;   // H2D landed / kernels done / D2H drained
-    uint8_t *d_in = nullptr, *d_out = nullptr;
-    int32_t *d_cls = nullptr, *d_bbox = nullptr;            // cnnacc_cam_bbox_batch's classes in and boxes out
-    size_t cap_in = 0, cap_out = 0, cap_pred = 0;
+    Event ev_in, ev_k, ev_out;                  // H2D landed / kernels done / D2H drained
+    Buf<uint8_t> d_in, d_out;
+    Buf<int32_t> d_cls, d_bbox;                 // cnnacc_cam_bbox_batch's classes in and boxes out
 };
 
 std::string g_create_error;
@@ -63,58 +99,62 @@ std::atomic<int64_t> g_pdl_seq{0};              // programmatic conv-stack launc
 
 }  // namespace
 
+// No user-provided default constructor: `new cnnacc_handle()` zero-initialises the members without an initialiser
+// (fused's weight arrays, one_map).
 struct cnnacc_handle {
     int device = 0;
-    cudaStream_t own_stream = nullptr, stream = nullptr;
-    cudaStream_t st_h2d = nullptr, st_k = nullptr, st_d2h = nullptr;   // one stream per engine for host-pointer batches
-    cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_a = nullptr, ev_b = nullptr, ev_done = nullptr;
+    Stream own_stream;
+    cudaStream_t stream = nullptr;                  // own_stream or the caller's (cnnacc_set_stream)
+    Stream st_h2d, st_k, st_d2h;                    // one stream per engine for host-pointer batches
+    Event ev_t0, ev_t1, ev_a, ev_b, ev_done;
     int sm_count = 0;
     bool weights_loaded = false, fc_loaded = false, tail_attr_set = false;
     int shifts[3] = {2, 4, 6};                  // SHIFT_L0..2 defaults, pynq_inference.py:83-85
     bool acc24 = false;                         // accumulator width: false = int32 (arm_cnn.c:31), true = 24-bit wrap (accumulator.v:15)
     uint8_t wbin[CNNACC_WEIGHT_BYTES];
     // device-side weights
-    uint32_t* d_wdirect = nullptr; size_t wdirect_off[3] = {0, 0, 0};
+    Buf<uint32_t> d_wdirect; size_t wdirect_off[3] = {0, 0, 0};
     FusedWeights fused;                         // packed operands of the fused kernel (conv_fused.cuh)
-    float *d_fcw = nullptr, *d_fcb = nullptr; int n_cls = 0;
+    Buf<float> d_fcw, d_fcb; int n_cls = 0;
     float fcw_host[kMaxClasses * 1024], fcb_host[kMaxClasses];   // what d_fcw / d_fcb hold: sharded calls compare members
     // workspaces (grown on demand) for the per-layer path and for infer_batch
-    uint8_t *d_l0 = nullptr, *d_l1 = nullptr, *d_feat = nullptr;
-    size_t cap_l0 = 0, cap_l1 = 0, cap_feat = 0;
+    Buf<uint8_t> d_l0, d_l1, d_feat;
     Slot slots[kSlots];
     // pre-processing (preprocess.cuh): INTER_AREA weight table of the last crop side seen
     int prep_side = 0; AreaTabHost prep_tab;
-    int *d_prep_start = nullptr, *d_prep_cnt = nullptr; float* d_prep_alpha = nullptr; size_t cap_prep_alpha = 0;
-    uint8_t* d_gray = nullptr; size_t cap_gray = 0;
+    Buf<int> d_prep_start, d_prep_cnt; Buf<float> d_prep_alpha;
+    Buf<uint8_t> d_gray;
     DescBuf rdesc[kDescRing]; int rdesc_next = 0;   // region calls (regions_impl)
     // merging calls (region_merge.cuh): device predictions of detect_objects' device-pointer path, and the detections of
     // host-pointer merges on the device and in pinned memory
-    uint8_t* d_mpred = nullptr; size_t cap_mpred = 0;
-    uint8_t *d_det = nullptr, *h_det = nullptr; size_t cap_det = 0;
+    Buf<uint8_t> d_mpred;
+    Buf<uint8_t> d_det; Buf<uint8_t, Mem::kPinned> h_det;
     bool merge_attr_set = false;
     // load_image_any (pil_resize.cuh): Pillow coefficient tables of the last (H, W) seen, on the device
     int pil_h = 0, pil_w = 0, pil_kh = 0, pil_kw = 0;
-    int32_t *d_pil_kx = nullptr, *d_pil_bx = nullptr, *d_pil_ky = nullptr, *d_pil_by = nullptr;
-    uint8_t *d_pil_tmp = nullptr, *d_pil_in = nullptr, *d_pil_out = nullptr; size_t cap_pil_tmp = 0, cap_pil_in = 0, cap_pil_out = 0;
+    Buf<int32_t> d_pil_kx, d_pil_bx, d_pil_ky, d_pil_by;
+    Buf<uint8_t> d_pil_tmp, d_pil_in, d_pil_out;
     // the prediction block of host-pointer calls (PredBlock): device block the kernels write, pinned block it is copied to
-    uint8_t *d_pred = nullptr, *h_pred = nullptr;
-    size_t cap_pred = 0;                            // images the two blocks hold
+    Buf<uint8_t> d_pred; Buf<uint8_t, Mem::kPinned> h_pred;
     // single-image protocol state
-    uint8_t *h_img = nullptr, *h_bram = nullptr;    // pinned + mapped: the batch-1 path runs zero-copy on them
-    int *h_done = nullptr, *h_done_dev = nullptr;   // mapped completion word of the batch-1 path and its device address
+    Buf<uint8_t, Mem::kMapped> h_img, h_bram;       // the batch-1 path runs zero-copy on them
+    Buf<int, Mem::kMapped> h_done;                  // completion word of the batch-1 path
+    int* h_done_dev = nullptr;                      // its device address
     int done_seq = 0;
     uint8_t *h_img_dev = nullptr, *h_bram_dev = nullptr;   // their device addresses
     CUtensorMap one_map;                            // tensor map over h_img (1 image), encoded once
     bool one_map_ok = false;
-    uint8_t *d_img1 = nullptr, *d_bram = nullptr;
+    Buf<uint8_t> d_img1, d_bram;
     bool image_loaded = false, started = false;
     int64_t launches = 0;
     PdlChain pdl;                                   // overlapped back-to-back conv-stack launches (pdl_chain.h)
     // cnnacc_run_batch_async: completion events of the last kMaxPending submitted calls, and the ring position the staging
     // slots continue from (asynchronous calls share one continuous ring across calls)
-    cudaEvent_t ev_ticket[CNNACC_MAX_PENDING] = {};
+    Event ev_ticket[CNNACC_MAX_PENDING];
     int64_t next_ticket = 0, ring_ci = 0;
     std::string err;
+
+    ~cnnacc_handle() { fused_free(fused); }
 };
 
 namespace {
@@ -130,12 +170,21 @@ int fail(cnnacc_handle* h, int code, const std::string& msg) {
             return fail((h), CNNACC_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); \
     } while (0)
 
-int grow(cnnacc_handle* h, uint8_t** p, size_t* cap, size_t need) {
-    if (*cap >= need) return 0;
-    if (*p) CU(h, cudaFree(*p));
-    *p = nullptr; *cap = 0;
-    CU(h, cudaMalloc(p, need));
-    *cap = need;
+// Makes b hold at least n elements: nothing when it does already, otherwise free, then allocate exactly n -- never both at
+// once, which would double the peak of the 512 MiB per-layer workspaces.  Contents are not kept.  On failure b is empty.
+template <class T, Mem K>
+int grow(cnnacc_handle* h, Buf<T, K>& b, size_t n) {
+    if (n <= b.cap) return 0;
+    const size_t bytes = n * sizeof(T);
+    void* p = nullptr;
+    cudaError_t e = b.release();
+    if (e == cudaSuccess)
+        e = K == Mem::kDevice ? cudaMalloc(&p, bytes)
+                              : cudaHostAlloc(&p, bytes, K == Mem::kMapped ? cudaHostAllocMapped : cudaHostAllocDefault);
+    if (e != cudaSuccess)
+        return fail(h, CNNACC_ERR_CUDA, "growing a buffer to " + std::to_string(bytes) + " bytes: " + cudaGetErrorString(e));
+    b.p = static_cast<T*>(p);
+    b.cap = n;
     return 0;
 }
 
@@ -177,7 +226,7 @@ int launch_direct_layer(cnnacc_handle* h, cudaStream_t stream, int layer, const 
     // image and tile share gridDim.x (2^31-1); gridDim.y (65535) would overflow at 8192x8192 (256 x 256 layer-0 tiles)
     if (n * tiles_x * tiles_y > 0x7fffffffLL) return fail(h, CNNACC_ERR_ARG, "too many tiles in one launch");
     dim3 grid((unsigned)(n * tiles_x * tiles_y), 1u, (unsigned)(kLayers[layer].oc / kDirOcb));
-    conv3x3_pool_direct_kernel<<<grid, 256, 0, stream>>>(in, out, h->d_wdirect + h->wdirect_off[layer],
+    conv3x3_pool_direct_kernel<<<grid, 256, 0, stream>>>(in, out, h->d_wdirect.p + h->wdirect_off[layer],
                                                          kLayers[layer].ic, kLayers[layer].oc, H, W,
                                                          h->shifts[layer], tiles_x, tiles_x * tiles_y, h->acc24 ? 1 : 0);
     h->launches++;
@@ -251,14 +300,14 @@ int64_t chunk_images(int H, int W) {
 int ensure_maps(cnnacc_handle* h, int64_t n, int H, int W) {
     int rc;
     // per-layer path: the two intermediate maps
-    if ((rc = grow(h, &h->d_l0, &h->cap_l0, (size_t)n * 16 * (H / 2) * (W / 2)))) return rc;
-    if ((rc = grow(h, &h->d_l1, &h->cap_l1, (size_t)n * 32 * (H / 4) * (W / 4)))) return rc;
+    if ((rc = grow(h, h->d_l0, (size_t)n * 16 * (H / 2) * (W / 2)))) return rc;
+    if ((rc = grow(h, h->d_l1, (size_t)n * 32 * (H / 4) * (W / 4)))) return rc;
     return 0;
 }
 
 TailArgs make_tail(const cnnacc_handle* h, float* d_probs, int32_t* d_cls, int32_t* d_bbox, bool cls_given, uint32_t flags) {
     TailArgs A;
-    A.fc_w = h->d_fcw; A.fc_b = h->d_fcb; A.n_cls = h->n_cls;
+    A.fc_w = h->d_fcw.p; A.fc_b = h->d_fcb.p; A.n_cls = h->n_cls;
     A.want_logits = (flags & CNNACC_FLAG_LOGITS) ? 1 : 0;
     A.probs = d_probs; A.bbox_out = d_bbox;
     A.cls_out = cls_given ? nullptr : d_cls;
@@ -292,7 +341,7 @@ int infer_device(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_imgs, i
         return 0;
     }
     int rc;
-    if ((rc = conv_stack_device(h, stream, d_imgs, m, CNNACC_IMG, CNNACC_IMG, d_feat_ws, flags, h->d_l0, h->d_l1))) return rc;
+    if ((rc = conv_stack_device(h, stream, d_imgs, m, CNNACC_IMG, CNNACC_IMG, d_feat_ws, flags, h->d_l0.p, h->d_l1.p))) return rc;
     return launch_tail(h, stream, d_feat_ws, m, A);
 }
 bool infer_needs_feat_ws(bool want_feats, uint32_t flags) {
@@ -304,7 +353,7 @@ int launch_cam_upsampled(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d
                          int32_t* d_bbox, uint8_t* d_cam) {
     if (n == 0) return 0;
     static const ResampleTab tab = make_resample_tab();
-    cam_bbox_upsampled_kernel<<<(unsigned)n, 256, 0, stream>>>(d_feats, h->d_fcw, h->n_cls, d_cls, d_bbox, d_cam, tab);
+    cam_bbox_upsampled_kernel<<<(unsigned)n, 256, 0, stream>>>(d_feats, h->d_fcw.p, h->n_cls, d_cls, d_bbox, d_cam, tab);
     h->launches++;
     CU(h, cudaGetLastError());
     return 0;
@@ -317,22 +366,18 @@ int launch_preprocess(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_fr
     if (S != h->prep_side) {
         CU(h, cudaDeviceSynchronize());                  // nothing in flight may still be reading the old table
         h->prep_tab = make_area_tab(S);
-        if (!h->d_prep_start) CU(h, cudaMalloc(&h->d_prep_start, kPrepOut * sizeof(int)));
-        if (!h->d_prep_cnt) CU(h, cudaMalloc(&h->d_prep_cnt, kPrepOut * sizeof(int)));
-        const size_t ab = h->prep_tab.alpha.size() * sizeof(float);
-        if (ab > h->cap_prep_alpha) {
-            cudaFree(h->d_prep_alpha); h->d_prep_alpha = nullptr; h->cap_prep_alpha = 0;
-            CU(h, cudaMalloc(&h->d_prep_alpha, ab));
-            h->cap_prep_alpha = ab;
-        }
-        CU(h, cudaMemcpy(h->d_prep_start, h->prep_tab.start.data(), kPrepOut * sizeof(int), cudaMemcpyHostToDevice));
-        CU(h, cudaMemcpy(h->d_prep_cnt, h->prep_tab.cnt.data(), kPrepOut * sizeof(int), cudaMemcpyHostToDevice));
-        CU(h, cudaMemcpy(h->d_prep_alpha, h->prep_tab.alpha.data(), ab, cudaMemcpyHostToDevice));
+        const size_t na = h->prep_tab.alpha.size();
+        int rc;
+        if ((rc = grow(h, h->d_prep_start, kPrepOut)) || (rc = grow(h, h->d_prep_cnt, kPrepOut)) || (rc = grow(h, h->d_prep_alpha, na)))
+            return rc;
+        CU(h, cudaMemcpy(h->d_prep_start.p, h->prep_tab.start.data(), kPrepOut * sizeof(int), cudaMemcpyHostToDevice));
+        CU(h, cudaMemcpy(h->d_prep_cnt.p, h->prep_tab.cnt.data(), kPrepOut * sizeof(int), cudaMemcpyHostToDevice));
+        CU(h, cudaMemcpy(h->d_prep_alpha.p, h->prep_tab.alpha.data(), na * sizeof(float), cudaMemcpyHostToDevice));
         h->prep_side = S;
     }
     PrepParams P;
     P.frames = d_frames; P.out = d_gray;
-    P.start = h->d_prep_start; P.cnt = h->d_prep_cnt; P.alpha = h->d_prep_alpha;
+    P.start = h->d_prep_start.p; P.cnt = h->d_prep_cnt.p; P.alpha = h->d_prep_alpha.p;
     P.fh = fh; P.fw = fw;
     P.x0 = fw > fh ? (fw - fh) / 2 : 0;                  // realtime_detect.py:583-589
     P.y0 = fh > fw ? (fh - fw) / 2 : 0;
@@ -365,7 +410,7 @@ int check_ready(cnnacc_handle* h) {
 // Waits for the handle's stream and the three ring streams.
 int sync_all(cnnacc_handle* h) {
     CU(h, cudaStreamSynchronize(h->stream));
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) CU(h, cudaStreamSynchronize(st));
+    for (const Stream* st : {&h->st_h2d, &h->st_k, &h->st_d2h}) CU(h, cudaStreamSynchronize(*st));
     return 0;
 }
 
@@ -387,7 +432,7 @@ struct HostCall {
 
     explicit HostCall(cnnacc_handle* h_, bool pipelined_ = false)
         : h(h_), pipelined(pipelined_), ring0(pipelined_ ? h_->ring_ci : 0) {}
-    ~HostCall() { if (armed) for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) cudaStreamSynchronize(st); }
+    ~HostCall() { if (armed) for (const Stream* st : {&h->st_h2d, &h->st_k, &h->st_d2h}) cudaStreamSynchronize(*st); }
     // a synchronous call starts on an idle handle (the ring is idle already unless asynchronous calls are pending)
     int begin() { return sync_all(h); }
     // the call's last operation is queued on `st`: wait for it and end the call; `fused`: the call ran the conv stack
@@ -399,14 +444,9 @@ struct HostCall {
     int acquire(Slot*& out, size_t in_bytes, size_t out_bytes, size_t n_pred = 0) {
         Slot& s = h->slots[(ring0 + ci) % kSlots];
         int rc;
-        if ((rc = grow(h, &s.d_in, &s.cap_in, in_bytes)) || (rc = grow(h, &s.d_out, &s.cap_out, out_bytes))) return rc;
-        if (n_pred > s.cap_pred) {
-            cudaFree(s.d_cls); cudaFree(s.d_bbox);
-            s.d_cls = s.d_bbox = nullptr; s.cap_pred = 0;
-            CU(h, cudaMalloc(&s.d_cls, n_pred * sizeof(int32_t)));
-            CU(h, cudaMalloc(&s.d_bbox, n_pred * 4 * sizeof(int32_t)));
-            s.cap_pred = n_pred;
-        }
+        if ((rc = grow(h, s.d_in, in_bytes)) || (rc = grow(h, s.d_out, out_bytes)) || (rc = grow(h, s.d_cls, n_pred)) ||
+            (rc = grow(h, s.d_bbox, n_pred * 4)))
+            return rc;
         if ((ci >= kSlots || pipelined) && (rc = wait_released(s, h->st_h2d))) return rc;   // an unrecorded event is complete
         ci++;
         if (pipelined) h->ring_ci = (ring0 + ci) % kSlots;
@@ -431,13 +471,11 @@ struct PredBlock {
     explicit PredBlock(cnnacc_handle* h_) : h(h_) {}
     // lay the block out for units [first, first + count), growing the handle's two buffers when they are too small
     int start(int64_t first, int64_t count) {
-        if ((size_t)count > h->cap_pred) {
+        const size_t bytes = (size_t)count * kPredBytesPerImage;
+        if (bytes > h->d_pred.cap || bytes > h->h_pred.cap) {
             CU(h, cudaStreamSynchronize(h->st_d2h));
-            cudaFree(h->d_pred); cudaFreeHost(h->h_pred);
-            h->d_pred = h->h_pred = nullptr; h->cap_pred = 0;
-            CU(h, cudaMalloc(&h->d_pred, (size_t)count * kPredBytesPerImage));
-            CU(h, cudaHostAlloc(&h->h_pred, (size_t)count * kPredBytesPerImage, cudaHostAllocDefault));
-            h->cap_pred = (size_t)count;
+            int rc;
+            if ((rc = grow(h, h->d_pred, bytes)) || (rc = grow(h, h->h_pred, bytes))) return rc;
         }
         s0 = first; m = count;
         return 0;
@@ -446,16 +484,16 @@ struct PredBlock {
     size_t off_probs() const { return (size_t)m * 16; }
     size_t off_cls() const { return off_probs() + (size_t)m * h->n_cls * 4; }
     // where the kernels write the predictions of unit u, s0 <= u < end()
-    int32_t* bbox(int64_t u) const { return reinterpret_cast<int32_t*>(h->d_pred) + (u - s0) * 4; }
-    float* probs(int64_t u) const { return reinterpret_cast<float*>(h->d_pred + off_probs()) + (u - s0) * h->n_cls; }
-    int32_t* cls(int64_t u) const { return reinterpret_cast<int32_t*>(h->d_pred + off_cls()) + (u - s0); }
+    int32_t* bbox(int64_t u) const { return reinterpret_cast<int32_t*>(h->d_pred.p) + (u - s0) * 4; }
+    float* probs(int64_t u) const { return reinterpret_cast<float*>(h->d_pred.p + off_probs()) + (u - s0) * h->n_cls; }
+    int32_t* cls(int64_t u) const { return reinterpret_cast<int32_t*>(h->d_pred.p + off_cls()) + (u - s0); }
     // the block, after the kernels queued on `st`, into the caller's arrays (indexed from unit 0); waits for st
     int flush(cudaStream_t st, float* probs_out, int32_t* cls_out, int32_t* bbox_out, bool cls_given) {
-        CU(h, cudaMemcpyAsync(h->h_pred, h->d_pred, off_cls() + (size_t)m * 4, cudaMemcpyDeviceToHost, st));
+        CU(h, cudaMemcpyAsync(h->h_pred.p, h->d_pred.p, off_cls() + (size_t)m * 4, cudaMemcpyDeviceToHost, st));
         CU(h, cudaStreamSynchronize(st));
-        if (bbox_out) std::memcpy(bbox_out + s0 * 4, h->h_pred, (size_t)m * 16);
-        if (probs_out) std::memcpy(probs_out + s0 * h->n_cls, h->h_pred + off_probs(), (size_t)m * h->n_cls * 4);
-        if (cls_out && !cls_given) std::memcpy(cls_out + s0, h->h_pred + off_cls(), (size_t)m * 4);
+        if (bbox_out) std::memcpy(bbox_out + s0 * 4, h->h_pred.p, (size_t)m * 16);
+        if (probs_out) std::memcpy(probs_out + s0 * h->n_cls, h->h_pred.p + off_probs(), (size_t)m * h->n_cls * 4);
+        if (cls_out && !cls_given) std::memcpy(cls_out + s0, h->h_pred.p + off_cls(), (size_t)m * 4);
         return 0;
     }
 };
@@ -472,7 +510,7 @@ int enqueue_host_batch(HostCall& call, const uint8_t* imgs, int64_t n, int H, in
     if (call.pipelined) {
         // earlier calls may still be using the slots: growing one (free + malloc) waits for the device first
         bool grows = false;
-        for (const Slot& s : h->slots) grows |= s.cap_in < hchunk * in_sz || s.cap_out < hchunk * out_sz;
+        for (const Slot& s : h->slots) grows |= s.d_in.cap < hchunk * in_sz || s.d_out.cap < hchunk * out_sz;
         if (grows) CU(h, cudaDeviceSynchronize());
     }
     int64_t m = 0;
@@ -480,11 +518,11 @@ int enqueue_host_batch(HostCall& call, const uint8_t* imgs, int64_t n, int H, in
         m = plan.next(i0, ci);
         Slot* s;
         if ((rc = call.acquire(s, hchunk * in_sz, hchunk * out_sz))) return rc;
-        CU(h, cudaMemcpyAsync(s->d_in, imgs + i0 * in_sz, m * in_sz, cudaMemcpyHostToDevice, h->st_h2d));
-        if ((rc = call.staged(*s)) || (rc = conv_stack_device(h, h->st_k, s->d_in, m, H, W, s->d_out, flags, h->d_l0, h->d_l1)) ||
+        CU(h, cudaMemcpyAsync(s->d_in.p, imgs + i0 * in_sz, m * in_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        if ((rc = call.staged(*s)) || (rc = conv_stack_device(h, h->st_k, s->d_in.p, m, H, W, s->d_out.p, flags, h->d_l0.p, h->d_l1.p)) ||
             (rc = call.computed(*s)))
             return rc;
-        CU(h, cudaMemcpyAsync(feats + i0 * out_sz, s->d_out, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+        CU(h, cudaMemcpyAsync(feats + i0 * out_sz, s->d_out.p, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
         if ((rc = call.released(*s, h->st_d2h))) return rc;
     }
     return 0;
@@ -573,11 +611,11 @@ int cnnacc_create(int device_id, cnnacc_handle** out) {
         return fail(nullptr, CNNACC_ERR_CUDA, std::string("no CUDA device: ") + cudaGetErrorString(e) +
                                                   " (this library has no CPU fallback)");
     if (device_id < 0 || device_id >= count) return fail(nullptr, CNNACC_ERR_ARG, "device_id out of range");
-    cnnacc_handle* h = new cnnacc_handle();
+    // on a failed step the handle is deleted with whatever it holds so far, device_id being current
+    std::unique_ptr<cnnacc_handle> h(new cnnacc_handle());
     h->device = device_id;
     auto bail = [&](const char* what, cudaError_t err) {
         g_create_error = std::string(what) + ": " + cudaGetErrorString(err);
-        cnnacc_destroy(h);                               // releases whatever was created so far (null members are skipped)
         return CNNACC_ERR_CUDA;
     };
     if ((e = cudaSetDevice(device_id)) != cudaSuccess) return bail("cudaSetDevice", e);
@@ -586,38 +624,34 @@ int cnnacc_create(int device_id, cnnacc_handle** out) {
     if (prop.major != 10) {
         g_create_error = "device is sm_" + std::to_string(prop.major * 10 + prop.minor) +
                          "; this library is built for sm_100a (B200) only";
-        cnnacc_destroy(h);
         return CNNACC_ERR_CUDA;
     }
     h->sm_count = prop.multiProcessorCount;
-    if ((e = cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
+    if ((e = h->own_stream.create(cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
     h->stream = h->own_stream;
-    cudaEvent_t* evs[] = {&h->ev_t0, &h->ev_t1, &h->ev_a, &h->ev_b, &h->ev_done};
-    for (auto ev : evs)
-        if ((e = cudaEventCreate(ev)) != cudaSuccess) return bail("cudaEventCreate", e);
+    for (Event* ev : {&h->ev_t0, &h->ev_t1, &h->ev_a, &h->ev_b, &h->ev_done})
+        if ((e = ev->create(cudaEventDefault)) != cudaSuccess) return bail("cudaEventCreate", e);
     for (auto& s : h->slots) {
-        for (auto ev : {&s.ev_in, &s.ev_k, &s.ev_out})
-            if ((e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+        for (Event* ev : {&s.ev_in, &s.ev_k, &s.ev_out})
+            if ((e = ev->create(cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
     }
     for (auto& ev : h->ev_ticket)
-        if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+        if ((e = ev.create(cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
     for (auto& b : h->rdesc)
-        if ((e = cudaEventCreateWithFlags(&b.ev, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
-    for (auto st : {&h->st_h2d, &h->st_k, &h->st_d2h})
-        if ((e = cudaStreamCreateWithFlags(st, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
-    if ((e = cudaHostAlloc(&h->h_img, CNNACC_IMG * CNNACC_IMG, cudaHostAllocMapped)) != cudaSuccess) return bail("cudaHostAlloc", e);
-    if ((e = cudaHostAlloc(&h->h_bram, kBramBytes, cudaHostAllocMapped)) != cudaSuccess) return bail("cudaHostAlloc", e);
-    if ((e = cudaHostGetDevicePointer(&h->h_img_dev, h->h_img, 0)) != cudaSuccess) return bail("cudaHostGetDevicePointer", e);
-    if ((e = cudaHostGetDevicePointer(&h->h_bram_dev, h->h_bram, 0)) != cudaSuccess) return bail("cudaHostGetDevicePointer", e);
-    if ((e = cudaHostAlloc(&h->h_done, 64, cudaHostAllocMapped)) != cudaSuccess) return bail("cudaHostAlloc", e);
-    *h->h_done = 0;
-    if ((e = cudaHostGetDevicePointer(&h->h_done_dev, h->h_done, 0)) != cudaSuccess) return bail("cudaHostGetDevicePointer", e);
-    if ((e = cudaHostAlloc(&h->h_pred, kSmallN * kPredBytesPerImage, cudaHostAllocDefault)) != cudaSuccess) return bail("cudaHostAlloc", e);
-    if ((e = cudaMalloc(&h->d_pred, kSmallN * kPredBytesPerImage)) != cudaSuccess) return bail("cudaMalloc", e);
-    h->cap_pred = kSmallN;
-    if ((e = cudaMalloc(&h->d_img1, CNNACC_IMG * CNNACC_IMG)) != cudaSuccess) return bail("cudaMalloc", e);
-    if ((e = cudaMalloc(&h->d_bram, kBramBytes)) != cudaSuccess) return bail("cudaMalloc", e);
-    *out = h;
+        if ((e = b.ev.create(cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+    for (Stream* st : {&h->st_h2d, &h->st_k, &h->st_d2h})
+        if ((e = st->create(cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
+    int rc;
+    if ((rc = grow(nullptr, h->h_img, CNNACC_IMG * CNNACC_IMG)) || (rc = grow(nullptr, h->h_bram, kBramBytes)) ||
+        (rc = grow(nullptr, h->h_done, 64 / sizeof(int))) || (rc = grow(nullptr, h->h_pred, kSmallN * kPredBytesPerImage)) ||
+        (rc = grow(nullptr, h->d_pred, kSmallN * kPredBytesPerImage)) || (rc = grow(nullptr, h->d_img1, CNNACC_IMG * CNNACC_IMG)) ||
+        (rc = grow(nullptr, h->d_bram, kBramBytes)))
+        return rc;
+    if ((e = cudaHostGetDevicePointer(&h->h_img_dev, h->h_img.p, 0)) != cudaSuccess) return bail("cudaHostGetDevicePointer", e);
+    if ((e = cudaHostGetDevicePointer(&h->h_bram_dev, h->h_bram.p, 0)) != cudaSuccess) return bail("cudaHostGetDevicePointer", e);
+    *h->h_done.p = 0;
+    if ((e = cudaHostGetDevicePointer(&h->h_done_dev, h->h_done.p, 0)) != cudaSuccess) return bail("cudaHostGetDevicePointer", e);
+    *out = h.release();
     return CNNACC_OK;
 }
 
@@ -625,27 +659,6 @@ int cnnacc_destroy(cnnacc_handle* h) {
     if (!h) return CNNACC_ERR_ARG;
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
-    for (auto& s : h->slots) {
-        cudaFree(s.d_in); cudaFree(s.d_out); cudaFree(s.d_cls); cudaFree(s.d_bbox);
-        for (auto ev : {s.ev_in, s.ev_k, s.ev_out}) if (ev) cudaEventDestroy(ev);
-    }
-    for (auto st : {h->st_h2d, h->st_k, h->st_d2h}) if (st) cudaStreamDestroy(st);
-    for (auto ev : h->ev_ticket) if (ev) cudaEventDestroy(ev);
-    for (auto& b : h->rdesc) {
-        cudaFreeHost(b.host); cudaFree(b.dev); cudaFreeHost(b.first_host); cudaFree(b.first_dev);
-        if (b.ev) cudaEventDestroy(b.ev);
-    }
-    cudaFree(h->d_mpred); cudaFree(h->d_det); cudaFreeHost(h->h_det);
-    cudaFree(h->d_prep_start); cudaFree(h->d_prep_cnt); cudaFree(h->d_prep_alpha); cudaFree(h->d_gray);
-    cudaFree(h->d_pil_kx); cudaFree(h->d_pil_bx); cudaFree(h->d_pil_ky); cudaFree(h->d_pil_by);
-    cudaFree(h->d_pil_tmp); cudaFree(h->d_pil_in); cudaFree(h->d_pil_out);
-    cudaFree(h->d_wdirect); cudaFree(h->d_fcw); cudaFree(h->d_fcb);
-    cudaFree(h->d_l0); cudaFree(h->d_l1); cudaFree(h->d_feat); cudaFree(h->d_img1); cudaFree(h->d_bram);
-    fused_free(h->fused);
-    cudaFreeHost(h->h_img); cudaFreeHost(h->h_bram); cudaFreeHost(h->h_done); cudaFreeHost(h->h_pred); cudaFree(h->d_pred);
-    cudaEvent_t evs[] = {h->ev_t0, h->ev_t1, h->ev_a, h->ev_b, h->ev_done};
-    for (auto ev : evs) if (ev) cudaEventDestroy(ev);
-    if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
     return CNNACC_OK;
 }
@@ -669,9 +682,10 @@ int cnnacc_load_weights(cnnacc_handle* h, const uint8_t* weights_bin, size_t n) 
     std::memcpy(h->wbin, weights_bin, n);
     std::vector<uint32_t> packed;
     pack_direct_weights(h->wbin, packed, h->wdirect_off);
-    if (!h->d_wdirect) CU(h, cudaMalloc(&h->d_wdirect, packed.size() * sizeof(uint32_t)));
-    CU(h, cudaMemcpy(h->d_wdirect, packed.data(), packed.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    int rc = fused_load_weights(h->fused, h->wbin);
+    int rc;
+    if ((rc = grow(h, h->d_wdirect, packed.size()))) return rc;
+    CU(h, cudaMemcpy(h->d_wdirect.p, packed.data(), packed.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    rc = fused_load_weights(h->fused, h->wbin);
     if (rc != 0) return fail(h, CNNACC_ERR_CUDA, std::string("fused_load_weights: ") + cudaGetErrorString((cudaError_t)rc));
     h->weights_loaded = true;
     return CNNACC_OK;
@@ -762,7 +776,7 @@ int cnnacc_run_batch(cnnacc_handle* h, const uint8_t* imgs, int64_t n, int H, in
         if (maps && (rc = ensure_maps(h, chunk, H, W))) return rc;
         for (int64_t i0 = 0; i0 < n; i0 += chunk) {
             const int64_t m = std::min(chunk, n - i0);
-            if ((rc = conv_stack_device(h, h->stream, imgs + i0 * in_sz, m, H, W, feats + i0 * out_sz, flags, h->d_l0, h->d_l1)))
+            if ((rc = conv_stack_device(h, h->stream, imgs + i0 * in_sz, m, H, W, feats + i0 * out_sz, flags, h->d_l0.p, h->d_l1.p)))
                 return rc;
         }
         return CNNACC_OK;
@@ -811,7 +825,7 @@ int cnnacc_load_image(cnnacc_handle* h, const uint8_t* img, size_t n) {
         return fail(h, CNNACC_ERR_ARG, "Expected 16384 pixels, got " + std::to_string(n));     // pynq_inference.py:214
     CU(h, cudaSetDevice(h->device));
     if (h->started) CU(h, cudaEventSynchronize(h->ev_done));   // s_axis_tready = !busy (…S00_AXI.v:390)
-    std::memcpy(h->h_img, img, n);
+    std::memcpy(h->h_img.p, img, n);
     h->image_loaded = true;
     return CNNACC_OK;
 }
@@ -821,10 +835,10 @@ int cnnacc_start(cnnacc_handle* h) {
     if ((rc = check_ready(h))) return rc;
     if (!h->image_loaded) return fail(h, CNNACC_ERR_STATE, "no image loaded (call cnnacc_load_image)");
     CU(h, cudaSetDevice(h->device));
-    uint8_t *l0 = h->d_bram, *l1 = h->d_bram + 16 * 4096, *l2 = l1 + 32 * 1024;
-    CU(h, cudaMemcpyAsync(h->d_img1, h->h_img, CNNACC_IMG * CNNACC_IMG, cudaMemcpyHostToDevice, h->stream));
-    if ((rc = conv_stack_device(h, h->stream, h->d_img1, 1, CNNACC_IMG, CNNACC_IMG, l2, CNNACC_FLAG_KEEP_MAPS, l0, l1))) return rc;
-    CU(h, cudaMemcpyAsync(h->h_bram, h->d_bram, kBramBytes, cudaMemcpyDeviceToHost, h->stream));
+    uint8_t *l0 = h->d_bram.p, *l1 = h->d_bram.p + 16 * 4096, *l2 = l1 + 32 * 1024;
+    CU(h, cudaMemcpyAsync(h->d_img1.p, h->h_img.p, CNNACC_IMG * CNNACC_IMG, cudaMemcpyHostToDevice, h->stream));
+    if ((rc = conv_stack_device(h, h->stream, h->d_img1.p, 1, CNNACC_IMG, CNNACC_IMG, l2, CNNACC_FLAG_KEEP_MAPS, l0, l1))) return rc;
+    CU(h, cudaMemcpyAsync(h->h_bram.p, h->d_bram.p, kBramBytes, cudaMemcpyDeviceToHost, h->stream));
     CU(h, cudaEventRecord(h->ev_done, h->stream));
     h->started = true;
     return CNNACC_OK;
@@ -863,7 +877,7 @@ int cnnacc_read_feature_map(cnnacc_handle* h, int channel, int num_values, uint8
     else                   { off = 16 * 4096 + 32 * 1024 + (size_t)(channel - 48) * 256; depth = 256; }
     if (num_values < 0 || (size_t)num_values > depth) return fail(h, CNNACC_ERR_ARG, "num_values exceeds the channel's BRAM depth");
     { int rc = check_fused_status(h); if (rc) return rc; }
-    std::memcpy(out, h->h_bram + off, (size_t)num_values);
+    std::memcpy(out, h->h_bram.p + off, (size_t)num_values);
     return CNNACC_OK;
 }
 
@@ -883,9 +897,9 @@ int cnnacc_infer_one(cnnacc_handle* h, const uint8_t* img, uint8_t* feat, float*
     if (!img || !feat) return fail(h, CNNACC_ERR_ARG, "NULL argument");
     CU(h, cudaSetDevice(h->device));
     if (h->started) CU(h, cudaEventSynchronize(h->ev_done));
-    uint8_t* h_l2 = h->h_bram + 16 * 4096 + 32 * 1024;
+    uint8_t* h_l2 = h->h_bram.p + 16 * 4096 + 32 * 1024;
     const auto t0 = std::chrono::steady_clock::now();
-    std::memcpy(h->h_img, img, CNNACC_FEAT_BYTES);
+    std::memcpy(h->h_img.p, img, CNNACC_FEAT_BYTES);
     // Zero-copy: the kernel TMA-loads the image straight from mapped pinned host memory and its 16 KiB bulk
     // store lands in mapped pinned host memory -- one launch, one stream sync, no copy-engine round trips.
     if (!h->one_map_ok) {
@@ -901,7 +915,7 @@ int cnnacc_infer_one(cnnacc_handle* h, const uint8_t* img, uint8_t* feat, float*
     // The kernel stores `seq` into a mapped host word after its feature store has landed: spinning on that word skips the
     // driver's wake-up path of a stream synchronise (~8 us of the ~36).  Bounded: after 2 s fall back to the synchronise.
     {
-        const volatile int* flag = h->h_done;
+        const volatile int* flag = h->h_done.p;
         const auto spin0 = std::chrono::steady_clock::now();
         for (unsigned it = 0; *flag != seq; it++) {
 #if defined(__x86_64__)
@@ -929,10 +943,10 @@ int cnnacc_load_classifier(cnnacc_handle* h, const float* fc_w, const float* fc_
         if (!(std::fabs(fc_w[i]) < 1.2676506002282294e30f)) return fail(h, CNNACC_ERR_ARG, "classifier weight not finite or |w| >= 2^100");
     CU(h, cudaSetDevice(h->device));
     CU(h, cudaDeviceSynchronize());
-    if (!h->d_fcw) CU(h, cudaMalloc(&h->d_fcw, (size_t)kMaxClasses * 1024 * sizeof(float)));
-    if (!h->d_fcb) CU(h, cudaMalloc(&h->d_fcb, kMaxClasses * sizeof(float)));
-    CU(h, cudaMemcpy(h->d_fcw, fc_w, (size_t)n_cls * 1024 * sizeof(float), cudaMemcpyHostToDevice));
-    CU(h, cudaMemcpy(h->d_fcb, fc_b, n_cls * sizeof(float), cudaMemcpyHostToDevice));
+    int rc;
+    if ((rc = grow(h, h->d_fcw, (size_t)kMaxClasses * 1024)) || (rc = grow(h, h->d_fcb, kMaxClasses))) return rc;
+    CU(h, cudaMemcpy(h->d_fcw.p, fc_w, (size_t)n_cls * 1024 * sizeof(float), cudaMemcpyHostToDevice));
+    CU(h, cudaMemcpy(h->d_fcb.p, fc_b, n_cls * sizeof(float), cudaMemcpyHostToDevice));
     std::memcpy(h->fcw_host, fc_w, (size_t)n_cls * 1024 * sizeof(float));
     std::memcpy(h->fcb_host, fc_b, n_cls * sizeof(float));
     h->n_cls = n_cls;
@@ -970,7 +984,7 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
         // one fused launch covers the whole call unless a workspace bounds the chunk
         const int64_t chunk = feat_ws ? std::min<int64_t>(n, 16384) : n;
         if (feat_ws) {
-            if ((rc = grow(h, &h->d_feat, &h->cap_feat, (size_t)chunk * img_sz))) return rc;
+            if ((rc = grow(h, h->d_feat, (size_t)chunk * img_sz))) return rc;
             if (maps && (rc = ensure_maps(h, chunk, CNNACC_IMG, CNNACC_IMG))) return rc;
         }
         for (int64_t i0 = 0; i0 < n; i0 += chunk) {
@@ -979,8 +993,8 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
                                          (bbox && !upsampled) ? bbox + i0 * 4 : nullptr, cls_given, flags);
             const uint8_t* f = src + i0 * img_sz;
             if (src_is_images) {
-                if ((rc = infer_device(h, h->stream, f, m, h->d_feat, upsampled, A, flags))) return rc;
-                f = h->d_feat;
+                if ((rc = infer_device(h, h->stream, f, m, h->d_feat.p, upsampled, A, flags))) return rc;
+                f = h->d_feat.p;
             } else if ((rc = launch_tail(h, h->stream, f, m, A))) return rc;
             if (upsampled && (rc = launch_cam_upsampled(h, h->stream, f, m, cls + i0, bbox + i0 * 4, nullptr))) return rc;
         }
@@ -992,11 +1006,11 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
     PredBlock pred(h);
     auto kernels = [&](cudaStream_t st, const Slot& s, int64_t i0, int64_t m) -> int {   // units [i0, i0 + m), staged in s
         const TailArgs A = make_tail(h, pred.probs(i0), pred.cls(i0), upsampled ? nullptr : pred.bbox(i0), cls_given, flags);
-        const uint8_t* f = s.d_in;
+        const uint8_t* f = s.d_in.p;
         int r;
         if (src_is_images) {
-            if ((r = infer_device(h, st, s.d_in, m, s.d_out, upsampled, A, flags))) return r;
-            f = s.d_out;
+            if ((r = infer_device(h, st, s.d_in.p, m, s.d_out.p, upsampled, A, flags))) return r;
+            f = s.d_out.p;
         } else if ((r = launch_tail(h, st, f, m, A))) return r;
         return upsampled ? launch_cam_upsampled(h, st, f, m, pred.cls(i0), pred.bbox(i0), nullptr) : 0;
     };
@@ -1006,7 +1020,7 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
         if ((rc = call.acquire(s, n * img_sz, feat_ws ? n * img_sz : 0))) return rc;
         if (maps && (rc = ensure_maps(h, n, CNNACC_IMG, CNNACC_IMG))) return rc;
         if ((rc = pred.start(0, n))) return rc;
-        CU(h, cudaMemcpyAsync(s->d_in, src, n * img_sz, cudaMemcpyHostToDevice, st));
+        CU(h, cudaMemcpyAsync(s->d_in.p, src, n * img_sz, cudaMemcpyHostToDevice, st));
         if (cls_given) CU(h, cudaMemcpyAsync(pred.cls(0), cls, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         if ((rc = kernels(st, *s, 0, n)) || (rc = pred.flush(st, probs, cls, bbox, cls_given))) return rc;
         return call.done(src_is_images);
@@ -1020,7 +1034,7 @@ static int predict_impl(cnnacc_handle* h, const uint8_t* src, int64_t n, bool sr
         for (int64_t i0 = s0; i0 < pred.end(); i0 += hchunk) {
             const int64_t m = std::min(hchunk, pred.end() - i0);
             if ((rc = call.acquire(s, hchunk * img_sz, feat_ws ? hchunk * img_sz : 0))) return rc;
-            CU(h, cudaMemcpyAsync(s->d_in, src + i0 * img_sz, m * img_sz, cudaMemcpyHostToDevice, h->st_h2d));
+            CU(h, cudaMemcpyAsync(s->d_in.p, src + i0 * img_sz, m * img_sz, cudaMemcpyHostToDevice, h->st_h2d));
             if (cls_given) CU(h, cudaMemcpyAsync(pred.cls(i0), cls + i0, m * sizeof(int32_t), cudaMemcpyHostToDevice, h->st_h2d));
             if ((rc = call.staged(*s)) || (rc = kernels(h->st_k, *s, i0, m)) || (rc = call.released(*s, h->st_k))) return rc;
         }
@@ -1060,13 +1074,13 @@ int cnnacc_pool_features(cnnacc_handle* h, const uint8_t* feats, int64_t n, floa
         const int64_t m = std::min(hchunk, n - i0);
         Slot* s;
         if ((rc = call.acquire(s, hchunk * feat_sz, hchunk * out_sz))) return rc;
-        CU(h, cudaMemcpyAsync(s->d_in, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        CU(h, cudaMemcpyAsync(s->d_in.p, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
         if ((rc = call.staged(*s))) return rc;
-        pool_features_kernel<<<(unsigned)m, 256, 0, h->st_k>>>(s->d_in, reinterpret_cast<float*>(s->d_out));
+        pool_features_kernel<<<(unsigned)m, 256, 0, h->st_k>>>(s->d_in.p, reinterpret_cast<float*>(s->d_out.p));
         h->launches++;
         CU(h, cudaGetLastError());
         if ((rc = call.computed(*s))) return rc;
-        CU(h, cudaMemcpyAsync(pooled + i0 * 1024, s->d_out, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+        CU(h, cudaMemcpyAsync(pooled + i0 * 1024, s->d_out.p, m * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
         if ((rc = call.released(*s, h->st_d2h))) return rc;
     }
     return call.finish(h->st_d2h, false);
@@ -1097,14 +1111,14 @@ int cnnacc_cam_bbox_batch(cnnacc_handle* h, const uint8_t* feats, int64_t n, con
         const int64_t m = std::min(hchunk, n - i0);
         Slot* s;
         if ((rc = call.acquire(s, hchunk * feat_sz, cam ? hchunk * cam_sz : 0, hchunk))) return rc;
-        CU(h, cudaMemcpyAsync(s->d_in, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
-        CU(h, cudaMemcpyAsync(s->d_cls, cls + i0, m * sizeof(int32_t), cudaMemcpyHostToDevice, h->st_h2d));
+        CU(h, cudaMemcpyAsync(s->d_in.p, feats + i0 * feat_sz, m * feat_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        CU(h, cudaMemcpyAsync(s->d_cls.p, cls + i0, m * sizeof(int32_t), cudaMemcpyHostToDevice, h->st_h2d));
         if ((rc = call.staged(*s)) ||
-            (rc = launch_cam_upsampled(h, h->st_k, s->d_in, m, s->d_cls, bbox ? s->d_bbox : nullptr, cam ? s->d_out : nullptr)) ||
+            (rc = launch_cam_upsampled(h, h->st_k, s->d_in.p, m, s->d_cls.p, bbox ? s->d_bbox.p : nullptr, cam ? s->d_out.p : nullptr)) ||
             (rc = call.computed(*s)))
             return rc;
-        if (bbox) CU(h, cudaMemcpyAsync(bbox + i0 * 4, s->d_bbox, m * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st_d2h));
-        if (cam)  CU(h, cudaMemcpyAsync(cam + i0 * cam_sz, s->d_out, m * cam_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+        if (bbox) CU(h, cudaMemcpyAsync(bbox + i0 * 4, s->d_bbox.p, m * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st_d2h));
+        if (cam)  CU(h, cudaMemcpyAsync(cam + i0 * cam_sz, s->d_out.p, m * cam_sz, cudaMemcpyDeviceToHost, h->st_d2h));
         if ((rc = call.released(*s, h->st_d2h))) return rc;
     }
     return call.finish(h->st_d2h, false);
@@ -1137,10 +1151,10 @@ static int prep_then_tail(cnnacc_handle* h, cudaStream_t st, const RegionPrep& b
     if (!detect) return 0;
     const size_t img_sz = CNNACC_FEAT_BYTES;
     const bool ups = (flags & CNNACC_FLAG_BBOX_UPSAMPLED) && d_bbox;
-    if (infer_needs_feat_ws(ups, 0) && (rc = grow(h, &h->d_feat, &h->cap_feat, (size_t)m * img_sz))) return rc;
+    if (infer_needs_feat_ws(ups, 0) && (rc = grow(h, h->d_feat, (size_t)m * img_sz))) return rc;
     const TailArgs A = make_tail(h, d_probs, d_cls, ups ? nullptr : d_bbox, false, flags);
-    if ((rc = infer_device(h, st, base.out, m, h->d_feat, ups, A, 0))) return rc;
-    if (ups && (rc = launch_cam_upsampled(h, st, h->d_feat, m, d_cls, d_bbox, nullptr))) return rc;
+    if ((rc = infer_device(h, st, base.out, m, h->d_feat.p, ups, A, 0))) return rc;
+    if (ups && (rc = launch_cam_upsampled(h, st, h->d_feat.p, m, d_cls, d_bbox, nullptr))) return rc;
     return 0;
 }
 
@@ -1151,20 +1165,10 @@ static int desc_acquire(cnnacc_handle* h, int64_t n, DescBuf** out, int64_t n_fi
     DescBuf& b = h->rdesc[h->rdesc_next];
     h->rdesc_next = (h->rdesc_next + 1) % kDescRing;
     CU(h, cudaEventSynchronize(b.ev));                   // an event never recorded counts as complete
-    if ((int64_t)b.cap < n) {
-        cudaFreeHost(b.host); cudaFree(b.dev);
-        b.host = nullptr; b.dev = nullptr; b.cap = 0;
-        CU(h, cudaHostAlloc(&b.host, (size_t)n * sizeof(int4), cudaHostAllocDefault));
-        CU(h, cudaMalloc(&b.dev, (size_t)n * sizeof(int4)));
-        b.cap = (size_t)n;
-    }
-    if ((int64_t)b.cap_first < n_first) {
-        cudaFreeHost(b.first_host); cudaFree(b.first_dev);
-        b.first_host = nullptr; b.first_dev = nullptr; b.cap_first = 0;
-        CU(h, cudaHostAlloc(&b.first_host, (size_t)n_first * sizeof(long long), cudaHostAllocDefault));
-        CU(h, cudaMalloc(&b.first_dev, (size_t)n_first * sizeof(long long)));
-        b.cap_first = (size_t)n_first;
-    }
+    int rc;
+    if ((rc = grow(h, b.host, (size_t)n)) || (rc = grow(h, b.dev, (size_t)n)) || (rc = grow(h, b.first_host, (size_t)n_first)) ||
+        (rc = grow(h, b.first_dev, (size_t)n_first)))
+        return rc;
     *out = &b;
     return 0;
 }
@@ -1266,31 +1270,26 @@ static int merge_to_host(cnnacc_handle* h, cudaStream_t st, MergeArgs A, const M
     const size_t D = (size_t)M.max_det, per_frame = 4 + D * 28;
     const int64_t step = std::max<int64_t>(1, std::min<int64_t>(fb - fa, ((size_t)8 << 20) / per_frame));
     const size_t need = (size_t)step * per_frame;
-    if (need > h->cap_det) {
-        cudaFree(h->d_det); cudaFreeHost(h->h_det);
-        h->d_det = h->h_det = nullptr; h->cap_det = 0;
-        CU(h, cudaMalloc(&h->d_det, need));
-        CU(h, cudaHostAlloc(&h->h_det, need, cudaHostAllocDefault));
-        h->cap_det = need;
-    }
+    int rc;
+    if ((rc = grow(h, h->d_det, need)) || (rc = grow(h, h->h_det, need))) return rc;
     for (int64_t g0 = fa; g0 < fb; g0 += step) {
         const int64_t m = std::min(step, fb - g0);
         const size_t md = (size_t)m * D, o_reg = md * 16, o_cls = o_reg + md * 4, o_score = o_cls + md * 4, o_n = o_score + md * 4;
-        A.det_box = reinterpret_cast<float4*>(h->d_det);
-        A.det_region = reinterpret_cast<int32_t*>(h->d_det + o_reg);
-        A.det_cls = reinterpret_cast<int32_t*>(h->d_det + o_cls);
-        A.det_score = reinterpret_cast<float*>(h->d_det + o_score);
-        A.n_det = reinterpret_cast<int32_t*>(h->d_det + o_n);
-        int rc;
+        uint8_t *d = h->d_det.p, *hd = h->h_det.p;
+        A.det_box = reinterpret_cast<float4*>(d);
+        A.det_region = reinterpret_cast<int32_t*>(d + o_reg);
+        A.det_cls = reinterpret_cast<int32_t*>(d + o_cls);
+        A.det_score = reinterpret_cast<float*>(d + o_score);
+        A.n_det = reinterpret_cast<int32_t*>(d + o_n);
         if ((rc = launch_merge(h, st, A, M, d_first, g0, g0 + m))) return rc;
-        CU(h, cudaMemcpyAsync(h->h_det, h->d_det, o_n + (size_t)m * 4, cudaMemcpyDeviceToHost, st));
+        CU(h, cudaMemcpyAsync(hd, d, o_n + (size_t)m * 4, cudaMemcpyDeviceToHost, st));
         CU(h, cudaStreamSynchronize(st));
         const size_t at = (size_t)g0 * D;
-        std::memcpy(M.n_det + g0, h->h_det + o_n, (size_t)m * 4);
-        if (M.det_box) std::memcpy(M.det_box + at * 4, h->h_det, md * 16);
-        if (M.det_region) std::memcpy(M.det_region + at, h->h_det + o_reg, md * 4);
-        if (M.det_cls) std::memcpy(M.det_cls + at, h->h_det + o_cls, md * 4);
-        if (M.det_score) std::memcpy(M.det_score + at, h->h_det + o_score, md * 4);
+        std::memcpy(M.n_det + g0, hd + o_n, (size_t)m * 4);
+        if (M.det_box) std::memcpy(M.det_box + at * 4, hd, md * 16);
+        if (M.det_region) std::memcpy(M.det_region + at, hd + o_reg, md * 4);
+        if (M.det_cls) std::memcpy(M.det_cls + at, hd + o_cls, md * 4);
+        if (M.det_score) std::memcpy(M.det_score + at, hd + o_score, md * 4);
     }
     return 0;
 }
@@ -1356,11 +1355,11 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         DescBuf* db = nullptr;
         if (!centre) {
             if ((rc = desc_acquire(h, n, &db, mg ? n_frames + 1 : 0))) return rc;
-            fill_desc(db->host, rg, n);
-            CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
+            fill_desc(db->host.p, rg, n);
+            CU(h, cudaMemcpyAsync(db->dev.p, db->host.p, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
             if (mg) {
-                std::memcpy(db->first_host, mg->first.data(), (size_t)(n_frames + 1) * sizeof(long long));
-                CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, (size_t)(n_frames + 1) * sizeof(long long),
+                std::memcpy(db->first_host.p, mg->first.data(), (size_t)(n_frames + 1) * sizeof(long long));
+                CU(h, cudaMemcpyAsync(db->first_dev.p, db->first_host.p, (size_t)(n_frames + 1) * sizeof(long long),
                                       cudaMemcpyHostToDevice, h->stream));
             }
         }
@@ -1368,25 +1367,25 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
             const int64_t chunk = std::min<int64_t>(n, 16384);
             uint8_t* g = gray128;
             int r;
-            if (!g && (r = grow(h, &h->d_gray, &h->cap_gray, (size_t)chunk * img_sz))) return r;
+            if (!g && (r = grow(h, h->d_gray, (size_t)chunk * img_sz))) return r;
             // detect_objects: the predictions of a piece go to a workspace laid out as PredBlock's, then the piece's frames
             // are merged; a piece is the whole frames that fit `chunk` regions (a frame has at most kMergeMaxPerFrame)
             const size_t w_probs = (size_t)chunk * 16, w_cls = w_probs + (size_t)chunk * nc * 4;
-            if (mg && (r = grow(h, &h->d_mpred, &h->cap_mpred, (size_t)chunk * kPredBytesPerImage))) return r;
+            if (mg && (r = grow(h, h->d_mpred, (size_t)chunk * kPredBytesPerImage))) return r;
             int64_t m = 0;
             for (int64_t i0 = 0, fa = 0; i0 < n; i0 += m) {
                 m = std::min(chunk, n - i0);
                 if (mg && i0 + m < n) m = mg->first[rg.frame(i0 + m)] - i0;
                 RegionPrep P = base;
                 P.frames = centre ? frames + i0 * frame_sz : frames;
-                P.desc = centre ? nullptr : db->dev + i0;
-                P.out = g ? g + i0 * img_sz : h->d_gray;
+                P.desc = centre ? nullptr : db->dev.p + i0;
+                P.out = g ? g + i0 * img_sz : h->d_gray.p;
                 if (mg) {
-                    int32_t* wb = reinterpret_cast<int32_t*>(h->d_mpred);
-                    float* wp = reinterpret_cast<float*>(h->d_mpred + w_probs);
-                    int32_t* wc = reinterpret_cast<int32_t*>(h->d_mpred + w_cls);
+                    int32_t* wb = reinterpret_cast<int32_t*>(h->d_mpred.p);
+                    float* wp = reinterpret_cast<float*>(h->d_mpred.p + w_probs);
+                    int32_t* wc = reinterpret_cast<int32_t*>(h->d_mpred.p + w_cls);
                     const int64_t fb = i0 + m == n ? n_frames : rg.frame(i0 + m);
-                    MergeArgs A = merge_args_of_predictions(db->dev, i0, wb, wp, wc, nc, *mg);
+                    MergeArgs A = merge_args_of_predictions(db->dev.p, i0, wb, wp, wc, nc, *mg);
                     A.n_det += fa;
                     const size_t o = (size_t)fa * mg->max_det;
                     if (A.det_region) A.det_region += o;
@@ -1394,7 +1393,7 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
                     if (A.det_score) A.det_score += o;
                     if (A.det_box) A.det_box += o;
                     if ((r = prep_then_tail(h, h->stream, P, m, detect, wp, wc, wb, flags)) ||
-                        (r = launch_merge(h, h->stream, A, *mg, db->first_dev, fa, fb)))
+                        (r = launch_merge(h, h->stream, A, *mg, db->first_dev.p, fa, fb)))
                         return r;
                     fa = fb;
                 } else if ((r = prep_then_tail(h, h->stream, P, m, detect, probs ? probs + i0 * nc : nullptr, cls ? cls + i0 : nullptr,
@@ -1437,13 +1436,13 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
         int64_t below = 0;                               // small: frames staged ahead of the chunk in the one buffer
         for (const RegionChunk& c : plan) {
             for (int64_t r = c.r0; r < c.r1; r++)
-                db->host[r] = make_int4((int)(rg.frame(r) - c.f0 + (small ? below : 0)), rg.x(r), rg.y(r), rg.wh(r));
+                db->host.p[r] = make_int4((int)(rg.frame(r) - c.f0 + (small ? below : 0)), rg.x(r), rg.y(r), rg.wh(r));
             below += c.f1 - c.f0;
         }
-        CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, small ? h->st_k : h->st_h2d));
+        CU(h, cudaMemcpyAsync(db->dev.p, db->host.p, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, small ? h->st_k : h->st_h2d));
         if (mg) {
-            std::memcpy(db->first_host, mg->first.data(), (size_t)(n_frames + 1) * sizeof(long long));
-            CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, (size_t)(n_frames + 1) * sizeof(long long), cudaMemcpyHostToDevice,
+            std::memcpy(db->first_host.p, mg->first.data(), (size_t)(n_frames + 1) * sizeof(long long));
+            CU(h, cudaMemcpyAsync(db->first_dev.p, db->first_host.p, (size_t)(n_frames + 1) * sizeof(long long), cudaMemcpyHostToDevice,
                                   small ? h->st_k : h->st_h2d));
         }
     }
@@ -1452,15 +1451,15 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
     int64_t det_f = 0;
     auto merge_block = [&](const PredBlock& pred, cudaStream_t st) -> int {
         const int64_t fb = pred.end() == n ? n_frames : rg.frame(pred.end());
-        const MergeArgs A = merge_args_of_predictions(db->dev, pred.s0, pred.bbox(pred.s0), pred.probs(pred.s0), pred.cls(pred.s0), nc, *mg);
-        const int r = merge_to_host(h, st, A, *mg, db->first_dev, det_f, fb);
+        const MergeArgs A = merge_args_of_predictions(db->dev.p, pred.s0, pred.bbox(pred.s0), pred.probs(pred.s0), pred.cls(pred.s0), nc, *mg);
+        const int r = merge_to_host(h, st, A, *mg, db->first_dev.p, det_f, fb);
         det_f = fb;
         return r;
     };
     auto region_base = [&](const uint8_t* d_frames, int64_t r, int64_t r_frame0, uint8_t* d_gray) {
         RegionPrep P = base;
         P.frames = centre ? d_frames + (r - r_frame0) * frame_sz : d_frames;
-        P.desc = centre ? nullptr : db->dev + r;
+        P.desc = centre ? nullptr : db->dev.p + r;
         P.out = d_gray;
         return P;
     };
@@ -1476,13 +1475,13 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
             size_t j = k + 1;
             while (j < plan.size() && plan[j].f0 == plan[j - 1].f1) j++;
             const size_t bytes = (size_t)(plan[j - 1].f1 - plan[k].f0) * frame_sz;
-            CU(h, cudaMemcpyAsync(s->d_in + off, frames + plan[k].f0 * frame_sz, bytes, cudaMemcpyHostToDevice, st));
+            CU(h, cudaMemcpyAsync(s->d_in.p + off, frames + plan[k].f0 * frame_sz, bytes, cudaMemcpyHostToDevice, st));
             off += bytes;
             k = j;
         }
-        if ((rc = prep_then_tail(h, st, region_base(s->d_in, 0, 0, s->d_out), n, detect, pred.probs(0), pred.cls(0), pred.bbox(0), flags)))
+        if ((rc = prep_then_tail(h, st, region_base(s->d_in.p, 0, 0, s->d_out.p), n, detect, pred.probs(0), pred.cls(0), pred.bbox(0), flags)))
             return rc;
-        if (gray128) CU(h, cudaMemcpyAsync(gray128, s->d_out, n * img_sz, cudaMemcpyDeviceToHost, st));
+        if (gray128) CU(h, cudaMemcpyAsync(gray128, s->d_out.p, n * img_sz, cudaMemcpyDeviceToHost, st));
         if (mg) rc = merge_block(pred, st);
         else if (detect) rc = pred.flush(st, probs, cls, bbox, false);
         if (db) CU(h, cudaEventRecord(db->ev, st));
@@ -1503,16 +1502,16 @@ static int regions_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n_frame
             bi++;
         }
         if ((rc = call.acquire(s, max_stage, per_launch * img_sz))) return rc;
-        CU(h, cudaMemcpyAsync(s->d_in, frames + c.f0 * frame_sz, (size_t)(c.f1 - c.f0) * frame_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        CU(h, cudaMemcpyAsync(s->d_in.p, frames + c.f0 * frame_sz, (size_t)(c.f1 - c.f0) * frame_sz, cudaMemcpyHostToDevice, h->st_h2d));
         if ((rc = call.staged(*s))) return rc;
         for (int64_t r = c.r0; r < c.r1; r += per_launch) {
             const int64_t m = std::min(per_launch, c.r1 - r);
             if (r > c.r0 && gray128 && (rc = call.wait_released(*s, h->st_k))) return rc;
-            if ((rc = prep_then_tail(h, h->st_k, region_base(s->d_in, r, c.r0, s->d_out), m, detect, detect ? pred.probs(r) : nullptr,
+            if ((rc = prep_then_tail(h, h->st_k, region_base(s->d_in.p, r, c.r0, s->d_out.p), m, detect, detect ? pred.probs(r) : nullptr,
                                      detect ? pred.cls(r) : nullptr, detect ? pred.bbox(r) : nullptr, flags)) ||
                 (rc = call.computed(*s)))
                 return rc;
-            if (gray128) CU(h, cudaMemcpyAsync(gray128 + r * img_sz, s->d_out, m * img_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+            if (gray128) CU(h, cudaMemcpyAsync(gray128 + r * img_sz, s->d_out.p, m * img_sz, cudaMemcpyDeviceToHost, h->st_d2h));
             if ((rc = call.released(*s, h->st_d2h))) return rc;
         }
     }
@@ -1566,14 +1565,14 @@ static int merge_impl(cnnacc_handle* h, const int32_t* regions, int64_t n, int64
         REQUIRE_ALIGNED(h, M.det_score, 4, "det_score");
         DescBuf* db = nullptr;
         if ((rc = desc_acquire(h, n, &db, n_frames + 1))) return rc;
-        fill_desc(db->host, rg, n);
-        std::memcpy(db->first_host, M.first.data(), first_bytes);
-        if (n) CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
-        CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, first_bytes, cudaMemcpyHostToDevice, h->stream));
-        A.desc = db->dev; A.r_pred0 = 0; A.score = scores; A.cls = cls; A.bbox = bbox;
+        fill_desc(db->host.p, rg, n);
+        std::memcpy(db->first_host.p, M.first.data(), first_bytes);
+        if (n) CU(h, cudaMemcpyAsync(db->dev.p, db->host.p, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, h->stream));
+        CU(h, cudaMemcpyAsync(db->first_dev.p, db->first_host.p, first_bytes, cudaMemcpyHostToDevice, h->stream));
+        A.desc = db->dev.p; A.r_pred0 = 0; A.score = scores; A.cls = cls; A.bbox = bbox;
         A.n_det = M.n_det; A.det_region = M.det_region; A.det_cls = M.det_cls; A.det_score = M.det_score;
         A.det_box = reinterpret_cast<float4*>(M.det_box);
-        rc = launch_merge(h, h->stream, A, M, db->first_dev, 0, n_frames);
+        rc = launch_merge(h, h->stream, A, M, db->first_dev.p, 0, n_frames);
         CU(h, cudaEventRecord(db->ev, h->stream));     // also after a failed launch: earlier ones may still read it
         return rc;
     }
@@ -1583,29 +1582,29 @@ static int merge_impl(cnnacc_handle* h, const int32_t* regions, int64_t n, int64
     cudaStream_t st = h->st_k;
     DescBuf* db = nullptr;
     if ((rc = desc_acquire(h, n, &db, n_frames + 1))) return rc;
-    fill_desc(db->host, rg, n);
-    std::memcpy(db->first_host, M.first.data(), first_bytes);
-    if (n) CU(h, cudaMemcpyAsync(db->dev, db->host, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, st));
-    CU(h, cudaMemcpyAsync(db->first_dev, db->first_host, first_bytes, cudaMemcpyHostToDevice, st));
+    fill_desc(db->host.p, rg, n);
+    std::memcpy(db->first_host.p, M.first.data(), first_bytes);
+    if (n) CU(h, cudaMemcpyAsync(db->dev.p, db->host.p, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, st));
+    CU(h, cudaMemcpyAsync(db->first_dev.p, db->first_host.p, first_bytes, cudaMemcpyHostToDevice, st));
     const std::vector<int64_t> blocks = frame_aligned_blocks([&](int64_t r) { return rg.frame(r); }, n, kPredSuper);
     int64_t most = 0;
     for (size_t k = 1; k < blocks.size(); k++) most = std::max(most, blocks[k] - blocks[k - 1]);
-    if (most && (rc = grow(h, &h->d_mpred, &h->cap_mpred, (size_t)most * 24))) return rc;
-    A.desc = db->dev;
+    if (most && (rc = grow(h, h->d_mpred, (size_t)most * 24))) return rc;
+    A.desc = db->dev.p;
     int64_t fa = 0;
     for (size_t k = 0; k < std::max<size_t>(1, blocks.size() - 1); k++) {
         const int64_t b0 = blocks[k], m = blocks.size() > 1 ? blocks[k + 1] - b0 : 0;
         const int64_t fb = b0 + m == n ? n_frames : rg.frame(b0 + m);
         if (m) {
-            CU(h, cudaMemcpyAsync(h->d_mpred, bbox + 4 * b0, (size_t)m * 16, cudaMemcpyHostToDevice, st));
-            CU(h, cudaMemcpyAsync(h->d_mpred + (size_t)m * 16, scores + b0, (size_t)m * 4, cudaMemcpyHostToDevice, st));
-            CU(h, cudaMemcpyAsync(h->d_mpred + (size_t)m * 20, cls + b0, (size_t)m * 4, cudaMemcpyHostToDevice, st));
+            CU(h, cudaMemcpyAsync(h->d_mpred.p, bbox + 4 * b0, (size_t)m * 16, cudaMemcpyHostToDevice, st));
+            CU(h, cudaMemcpyAsync(h->d_mpred.p + (size_t)m * 16, scores + b0, (size_t)m * 4, cudaMemcpyHostToDevice, st));
+            CU(h, cudaMemcpyAsync(h->d_mpred.p + (size_t)m * 20, cls + b0, (size_t)m * 4, cudaMemcpyHostToDevice, st));
         }
         A.r_pred0 = b0;
-        A.bbox = reinterpret_cast<const int32_t*>(h->d_mpred);
-        A.score = reinterpret_cast<const float*>(h->d_mpred + (size_t)m * 16);
-        A.cls = reinterpret_cast<const int32_t*>(h->d_mpred + (size_t)m * 20);
-        rc = merge_to_host(h, st, A, M, db->first_dev, fa, fb);
+        A.bbox = reinterpret_cast<const int32_t*>(h->d_mpred.p);
+        A.score = reinterpret_cast<const float*>(h->d_mpred.p + (size_t)m * 16);
+        A.cls = reinterpret_cast<const int32_t*>(h->d_mpred.p + (size_t)m * 20);
+        rc = merge_to_host(h, st, A, M, db->first_dev.p, fa, fb);
         if (rc) break;
         fa = fb;
     }
@@ -1727,12 +1726,13 @@ int cnnacc_probe_int8_peak(cnnacc_handle* h, double target_ms, double* tops, dou
     if (!h || !tops) return fail(h, CNNACC_ERR_ARG, "NULL argument");
     if (!(target_ms > 0.0) || target_ms > 2000.0) return fail(h, CNNACC_ERR_ARG, "target_ms outside (0, 2000]");
     CU(h, cudaSetDevice(h->device));
-    int* d_status = nullptr;
-    CU(h, cudaMalloc(&d_status, sizeof(int)));
-    CU(h, cudaMemset(d_status, 0, sizeof(int)));
+    int rc;
+    Buf<int> d_status;
+    if ((rc = grow(h, d_status, 1))) return rc;
+    CU(h, cudaMemset(d_status.p, 0, sizeof(int)));
     auto run = [&](int iters, float* ms) -> int {
         CU(h, cudaEventRecord(h->ev_a, h->stream));
-        int8_peak_probe_kernel<<<h->sm_count, 32, kProbeSmem, h->stream>>>(iters, d_status);
+        int8_peak_probe_kernel<<<h->sm_count, 32, kProbeSmem, h->stream>>>(iters, d_status.p);
         h->launches++;
         CU(h, cudaGetLastError());
         CU(h, cudaEventRecord(h->ev_b, h->stream));
@@ -1740,16 +1740,14 @@ int cnnacc_probe_int8_peak(cnnacc_handle* h, double target_ms, double* tops, dou
         CU(h, cudaEventElapsedTime(ms, h->ev_a, h->ev_b));
         return 0;
     };
-    int rc; float ms = 0.f;
+    float ms = 0.f;
     const int iters0 = 1 << 15;                                          // calibration: ~2 ms
-    if ((rc = run(iters0, &ms)) || (rc = run(iters0, &ms))) { cudaFree(d_status); return rc; }
+    if ((rc = run(iters0, &ms)) || (rc = run(iters0, &ms))) return rc;
     double want = (double)iters0 * target_ms / std::max(ms, 1e-3f);
     const int iters = (int)std::min<double>(1 << 30, std::max<double>(iters0, want)) & ~7;
-    if ((rc = run(iters, &ms))) { cudaFree(d_status); return rc; }
+    if ((rc = run(iters, &ms))) return rc;
     int st = 0;
-    const cudaError_t e_st = cudaMemcpy(&st, d_status, sizeof(int), cudaMemcpyDeviceToHost);
-    cudaFree(d_status);
-    CU(h, e_st);
+    CU(h, cudaMemcpy(&st, d_status.p, sizeof(int), cudaMemcpyDeviceToHost));
     if (st) return fail(h, CNNACC_ERR_CUDA, "int8 peak probe timed out");
     *tops = (double)h->sm_count * iters * kProbeOpsPerMma / (ms * 1e-3) / 1e12;
     if (ms_out) *ms_out = ms;
@@ -1779,14 +1777,14 @@ int cnnacc_image_to_gray128(cnnacc_handle* h, const uint8_t* img, int64_t n, int
     if (H != h->pil_h || W != h->pil_w) {                // Pillow's coefficient tables depend on the input size
         CU(h, cudaDeviceSynchronize());
         const PilTabHost tx = make_pil_tab(W), ty = make_pil_tab(H);
-        for (int32_t** p : {&h->d_pil_kx, &h->d_pil_bx, &h->d_pil_ky, &h->d_pil_by}) { cudaFree(*p); *p = nullptr; }
         h->pil_h = h->pil_w = 0;
-        CU(h, cudaMalloc(&h->d_pil_kx, tx.k.size() * 4)); CU(h, cudaMalloc(&h->d_pil_bx, tx.bounds.size() * 4));
-        CU(h, cudaMalloc(&h->d_pil_ky, ty.k.size() * 4)); CU(h, cudaMalloc(&h->d_pil_by, ty.bounds.size() * 4));
-        CU(h, cudaMemcpy(h->d_pil_kx, tx.k.data(), tx.k.size() * 4, cudaMemcpyHostToDevice));
-        CU(h, cudaMemcpy(h->d_pil_bx, tx.bounds.data(), tx.bounds.size() * 4, cudaMemcpyHostToDevice));
-        CU(h, cudaMemcpy(h->d_pil_ky, ty.k.data(), ty.k.size() * 4, cudaMemcpyHostToDevice));
-        CU(h, cudaMemcpy(h->d_pil_by, ty.bounds.data(), ty.bounds.size() * 4, cudaMemcpyHostToDevice));
+        if ((rc = grow(h, h->d_pil_kx, tx.k.size())) || (rc = grow(h, h->d_pil_bx, tx.bounds.size())) ||
+            (rc = grow(h, h->d_pil_ky, ty.k.size())) || (rc = grow(h, h->d_pil_by, ty.bounds.size())))
+            return rc;
+        CU(h, cudaMemcpy(h->d_pil_kx.p, tx.k.data(), tx.k.size() * 4, cudaMemcpyHostToDevice));
+        CU(h, cudaMemcpy(h->d_pil_bx.p, tx.bounds.data(), tx.bounds.size() * 4, cudaMemcpyHostToDevice));
+        CU(h, cudaMemcpy(h->d_pil_ky.p, ty.k.data(), ty.k.size() * 4, cudaMemcpyHostToDevice));
+        CU(h, cudaMemcpy(h->d_pil_by.p, ty.bounds.data(), ty.bounds.size() * 4, cudaMemcpyHostToDevice));
         h->pil_kw = tx.ksize; h->pil_kh = ty.ksize; h->pil_h = H; h->pil_w = W;
     }
     const size_t in_bytes = (size_t)n * H * W * C, out_bytes = (size_t)n * kPilOut * kPilOut;
@@ -1795,10 +1793,10 @@ int cnnacc_image_to_gray128(cnnacc_handle* h, const uint8_t* img, int64_t n, int
     const uint8_t* d_in = img;
     uint8_t* d_out = gray128;
     if (!dev) {
-        if ((rc = grow(h, &h->d_pil_in, &h->cap_pil_in, in_bytes))) return rc;
-        if ((rc = grow(h, &h->d_pil_out, &h->cap_pil_out, out_bytes))) return rc;
-        CU(h, cudaMemcpyAsync(h->d_pil_in, img, in_bytes, cudaMemcpyHostToDevice, st));
-        d_in = h->d_pil_in; d_out = h->d_pil_out;
+        if ((rc = grow(h, h->d_pil_in, in_bytes))) return rc;
+        if ((rc = grow(h, h->d_pil_out, out_bytes))) return rc;
+        CU(h, cudaMemcpyAsync(h->d_pil_in.p, img, in_bytes, cudaMemcpyHostToDevice, st));
+        d_in = h->d_pil_in.p; d_out = h->d_pil_out.p;
     }
     const unsigned nu = (unsigned)n;
     if (H > 100 * W && H > kPilOut) {
@@ -1806,13 +1804,13 @@ int cnnacc_image_to_gray128(cnnacc_handle* h, const uint8_t* img, int64_t n, int
         // folded in, writes [n][128][W] -- the result itself when W == 128 -- and the horizontal pass reads that
         uint8_t* d_tmp = d_out;
         if (W != kPilOut) {
-            if ((rc = grow(h, &h->d_pil_tmp, &h->cap_pil_tmp, (size_t)n * kPilOut * W))) return rc;
-            d_tmp = h->d_pil_tmp;
+            if ((rc = grow(h, h->d_pil_tmp, (size_t)n * kPilOut * W))) return rc;
+            d_tmp = h->d_pil_tmp.p;
         }
-        pil_vertical_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_in, d_tmp, h->d_pil_ky, h->d_pil_by, h->pil_kh, H, W, C);
+        pil_vertical_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_in, d_tmp, h->d_pil_ky.p, h->d_pil_by.p, h->pil_kh, H, W, C);
         h->launches++;
         if (W != kPilOut) {
-            pil_horizontal_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_tmp, d_out, h->d_pil_kx, h->d_pil_bx, h->pil_kw, kPilOut, W, 1, 0);
+            pil_horizontal_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_tmp, d_out, h->d_pil_kx.p, h->d_pil_bx.p, h->pil_kw, kPilOut, W, 1, 0);
             h->launches++;
         }
     } else {
@@ -1820,13 +1818,13 @@ int cnnacc_image_to_gray128(cnnacc_handle* h, const uint8_t* img, int64_t n, int
         // the horizontal pass (or, at W == 128, the plain gray conversion) writes [n][H][128]: the result itself when H == 128
         uint8_t* d_tmp = d_out;
         if (need_v) {
-            if ((rc = grow(h, &h->d_pil_tmp, &h->cap_pil_tmp, (size_t)n * H * kPilOut))) return rc;
-            d_tmp = h->d_pil_tmp;
+            if ((rc = grow(h, h->d_pil_tmp, (size_t)n * H * kPilOut))) return rc;
+            d_tmp = h->d_pil_tmp.p;
         }
-        pil_horizontal_kernel<<<dim3((unsigned)H, nu), kPilOut, 0, st>>>(d_in, d_tmp, h->d_pil_kx, h->d_pil_bx, h->pil_kw, H, W, C, W == kPilOut);
+        pil_horizontal_kernel<<<dim3((unsigned)H, nu), kPilOut, 0, st>>>(d_in, d_tmp, h->d_pil_kx.p, h->d_pil_bx.p, h->pil_kw, H, W, C, W == kPilOut);
         h->launches++;
         if (need_v) {
-            pil_vertical_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_tmp, d_out, h->d_pil_ky, h->d_pil_by, h->pil_kh, H, kPilOut, 1);
+            pil_vertical_kernel<<<dim3(kPilOut, nu), kPilOut, 0, st>>>(d_tmp, d_out, h->d_pil_ky.p, h->d_pil_by.p, h->pil_kh, H, kPilOut, 1);
             h->launches++;
         }
     }
