@@ -63,6 +63,10 @@ SYMBOLS = {
                                         _c.c_float, _c.c_int] + [_c.c_void_p] * 5 + [_c.c_uint32]),
     "cnnacc_merge_regions_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_float,
                                              _c.c_float, _c.c_int] + [_c.c_void_p] * 5 + [_c.c_uint32]),
+    "cnnacc_scan_frames": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p, _c.c_void_p,
+                                      _c.c_void_p, _c.c_uint32]),
+    "cnnacc_scan_objects": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_float, _c.c_float,
+                                       _c.c_int] + [_c.c_void_p] * 5 + [_c.c_uint32]),
     "cnnacc_region_plan_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int]),
     "cnnacc_rect_plan_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int]),
     "cnnacc_area_tab_host": (_c.c_int, [_c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_int]),

@@ -598,6 +598,55 @@ class CNNAccelerator:
                                                         flags | kind))
         return _callers_regions(dets, order)
 
+    def scan_frames(self, frames, stride=64, logits=False):
+        """Classify every 128x128 window of whole frames from one conv pass per frame: frames [F,h,w,3] u8 BGR (numpy, or a
+        contiguous CUDA uint8 tensor run on torch's current stream), h and w multiples of 16 in 128..8192, stride a positive
+        multiple of 8.  The windows are grid_regions(F, h, w, 128, stride), in that order.  Each frame is converted to gray
+        and run through the conv stack once (run_batch at h x w); window (f, x, y) gets classify_batch's predictions for the
+        16x16 cells of that map at (x/8, y/8), bit for bit, its box on the window's 128 grid (region_boxes_to_frame maps it).
+        Not detect_regions on the same squares: a region is zero-padded at its own border, a scan window sees the frame's
+        pixels beyond it, so the two agree on the inner 14x14 cells (and on the sides where the window meets the frame edge);
+        on 128x128 frames they are the same.  logits=True: the second element holds the raw logits instead of the softmax.
+        -> (cls [R] i32, probs [R,n_cls] f32, bbox [R,4] i32), numpy or torch like frames."""
+        n_cls = self._classes()
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
+        nf, fh, fw = self._scan_shape(frames, stride)
+        cls, probs, box = _pred_outputs(new, nf * self._scan_windows(fh, fw, stride), n_cls)
+        with ctx:
+            self._check(self._libc.cnnacc_scan_frames(self._h, ptr(frames), nf, fh, fw, int(stride), ptr(probs), ptr(cls), ptr(box),
+                                                      _pred_flags("vec", logits) | kind))
+        return cls, probs, box
+
+    def scan_objects(self, frames, stride=64, score_min=0.0, iou_max=0.5, max_det=100, class_agnostic=False, logits=False):
+        """scan_frames followed by detect_objects' per-frame greedy NMS on the GPU, the windows grid_regions(F, h, w, 128,
+        stride) being the regions: exactly merge_regions(grid_regions(...), cls, probs[r, cls[r]], bbox, F, ...) on
+        scan_frames' outputs (see scan_frames for how a window differs from a detect_regions region).  At most 16384 windows
+        per frame.  -> as detect_objects, with region indexing the window order; numpy or torch like frames."""
+        flags = _pred_flags("vec", logits) | _merge_flags(max_det, class_agnostic)
+        self._classes()
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
+        nf, fh, fw = self._scan_shape(frames, stride)
+        dets = _det_outputs(new, nf, int(max_det))
+        with ctx:
+            self._check(self._libc.cnnacc_scan_objects(self._h, ptr(frames), nf, fh, fw, int(stride), float(score_min),
+                                                       float(iou_max), int(max_det), *[ptr(a) for a in dets], flags | kind))
+        return dets
+
+    @staticmethod
+    def _scan_shape(frames, stride):
+        if frames.ndim != 4 or frames.shape[3] != 3:
+            raise ValueError("expected [F,h,w,3] BGR frames")
+        if int(stride) != stride:
+            raise ValueError("stride must be an integer")
+        return frames.shape[:3]
+
+    @staticmethod
+    def _scan_windows(fh, fw, stride):
+        """Windows per frame of grid_regions(1, fh, fw, 128, stride); 0 where the library refuses the call anyway."""
+        if stride < 1 or min(fh, fw) < 128:
+            return 0
+        return len(_tile_origins(fh, 128, stride)) * len(_tile_origins(fw, 128, stride))
+
     def infer_one(self, gray128):
         """One image, lowest latency.  -> (feat (64,256) u8, conv_ms, read_ms)."""
         img = gray128 if (type(gray128) is np.ndarray and gray128.dtype == np.uint8 and gray128.flags.c_contiguous) \

@@ -108,7 +108,7 @@ struct cnnacc_handle {
     Stream st_h2d, st_k, st_d2h;                    // one stream per engine for host-pointer batches
     Event ev_t0, ev_t1, ev_a, ev_b, ev_done;
     int sm_count = 0;
-    bool weights_loaded = false, fc_loaded = false, tail_attr_set = false;
+    bool weights_loaded = false, fc_loaded = false, tail_attr_set = false, scan_attr_set = false;
     int shifts[3] = {2, 4, 6};                  // SHIFT_L0..2 defaults, pynq_inference.py:83-85
     bool acc24 = false;                         // accumulator width: false = int32 (arm_cnn.c:31), true = 24-bit wrap (accumulator.v:15)
     uint8_t wbin[CNNACC_WEIGHT_BYTES];
@@ -124,6 +124,8 @@ struct cnnacc_handle {
     int prep_side = 0; AreaTabHost prep_tab;
     Buf<int> d_prep_start, d_prep_cnt; Buf<float> d_prep_alpha;
     Buf<uint8_t> d_gray;
+    // scanning calls (cnnacc_scan_frames / cnnacc_scan_objects): full-resolution gray frames and their feature maps
+    Buf<uint8_t> d_scan_gray, d_scan_feat;
     DescBuf rdesc[kDescRing]; int rdesc_next = 0;   // region calls (regions_impl)
     // merging calls (region_merge.cuh): device predictions of detect_objects' device-pointer path, and the detections of
     // host-pointer merges on the device and in pinned memory
@@ -315,18 +317,24 @@ TailArgs make_tail(const cnnacc_handle* h, float* d_probs, int32_t* d_cls, int32
     return A;
 }
 
-// classify_vec + bbox_vec on n device-resident feature maps (tail.cuh)
-int launch_tail(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_feats, int64_t n, const TailArgs& A) {
+// classify_vec + bbox_vec on n device-resident feature maps that `maps` fetches (tail.cuh); attr_set: the handle's flag of
+// this kernel instance's shared-memory attribute
+template <class Maps>
+int launch_tail_kernel(cnnacc_handle* h, cudaStream_t stream, const Maps& maps, int64_t n, const TailArgs& A, bool& attr_set) {
     if (n == 0) return 0;
-    if (!h->tail_attr_set) {
-        CU(h, cudaFuncSetAttribute(classify_bbox_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTailSmem));
-        h->tail_attr_set = true;
+    if (!attr_set) {
+        CU(h, cudaFuncSetAttribute(classify_bbox_kernel<Maps>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTailSmem));
+        attr_set = true;
     }
     const unsigned grid = (unsigned)std::min<int64_t>((n + kTailGroups - 1) / kTailGroups, h->sm_count);
-    classify_bbox_kernel<<<grid, kTailGroups * kTailThreads, kTailSmem, stream>>>(d_feats, (long long)n, A);
+    classify_bbox_kernel<Maps><<<grid, kTailGroups * kTailThreads, kTailSmem, stream>>>(maps, (long long)n, A);
     h->launches++;
     CU(h, cudaGetLastError());
     return 0;
+}
+// ... on n compact 16 KiB maps
+int launch_tail(cnnacc_handle* h, cudaStream_t stream, const uint8_t* d_feats, int64_t n, const TailArgs& A) {
+    return launch_tail_kernel(h, stream, CompactMaps{d_feats}, n, A, h->tail_attr_set);
 }
 
 // Conv stack + tail for m device-resident 128x128 images on `stream`.  The fused kernel's tail warps produce the
@@ -1648,6 +1656,182 @@ int cnnacc_merge_regions_host(const int32_t* regions, int64_t n_regions, int64_t
                                     M.agnostic, det_region ? det_region + f * D : nullptr, det_cls ? det_cls + f * D : nullptr,
                                     det_score ? det_score + f * D : nullptr, det_box ? det_box + f * D * 4 : nullptr);
     return CNNACC_OK;
+}
+
+// ---- scanning whole frames (cnnacc_scan_frames / cnnacc_scan_objects) ---------------------------------------------------
+
+// Scan windows along a side of `side` pixels: 0, stride, 2 stride, ... plus one flush with the far edge when that is missing.
+static int scan_count(int side, int stride) {
+    const int last = side - CNNACC_IMG;
+    return last / stride + 1 + (last % stride != 0);
+}
+
+// Gray, conv stack once per frame, then every window's predictions read straight out of the frame's feature map; with `mg`
+// (scan_objects) the predictions stay on the device and are merged per frame with the windows as (f, x, y, 128) regions.
+static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, int stride, float* probs, int32_t* cls,
+                     int32_t* bbox, uint32_t flags, MergeSpec* mg) {
+    int rc;
+    if (!h) return CNNACC_ERR_ARG;
+    if ((rc = check_ready(h))) return rc;
+    if (!h->fc_loaded) return fail(h, CNNACC_ERR_STATE, "classifier not loaded (call cnnacc_load_classifier)");
+    if (n < 0) return fail(h, CNNACC_ERR_ARG, "negative n");
+    if (!valid_hw(fh, fw) || fh < CNNACC_IMG || fw < CNNACC_IMG)
+        return fail(h, CNNACC_ERR_ARG, "frame sides must be multiples of 16 in 128..8192");
+    if (stride < 8 || stride % 8) return fail(h, CNNACC_ERR_ARG, "stride must be a positive multiple of 8");
+    if (flags & (CNNACC_FLAG_BBOX_UPSAMPLED | CNNACC_FLAG_RECTS | CNNACC_FLAG_DIRECT | CNNACC_FLAG_KEEP_MAPS | CNNACC_FLAG_TWO_KERNELS))
+        return fail(h, CNNACC_ERR_ARG, "BBOX_UPSAMPLED / RECTS / DIRECT / KEEP_MAPS / TWO_KERNELS have no scanning form");
+    const int nx = scan_count(fw, stride), ny = scan_count(fh, stride);
+    const int64_t per = (int64_t)nx * ny;
+    if (n > 0x7fffffffLL / per) return fail(h, CNNACC_ERR_ARG, "more than 2^31-1 windows in one call");
+    if (mg) {
+        if (!mg->n_det) return fail(h, CNNACC_ERR_ARG, "NULL n_det");
+        if (const char* why = merge_limits_error(mg->iou_max, mg->max_det)) return fail(h, CNNACC_ERR_ARG, why);
+        if (per > kMergeMaxPerFrame) return fail(h, CNNACC_ERR_ARG, "more than 16384 windows per frame in a merging call");
+    }
+    if (n == 0) return CNNACC_OK;
+    if (!frames) return fail(h, CNNACC_ERR_ARG, "NULL frame pointer");
+    CU(h, cudaSetDevice(h->device));
+    const size_t frame_sz = (size_t)fh * fw * 3, plane = (size_t)fh * fw;   // a gray frame and its map are both fh * fw bytes
+    const int nc = h->n_cls;
+    ScanWindows win;
+    win.ho = fh / 8; win.wo = fw / 8; win.nx = nx; win.ny = ny; win.step = stride / 8;
+    win.umax = (fw - CNNACC_IMG) / 8; win.vmax = (fh - CNNACC_IMG) / 8;
+    // gray and feature workspaces for k frames (the window gather may read 16 bytes past the last map)
+    auto grow_ws = [&](int64_t k) -> int {
+        int r;
+        if ((r = grow(h, h->d_scan_gray, (size_t)k * plane)) || (r = grow(h, h->d_scan_feat, (size_t)k * plane + 16))) return r;
+        return 0;
+    };
+    // gray -> conv stack -> window tail for k frames staged at d_frames; p / c / b: the predictions of their first window
+    auto kernels = [&](cudaStream_t st, const uint8_t* d_frames, int64_t k, float* p, int32_t* c, int32_t* b) -> int {
+        const long long quads = (long long)(k * plane / 4);
+        gray_full_kernel<<<(unsigned)std::min<long long>((quads + 255) / 256, 16LL * h->sm_count), 256, 0, st>>>(
+            d_frames, h->d_scan_gray.p, quads);
+        h->launches++;
+        CU(h, cudaGetLastError());
+        int r;
+        if ((r = conv_stack_device(h, st, h->d_scan_gray.p, k, fh, fw, h->d_scan_feat.p, 0, nullptr, nullptr))) return r;
+        ScanWindows w = win;
+        w.feats = h->d_scan_feat.p;
+        return launch_tail_kernel(h, st, w, k * per, make_tail(h, p, c, b, false, flags), h->scan_attr_set);
+    };
+    // the merge's region descriptors (f, x, y, 128) and per-frame ranges, uploaded on st
+    DescBuf* db = nullptr;
+    auto upload_desc = [&](cudaStream_t st) -> int {
+        int r;
+        if ((r = desc_acquire(h, n * per, &db, n + 1))) return r;
+        mg->first.resize((size_t)n + 1);
+        for (int64_t f = 0; f <= n; f++) mg->first[f] = f * per;
+        int4* d = db->host.p;
+        for (int64_t f = 0; f < n; f++)
+            for (int iy = 0; iy < ny; iy++)
+                for (int ix = 0; ix < nx; ix++)
+                    *d++ = make_int4((int)f, std::min(ix * stride, fw - CNNACC_IMG), std::min(iy * stride, fh - CNNACC_IMG), CNNACC_IMG);
+        std::memcpy(db->first_host.p, mg->first.data(), (size_t)(n + 1) * sizeof(long long));
+        CU(h, cudaMemcpyAsync(db->dev.p, db->host.p, (size_t)(n * per) * sizeof(int4), cudaMemcpyHostToDevice, st));
+        CU(h, cudaMemcpyAsync(db->first_dev.p, db->first_host.p, (size_t)(n + 1) * sizeof(long long), cudaMemcpyHostToDevice, st));
+        return 0;
+    };
+
+    if (flags & CNNACC_FLAG_DEVICE_PTRS) {
+        REQUIRE_ALIGNED(h, bbox, 16, "bbox");
+        REQUIRE_ALIGNED(h, probs, 4, "probs");
+        REQUIRE_ALIGNED(h, cls, 4, "cls");
+        if (mg) {
+            REQUIRE_ALIGNED(h, mg->det_box, 16, "det_box");
+            REQUIRE_ALIGNED(h, mg->n_det, 4, "n_det");
+            REQUIRE_ALIGNED(h, mg->det_region, 4, "det_region");
+            REQUIRE_ALIGNED(h, mg->det_cls, 4, "det_cls");
+            REQUIRE_ALIGNED(h, mg->det_score, 4, "det_score");
+        }
+        // pieces of whole frames: gray and feature workspaces of at most 256 MiB each, at most kPredSuper windows
+        const int64_t chunk = std::min<int64_t>(n, std::max<int64_t>(1, std::min<int64_t>(((size_t)256 << 20) / plane, kPredSuper / per)));
+        if ((rc = grow_ws(chunk))) return rc;
+        const size_t cw = (size_t)(chunk * per), w_probs = cw * 16, w_cls = w_probs + cw * nc * 4;   // PredBlock's layout
+        if (mg && ((rc = grow(h, h->d_mpred, cw * kPredBytesPerImage)) || (rc = upload_desc(h->stream)))) return rc;
+        auto run = [&]() -> int {
+            int r;
+            for (int64_t f0 = 0; f0 < n; f0 += chunk) {
+                const int64_t k = std::min(chunk, n - f0), w0 = f0 * per;
+                if (!mg) {
+                    if ((r = kernels(h->stream, frames + f0 * frame_sz, k, probs ? probs + w0 * nc : nullptr, cls ? cls + w0 : nullptr,
+                                     bbox ? bbox + w0 * 4 : nullptr)))
+                        return r;
+                    continue;
+                }
+                int32_t* wb = reinterpret_cast<int32_t*>(h->d_mpred.p);
+                float* wp = reinterpret_cast<float*>(h->d_mpred.p + w_probs);
+                int32_t* wc = reinterpret_cast<int32_t*>(h->d_mpred.p + w_cls);
+                MergeArgs A = merge_args_of_predictions(db->dev.p, w0, wb, wp, wc, nc, *mg);
+                A.n_det += f0;
+                const size_t o = (size_t)f0 * mg->max_det;
+                if (A.det_region) A.det_region += o;
+                if (A.det_cls) A.det_cls += o;
+                if (A.det_score) A.det_score += o;
+                if (A.det_box) A.det_box += o;
+                if ((r = kernels(h->stream, frames + f0 * frame_sz, k, wp, wc, wb)) ||
+                    (r = launch_merge(h, h->stream, A, *mg, db->first_dev.p, f0, f0 + k)))
+                    return r;
+            }
+            return 0;
+        };
+        rc = run();
+        if (db) CU(h, cudaEventRecord(db->ev, h->stream));   // also after a failed launch: earlier ones may still read it
+        return rc;
+    }
+
+    // Host pointers: prediction blocks of whole frames (a frame has fewer than kPredSuper windows), staged in chunks of about
+    // 16 MiB of frames (a larger frame alone) through the ring.
+    HostCall call(h);
+    if ((rc = call.begin())) return rc;
+    const std::vector<int64_t> blocks = frame_aligned_blocks([per](int64_t r) { return r / per; }, n * per, kPredSuper);
+    const int64_t fpc = std::min<int64_t>(n, std::max<int64_t>(1, (int64_t)(kRegionChunkBytes / frame_sz)));
+    const bool small = blocks.size() == 2 && n <= fpc;    // latency path: one chunk, one stream, one result copy
+    cudaStream_t st = small ? h->st_k : h->st_h2d;
+    if ((rc = grow_ws(fpc)) || (mg && (rc = upload_desc(st)))) return rc;
+    PredBlock pred(h);
+    auto finish_block = [&](cudaStream_t s, int64_t fa, int64_t fb) -> int {
+        if (!mg) return pred.flush(s, probs, cls, bbox, false);
+        const MergeArgs A = merge_args_of_predictions(db->dev.p, pred.s0, pred.bbox(pred.s0), pred.probs(pred.s0), pred.cls(pred.s0), nc, *mg);
+        return merge_to_host(h, s, A, *mg, db->first_dev.p, fa, fb);
+    };
+    Slot* s;
+    if (small) {
+        if ((rc = call.acquire(s, n * frame_sz, 0)) || (rc = pred.start(0, n * per))) return rc;
+        CU(h, cudaMemcpyAsync(s->d_in.p, frames, n * frame_sz, cudaMemcpyHostToDevice, st));
+        if (!(rc = kernels(st, s->d_in.p, n, pred.probs(0), pred.cls(0), pred.bbox(0)))) rc = finish_block(st, 0, n);
+    } else {
+        for (size_t bi = 0; !rc && bi + 1 < blocks.size(); bi++) {
+            const int64_t fa = blocks[bi] / per, fb = blocks[bi + 1] / per;
+            if ((rc = pred.start(blocks[bi], blocks[bi + 1] - blocks[bi]))) break;
+            for (int64_t f0 = fa; !rc && f0 < fb; f0 += fpc) {
+                const int64_t k = std::min(fpc, fb - f0);
+                if ((rc = call.acquire(s, fpc * frame_sz, 0))) break;
+                CU(h, cudaMemcpyAsync(s->d_in.p, frames + f0 * frame_sz, k * frame_sz, cudaMemcpyHostToDevice, h->st_h2d));
+                if (!(rc = call.staged(*s)) && !(rc = kernels(h->st_k, s->d_in.p, k, pred.probs(f0 * per), pred.cls(f0 * per),
+                                                               pred.bbox(f0 * per))))
+                    rc = call.released(*s, h->st_k);
+            }
+            if (!rc) rc = finish_block(h->st_k, fa, fb);
+        }
+        st = h->st_k;
+    }
+    if (db) CU(h, cudaEventRecord(db->ev, st));
+    if (rc) return rc;
+    return call.done(true);                               // finish_block waited for st
+}
+
+int cnnacc_scan_frames(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, int stride, float* probs, int32_t* cls,
+                       int32_t* bbox, uint32_t flags) {
+    return scan_impl(h, frames, n, fh, fw, stride, probs, cls, bbox, flags, nullptr);
+}
+
+int cnnacc_scan_objects(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, int stride, float score_min, float iou_max,
+                        int max_det, int32_t* n_det, int32_t* det_region, int32_t* det_cls, float* det_score, float* det_box,
+                        uint32_t flags) {
+    if (!h) return CNNACC_ERR_ARG;
+    MergeSpec M = make_merge_spec(score_min, iou_max, max_det, n_det, det_region, det_cls, det_score, det_box, flags);
+    return scan_impl(h, frames, n, fh, fw, stride, nullptr, nullptr, nullptr, flags, &M);
 }
 
 static int region_plan_host(const RegionRecords& rg, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t* chunks, int cap) {

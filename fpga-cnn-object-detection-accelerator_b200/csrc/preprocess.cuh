@@ -115,6 +115,19 @@ __device__ __forceinline__ int bgr2gray(const uint8_t* p) {
     return (3735 * (int)__ldg(p) + 19235 * (int)__ldg(p + 1) + 9798 * (int)__ldg(p + 2) + (1 << 14)) >> 15;
 }
 
+// cvtColor(COLOR_BGR2GRAY) at full resolution (cnnacc_scan_frames): [n][fh][fw][3] -> [n][fh][fw], four pixels per thread.
+// quads = n * fh * fw / 4 (fw is a multiple of 16); the output is 4-byte aligned, the frames may have any alignment.
+__global__ void __launch_bounds__(256)
+gray_full_kernel(const uint8_t* __restrict__ frames, uint8_t* __restrict__ gray, long long quads)
+{
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < quads; q += (long long)gridDim.x * blockDim.x) {
+        const uint8_t* p = frames + (size_t)q * 12;
+        const uint32_t v = (uint32_t)bgr2gray(p) | (uint32_t)bgr2gray(p + 3) << 8 | (uint32_t)bgr2gray(p + 6) << 16 |
+                           (uint32_t)bgr2gray(p + 9) << 24;
+        reinterpret_cast<uint32_t*>(gray)[q] = v;
+    }
+}
+
 __global__ void __launch_bounds__(kPrepOut)
 preprocess_bgr_kernel(const PrepParams P)
 {

@@ -5,7 +5,8 @@
 //   * conv_fused.cuh: four extra warps of the conv-stack kernel run it on the layer-2 staging buffer while the tensor
 //     core and the epilogue warps are already busy with the next image -- the features never leave the SM and, when the
 //     caller passes no feature pointer, HBM sees 44 B per image instead of 16 KiB out + 16 KiB back in;
-//   * classify_bbox_kernel below (features-in entry point, cnnacc_classify_batch): eight such groups per CTA.
+//   * classify_bbox_kernel below (features-in entry point, cnnacc_classify_batch and, on windows of a frame's map,
+//     cnnacc_scan_frames): eight such groups per CTA.
 // Both produce bit-identical predictions because they are the same code on the same bytes.
 //
 // Reference (all /root/reference/software/realtime_detect.py):
@@ -359,15 +360,62 @@ __device__ __forceinline__ void tail_back(float (&cam)[4], TailScratch* sc, cons
     trace(8);
 }
 
-// Features-in entry point (cnnacc_classify_batch): persistent CTAs of seven 128-thread groups; a group copies its image's
-// 16 KiB map into its own shared-memory slot (8 independent 128-bit loads per thread), runs tail_front on it, and its first two
-// warps then run tail_back while the other two already fetch the next image.
+// Features-in entry point: persistent CTAs of seven 128-thread groups; a group copies its item's 16 KiB map into its own
+// shared-memory slot (8 independent 128-bit loads per thread), runs tail_front on it, and its first two warps then run
+// tail_back while the other two already fetch the next item.  Where an item's map comes from is the one thing that varies:
+//   CompactMaps  cnnacc_classify_batch: item img is the 16 KiB map feats[img];
+//   ScanWindows  cnnacc_scan_frames: item img is a 16 x 16 window of a frame's [64][ho][wo] map, gathered in place.
+// Both hand the same slot layout to the same tail_front / tail_back, so a window's predictions are classify_batch's on the
+// window's map, bit for bit.  load(img, T, v): thread T's eight 16-byte rows, row T + 128 r = channel (T >> 4) + 8 r, map row
+// T & 15.
+struct CompactMaps {
+    const uint8_t* feats;
+    __device__ __forceinline__ void load(long long img, int T, uint4 (&v)[8]) const {
+        const uint4* src = reinterpret_cast<const uint4*>(feats + (size_t)img * 16384);
+#pragma unroll
+        for (int r = 0; r < 8; r++) v[r] = __ldcs(src + T + kTailThreads * r);       // read once: streaming
+    }
+};
+
+// The 16 bytes at byte offset sh (0..15) of the 32 bytes a:b.
+__device__ __forceinline__ uint4 bytes_at(const uint4 a, const uint4 b, int sh) {
+    uint32_t w0 = a.x, w1 = a.y, w2 = a.z, w3 = a.w, w4 = b.x, w5 = b.y, w6 = b.z, w7 = b.w;
+    if (sh & 8) { w0 = w2; w1 = w3; w2 = w4; w3 = w5; w4 = w6; w5 = w7; }
+    if (sh & 4) { w0 = w1; w1 = w2; w2 = w3; w3 = w4; w4 = w5; }
+    const uint32_t s = 8u * (sh & 3);
+    return make_uint4(__funnelshift_r(w0, w1, s), __funnelshift_r(w1, w2, s), __funnelshift_r(w2, w3, s), __funnelshift_r(w3, w4, s));
+}
+
+// Window (ix, iy) of frame f is the map's cells [v, v + 16) x [u, u + 16), u = min(ix step, umax), v = min(iy step, vmax):
+// the 128 x 128 pixels at (8u, 8v).  Windows are numbered frame-major, then row, then column, so the seven groups of a CTA
+// take horizontally adjacent windows, which share 15/16 of their bytes: L1 serves most of the gather.  A row of a window
+// starts at any byte (u may be odd): it is read as the two aligned 16-byte blocks around it and shifted into place.  With
+// ho and wo even, a channel plane is a multiple of 4 bytes, so the shift is the same for all eight rows of a thread.  The
+// second block of a row that starts aligned lies past the row: the workspace has 16 bytes of slack after the last map.
+struct ScanWindows {
+    const uint8_t* feats;                       // [k][64][ho][wo], 16-byte aligned
+    int ho, wo, nx, ny, step, umax, vmax;       // map size, windows per row / column, stride / 8, last origins in cells
+    __device__ __forceinline__ void load(long long img, int T, uint4 (&v)[8]) const {
+        const long long per = (long long)nx * ny, f = img / per;
+        const int rem = (int)(img - f * per), iy = rem / nx, ix = rem - iy * nx;
+        const size_t plane = (size_t)ho * wo;
+        const uint8_t* p = feats + (size_t)f * 64 * plane + (size_t)(min(iy * step, vmax) + (T & 15)) * wo +
+                           min(ix * step, umax) + (size_t)(T >> 4) * plane;
+        const int sh = (int)(reinterpret_cast<uintptr_t>(p) & 15);
+        const uint4* a = reinterpret_cast<const uint4*>(p - sh);
+        const size_t step8 = 8 * plane / 16;                // channel c -> c + 8, in 16-byte blocks
+#pragma unroll
+        for (int r = 0; r < 8; r++) v[r] = bytes_at(__ldg(a + r * step8), __ldg(a + r * step8 + 1), sh);
+    }
+};
+
 constexpr int kTailGroups = 7;                          // 7 x (one 128-thread + one 64-thread named barrier) = 14 of the 15 ids
 constexpr int kTailSmemW = kMaxClasses * 4096;          // every classifier row, shared by the groups
 constexpr int kTailSmem = kTailGroups * (16384 + kTailScratchBytes) + kTailSmemW;
 
+template <class Maps>
 __global__ void __launch_bounds__(kTailGroups * kTailThreads, 1)
-classify_bbox_kernel(const uint8_t* __restrict__ feats, long long n, const TailArgs A)
+classify_bbox_kernel(const Maps maps, long long n, const TailArgs A)
 {
     extern __shared__ __align__(16) uint8_t tail_smem[];
     const int g = threadIdx.x / kTailThreads, T = threadIdx.x % kTailThreads;
@@ -383,10 +431,8 @@ classify_bbox_kernel(const uint8_t* __restrict__ feats, long long n, const TailA
     W.bias = (T & 31) < A.n_cls ? __ldg(A.fc_b + (T & 31)) : 0.f;
     __syncthreads();
     for (long long img = (long long)blockIdx.x * kTailGroups + g; img < n; img += (long long)gridDim.x * kTailGroups) {
-        const uint4* src = reinterpret_cast<const uint4*>(feats + (size_t)img * 16384);
         uint4 v[8];
-#pragma unroll
-        for (int r = 0; r < 8; r++) v[r] = __ldcs(src + T + kTailThreads * r);       // read once: streaming
+        maps.load(img, T, v);
         // (the previous image's tail_front ended with a group barrier after its last read of stg, and its tail_back
         // threads have read sc->cam before they come back here: both buffers are free)
 #pragma unroll

@@ -270,6 +270,38 @@ int cnnacc_merge_regions_host(const int32_t *regions, int64_t n_regions, int64_t
                               const float *scores, const int32_t *cls, const int32_t *bbox, float score_min, float iou_max,
                               int max_det, int32_t *n_det, int32_t *det_region, int32_t *det_cls, float *det_score,
                               float *det_box, uint32_t flags);
+/* ---- scanning whole frames: every 128x128 window at a multiple-of-8 stride from one conv pass per frame -----------------
+ * frames [n][fh][fw][3] u8 BGR, fh and fw multiples of 16 in 128..8192 (so 1920x1080 frames are refused: 1080 is not a
+ * multiple of 16, exactly as cnnacc_run_batch refuses them), stride a positive multiple of 8.
+ * Windows: x = 0, stride, 2 stride, ... plus one window flush with the right edge (x = fw - 128) when that position is
+ * missing, so nx = (fw - 128) / stride + 1 + ((fw - 128) % stride != 0); the same for y and ny.  Window r of the call is
+ * (f, x, y) with r = (f * ny + iy) * nx + ix: frame-major, then y, then x -- the order of grid_regions(n, fh, fw, 128, stride)
+ * in the Python package.  Outputs are indexed by window in that order.
+ * What a window computes:
+ *   gray[f] = cvtColor(frames[f], COLOR_BGR2GRAY) at full resolution (OpenCV's 15-bit fixed point, as preprocess_bgr)
+ *   feat[f] = cnnacc_run_batch(gray[f]) at fh x fw: [64][fh/8][fw/8], with the handle's shifts and accumulator width
+ *   window (f, x, y) -> cls / probs (logits with CNNACC_FLAG_LOGITS) / bbox = cnnacc_classify_batch of the 64x16x16 map
+ *                       feat[f][:, y/8 : y/8+16, x/8 : x/8+16], bit for bit; the box is on the window's 128 grid
+ * This is NOT detect_regions on the same squares.  A region is pre-processed as an image of its own, so its conv stack pads
+ * with zeros at the region's border; a scan window sees the frame's real pixels beyond its border.  Their maps agree on the
+ * inner 14x14 cells, and on the outer ring only on the sides where the window's edge is the frame's edge; on a 128x128 frame
+ * the two are the same computation.  The gain: each pixel goes through the conv stack once per frame, not once per window.
+ * scan_frames : probs [R][n_cls] f32, cls [R] i32, bbox [R][4] i32 for R = n * nx * ny windows; any output may be NULL.
+ * scan_objects: scan_frames followed by the merge above, the windows being the regions (f, x, y, 128), score[r] =
+ *               probs[r][cls[r]] (the logit with CNNACC_FLAG_LOGITS); det_region indexes the window order.  The result is
+ *               exactly merge_regions on those regions and scan_frames' outputs.  Per-window predictions never leave the GPU.
+ * Host pointers: frames are staged in chunks of about 16 MiB (a larger frame alone).  Device pointers
+ * (CNNACC_FLAG_DEVICE_PTRS): asynchronous on the handle's stream, with detect_regions' alignment rules.  CNNACC_FLAG_LOGITS
+ * and, for scan_objects, CNNACC_FLAG_CLASS_AGNOSTIC are honoured.
+ *   -2, nothing launched: n < 0, fh or fw not a multiple of 16 or outside 128..8192, stride not a positive multiple of 8,
+ *       more than 2^31-1 windows in the call, CNNACC_FLAG_BBOX_UPSAMPLED / _RECTS / _DIRECT / _KEEP_MAPS / _TWO_KERNELS,
+ *       frames NULL with n > 0; for scan_objects also more than CNNACC_MERGE_MAX_PER_FRAME windows per frame and the
+ *       merge's own refusals.  -4 without weights or without a classifier.  n == 0 returns 0. */
+int cnnacc_scan_frames(cnnacc_handle *h, const uint8_t *frames, int64_t n, int fh, int fw, int stride,
+                       float *probs, int32_t *cls, int32_t *bbox, uint32_t flags);
+int cnnacc_scan_objects(cnnacc_handle *h, const uint8_t *frames, int64_t n, int fh, int fw, int stride,
+                        float score_min, float iou_max, int max_det, int32_t *n_det, int32_t *det_region,
+                        int32_t *det_cls, float *det_score, float *det_box, uint32_t flags);
 /* Host-only view of the staging plan of a host-pointer region call (csrc/region_plan.h): chunk i stages frames
  * [chunks[4i], chunks[4i+1]) with one copy and runs regions [chunks[4i+2], chunks[4i+3]) on them.  Returns the number of chunks
  * (<= cap), or -2 for a region array the real call refuses, or when cap is too small.  No GPU needed. */

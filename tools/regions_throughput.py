@@ -18,8 +18,14 @@ device-resident on
   aspect  (d) 157 rectangles per frame: 128x128, 256x128 and 128x256 at stride 64 (grid_rects)
   random  (e) 48 seeded random rectangles per frame, 128..640 wide and 128..480 tall
 beside grid (a) as squares in the same run, and batch-1 p50 / p99 of one VGA frame with aspect (d).
+--scan measures the scanning calls (one conv pass per frame, every 128x128 window at a stride): scan_frames at strides 64,
+32, 16 and 8 host-fed and device-resident, alternated with detect_regions on the same grid_regions windows at 64 and 32;
+scan_objects at 64 and 8 with score_min 0 and with the 97th percentile of the window scores; batch-1 p50 / p99 of one pageable
+frame through scan_frames and scan_objects; the device-time split of scan_frames at stride 8 into gray, conv and window tail
+(torch.profiler kernel times, in a pass of its own); how often scan and detect_regions agree on the class of the same window.
 
-    python tools/regions_throughput.py [--frames 2048] [--dev-frames 1024] [--seconds 2] [--objects | --rects] [--out FILE]
+    python tools/regions_throughput.py [--frames 2048] [--dev-frames 1024] [--seconds 2] [--objects | --rects | --scan]
+                                       [--out FILE]
 """
 import argparse
 import ctypes
@@ -89,6 +95,7 @@ def main():
     ap.add_argument("--out", default=None)
     ap.add_argument("--objects", action="store_true", help="measure the merging calls (detect_objects / merge_regions)")
     ap.add_argument("--rects", action="store_true", help="measure rectangle regions (detect_regions / detect_objects)")
+    ap.add_argument("--scan", action="store_true", help="measure the scanning calls (scan_frames / scan_objects)")
     a = ap.parse_args()
     import torch
     dev = torch.device("cuda", 0)
@@ -115,6 +122,9 @@ def main():
         return write(a, lines)
     if a.rects:
         rects(a, acc, host, emit)
+        return write(a, lines)
+    if a.scan:
+        scan(a, acc, host, emit)
         return write(a, lines)
 
     # host-fed
@@ -290,6 +300,98 @@ def rects(a, acc, host, emit):
             ts.append(time.perf_counter() - t0)
         ts = np.array(ts) * 1e6
         emit({"what": "batch1", "path": path, "p50_us": float(np.percentile(ts, 50)), "p99_us": float(np.percentile(ts, 99))})
+
+
+def batch1(emit, path, fn):
+    """p50 / p99 wall time of fn over 2000 calls after 50 warm-up calls."""
+    for _ in range(50):
+        fn()
+    ts = []
+    for _ in range(2000):
+        t0 = time.perf_counter()
+        fn()
+        ts.append(time.perf_counter() - t0)
+    ts = np.array(ts) * 1e6
+    emit({"what": "batch1", "path": path, "p50_us": float(np.percentile(ts, 50)), "p99_us": float(np.percentile(ts, 99))})
+
+
+def scan(a, acc, host, emit):
+    """scan_frames / scan_objects beside detect_regions on the same windows, host-fed and device-resident, each comparison
+    alternated twice in this run; batch 1; the stride-8 device-time split; class agreement with detect_regions."""
+    import torch
+    dev = torch.device("cuda", 0)
+    t = torch.from_numpy(host[:a.dev_frames]).to(dev)
+    nd = a.dev_frames
+    strides = (64, 32, 16, 8)
+    for where, frames, n, measure, unit in (("host_fed", host, a.frames, lambda fn: 1.0 / wall_rate(fn, a.seconds), "s"),
+                                            ("device_resident", t, nd, lambda fn: event_ms(fn, a.seconds) / 1e3, "s")):
+        secs = {}
+        for rep in range(2):
+            for stride in strides:
+                secs.setdefault(("scan_frames", stride), []).append(measure(lambda: acc.scan_frames(frames, stride)))
+                if stride in (64, 32):
+                    reg = fc.grid_regions(n, H, W, 128, stride)
+                    secs.setdefault(("detect_regions", stride), []).append(measure(lambda: acc.detect_regions(frames, reg)))
+        for (path, stride), v in secs.items():
+            windows = n * len(fc.grid_regions(1, H, W, 128, stride))
+            emit({"what": where, "path": path, "stride": stride, "windows_per_frame": windows // n, "s_runs": v,
+                  "frames_per_s": n / min(v), "windows_per_s": windows / min(v), "us_per_frame": min(v) / n * 1e6})
+        for stride in (64, 32):
+            emit({"what": where, "ratio": "scan_frames/detect_regions (frames/s)", "stride": stride,
+                  "value": min(secs[("detect_regions", stride)]) / min(secs[("scan_frames", stride)])})
+        if where == "device_resident":
+            ok = min(secs[("scan_frames", 64)]) <= min(secs[("detect_regions", 64)])
+            emit({"what": where, "gate": "scan_frames stride 64 not slower than detect_regions on the same 63 windows",
+                  "pass": bool(ok)})
+        # scan_objects at 64 and 8: every window a candidate, and only the top 3 % of window scores
+        secs = {}
+        for stride in (64, 8):
+            cls, probs, _ = acc.scan_frames(t[:64], stride)
+            sc = probs[torch.arange(len(cls), device=dev), cls.long()].cpu().numpy()
+            thr = float(np.percentile(sc, 97))
+            for rep in range(2):
+                for score_min in (0.0, thr):
+                    kw = dict(score_min=score_min, iou_max=0.5, max_det=100)
+                    secs.setdefault((stride, score_min), []).append(measure(lambda: acc.scan_objects(frames, stride, **kw)))
+                    secs.setdefault((stride, "scan_frames"), []).append(measure(lambda: acc.scan_frames(frames, stride)))
+        for (stride, what), v in secs.items():
+            emit({"what": where, "path": "scan_frames" if what == "scan_frames" else "scan_objects", "stride": stride,
+                  **({} if what == "scan_frames" else {"score_min": what, "candidates": "all" if what == 0.0 else "top 3 %"}),
+                  "s_runs": v, "frames_per_s": n / min(v), "us_per_frame": min(v) / n * 1e6})
+    # how often a scan window and the detect_regions region on the same square agree on the class (information only)
+    for stride in (64, 32):
+        reg = fc.grid_regions(64, H, W, 128, stride)
+        c_scan = acc.scan_frames(t[:64], stride)[0].cpu().numpy()
+        c_reg = acc.detect_regions(t[:64], reg)[0].cpu().numpy()
+        emit({"what": "agreement", "stride": stride, "windows": len(reg), "same_class": float((c_scan == c_reg).mean())})
+    # device-time split at stride 8 (kernel times from torch.profiler, a pass of its own)
+    from torch.profiler import ProfilerActivity, profile
+    acc.scan_frames(t, 8)
+    torch.cuda.synchronize()
+    reps = 5
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            acc.scan_frames(t, 8)
+        torch.cuda.synchronize()
+    split = {}
+    for e in prof.key_averages():
+        us = e.device_time_total if hasattr(e, "device_time_total") else e.cuda_time_total
+        if us <= 0:
+            continue
+        name = e.key
+        part = ("gray" if "gray_full_kernel" in name else "window_tail" if "ScanWindows" in name
+                else "conv" if "fused" in name else "other")
+        split[part] = split.get(part, 0.0) + us / reps / nd
+    emit({"what": "device_split", "path": "scan_frames", "stride": 8, "frames": nd, "us_per_frame": split,
+          "kernels": sorted({e.key for e in prof.key_averages()})})
+    del t
+    torch.cuda.synchronize()
+    one = np.ascontiguousarray(host[:1])
+    batch1(emit, "scan_frames_stride64", lambda: acc.scan_frames(one, 64))
+    batch1(emit, "scan_objects_stride64", lambda: acc.scan_objects(one, 64))
+    batch1(emit, "scan_frames_stride8", lambda: acc.scan_frames(one, 8))
+    batch1(emit, "scan_objects_stride8", lambda: acc.scan_objects(one, 8))
+    batch1(emit, "detect_regions_grid63", lambda: acc.detect_regions(one, fc.grid_regions(1, H, W, 128, 64)))
 
 
 if __name__ == "__main__":
