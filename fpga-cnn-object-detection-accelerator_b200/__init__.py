@@ -8,8 +8,8 @@ from . import _lib
 from ._lib import build, load
 from .accelerator import (ARMEngine, B200Engine, CNNAccelerator, Classifier, MultiAccelerator, NAMES, alloc_host, bbox_vec,
                           classify_vec, dump_features, grid_rects, grid_regions, load_arm_cnn_lib, load_features, load_image_any,
-                          region_boxes_to_frame, register_host, train_linear_classifier)
+                          pyramid_levels, pyramid_windows, region_boxes_to_frame, register_host, train_linear_classifier)
 
 __all__ = ["ARMEngine", "B200Engine", "CNNAccelerator", "Classifier", "MultiAccelerator", "dump_features", "load_features", "NAMES", "alloc_host", "register_host", "load_image_any", "train_linear_classifier", "bbox_vec", "classify_vec",
-           "grid_regions", "grid_rects", "region_boxes_to_frame",
+           "grid_regions", "grid_rects", "pyramid_levels", "pyramid_windows", "region_boxes_to_frame",
            "load_arm_cnn_lib", "build", "load", "_lib"]

@@ -14,6 +14,7 @@ FLAG_TWO_KERNELS = 0x40
 FLAG_CLASS_AGNOSTIC = 0x80
 FLAG_RECTS = 0x100
 MERGE_MAX_DET, MERGE_MAX_PER_FRAME = 1024, 16384
+PYRAMID_MAX_LEVELS = 16
 MAX_PENDING = 8
 
 # every symbol include/cnnacc.h declares: name -> (restype, argtypes)
@@ -67,6 +68,13 @@ SYMBOLS = {
                                       _c.c_void_p, _c.c_uint32]),
     "cnnacc_scan_objects": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_float, _c.c_float,
                                        _c.c_int] + [_c.c_void_p] * 5 + [_c.c_uint32]),
+    "cnnacc_preprocess_pyramid": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int, _c.c_void_p,
+                                             _c.c_uint32]),
+    "cnnacc_scan_pyramid": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int, _c.c_int,
+                                       _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_uint32]),
+    "cnnacc_scan_pyramid_objects": (_c.c_int, [_H, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int, _c.c_int,
+                                               _c.c_float, _c.c_float, _c.c_int] + [_c.c_void_p] * 5 + [_c.c_uint32]),
+    "cnnacc_pyramid_windows_host": (_c.c_int, [_c.c_int, _c.c_int, _c.c_void_p, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int64]),
     "cnnacc_region_plan_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int]),
     "cnnacc_rect_plan_host": (_c.c_int, [_c.c_void_p, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int]),
     "cnnacc_area_tab_host": (_c.c_int, [_c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_int]),

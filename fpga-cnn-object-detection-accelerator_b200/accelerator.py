@@ -647,6 +647,58 @@ class CNNAccelerator:
             return 0
         return len(_tile_origins(fh, 128, stride)) * len(_tile_origins(fw, 128, stride))
 
+    def preprocess_pyramid(self, frames, levels):
+        """The gray levels of an image pyramid: frames [F,h,w,3] u8 BGR (numpy, or a contiguous CUDA uint8 tensor run on
+        torch's current stream), h and w in 128..8192; levels a sequence of (w_l, h_l), multiples of 16 with 128 <= w_l <= w
+        and 128 <= h_l <= h, at most 16 (pyramid_levels gives the isotropic ones).  Level l of frame f is
+        cv2.resize(cv2.cvtColor(frame, COLOR_BGR2GRAY), (w_l, h_l), interpolation=INTER_AREA), byte for byte.
+        -> [F, sum of h_l * w_l] u8, frame-major, then level (reshape level l's slice to (h_l, w_l)); numpy or torch like frames."""
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
+        nf, fh, fw = self._scan_shape(frames, 8)
+        lv = _levels_array(levels)
+        gray = new((nf, int((lv[:, 0].astype(np.int64) * lv[:, 1]).sum())), np.uint8)
+        with ctx:
+            self._check(self._libc.cnnacc_preprocess_pyramid(self._h, ptr(frames), nf, fh, fw, _vp(lv), len(lv), ptr(gray), kind))
+        return gray
+
+    def scan_pyramid(self, frames, levels, stride=16, logits=False):
+        """Classify every 128x128 window of every level of an image pyramid, one conv pass per level: frames and levels as
+        preprocess_pyramid, stride a positive multiple of 8 in level pixels.  A level's windows are scan_frames' windows of
+        its gray (preprocess_pyramid); window r is numbered frame-major, then level in the given order, then y, then x, and
+        gets classify_batch's predictions for the 16x16 cells at (x/8, y/8) of run_batch(level gray), bit for bit, its box on
+        the window's 128 grid.  pyramid_windows(F, h, w, levels, stride) lists the windows' frame rectangles, which must all
+        be whole pixels (else ValueError); region_boxes_to_frame maps the boxes onto the frame.  A single level (w, h) is
+        scan_frames.  Not detect_regions on those rectangles: a window is resized with the whole frame and sees the frame
+        beyond its border.  -> (cls [R] i32, probs [R,n_cls] f32, bbox [R,4] i32), numpy or torch like frames."""
+        n_cls = self._classes()
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
+        nf, fh, fw = self._scan_shape(frames, stride)
+        lv = _levels_array(levels)
+        per = max(0, _lib.load().cnnacc_pyramid_windows_host(fh, fw, _vp(lv), len(lv), int(stride), None, 0))
+        cls, probs, box = _pred_outputs(new, nf * per, n_cls)
+        with ctx:
+            self._check(self._libc.cnnacc_scan_pyramid(self._h, ptr(frames), nf, fh, fw, _vp(lv), len(lv), int(stride), ptr(probs),
+                                                       ptr(cls), ptr(box), _pred_flags("vec", logits) | kind))
+        return cls, probs, box
+
+    def scan_pyramid_objects(self, frames, levels, stride=16, score_min=0.0, iou_max=0.5, max_det=100, class_agnostic=False,
+                             logits=False):
+        """scan_pyramid followed by detect_objects' per-frame greedy NMS on the GPU, the windows' frame rectangles
+        pyramid_windows(F, h, w, levels, stride) being the regions: exactly merge_regions(pyramid_windows(...), cls,
+        probs[r, cls[r]], bbox, F, ...) on scan_pyramid's outputs.  At most 16384 windows per frame.  -> as detect_objects,
+        with region indexing the window order; numpy or torch like frames."""
+        flags = _pred_flags("vec", logits) | _merge_flags(max_det, class_agnostic)
+        self._classes()
+        frames, new, ptr, kind, ctx = self._host_or_device(frames)
+        nf, fh, fw = self._scan_shape(frames, stride)
+        lv = _levels_array(levels)
+        dets = _det_outputs(new, nf, int(max_det))
+        with ctx:
+            self._check(self._libc.cnnacc_scan_pyramid_objects(self._h, ptr(frames), nf, fh, fw, _vp(lv), len(lv), int(stride),
+                                                               float(score_min), float(iou_max), int(max_det),
+                                                               *[ptr(a) for a in dets], flags | kind))
+        return dets
+
     def infer_one(self, gray128):
         """One image, lowest latency.  -> (feat (64,256) u8, conv_ms, read_ms)."""
         img = gray128 if (type(gray128) is np.ndarray and gray128.dtype == np.uint8 and gray128.flags.c_contiguous) \
@@ -717,6 +769,50 @@ def grid_rects(n_frames, fh, fw, sizes, strides):
     out[:, :, 0] = np.arange(int(n_frames), dtype=np.int32)[:, None]
     out[:, :, 1:] = tiles[None]
     return out.reshape(-1, 5)
+
+
+def _levels_array(levels):
+    """Pyramid levels as the library takes them: an (L, 2) C-contiguous int32 array of (w, h)."""
+    lv = np.asarray(levels)
+    if lv.ndim != 2 or lv.shape[1] != 2 or not (lv.size == 0 or np.issubdtype(lv.dtype, np.integer)):
+        raise ValueError("levels must be a sequence of (w, h) integer pairs")
+    if lv.size and (lv.min() < 0 or lv.max() > 8192):
+        raise ValueError("level sides must be in 0..8192 to be passed on (the library checks the rest)")
+    return np.ascontiguousarray(lv, dtype=np.int32)
+
+
+def pyramid_windows(n_frames, fh, fw, levels, stride):
+    """The windows of scan_pyramid on n_frames frames of fh x fw as frame rectangles (frame, x fw / w_l, y fh / h_l,
+    128 fw / w_l, 128 fh / h_l), in window order (frame, then level in the given order, then y, then x): the regions that
+    merge_regions and region_boxes_to_frame take for scan_pyramid's outputs.  ValueError where scan_pyramid refuses the
+    levels or stride.  -> (R, 5) int32."""
+    lib = _lib.load()
+    lv = _levels_array(levels)
+    per = lib.cnnacc_pyramid_windows_host(int(fh), int(fw), _vp(lv), len(lv), int(stride), None, 0)
+    if per < 0:
+        raise ValueError(f"levels {lv.tolist()} / stride {stride} do not make a pyramid scan of {fh}x{fw} frames")
+    one = np.empty((per, 5), dtype=np.int32)
+    lib.cnnacc_pyramid_windows_host(int(fh), int(fw), _vp(lv), len(lv), int(stride), _vp(one), per)
+    out = np.repeat(one[None], int(n_frames), axis=0)
+    out[:, :, 0] = np.arange(int(n_frames), dtype=np.int32)[:, None]
+    return out.reshape(-1, 5)
+
+
+def pyramid_levels(fh, fw, stride):
+    """The isotropic levels scan_pyramid takes for fh x fw frames at this stride, largest first: every (w, h) with
+    h = w fh / fw exactly, both multiples of 16, 128 <= w <= fw and 128 <= h <= fh, whose windows land on whole frame
+    pixels (pyramid_windows).  The frame itself comes first when its sides are multiples of 16.  -> [(w, h), ...]."""
+    lib = _lib.load()
+    out = []
+    for w in range(fw - fw % 16, 127, -16):
+        if (w * fh) % fw:
+            continue
+        h = w * fh // fw
+        if h % 16 or h < 128:
+            continue
+        if lib.cnnacc_pyramid_windows_host(int(fh), int(fw), _vp(np.array([[w, h]], np.int32)), 1, int(stride), None, 0) > 0:
+            out.append((w, h))
+    return out
 
 
 def region_boxes_to_frame(regions, bbox):

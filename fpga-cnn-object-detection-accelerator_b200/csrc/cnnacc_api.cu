@@ -22,6 +22,7 @@
 #include "cam_upsampled.cuh"
 #include "preprocess.cuh"
 #include "regions.cuh"
+#include "pyramid.cuh"
 #include "region_plan.h"
 #include "region_merge.cuh"
 #include "pil_resize.cuh"
@@ -108,7 +109,7 @@ struct cnnacc_handle {
     Stream st_h2d, st_k, st_d2h;                    // one stream per engine for host-pointer batches
     Event ev_t0, ev_t1, ev_a, ev_b, ev_done;
     int sm_count = 0;
-    bool weights_loaded = false, fc_loaded = false, tail_attr_set = false, scan_attr_set = false;
+    bool weights_loaded = false, fc_loaded = false, tail_attr_set = false, scan_attr_set = false, pyramid_attr_set = false;
     int shifts[3] = {2, 4, 6};                  // SHIFT_L0..2 defaults, pynq_inference.py:83-85
     bool acc24 = false;                         // accumulator width: false = int32 (arm_cnn.c:31), true = 24-bit wrap (accumulator.v:15)
     uint8_t wbin[CNNACC_WEIGHT_BYTES];
@@ -1658,7 +1659,8 @@ int cnnacc_merge_regions_host(const int32_t* regions, int64_t n_regions, int64_t
     return CNNACC_OK;
 }
 
-// ---- scanning whole frames (cnnacc_scan_frames / cnnacc_scan_objects) ---------------------------------------------------
+// ---- scanning whole frames and image pyramids (cnnacc_scan_frames / cnnacc_scan_objects, cnnacc_preprocess_pyramid /
+// cnnacc_scan_pyramid / cnnacc_scan_pyramid_objects) ---------------------------------------------------------------------
 
 // Scan windows along a side of `side` pixels: 0, stride, 2 stride, ... plus one flush with the far edge when that is missing.
 static int scan_count(int side, int stride) {
@@ -1666,22 +1668,110 @@ static int scan_count(int side, int stride) {
     return last / stride + 1 + (last % stride != 0);
 }
 
-// Gray, conv stack once per frame, then every window's predictions read straight out of the frame's feature map; with `mg`
-// (scan_objects) the predictions stay on the device and are merged per frame with the windows as (f, x, y, 128) regions.
-static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, int stride, float* probs, int32_t* cls,
-                     int32_t* bbox, uint32_t flags, MergeSpec* mg) {
+// The checked levels of a pyramid call (include/cnnacc.h); cnnacc_scan_frames is the one level (fw, fh).  Level l of a frame
+// holds its windows first[l] .. first[l + 1] - 1 and w[l] * h[l] gray pixels (and map bytes) at px[l] of the frame's total.
+static_assert(kPyramidMaxLevels == CNNACC_PYRAMID_MAX_LEVELS && kScanMaxLevels == CNNACC_PYRAMID_MAX_LEVELS, "level limits");
+
+struct PyramidPlan {
+    int fh = 0, fw = 0, n_levels = 0, stride = 0;
+    int w[kPyramidMaxLevels] = {}, h[kPyramidMaxLevels] = {}, nx[kPyramidMaxLevels] = {}, ny[kPyramidMaxLevels] = {};
+    int64_t first[kPyramidMaxLevels + 1] = {};
+    size_t px[kPyramidMaxLevels + 1] = {};
+    bool identity(int l) const { return w[l] == fw && h[l] == fh; }   // the gray frame itself: no resize, no copy
+    int box(int l) const { return area_fast_axis(fw, w[l]) && area_fast_axis(fh, h[l]); }   // OpenCV's integer path
+    int64_t per() const { return first[n_levels]; }                 // windows per frame
+    size_t level_px() const { return px[n_levels]; }
+    // the frame rectangle (x, y, w, h) of window (ix, iy) of level l
+    int4 rect(int l, int ix, int iy) const {
+        const int64_t x = std::min(ix * stride, w[l] - CNNACC_IMG), y = std::min(iy * stride, h[l] - CNNACC_IMG);
+        return make_int4((int)(x * fw / w[l]), (int)(y * fh / h[l]), CNNACC_IMG * fw / w[l], CNNACC_IMG * fh / h[l]);
+    }
+};
+
+// Do the windows of a level of side D land on whole pixels of the frame's side S: 128 S / D and o S / D an integer for every
+// window origin o (the actual origins, flush one included, not just the stride)?
+static bool whole_pixels(int S, int D, int stride) {
+    if ((int64_t)CNNACC_IMG * S % D) return false;
+    for (int ix = 0, n = scan_count(D, stride); ix < n; ix++)
+        if ((int64_t)std::min(ix * stride, D - CNNACC_IMG) * S % D) return false;
+    return true;
+}
+
+// nullptr with *P filled when frames of fh x fw, levels [L][2] (w, h) and stride (0: no windows, cnnacc_preprocess_pyramid)
+// make a pyramid call, else why not.
+static const char* pyramid_error(int fh, int fw, const int32_t* levels, int L, int stride, PyramidPlan* P) {
+    if (fh < kRegionMinSide || fh > kRegionMaxSide || fw < kRegionMinSide || fw > kRegionMaxSide) return "frame sides must be in 128..8192";
+    if (L < 1 || L > kPyramidMaxLevels) return "1..16 levels";
+    if (!levels) return "NULL levels";
+    if (stride && (stride < 8 || stride % 8)) return "stride must be a positive multiple of 8";
+    P->fh = fh; P->fw = fw; P->n_levels = L; P->stride = stride;
+    for (int l = 0; l < L; l++) {
+        const int w = levels[2 * l], hl = levels[2 * l + 1];
+        if (w % 16 || hl % 16 || w < CNNACC_IMG || hl < CNNACC_IMG || w > fw || hl > fh)
+            return "level sides must be multiples of 16 with 128 <= w <= fw and 128 <= h <= fh";
+        P->w[l] = w; P->h[l] = hl;
+        P->px[l + 1] = P->px[l] + (size_t)w * hl;
+        if (stride) {
+            if (!whole_pixels(fw, w, stride) || !whole_pixels(fh, hl, stride))
+                return "a window's frame rectangle (x fw / w, y fh / h, 128 fw / w, 128 fh / h) is not in whole pixels";
+            P->nx[l] = scan_count(w, stride); P->ny[l] = scan_count(hl, stride);
+        }
+        P->first[l + 1] = P->first[l] + (int64_t)P->nx[l] * P->ny[l];
+    }
+    return nullptr;
+}
+
+// gray_full_kernel over k frames of `plane` pixels
+static int launch_gray(cnnacc_handle* h, cudaStream_t st, const uint8_t* d_frames, int64_t k, size_t plane, uint8_t* d_gray) {
+    const long long pixels = (long long)(k * plane), quads = pixels / 4;
+    gray_full_kernel<<<(unsigned)std::max<long long>(1, std::min<long long>((quads + 255) / 256, 16LL * h->sm_count)), 256, 0, st>>>(
+        d_frames, d_gray, pixels);
+    h->launches++;
+    CU(h, cudaGetLastError());
+    return 0;
+}
+
+// pyramid_levels_kernel on k gray frames: R's levels, `rows` rows in all
+static int launch_levels(cnnacc_handle* h, cudaStream_t st, PyramidPrep R, int rows, int64_t k) {
+    const size_t plane = (size_t)R.fh * R.fw;
+    for (int64_t g0 = 0; g0 < k; g0 += 65535) {          // gridDim.y limit
+        PyramidPrep P = R;
+        P.gray += g0 * plane;
+        for (int l = 0; l < P.n_levels; l++) P.lv[l].off += g0 * P.lv[l].fstride;
+        pyramid_levels_kernel<<<dim3((unsigned)rows, (unsigned)std::min<int64_t>(65535, k - g0)), kPrepOut, 0, st>>>(P);
+        h->launches++;
+    }
+    CU(h, cudaGetLastError());
+    return 0;
+}
+
+static constexpr uint32_t kNoScanForm = CNNACC_FLAG_BBOX_UPSAMPLED | CNNACC_FLAG_RECTS | CNNACC_FLAG_DIRECT | CNNACC_FLAG_KEEP_MAPS |
+                                        CNNACC_FLAG_TWO_KERNELS;
+
+// Gray once per frame, the pyramid's levels, the conv stack once per level, then every window's predictions read straight
+// out of its level's feature map; with `mg` (the _objects calls) the predictions stay on the device and are merged per frame
+// with the windows' frame rectangles as the regions.  levels == nullptr: cnnacc_scan_frames (the one level fw x fh).
+static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, const int32_t* levels, int n_levels,
+                     int stride, float* probs, int32_t* cls, int32_t* bbox, uint32_t flags, MergeSpec* mg) {
     int rc;
     if (!h) return CNNACC_ERR_ARG;
     if ((rc = check_ready(h))) return rc;
     if (!h->fc_loaded) return fail(h, CNNACC_ERR_STATE, "classifier not loaded (call cnnacc_load_classifier)");
     if (n < 0) return fail(h, CNNACC_ERR_ARG, "negative n");
-    if (!valid_hw(fh, fw) || fh < CNNACC_IMG || fw < CNNACC_IMG)
-        return fail(h, CNNACC_ERR_ARG, "frame sides must be multiples of 16 in 128..8192");
-    if (stride < 8 || stride % 8) return fail(h, CNNACC_ERR_ARG, "stride must be a positive multiple of 8");
-    if (flags & (CNNACC_FLAG_BBOX_UPSAMPLED | CNNACC_FLAG_RECTS | CNNACC_FLAG_DIRECT | CNNACC_FLAG_KEEP_MAPS | CNNACC_FLAG_TWO_KERNELS))
+    PyramidPlan P;
+    if (!levels) {
+        if (!valid_hw(fh, fw) || fh < CNNACC_IMG || fw < CNNACC_IMG)
+            return fail(h, CNNACC_ERR_ARG, "frame sides must be multiples of 16 in 128..8192");
+        if (stride < 8 || stride % 8) return fail(h, CNNACC_ERR_ARG, "stride must be a positive multiple of 8");
+        const int32_t one[2] = {fw, fh};
+        pyramid_error(fh, fw, one, 1, stride, &P);        // passes: the identity level of a valid frame
+    } else {
+        if (stride < 1) return fail(h, CNNACC_ERR_ARG, "stride must be a positive multiple of 8");
+        if (const char* why = pyramid_error(fh, fw, levels, n_levels, stride, &P)) return fail(h, CNNACC_ERR_ARG, why);
+    }
+    if (flags & kNoScanForm)
         return fail(h, CNNACC_ERR_ARG, "BBOX_UPSAMPLED / RECTS / DIRECT / KEEP_MAPS / TWO_KERNELS have no scanning form");
-    const int nx = scan_count(fw, stride), ny = scan_count(fh, stride);
-    const int64_t per = (int64_t)nx * ny;
+    const int64_t per = P.per();
     if (n > 0x7fffffffLL / per) return fail(h, CNNACC_ERR_ARG, "more than 2^31-1 windows in one call");
     if (mg) {
         if (!mg->n_det) return fail(h, CNNACC_ERR_ARG, "NULL n_det");
@@ -1691,31 +1781,55 @@ static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh,
     if (n == 0) return CNNACC_OK;
     if (!frames) return fail(h, CNNACC_ERR_ARG, "NULL frame pointer");
     CU(h, cudaSetDevice(h->device));
-    const size_t frame_sz = (size_t)fh * fw * 3, plane = (size_t)fh * fw;   // a gray frame and its map are both fh * fw bytes
+    const int L = P.n_levels;
+    const size_t frame_sz = (size_t)fh * fw * 3, plane = (size_t)fh * fw;
+    size_t resized = 0;                                   // gray pixels per frame of the levels that are resized
+    for (int l = 0; l < L; l++) resized += P.identity(l) ? 0 : (size_t)P.w[l] * P.h[l];
     const int nc = h->n_cls;
-    ScanWindows win;
-    win.ho = fh / 8; win.wo = fw / 8; win.nx = nx; win.ny = ny; win.step = stride / 8;
-    win.umax = (fw - CNNACC_IMG) / 8; win.vmax = (fh - CNNACC_IMG) / 8;
-    // gray and feature workspaces for k frames (the window gather may read 16 bytes past the last map)
+    // Workspaces for k frames: d_scan_gray holds the gray frames, then (from a 256-byte boundary) each resized level as
+    // [k][h][w]; d_scan_feat holds each level's maps as [k][64][h/8][w/8].  w * h is a multiple of 256, so every level
+    // starts 16-byte aligned.  The window gather may read 16 bytes past the last map.
+    auto gray_base = [&](int64_t k) { return (k * plane + 255) / 256 * 256; };
     auto grow_ws = [&](int64_t k) -> int {
         int r;
-        if ((r = grow(h, h->d_scan_gray, (size_t)k * plane)) || (r = grow(h, h->d_scan_feat, (size_t)k * plane + 16))) return r;
+        if ((r = grow(h, h->d_scan_gray, gray_base(k) + k * resized)) || (r = grow(h, h->d_scan_feat, k * P.level_px() + 16))) return r;
         return 0;
     };
-    // gray -> conv stack -> window tail for k frames staged at d_frames; p / c / b: the predictions of their first window
+    // gray -> levels -> conv stack per level -> window tail for k frames staged at d_frames; p / c / b: the predictions of
+    // their first window
     auto kernels = [&](cudaStream_t st, const uint8_t* d_frames, int64_t k, float* p, int32_t* c, int32_t* b) -> int {
-        const long long quads = (long long)(k * plane / 4);
-        gray_full_kernel<<<(unsigned)std::min<long long>((quads + 255) / 256, 16LL * h->sm_count), 256, 0, st>>>(
-            d_frames, h->d_scan_gray.p, quads);
-        h->launches++;
-        CU(h, cudaGetLastError());
         int r;
-        if ((r = conv_stack_device(h, st, h->d_scan_gray.p, k, fh, fw, h->d_scan_feat.p, 0, nullptr, nullptr))) return r;
-        ScanWindows w = win;
-        w.feats = h->d_scan_feat.p;
-        return launch_tail_kernel(h, st, w, k * per, make_tail(h, p, c, b, false, flags), h->scan_attr_set);
+        if ((r = launch_gray(h, st, d_frames, k, plane, h->d_scan_gray.p))) return r;
+        PyramidPrep R;
+        R.gray = h->d_scan_gray.p; R.out = h->d_scan_gray.p; R.fh = fh; R.fw = fw; R.n_levels = 0;
+        const uint8_t* in[kPyramidMaxLevels];
+        size_t o = gray_base(k);
+        int rows = 0;
+        for (int l = 0; l < L; l++) {
+            if (P.identity(l)) { in[l] = h->d_scan_gray.p; continue; }
+            R.lv[R.n_levels++] = PyramidLevel{P.w[l], P.h[l], rows, P.box(l), o, (size_t)P.w[l] * P.h[l]};
+            in[l] = h->d_scan_gray.p + o;
+            rows += P.h[l];
+            o += k * P.w[l] * P.h[l];
+        }
+        if (R.n_levels && (r = launch_levels(h, st, R, rows, k))) return r;
+        ScanLevel lv[kScanMaxLevels];
+        for (int l = 0; l < L; l++) {
+            uint8_t* maps = h->d_scan_feat.p + k * P.px[l];
+            if ((r = conv_stack_device(h, st, in[l], k, P.h[l], P.w[l], maps, 0, nullptr, nullptr))) return r;
+            lv[l] = ScanLevel{maps, P.h[l] / 8, P.w[l] / 8, P.nx[l], (P.w[l] - CNNACC_IMG) / 8, (P.h[l] - CNNACC_IMG) / 8,
+                              (int)P.first[l]};
+        }
+        const TailArgs A = make_tail(h, p, c, b, false, flags);
+        if (L == 1) {
+            ScanWindows<true> win{(int)per, stride / 8, 1, {lv[0]}};
+            return launch_tail_kernel(h, st, win, k * per, A, h->scan_attr_set);
+        }
+        ScanWindows<false> win{(int)per, stride / 8, L, {}};
+        std::copy(lv, lv + L, win.lv);
+        return launch_tail_kernel(h, st, win, k * per, A, h->pyramid_attr_set);
     };
-    // the merge's region descriptors (f, x, y, 128) and per-frame ranges, uploaded on st
+    // the merge's region descriptors (f, x, y, w | h << 16) -- the windows' frame rectangles -- and per-frame ranges, uploaded on st
     DescBuf* db = nullptr;
     auto upload_desc = [&](cudaStream_t st) -> int {
         int r;
@@ -1724,9 +1838,12 @@ static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh,
         for (int64_t f = 0; f <= n; f++) mg->first[f] = f * per;
         int4* d = db->host.p;
         for (int64_t f = 0; f < n; f++)
-            for (int iy = 0; iy < ny; iy++)
-                for (int ix = 0; ix < nx; ix++)
-                    *d++ = make_int4((int)f, std::min(ix * stride, fw - CNNACC_IMG), std::min(iy * stride, fh - CNNACC_IMG), CNNACC_IMG);
+            for (int l = 0; l < L; l++)
+                for (int iy = 0; iy < P.ny[l]; iy++)
+                    for (int ix = 0; ix < P.nx[l]; ix++) {
+                        const int4 q = P.rect(l, ix, iy);
+                        *d++ = make_int4((int)f, q.x, q.y, q.z | q.w << 16);
+                    }
         std::memcpy(db->first_host.p, mg->first.data(), (size_t)(n + 1) * sizeof(long long));
         CU(h, cudaMemcpyAsync(db->dev.p, db->host.p, (size_t)(n * per) * sizeof(int4), cudaMemcpyHostToDevice, st));
         CU(h, cudaMemcpyAsync(db->first_dev.p, db->first_host.p, (size_t)(n + 1) * sizeof(long long), cudaMemcpyHostToDevice, st));
@@ -1745,7 +1862,8 @@ static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh,
             REQUIRE_ALIGNED(h, mg->det_score, 4, "det_score");
         }
         // pieces of whole frames: gray and feature workspaces of at most 256 MiB each, at most kPredSuper windows
-        const int64_t chunk = std::min<int64_t>(n, std::max<int64_t>(1, std::min<int64_t>(((size_t)256 << 20) / plane, kPredSuper / per)));
+        const size_t ws_frame = std::max(plane + resized, P.level_px());
+        const int64_t chunk = std::min<int64_t>(n, std::max<int64_t>(1, std::min<int64_t>(((size_t)256 << 20) / ws_frame, kPredSuper / per)));
         if ((rc = grow_ws(chunk))) return rc;
         const size_t cw = (size_t)(chunk * per), w_probs = cw * 16, w_cls = w_probs + cw * nc * 4;   // PredBlock's layout
         if (mg && ((rc = grow(h, h->d_mpred, cw * kPredBytesPerImage)) || (rc = upload_desc(h->stream)))) return rc;
@@ -1780,11 +1898,13 @@ static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh,
         return rc;
     }
 
-    // Host pointers: prediction blocks of whole frames (a frame has fewer than kPredSuper windows), staged in chunks of about
-    // 16 MiB of frames (a larger frame alone) through the ring.
+    // Host pointers: prediction blocks of whole frames, staged in chunks of about 16 MiB of frames (a larger frame alone)
+    // through the ring.  A block holds up to kPredSuper windows, or one frame when a frame has more (a pyramid of an 8192 x
+    // 8192 frame at stride 8 has 1.34 M): a block never ends inside a frame, since every frame's kernels write its block.
     HostCall call(h);
     if ((rc = call.begin())) return rc;
-    const std::vector<int64_t> blocks = frame_aligned_blocks([per](int64_t r) { return r / per; }, n * per, kPredSuper);
+    const std::vector<int64_t> blocks =
+        frame_aligned_blocks([per](int64_t r) { return r / per; }, n * per, std::max<int64_t>(kPredSuper, per));
     const int64_t fpc = std::min<int64_t>(n, std::max<int64_t>(1, (int64_t)(kRegionChunkBytes / frame_sz)));
     const bool small = blocks.size() == 2 && n <= fpc;    // latency path: one chunk, one stream, one result copy
     cudaStream_t st = small ? h->st_k : h->st_h2d;
@@ -1823,7 +1943,7 @@ static int scan_impl(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh,
 
 int cnnacc_scan_frames(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, int stride, float* probs, int32_t* cls,
                        int32_t* bbox, uint32_t flags) {
-    return scan_impl(h, frames, n, fh, fw, stride, probs, cls, bbox, flags, nullptr);
+    return scan_impl(h, frames, n, fh, fw, nullptr, 1, stride, probs, cls, bbox, flags, nullptr);
 }
 
 int cnnacc_scan_objects(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, int stride, float score_min, float iou_max,
@@ -1831,7 +1951,91 @@ int cnnacc_scan_objects(cnnacc_handle* h, const uint8_t* frames, int64_t n, int 
                         uint32_t flags) {
     if (!h) return CNNACC_ERR_ARG;
     MergeSpec M = make_merge_spec(score_min, iou_max, max_det, n_det, det_region, det_cls, det_score, det_box, flags);
-    return scan_impl(h, frames, n, fh, fw, stride, nullptr, nullptr, nullptr, flags, &M);
+    return scan_impl(h, frames, n, fh, fw, nullptr, 1, stride, nullptr, nullptr, nullptr, flags, &M);
+}
+
+int cnnacc_scan_pyramid(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, const int32_t* levels, int n_levels,
+                        int stride, float* probs, int32_t* cls, int32_t* bbox, uint32_t flags) {
+    if (!h) return CNNACC_ERR_ARG;
+    if (!levels) return fail(h, CNNACC_ERR_ARG, "NULL levels");
+    return scan_impl(h, frames, n, fh, fw, levels, n_levels, stride, probs, cls, bbox, flags, nullptr);
+}
+
+int cnnacc_scan_pyramid_objects(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, const int32_t* levels,
+                                int n_levels, int stride, float score_min, float iou_max, int max_det, int32_t* n_det,
+                                int32_t* det_region, int32_t* det_cls, float* det_score, float* det_box, uint32_t flags) {
+    if (!h) return CNNACC_ERR_ARG;
+    if (!levels) return fail(h, CNNACC_ERR_ARG, "NULL levels");
+    MergeSpec M = make_merge_spec(score_min, iou_max, max_det, n_det, det_region, det_cls, det_score, det_box, flags);
+    return scan_impl(h, frames, n, fh, fw, levels, n_levels, stride, nullptr, nullptr, nullptr, flags, &M);
+}
+
+// The pyramid's gray levels alone, [n][sum of h * w] frame-major, then level: gray once per frame, then every level (an
+// identity level is copied) in one launch per piece.
+int cnnacc_preprocess_pyramid(cnnacc_handle* h, const uint8_t* frames, int64_t n, int fh, int fw, const int32_t* levels,
+                              int n_levels, uint8_t* gray, uint32_t flags) {
+    int rc;
+    if (!h) return CNNACC_ERR_ARG;
+    if (n < 0) return fail(h, CNNACC_ERR_ARG, "negative n");
+    PyramidPlan P;
+    if (const char* why = pyramid_error(fh, fw, levels, n_levels, 0, &P)) return fail(h, CNNACC_ERR_ARG, why);
+    if (flags & kNoScanForm)
+        return fail(h, CNNACC_ERR_ARG, "BBOX_UPSAMPLED / RECTS / DIRECT / KEEP_MAPS / TWO_KERNELS have no pyramid form");
+    if (n == 0) return CNNACC_OK;
+    if (!frames || !gray) return fail(h, CNNACC_ERR_ARG, "NULL frame / output pointer");
+    CU(h, cudaSetDevice(h->device));
+    const size_t frame_sz = (size_t)fh * fw * 3, plane = (size_t)fh * fw, out_sz = P.level_px();
+    PyramidPrep R;
+    R.fh = fh; R.fw = fw; R.n_levels = P.n_levels;
+    int rows = 0;
+    for (int l = 0; l < P.n_levels; l++) {
+        R.lv[l] = PyramidLevel{P.w[l], P.h[l], rows, P.box(l), P.px[l], out_sz};
+        rows += P.h[l];
+    }
+    // gray of k frames at d_frames, then their levels into out
+    auto kernels = [&](cudaStream_t st, const uint8_t* d_frames, int64_t k, uint8_t* out) -> int {
+        int r;
+        if ((r = launch_gray(h, st, d_frames, k, plane, h->d_scan_gray.p))) return r;
+        R.gray = h->d_scan_gray.p; R.out = out;
+        return launch_levels(h, st, R, rows, k);
+    };
+    if (flags & CNNACC_FLAG_DEVICE_PTRS) {
+        const int64_t chunk = std::min<int64_t>(n, std::max<int64_t>(1, ((size_t)256 << 20) / plane));   // gray workspace <= 256 MiB
+        if ((rc = grow(h, h->d_scan_gray, chunk * plane))) return rc;
+        for (int64_t f0 = 0; f0 < n; f0 += chunk)
+            if ((rc = kernels(h->stream, frames + f0 * frame_sz, std::min(chunk, n - f0), gray + f0 * out_sz))) return rc;
+        return CNNACC_OK;
+    }
+    // Host pointers: chunks of about 16 MiB of frames (a larger frame alone) through the ring, levels copied out per chunk
+    HostCall call(h);
+    if ((rc = call.begin())) return rc;
+    const int64_t fpc = std::min<int64_t>(n, std::max<int64_t>(1, (int64_t)(kRegionChunkBytes / frame_sz)));
+    if ((rc = grow(h, h->d_scan_gray, fpc * plane))) return rc;
+    Slot* s;
+    for (int64_t f0 = 0; f0 < n; f0 += fpc) {
+        const int64_t k = std::min(fpc, n - f0);
+        if ((rc = call.acquire(s, fpc * frame_sz, fpc * out_sz))) return rc;
+        CU(h, cudaMemcpyAsync(s->d_in.p, frames + f0 * frame_sz, k * frame_sz, cudaMemcpyHostToDevice, h->st_h2d));
+        if ((rc = call.staged(*s)) || (rc = kernels(h->st_k, s->d_in.p, k, s->d_out.p)) || (rc = call.computed(*s))) return rc;
+        CU(h, cudaMemcpyAsync(gray + f0 * out_sz, s->d_out.p, k * out_sz, cudaMemcpyDeviceToHost, h->st_d2h));
+        if ((rc = call.released(*s, h->st_d2h))) return rc;
+    }
+    return call.finish(h->st_d2h, false);
+}
+
+int cnnacc_pyramid_windows_host(int fh, int fw, const int32_t* levels, int n_levels, int stride, int32_t* rects, int64_t cap) {
+    PyramidPlan P;
+    if (stride < 1 || pyramid_error(fh, fw, levels, n_levels, stride, &P)) return CNNACC_ERR_ARG;
+    if (rects) {
+        if (cap < P.per()) return CNNACC_ERR_ARG;
+        for (int l = 0; l < P.n_levels; l++)
+            for (int iy = 0; iy < P.ny[l]; iy++)
+                for (int ix = 0; ix < P.nx[l]; ix++) {
+                    const int4 q = P.rect(l, ix, iy);
+                    *rects++ = 0; *rects++ = q.x; *rects++ = q.y; *rects++ = q.z; *rects++ = q.w;
+                }
+    }
+    return (int)P.per();
 }
 
 static int region_plan_host(const RegionRecords& rg, int64_t n_regions, int64_t n_frames, int fh, int fw, int64_t* chunks, int cap) {
@@ -1859,7 +2063,7 @@ int cnnacc_area_tab_host(int side, int* start, int* cnt, float* alpha, int taps_
     if (side < kRegionMinSide || side > kRegionMaxSide || !start || !cnt || !alpha || taps_cap < 1) return CNNACC_ERR_ARG;
     int taps = 0;
     for (int d = 0; d < kPrepOut; d++) {
-        const AreaTaps a = area_taps(side, d, side % kPrepOut == 0);
+        const AreaTaps a = area_taps(side, kPrepOut, d, side % kPrepOut == 0);
         if (a.n > taps_cap) return CNNACC_ERR_ARG;
         taps = std::max(taps, a.n);
         start[d] = a.first; cnt[d] = a.n;

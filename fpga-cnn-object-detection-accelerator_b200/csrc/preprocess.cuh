@@ -35,30 +35,47 @@ struct AreaTabHost {
     std::vector<float> alpha;                  // [128][taps]
 };
 
-// The INTER_AREA taps of output index d for a side S (128..8192) of the source: OpenCV's computeResizeAreaTab(ssize = S,
-// dsize = 128, scale = S/128.) for one d, in its order (double arithmetic, then float).  The taps are the consecutive source
-// indices first .. first+n-1; tap i weighs area_tap_weight(t, i).  `box`: the source takes OpenCV's integer path
-// (ResizeAreaFast), which OpenCV decides from both sides (both multiples of 128); then S = 128 k gives k taps of weight 1
-// (the kernels sum integers instead).  Without it an integer S still takes the table: k taps of (float)(1.0 / k).  Host (make_area_tab, cnnacc_area_tab_host) and device (regions.cuh) get the same bits: scale = S/128
-// is exact, so are d * scale, fsx1 + scale and S - fsx1 for S <= 8192 (at most 20 significant bits) -- an FMA the compiler
-// forms from them rounds nothing -- ceil / floor / min are exact, and the three divisions are correctly rounded in IEEE double
-// on both sides.  Up to 65 taps per output at S = 8191: the weights stay three scalars (first partial, 1/cell, last partial)
-// instead of a table in registers.
+// The INTER_AREA taps of output index d for a side S of the source resized to D (128 <= D <= S <= 8192): OpenCV's
+// computeResizeAreaTab(ssize = S, dsize = D, scale = S/D) for one d, in its order (double arithmetic, then float).  The taps
+// are the consecutive source indices first .. first+n-1; tap i weighs area_tap_weight(t, i).  `box`: the source takes
+// OpenCV's integer path (ResizeAreaFast), which OpenCV decides from both sides (both integer multiples); then S = D k gives k
+// taps of weight 1 (the kernels sum integers instead).  Without it an integer S still takes the table: k taps of
+// (float)(1.0 / k).  Host (make_area_tab, cnnacc_area_tab_host, cnnacc_pyramid_windows_host's checks) and device
+// (regions.cuh, pyramid.cuh) get the same bits: d * scale and fsx1 + scale are each rounded once (area_mul / area_add: the
+// device code may not contract them into an FMA, which would round d * scale + scale once -- for D = 128 every one of these
+// is exact, for other D it is not), ceil / floor / min are exact, and the subtractions and three divisions are correctly
+// rounded in IEEE double on both sides.  Up to 65 taps per output at S = 8191, D = 128: the weights stay three scalars
+// (first partial, 1/cell, last partial) instead of a table in registers.
 struct AreaTaps {
     int first, n;
     bool head, tail;                 // tap 0 / tap n-1 is a partial cell
     float a_head, a_mid, a_tail;
 };
 
-__host__ __device__ __forceinline__ AreaTaps area_taps(int S, int d, bool box) {
+__host__ __device__ __forceinline__ double area_mul(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+__host__ __device__ __forceinline__ double area_add(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+
+__host__ __device__ __forceinline__ AreaTaps area_taps(int S, int D, int d, bool box) {
     AreaTaps t;
     if (box) {
-        const int k = S / kPrepOut;
+        const int k = S / D;
         t.first = d * k; t.n = k; t.head = t.tail = false; t.a_head = t.a_mid = t.a_tail = 1.f;
         return t;
     }
-    const double scale = (double)S / kPrepOut;
-    const double fsx1 = d * scale, fsx2 = fsx1 + scale;
+    const double scale = (double)S / D;
+    const double fsx1 = area_mul(d, scale), fsx2 = area_add(fsx1, scale);
     const double cell = scale < S - fsx1 ? scale : S - fsx1;
     int sx1 = (int)ceil(fsx1), sx2 = (int)floor(fsx2);
     sx2 = sx2 < S - 1 ? sx2 : S - 1;
@@ -92,7 +109,7 @@ inline AreaTabHost make_area_tab(int S) {
     }
     t.alpha.assign((size_t)kPrepOut * t.taps, 1.f);
     for (int d = 0; d < kPrepOut; d++) {
-        const AreaTaps a = area_taps(S, d, S % kPrepOut == 0);
+        const AreaTaps a = area_taps(S, kPrepOut, d, S % kPrepOut == 0);
         t.start[d] = a.first; t.cnt[d] = a.n;
         if (t.mode == kPrepFrac)
             for (int i = 0; i < t.taps; i++) t.alpha[(size_t)d * t.taps + i] = i < a.n ? area_tap_weight(a, i) : 0.f;
@@ -115,16 +132,22 @@ __device__ __forceinline__ int bgr2gray(const uint8_t* p) {
     return (3735 * (int)__ldg(p) + 19235 * (int)__ldg(p + 1) + 9798 * (int)__ldg(p + 2) + (1 << 14)) >> 15;
 }
 
-// cvtColor(COLOR_BGR2GRAY) at full resolution (cnnacc_scan_frames): [n][fh][fw][3] -> [n][fh][fw], four pixels per thread.
-// quads = n * fh * fw / 4 (fw is a multiple of 16); the output is 4-byte aligned, the frames may have any alignment.
+// cvtColor(COLOR_BGR2GRAY) at full resolution (cnnacc_scan_frames, the pyramid calls): [n][fh][fw][3] -> [n][fh][fw] as
+// one contiguous plane of `pixels` = n * fh * fw, four pixels per thread and the last pixels % 4 by the first threads of
+// block 0.  The output is 4-byte aligned, the frames may have any alignment.
 __global__ void __launch_bounds__(256)
-gray_full_kernel(const uint8_t* __restrict__ frames, uint8_t* __restrict__ gray, long long quads)
+gray_full_kernel(const uint8_t* __restrict__ frames, uint8_t* __restrict__ gray, long long pixels)
 {
+    const long long quads = pixels >> 2;
     for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < quads; q += (long long)gridDim.x * blockDim.x) {
         const uint8_t* p = frames + (size_t)q * 12;
         const uint32_t v = (uint32_t)bgr2gray(p) | (uint32_t)bgr2gray(p + 3) << 8 | (uint32_t)bgr2gray(p + 6) << 16 |
                            (uint32_t)bgr2gray(p + 9) << 24;
         reinterpret_cast<uint32_t*>(gray)[q] = v;
+    }
+    if (blockIdx.x == 0 && threadIdx.x < (pixels & 3)) {
+        const long long i = quads * 4 + threadIdx.x;
+        gray[i] = (uint8_t)bgr2gray(frames + (size_t)i * 3);
     }
 }
 

@@ -33,7 +33,7 @@ preprocess_regions_kernel(const RegionPrep P)
     const int4 d = __ldg(P.desc + r);
     const int frame = d.x, x0 = d.y, y0 = d.z, W = desc_w(d.w), H = desc_h(d.w);
     const bool box = W % kPrepOut == 0 && H % kPrepOut == 0;
-    const AreaTaps tx = area_taps(W, dx, box), ty = area_taps(H, dy, box);
+    const AreaTaps tx = area_taps(W, kPrepOut, dx, box), ty = area_taps(H, kPrepOut, dy, box);
     const uint8_t* src = P.frames + (size_t)frame * P.fh * P.fw * 3 + ((size_t)(y0 + ty.first) * P.fw + (x0 + tx.first)) * 3;
     const size_t pitch = (size_t)P.fw * 3;
     int v;

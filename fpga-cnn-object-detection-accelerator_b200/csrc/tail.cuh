@@ -364,7 +364,8 @@ __device__ __forceinline__ void tail_back(float (&cam)[4], TailScratch* sc, cons
 // shared-memory slot (8 independent 128-bit loads per thread), runs tail_front on it, and its first two warps then run
 // tail_back while the other two already fetch the next item.  Where an item's map comes from is the one thing that varies:
 //   CompactMaps  cnnacc_classify_batch: item img is the 16 KiB map feats[img];
-//   ScanWindows  cnnacc_scan_frames: item img is a 16 x 16 window of a frame's [64][ho][wo] map, gathered in place.
+//   ScanWindows  cnnacc_scan_frames / cnnacc_scan_pyramid: item img is a 16 x 16 window of a frame's [64][ho][wo] map
+//                (of one of its pyramid levels), gathered in place.
 // Both hand the same slot layout to the same tail_front / tail_back, so a window's predictions are classify_batch's on the
 // window's map, bit for bit.  load(img, T, v): thread T's eight 16-byte rows, row T + 128 r = channel (T >> 4) + 8 r, map row
 // T & 15.
@@ -386,21 +387,40 @@ __device__ __forceinline__ uint4 bytes_at(const uint4 a, const uint4 b, int sh) 
     return make_uint4(__funnelshift_r(w0, w1, s), __funnelshift_r(w1, w2, s), __funnelshift_r(w2, w3, s), __funnelshift_r(w3, w4, s));
 }
 
-// Window (ix, iy) of frame f is the map's cells [v, v + 16) x [u, u + 16), u = min(ix step, umax), v = min(iy step, vmax):
-// the 128 x 128 pixels at (8u, 8v).  Windows are numbered frame-major, then row, then column, so the seven groups of a CTA
-// take horizontally adjacent windows, which share 15/16 of their bytes: L1 serves most of the gather.  A row of a window
-// starts at any byte (u may be odd): it is read as the two aligned 16-byte blocks around it and shifted into place.  With
-// ho and wo even, a channel plane is a multiple of 4 bytes, so the shift is the same for all eight rows of a thread.  The
-// second block of a row that starts aligned lies past the row: the workspace has 16 bytes of slack after the last map.
-struct ScanWindows {
+// Window (ix, iy) of a level of frame f is the level map's cells [v, v + 16) x [u, u + 16), u = min(ix step, umax),
+// v = min(iy step, vmax): the 128 x 128 level pixels at (8u, 8v).  Windows are numbered frame-major, then level, then row,
+// then column, so the seven groups of a CTA take horizontally adjacent windows, which share 15/16 of their bytes: L1 serves
+// most of the gather.  A row of a window starts at any byte (u may be odd): it is read as the two aligned 16-byte blocks
+// around it and shifted into place.  With ho and wo even, a channel plane is a multiple of 4 bytes, so the shift is the same
+// for all eight rows of a thread.  The second block of a row that starts aligned lies past the row: the workspace has 16
+// bytes of slack after the last map.  cnnacc_scan_frames is the one-level case (the frame's own map).
+constexpr int kScanMaxLevels = 16;
+struct ScanLevel {
     const uint8_t* feats;                       // [k][64][ho][wo], 16-byte aligned
-    int ho, wo, nx, ny, step, umax, vmax;       // map size, windows per row / column, stride / 8, last origins in cells
+    int ho, wo, nx, umax, vmax, first;          // map size, windows per row, last origins in cells, first window in a frame
+};
+// kOneLevel: the instance of one-level calls (cnnacc_scan_frames), which looks up no level; the other walks the table.
+template <bool kOneLevel>
+struct ScanWindows {
+    int per, step, n_levels;                    // windows per frame, stride / 8, levels
+    ScanLevel lv[kOneLevel ? 1 : kScanMaxLevels];
     __device__ __forceinline__ void load(long long img, int T, uint4 (&v)[8]) const {
-        const long long per = (long long)nx * ny, f = img / per;
-        const int rem = (int)(img - f * per), iy = rem / nx, ix = rem - iy * nx;
-        const size_t plane = (size_t)ho * wo;
-        const uint8_t* p = feats + (size_t)f * 64 * plane + (size_t)(min(iy * step, vmax) + (T & 15)) * wo +
-                           min(ix * step, umax) + (size_t)(T >> 4) * plane;
+        const long long f = img / per;
+        const int rem = (int)(img - f * per);
+        if constexpr (kOneLevel) {
+            gather(lv[0], f, rem, T, v);
+        } else {
+            int l = 0;
+            while (l + 1 < n_levels && rem >= lv[l + 1].first) l++;
+            gather(lv[l], f, rem - lv[l].first, T, v);
+        }
+    }
+    // window rem of level L of frame f
+    __device__ __forceinline__ void gather(const ScanLevel& L, long long f, int rem, int T, uint4 (&v)[8]) const {
+        const int iy = rem / L.nx, ix = rem - iy * L.nx;
+        const size_t plane = (size_t)L.ho * L.wo;
+        const uint8_t* p = L.feats + (size_t)f * 64 * plane + (size_t)(min(iy * step, L.vmax) + (T & 15)) * L.wo +
+                           min(ix * step, L.umax) + (size_t)(T >> 4) * plane;
         const int sh = (int)(reinterpret_cast<uintptr_t>(p) & 15);
         const uint4* a = reinterpret_cast<const uint4*>(p - sh);
         const size_t step8 = 8 * plane / 16;                // channel c -> c + 8, in 16-byte blocks
@@ -415,7 +435,7 @@ constexpr int kTailSmem = kTailGroups * (16384 + kTailScratchBytes) + kTailSmemW
 
 template <class Maps>
 __global__ void __launch_bounds__(kTailGroups * kTailThreads, 1)
-classify_bbox_kernel(const Maps maps, long long n, const TailArgs A)
+classify_bbox_kernel(const __grid_constant__ Maps maps, long long n, const TailArgs A)
 {
     extern __shared__ __align__(16) uint8_t tail_smem[];
     const int g = threadIdx.x / kTailThreads, T = threadIdx.x % kTailThreads;

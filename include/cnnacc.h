@@ -229,6 +229,9 @@ int cnnacc_detect_regions(cnnacc_handle *h, const uint8_t *frames, int64_t n_fra
  *   otherwise (an axis is fractional)      ResizeArea's float accumulation, x taps from computeResizeAreaTab(w) and y taps
  *                                          from computeResizeAreaTab(h); an integer axis takes that table too (kx taps of
  *                                          (float)(1.0/kx) each)
+ * One exception: a side of exactly 6272 = 49 x 128 pixels counts as an integer axis here, while OpenCV (whose test is
+ * 1 / (128 / side) within DBL_EPSILON of an integer, and 1.0 / (1.0 / 49) != 49 in double) takes the table for it; single
+ * outputs can then differ from cv2.resize by 1.  The pyramid calls below follow OpenCV's test.
  * cls / probs / bbox are what infer_batch gives for that gray128; boxes stay on the rectangle's 128 grid.  The merge maps
  * them with X = 128 x + clamp(bx) w and Y = 128 y + clamp(by) h.
  *   -2, nothing launched: as for squares with w and h in place of side -- w or h outside 128..8192, x < 0, y < 0,
@@ -302,6 +305,48 @@ int cnnacc_scan_frames(cnnacc_handle *h, const uint8_t *frames, int64_t n, int f
 int cnnacc_scan_objects(cnnacc_handle *h, const uint8_t *frames, int64_t n, int fh, int fw, int stride,
                         float score_min, float iou_max, int max_det, int32_t *n_det, int32_t *det_region,
                         int32_t *det_cls, float *det_score, float *det_box, uint32_t flags);
+/* ---- scanning image pyramids: the windows of several downscaled levels of each frame, one conv pass per level ------------
+ * frames [n][fh][fw][3] u8 BGR, fh and fw any integers in 128..8192.  levels [L][2] int32 (w, h) in host memory,
+ * 1 <= L <= CNNACC_PYRAMID_MAX_LEVELS: each level has w and h multiples of 16 with 128 <= w <= fw and 128 <= h <= fh
+ * (downscales only; a level may be anisotropic).  stride: a positive multiple of 8, in level pixels, the same at every level.
+ * Level gray (byte for byte):
+ *   gray_l[f] = cv2.resize(cv2.cvtColor(frames[f], COLOR_BGR2GRAY), (w, h), interpolation=INTER_AREA)
+ * with OpenCV's choice of arithmetic from both scales, as for the rectangle regions with 128 replaced by w / h: a copy when the
+ * level is the frame size; (sum + 2) >> 2 at 2x2; rint(float(sum) * (1.f / (kx * ky))) for other integer pairs; otherwise
+ * ResizeArea with x taps from computeResizeAreaTab(fw -> w) and y taps from (fh -> h).  An axis counts as integer as OpenCV
+ * decides it: 1 / (w / fw) in double within DBL_EPSILON of an integer, so a 49x axis (1.0 / (1.0 / 49) != 49) takes the table.
+ * Windows of a level: x in the origins of cnnacc_scan_frames along w (0, stride, 2 stride, ... plus the one flush with the far
+ * edge), y likewise along h.  Window r of the call is numbered frame-major, then level in the given order, then y, then x.
+ * What a window computes: cnnacc_classify_batch of the 64x16x16 cells at (x/8, y/8) of cnnacc_run_batch(gray_l[f]), bit for
+ * bit; its box is on the window's 128 grid.  Its frame rectangle is (f, x fw / w, y fh / h, 128 fw / w, 128 fh / h): the call
+ * is refused unless all four are integers for every window of every level (the actual origins are checked, so a level with
+ * one window position is never refused for its stride), so the rectangle merge maps every box exactly.  A single level
+ * (fw, fh) gives exactly cnnacc_scan_frames' outputs.
+ * This is NOT detect_regions on the same rectangles: a region is cropped and then resized, a pyramid window is resized with
+ * the whole frame and sees the frame beyond its border (see cnnacc_scan_frames).
+ * preprocess_pyramid  : gray [n][sum of h * w] u8, frame-major, then level (the weights are not needed).
+ * scan_pyramid        : probs [R][n_cls] f32, cls [R] i32, bbox [R][4] i32 for R = n * (windows per frame); any may be NULL.
+ * scan_pyramid_objects: scan_pyramid followed by the merge above with CNNACC_FLAG_RECTS, the windows' frame rectangles being
+ *                       the regions and score[r] = probs[r][cls[r]] (the logit with CNNACC_FLAG_LOGITS): exactly
+ *                       merge_regions on those rectangles and scan_pyramid's outputs.  Predictions never leave the GPU.
+ * Host and device pointers, alignment, CNNACC_FLAG_LOGITS and CNNACC_FLAG_CLASS_AGNOSTIC as for the scan_frames calls.
+ *   -2, nothing launched: n < 0, a frame side outside 128..8192, L outside 1..16 or levels NULL, a level that breaks the
+ *       rules above, a window rectangle not in whole frame pixels, stride not a positive multiple of 8, more than 2^31-1
+ *       windows in the call, the flags cnnacc_scan_frames refuses, frames (or gray) NULL with n > 0; for the _objects call
+ *       also more than CNNACC_MERGE_MAX_PER_FRAME windows per frame and the merge's own refusals.  preprocess_pyramid takes
+ *       no stride and has no windows to check.  -4 without weights or without a classifier (scan calls).  n == 0 returns 0. */
+#define CNNACC_PYRAMID_MAX_LEVELS 16
+int cnnacc_preprocess_pyramid(cnnacc_handle *h, const uint8_t *frames, int64_t n, int fh, int fw, const int32_t *levels,
+                              int n_levels, uint8_t *gray, uint32_t flags);
+int cnnacc_scan_pyramid(cnnacc_handle *h, const uint8_t *frames, int64_t n, int fh, int fw, const int32_t *levels,
+                        int n_levels, int stride, float *probs, int32_t *cls, int32_t *bbox, uint32_t flags);
+int cnnacc_scan_pyramid_objects(cnnacc_handle *h, const uint8_t *frames, int64_t n, int fh, int fw, const int32_t *levels,
+                                int n_levels, int stride, float score_min, float iou_max, int max_det, int32_t *n_det,
+                                int32_t *det_region, int32_t *det_cls, float *det_score, float *det_box, uint32_t flags);
+/* Host-only: the windows per frame of a pyramid call with these frame sides, levels and stride, or -2 where the call refuses
+ * them (the same checks).  With rects, also writes their frame rectangles [R][5] (0, x, y, w, h) in window order (cap >= R,
+ * else -2).  No GPU needed. */
+int cnnacc_pyramid_windows_host(int fh, int fw, const int32_t *levels, int n_levels, int stride, int32_t *rects, int64_t cap);
 /* Host-only view of the staging plan of a host-pointer region call (csrc/region_plan.h): chunk i stages frames
  * [chunks[4i], chunks[4i+1]) with one copy and runs regions [chunks[4i+2], chunks[4i+3]) on them.  Returns the number of chunks
  * (<= cap), or -2 for a region array the real call refuses, or when cap is too small.  No GPU needed. */

@@ -23,8 +23,18 @@ beside grid (a) as squares in the same run, and batch-1 p50 / p99 of one VGA fra
 scan_objects at 64 and 8 with score_min 0 and with the 97th percentile of the window scores; batch-1 p50 / p99 of one pageable
 frame through scan_frames and scan_objects; the device-time split of scan_frames at stride 8 into gray, conv and window tail
 (torch.profiler kernel times, in a pass of its own); how often scan and detect_regions agree on the class of the same window.
+--pyramid measures the pyramid calls: scan_pyramid on the VGA four-level set (640x480, 512x384, 320x240, 256x192) at strides
+8, 16 and 32 and on 1920x1080 frames with the six-level set (1536x864 .. 256x144) at stride 16, device-resident us per frame
+and host-fed frames/s, alternated twice with detect_regions on the same frame rectangles (VGA stride 32 and 16); the
+device-time split of scan_pyramid_objects into gray, level resize, conv, window tail and merge (torch.profiler, a pass of its
+own) and the conv time of each level alone (run_batch on its gray); batch-1 p50 / p99 of one pageable frame.
+--scan-rates --vs-lib LIB compares scan_frames (device-resident us per frame and host-fed frames/s at strides 64 and 8) with
+this tree's library and with another build of it, LIB (for example the parent commit's, built in a worktree:
+`git worktree add /tmp/parent HEAD~1 && make -C /tmp/parent/fpga-cnn-object-detection-accelerator_b200/csrc`), in
+subprocesses alternated --runs times, so both see the same card in the same command.
 
-    python tools/regions_throughput.py [--frames 2048] [--dev-frames 1024] [--seconds 2] [--objects | --rects | --scan]
+    python tools/regions_throughput.py [--frames 2048] [--dev-frames 1024] [--seconds 2] [--objects | --rects | --scan | --pyramid |
+                                        --scan-rates [--vs-lib LIB --runs 2]]
                                        [--out FILE]
 """
 import argparse
@@ -96,7 +106,13 @@ def main():
     ap.add_argument("--objects", action="store_true", help="measure the merging calls (detect_objects / merge_regions)")
     ap.add_argument("--rects", action="store_true", help="measure rectangle regions (detect_regions / detect_objects)")
     ap.add_argument("--scan", action="store_true", help="measure the scanning calls (scan_frames / scan_objects)")
+    ap.add_argument("--pyramid", action="store_true", help="measure the pyramid calls (scan_pyramid / scan_pyramid_objects)")
+    ap.add_argument("--scan-rates", action="store_true", help="scan_frames rates at strides 64 and 8 only")
+    ap.add_argument("--vs-lib", default=None, help="with --scan-rates: alternate with this other libcnnacc.so")
+    ap.add_argument("--runs", type=int, default=2)
     a = ap.parse_args()
+    if a.scan_rates:
+        return scan_rates(a)
     import torch
     dev = torch.device("cuda", 0)
     meta = {"card": card(), "frame": [H, W], "host_frames": a.frames, "dev_frames": a.dev_frames}
@@ -125,6 +141,9 @@ def main():
         return write(a, lines)
     if a.scan:
         scan(a, acc, host, emit)
+        return write(a, lines)
+    if a.pyramid:
+        pyramid(a, acc, host, emit)
         return write(a, lines)
 
     # host-fed
@@ -392,6 +411,133 @@ def scan(a, acc, host, emit):
     batch1(emit, "scan_frames_stride8", lambda: acc.scan_frames(one, 8))
     batch1(emit, "scan_objects_stride8", lambda: acc.scan_objects(one, 8))
     batch1(emit, "detect_regions_grid63", lambda: acc.detect_regions(one, fc.grid_regions(1, H, W, 128, 64)))
+
+
+def scan_rates(a):
+    """scan_frames device-resident us per frame and host-fed frames/s at strides 64 and 8 over --frames VGA frames, with the
+    library CNNACC_LIB_PATH names (this tree's when unset); with --vs-lib, subprocesses alternate this tree's library and
+    that one --runs times."""
+    if a.vs_lib:
+        lines = []
+        for run in range(a.runs):
+            for lib in (a.vs_lib, None):
+                env = {k: v for k, v in os.environ.items() if k != "CNNACC_LIB_PATH"}
+                if lib:
+                    env["CNNACC_LIB_PATH"] = os.path.abspath(lib)
+                cmd = [sys.executable, os.path.abspath(__file__), "--scan-rates", "--frames", str(a.frames), "--seconds",
+                       str(a.seconds)]
+                out = subprocess.run(cmd, env=env, capture_output=True, text=True, check=True).stdout
+                d = {**json.loads(out.strip().splitlines()[-1]), "run": run, "library": lib or "this tree"}
+                lines.append(d)
+                print(json.dumps(d), flush=True)
+        return write(a, lines)
+    import ctypes as c
+    import torch
+    if os.environ.get("CNNACC_LIB_PATH"):               # another build may predate some of this tree's symbols
+        other = c.CDLL(os.environ["CNNACC_LIB_PATH"])
+        for name in [k for k in fc._lib.SYMBOLS if not hasattr(other, k)]:
+            fc._lib.SYMBOLS.pop(name)
+    acc = fc.CNNAccelerator()
+    acc.load_weights(os.path.join(ROOT, "tests", "golden", "weights.bin"))
+    acc.set_shifts(7, 10, 11)
+    acc.load_classifier(*inputs.make_fc())
+    host = fc.alloc_host((a.frames, H, W, 3))
+    host[:] = inputs.make_frames(("smooth", 1), 1, H, W)
+    t = torch.from_numpy(host).cuda()
+    d = {"card": card(), "frame": [H, W], "frames": a.frames}
+    for stride in (64, 8):
+        d[f"dev_us_per_frame_s{stride}"] = event_ms(lambda: acc.scan_frames(t, stride), a.seconds) / a.frames * 1e3
+        d[f"host_frames_per_s_s{stride}"] = wall_rate(lambda: acc.scan_frames(host, stride), a.seconds) * a.frames
+    print(json.dumps(d), flush=True)
+
+
+VGA_LEVELS = [(640, 480), (512, 384), (320, 240), (256, 192)]
+P1080_LEVELS = [(1536, 864), (1280, 720), (1024, 576), (768, 432), (512, 288), (256, 144)]
+
+
+def profile_split(acc, fn, n, reps=5):
+    """us per frame of fn's kernels by part (torch.profiler CUDA kernel times, a pass of its own)."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            fn()
+        torch.cuda.synchronize()
+    split = {}
+    for e in prof.key_averages():
+        us = e.device_time_total if hasattr(e, "device_time_total") else e.cuda_time_total
+        if us <= 0:
+            continue
+        name = e.key
+        part = ("gray" if "gray_full_kernel" in name else "level_resize" if "pyramid_levels_kernel" in name
+                else "window_tail" if "ScanWindows" in name else "merge" if "merge" in name
+                else "conv" if "fused" in name else "other")
+        split[part] = split.get(part, 0.0) + us / reps / n
+    return split, sorted({e.key for e in prof.key_averages()})
+
+
+def pyramid(a, acc, host, emit):
+    """scan_pyramid beside detect_regions on the same rectangles, host-fed and device-resident, alternated twice in this
+    run; the 1080p six-level set; the device-time split and per-level conv; batch 1."""
+    import torch
+    dev = torch.device("cuda", 0)
+    t = torch.from_numpy(host[:a.dev_frames]).to(dev)
+    nd = a.dev_frames
+    for where, frames, n, measure in (("host_fed", host, a.frames, lambda fn: 1.0 / wall_rate(fn, a.seconds)),
+                                      ("device_resident", t, nd, lambda fn: event_ms(fn, a.seconds) / 1e3)):
+        secs = {}
+        for rep in range(2):
+            for stride in (8, 16, 32):
+                secs.setdefault(("scan_pyramid", stride), []).append(measure(lambda: acc.scan_pyramid(frames, VGA_LEVELS, stride)))
+                if stride in (16, 32) and where == "device_resident":
+                    k = min(n, 64)                              # detect_regions converts and convolves every window on its own
+                    reg = fc.pyramid_windows(k, H, W, VGA_LEVELS, stride)
+                    secs.setdefault(("detect_regions", stride), []).append(
+                        measure(lambda: acc.detect_regions(frames[:k], reg)) * n / k)
+        for (path, stride), v in secs.items():
+            per = len(fc.pyramid_windows(1, H, W, VGA_LEVELS, stride))
+            emit({"what": where, "path": path, "levels": VGA_LEVELS, "stride": stride, "windows_per_frame": per, "s_runs": v,
+                  "frames_per_s": n / min(v), "windows_per_s": n * per / min(v), "us_per_frame": min(v) / n * 1e6})
+        if where == "device_resident":
+            for stride in (16, 32):
+                emit({"what": where, "ratio": "scan_pyramid/detect_regions (frames/s), same rectangles", "stride": stride,
+                      "value": min(secs[("detect_regions", stride)]) / min(secs[("scan_pyramid", stride)])})
+    split, kernels = profile_split(acc, lambda: acc.scan_pyramid_objects(t, VGA_LEVELS, 16), nd)
+    emit({"what": "device_split", "path": "scan_pyramid_objects", "levels": VGA_LEVELS, "stride": 16, "score_min": 0.0,
+          "frames": nd, "us_per_frame": split, "kernels": kernels})
+    gray = acc.preprocess_pyramid(t, VGA_LEVELS)
+    o = 0
+    for w, h in VGA_LEVELS:
+        g = gray[:, o:o + w * h].reshape(nd, h, w).contiguous()
+        o += w * h
+        emit({"what": "device_split", "path": "run_batch of one level's gray", "level": [w, h],
+              "us_per_frame": event_ms(lambda: acc.run_batch(g), a.seconds) / nd * 1e3})
+    del gray, g, t
+    torch.cuda.synchronize()
+    # 1920x1080 frames, six levels at stride 16
+    n_hd = max(1, min(a.dev_frames // 8, 128))
+    hd = fc.alloc_host((n_hd, 1080, 1920, 3))
+    hd[:] = inputs.make_frames(("smooth", 3), 1, 1080, 1920)
+    td = torch.from_numpy(hd).to(dev)
+    per = len(fc.pyramid_windows(1, 1080, 1920, P1080_LEVELS, 16))
+    for where, frames, measure in (("host_fed", hd, lambda fn: 1.0 / wall_rate(fn, a.seconds)),
+                                   ("device_resident", td, lambda fn: event_ms(fn, a.seconds) / 1e3)):
+        v = [measure(lambda: acc.scan_pyramid(frames, P1080_LEVELS, 16)) for _ in range(2)]
+        emit({"what": where, "path": "scan_pyramid", "frame": [1080, 1920], "levels": P1080_LEVELS, "stride": 16,
+              "windows_per_frame": per, "s_runs": v, "frames_per_s": n_hd / min(v), "us_per_frame": min(v) / n_hd * 1e6})
+    split, kernels = profile_split(acc, lambda: acc.scan_pyramid_objects(td, P1080_LEVELS, 16), n_hd)
+    emit({"what": "device_split", "path": "scan_pyramid_objects", "frame": [1080, 1920], "levels": P1080_LEVELS, "stride": 16,
+          "score_min": 0.0, "frames": n_hd, "us_per_frame": split, "kernels": kernels})
+    del td
+    torch.cuda.synchronize()
+    one = np.ascontiguousarray(host[:1])
+    one_hd = np.ascontiguousarray(hd[:1])
+    batch1(emit, "scan_pyramid_vga_stride16", lambda: acc.scan_pyramid(one, VGA_LEVELS, 16))
+    batch1(emit, "scan_pyramid_objects_vga_stride16", lambda: acc.scan_pyramid_objects(one, VGA_LEVELS, 16))
+    batch1(emit, "scan_pyramid_1080p_stride16", lambda: acc.scan_pyramid(one_hd, P1080_LEVELS, 16))
+    batch1(emit, "scan_frames_vga_stride16", lambda: acc.scan_frames(one, 16))
 
 
 if __name__ == "__main__":
